@@ -485,10 +485,54 @@ class Timing:
         return float(t.item())
 
 
-def device_resident_leg(T: Timing, D, rank, frames, B, DL, steps, warmup, clocks=None):
+DUMP_CAP_BYTES = 64 << 20   # --dump-outputs writes at most this much
+
+
+def dump_outputs(out_dir, dlanes, B):
+    """Writes what the detectors return for their last batch as DIR/<name>.npy (float64), one row per frame or per
+    detection, lanes in order: frames are numbered lane * B + frame.  Detections keep the engine's order (by id).
+    Past DUMP_CAP_BYTES, every array keeps the same fixed, seeded fraction of its rows (frame_index and det_frame say
+    which frames they are)."""
+    os.makedirs(out_dir, exist_ok=True)
+    infos, per_frame = [], []
+    for d in dlanes:
+        for f in range(B):
+            i = d.FrameInfo(f)
+            infos.append([getattr(i, n) for n, _ in i._fields_])
+            per_frame.append(d.Detections(f))
+    det = np.concatenate(per_frame)
+    frame_rows = {
+        "frame_index": np.arange(len(infos)),
+        "frame_info": np.array(infos),   # b200tag_frame_info fields in their C order (status, num_points, ...)
+    }
+    det_rows = {
+        "det_frame": np.concatenate([np.full(len(x), g) for g, x in enumerate(per_frame)]),
+        "det_id": det["id"],
+        "det_hamming": det["hamming"],
+        "det_decision_margin": det["decision_margin"],
+        "det_center": det["c"],
+        "det_corners": det["p"],
+        "det_homography": det["H"].reshape(-1, 3, 3),
+    }
+    groups = [frame_rows, det_rows]
+    total = sum(8 * a.size for g in groups for a in g.values())
+    budget = DUMP_CAP_BYTES - 4096 * sum(len(g) for g in groups)   # room for the .npy headers
+    if total > budget:
+        rng = np.random.default_rng(0)
+        for g in groups:
+            n = len(next(iter(g.values())))
+            keep = np.sort(rng.choice(n, size=int(n * budget / total), replace=False))
+            g.update({name: a[keep] for name, a in g.items()})
+    for g in groups:
+        for name, a in g.items():
+            np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
+def device_resident_leg(T: Timing, D, rank, frames, B, DL, steps, warmup, clocks=None, dump_dir=None):
     """`DL` detectors, one CUDA stream each, take turns on batches that already sit in HBM: while the host collects
     lane k's results (the only host work between two batches) lane k+1's kernels keep the GPU busy.  One step = one
-    batch per lane.  Returns the first detector (kept open, warm) and the device batch for the profiling leg."""
+    batch per lane.  Returns the first detector (kept open, warm) and the device batch for the profiling leg.
+    With `dump_dir`, every lane's results of the last step are written there after the timed region."""
     torch, local = T.torch, T.local
     host_batch = np.stack([frames[(i + rank * 3) % len(frames)] for i in range(B)])
     dev_batch = torch.from_numpy(host_batch).cuda()
@@ -520,6 +564,8 @@ def device_resident_leg(T: Timing, D, rank, frames, B, DL, steps, warmup, clocks
     ms = T.max_ranks(max(e0.elapsed_time(ev) for ev in e_end))
     # per-step spread: lane 0's batch-to-batch intervals (its stream is busy back to back in steady state)
     gaps = [marks[k - 1].elapsed_time(marks[k]) for k in range(1, steps)]
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, dlanes, B)
     for d in dlanes[1:]:
         d.close()
     return det, dev_batch, host_batch, ms, gaps, infos
@@ -645,7 +691,8 @@ def run_ours(args):
     clocks = ClockSampler(local)
 
     # --- device-resident throughput (the line's `value`) ------------------------------------------
-    det, dev_batch, host_batch, ms, gaps, infos = device_resident_leg(T, D, rank, frames, B, DL, args.steps, args.warmup, clocks)
+    det, dev_batch, host_batch, ms, gaps, infos = device_resident_leg(T, D, rank, frames, B, DL, args.steps, args.warmup, clocks,
+                                                                      args.dump_outputs)
     value = B * DL * args.steps * world / (ms * 1e-3)
     ndet_per_batch = sum(len(det.Detections(f)) for f in range(B))
     P = float(np.mean([i.num_points for i in infos]))
@@ -782,7 +829,11 @@ def main():
                     help="BASELINE.json config to measure; the contract line is config 2 (the default)")
     ap.add_argument("--format", default=None, choices=["gray", "yuyv", "bgr"],
                     help="pixel format of the frames (default: the config's own; the contract line is YUYV)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the device-resident leg's results of its last step (rank 0, every lane) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     select_config(args.config)
     if args.format:
         global FMT, WORKLOAD
