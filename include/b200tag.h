@@ -310,6 +310,25 @@ typedef struct b200tag_tag_position {
 int b200tag_locate_tags(const b200tag_detection *dets, int count, double tagsize, double fx, double fy, double cx,
                         double cy, const double *rotation, const double *offset, b200tag_tag_position *out);
 
+/* The same step on the device, inside every detect call: a kernel at the end of the detection graph estimates the pose
+ * of every detection, and the results come back with the detections.  Off by default; a detector that never turns it
+ * on launches, allocates and returns exactly what it would without it.
+ * b200tag_set_pose_estimation turns it on (tagsize > 0) or off (tagsize == 0), with the same arguments and meaning as
+ * b200tag_locate_tags; rotation / offset may be NULL.  B200TAG_E_INVALID (state unchanged) unless tagsize >= 0 and fx,
+ * fy are non-zero.  Takes effect from the next detect call; adds one kernel to b200tag_kernels_per_batch. */
+int b200tag_set_pose_estimation(b200tag_detector *det, double tagsize, double fx, double fy, double cx, double cy,
+                                const double *rotation, const double *offset);
+/* Poses of frame `frame` of the last call, parallel to b200tag_detections(det, frame): element i is the pose of
+ * detection i.  NULL and *count = 0 when the last call ran without the pose step.  Owned by the detector, valid until
+ * the next detect call. */
+const b200tag_pose *b200tag_poses(const b200tag_detector *det, int frame, int *count);
+/* The same detections as b200tag_locate_tags returns them (closest first, .index into b200tag_detections). */
+const b200tag_tag_position *b200tag_tag_positions(const b200tag_detector *det, int frame, int *count);
+/* Test hook, as b200tag_debug_math: the device pose kernel on caller-supplied records (current device); arguments and
+ * results as b200tag_estimate_poses. */
+int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count, double tagsize, double fx, double fy,
+                                        double cx, double cy, b200tag_pose *out);
+
 /* Pinned host staging memory, so b200tag_detect* can overlap H2D with compute. */
 void *b200tag_alloc_pinned(size_t bytes);
 /* Write-combined pinned memory: for buffers the CPU (or a capture driver) only ever WRITES, such as a camera ring

@@ -10,9 +10,9 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libb200tag.so")
 
-CU_SOURCES = ["kernels_frontend.cu", "kernels_blobs.cu", "kernels_decode.cu", "kernels_jpeg.cu", "detector.cu"]
+CU_SOURCES = ["kernels_frontend.cu", "kernels_blobs.cu", "kernels_decode.cu", "kernels_jpeg.cu", "kernels_pose.cu", "detector.cu"]
 CC_SOURCES = ["pose.cc", "jpeg_host.cc"]   # host-only parts of the C ABI
-HEADERS = ["dev_types.h", "kernels.h", "jpeg.h", "jpeg_core.h", "tag_families_data.h", os.path.join("..", "..", "include", "b200tag.h")]
+HEADERS = ["dev_types.h", "kernels.h", "jpeg.h", "jpeg_core.h", "pose_core.h", "tag_families_data.h", os.path.join("..", "..", "include", "b200tag.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

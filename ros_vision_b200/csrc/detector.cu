@@ -28,6 +28,7 @@
 #include "jpeg.h"
 #include "jpeg_core.h"
 #include "kernels.h"
+#include "pose_core.h"
 
 #include "tag_families_data.h"
 
@@ -117,6 +118,16 @@ struct b200tag_detector {
   void *d_families = nullptr;  // DevFamily[nfamilies] followed by the code tables
   int min_width_at_border = 8;
   bool normal_border = true, reversed_border = false;
+  // the pose step (b200tag_set_pose_estimation): on while tagsize > 0
+  struct PoseSettings {
+    double tagsize = 0, fx = 0, fy = 0, cx = 0, cy = 0;
+    double rotation[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, offset[3] = {0, 0, 0};
+  };
+  PoseSettings pose, last_pose;                // current; what the last enqueue ran with
+  b200tag_pose *h_poses = nullptr;             // pinned + mapped, parallel to h_dets; allocated when first turned on
+  b200tag_pose *d_poses_alias = nullptr;
+  std::vector<std::vector<b200tag_pose>> poses;                   // parallel to dets
+  std::vector<std::vector<b200tag_tag_position>> positions;       // closest first
 };
 
 namespace b200tag {
@@ -230,34 +241,45 @@ bool det_less(const b200tag_detection &a, const b200tag_detection &b) {  // dete
   if (a.family != b.family) return a.family < b.family;
   return a.hamming < b.hamming;
 }
-void reconcile(std::vector<b200tag_detection> &d) {
-  std::sort(d.begin(), d.end(), det_less);  // device append order is arbitrary: fix it first
-  int n = static_cast<int>(d.size());
+// A detection with the pose the device computed for it: reconcile moves both together.
+struct DetPose {
+  b200tag_detection det;
+  b200tag_pose pose;
+};
+const b200tag_detection &rec(const b200tag_detection &d) { return d; }
+const b200tag_detection &rec(const DetPose &d) { return d.det; }
+
+template <class T>
+void reconcile(std::vector<T> &v) {
+  // device append order is arbitrary: fix it first
+  std::sort(v.begin(), v.end(), [](const T &a, const T &b) { return det_less(rec(a), rec(b)); });
+  auto d = [&v](int i) -> const b200tag_detection & { return rec(v[i]); };
+  int n = static_cast<int>(v.size());
   for (int i0 = 0; i0 < n; i0++) {
     for (int i1 = i0 + 1; i1 < n; i1++) {
-      if (d[i0].id != d[i1].id || d[i0].family != d[i1].family) continue;
-      if (!polys_overlap(d[i0].p, d[i1].p)) continue;
+      if (d(i0).id != d(i1).id || d(i0).family != d(i1).family) continue;
+      if (!polys_overlap(d(i0).p, d(i1).p)) continue;
       int pref = 0;
-      pref = prefer_smaller(pref, d[i0].hamming, d[i1].hamming);
-      pref = prefer_smaller(pref, -d[i0].decision_margin, -d[i1].decision_margin);
+      pref = prefer_smaller(pref, d(i0).hamming, d(i1).hamming);
+      pref = prefer_smaller(pref, -d(i0).decision_margin, -d(i1).decision_margin);
       for (int i = 0; i < 4; i++) {
-        pref = prefer_smaller(pref, d[i0].p[i][0], d[i1].p[i][0]);
-        pref = prefer_smaller(pref, d[i0].p[i][1], d[i1].p[i][1]);
+        pref = prefer_smaller(pref, d(i0).p[i][0], d(i1).p[i][0]);
+        pref = prefer_smaller(pref, d(i0).p[i][1], d(i1).p[i][1]);
       }
       if (pref < 0) {
-        d[i1] = d[n - 1];
+        v[i1] = v[n - 1];
         n--;
         i1--;
       } else {
-        d[i0] = d[n - 1];
+        v[i0] = v[n - 1];
         n--;
         i0--;
         break;
       }
     }
   }
-  d.resize(n);
-  std::sort(d.begin(), d.end(), det_less);
+  v.resize(n);
+  std::sort(v.begin(), v.end(), [](const T &a, const T &b) { return det_less(rec(a), rec(b)); });
 }
 
 int validate(const b200tag_config &c, std::string *why) {
@@ -314,8 +336,26 @@ int finish_impl(b200tag_detector *det) {
     const Counters &c = det->h_counters[f];
     const uint32_t nd = std::min(c.num_detections, det->fp.det_cap);
     const b200tag_detection *src = det->h_dets + static_cast<size_t>(f) * det->fp.det_cap;
-    det->dets[f].assign(src, src + nd);
-    reconcile(det->dets[f]);
+    if (det->last_pose.tagsize > 0) {
+      const b200tag_pose *ps = det->h_poses + static_cast<size_t>(f) * det->fp.det_cap;
+      std::vector<DetPose> both(nd);
+      for (uint32_t i = 0; i < nd; i++) both[i] = DetPose{src[i], ps[i]};
+      reconcile(both);
+      det->dets[f].resize(both.size());
+      det->poses[f].resize(both.size());
+      for (size_t i = 0; i < both.size(); i++) {
+        det->dets[f][i] = both[i].det;
+        det->poses[f][i] = both[i].pose;
+      }
+      det->positions[f].resize(both.size());
+      locate_from_poses(det->dets[f].data(), det->poses[f].data(), static_cast<int>(both.size()), det->last_pose.rotation,
+                        det->last_pose.offset, det->positions[f].data());
+    } else {
+      det->dets[f].assign(src, src + nd);
+      reconcile(det->dets[f]);
+      det->poses[f].clear();
+      det->positions[f].clear();
+    }
     det->quads_valid[f] = false;
     if (c.status) rc = B200TAG_E_OVERFLOW;
   }
@@ -342,6 +382,11 @@ int record_sequence(b200tag_detector *det, const void *device_images, size_t str
   launches += launch_frontend(p, count, det->stream, kt);
   launches += launch_blobs(p, count, det->stream, kt, kt ? nullptr : &det->side);  // per-kernel timing runs serially
   launches += launch_decode(p, count, det->stream, kt);
+  if (det->pose.tagsize > 0) {
+    const auto &ps = det->pose;
+    const PoseLaunch pl{det->d_dets_alias, det->d_poses_alias, p.counters, p.det_cap, 0, ps.tagsize, ps.fx, ps.fy, ps.cx, ps.cy};
+    launches += launch_pose(pl, count, det->stream, kt);
+  }
   *launches_out = launches;
   CK(cudaMemcpyAsync(det->h_counters, p.counters, sizeof(Counters) * count, cudaMemcpyDeviceToHost, det->stream));
   return 0;
@@ -388,6 +433,7 @@ int enqueue_impl(b200tag_detector *det, const void *device_images, size_t stride
   }
   det->kernels_per_batch = launches;
   CK(cudaGetLastError());
+  det->last_pose = det->pose;
   det->last_count = count;
   det->pending = true;
   return 0;
@@ -711,6 +757,8 @@ int b200tag_create_families(const b200tag_config *cfg, const b200tag_family *fam
   launch_hash_clear(p, B, det->stream);
   if (!ck(cudaStreamSynchronize(det->stream), "initial hash clear")) return fail(B200TAG_E_CUDA);
   det->dets.resize(B);
+  det->poses.resize(B);
+  det->positions.resize(B);
   det->quads.resize(B);
   det->quads_valid.assign(B, false);
   memset(det->h_counters, 0, sizeof(Counters) * B);
@@ -746,6 +794,7 @@ void b200tag_destroy(b200tag_detector *det) {
   if (det->d_families) cudaFree(det->d_families);
   if (det->h_counters) cudaFreeHost(det->h_counters);
   if (det->h_dets) cudaFreeHost(det->h_dets);
+  if (det->h_poses) cudaFreeHost(det->h_poses);
   delete det;
 }
 
@@ -1166,6 +1215,20 @@ const b200tag_detection *b200tag_detections(const b200tag_detector *det, int fra
   return det->dets[frame].data();
 }
 
+const b200tag_pose *b200tag_poses(const b200tag_detector *det, int frame, int *count) {
+  if (count) *count = 0;
+  if (!det || frame < 0 || frame >= det->last_count || det->pending || !(det->last_pose.tagsize > 0)) return nullptr;
+  if (count) *count = static_cast<int>(det->poses[frame].size());
+  return det->poses[frame].data();
+}
+
+const b200tag_tag_position *b200tag_tag_positions(const b200tag_detector *det, int frame, int *count) {
+  if (count) *count = 0;
+  if (!det || frame < 0 || frame >= det->last_count || det->pending || !(det->last_pose.tagsize > 0)) return nullptr;
+  if (count) *count = static_cast<int>(det->positions[frame].size());
+  return det->positions[frame].data();
+}
+
 int b200tag_frame_info_get(const b200tag_detector *det, int frame, b200tag_frame_info *info) {
   if (!det || !info || frame < 0 || frame >= det->last_count || det->pending) return B200TAG_E_INVALID;
   const Counters &c = det->h_counters[frame];
@@ -1294,6 +1357,32 @@ int b200tag_set_camera(b200tag_detector *det, double fx, double cx, double fy, d
   return 0;
 }
 
+int b200tag_set_pose_estimation(b200tag_detector *det, double tagsize, double fx, double fy, double cx, double cy,
+                                const double *rotation, const double *offset) {
+  if (!det || !(tagsize >= 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
+  DeviceGuard on_device(det->device);
+  if (tagsize > 0 && !det->h_poses) {
+    const size_t bytes = sizeof(b200tag_pose) * det->fp.det_cap * static_cast<size_t>(det->cfg.max_batch);
+    b200tag_pose *h = nullptr, *d = nullptr;
+    CK(cudaHostAlloc(reinterpret_cast<void **>(&h), bytes, cudaHostAllocMapped));
+    if (cudaHostGetDevicePointer(reinterpret_cast<void **>(&d), h, 0) != cudaSuccess) {
+      cudaGetLastError();
+      cudaFreeHost(h);
+      det->err = "cudaHostGetDevicePointer(poses) failed";
+      return B200TAG_E_CUDA;
+    }
+    det->h_poses = h;
+    det->d_poses_alias = d;
+  }
+  drop_graphs(det);  // the parameters are baked into the captured launches
+  b200tag_detector::PoseSettings &ps = det->pose;
+  ps.tagsize = tagsize; ps.fx = fx; ps.fy = fy; ps.cx = cx; ps.cy = cy;
+  static const double kEye[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, kZero[3] = {0, 0, 0};
+  memcpy(ps.rotation, rotation ? rotation : kEye, sizeof(ps.rotation));
+  memcpy(ps.offset, offset ? offset : kZero, sizeof(ps.offset));
+  return 0;
+}
+
 int b200tag_set_distortion(b200tag_detector *det, double k1, double k2, double p1, double p2, double k3) {
   if (!det) return B200TAG_E_INVALID;
   DeviceGuard on_device(det->device);
@@ -1367,6 +1456,28 @@ int b200tag_debug_math(int op, const float *a, const float *b, float *out, int n
   if (!rc) {
     b200tag::k_debug_math<<<(n + 255) / 256, 256>>>(op, d, d + n, d + 2 * static_cast<size_t>(n), n);
     if (cudaMemcpy(out, d + 2 * static_cast<size_t>(n), sizeof(float) * n, cudaMemcpyDeviceToHost) != cudaSuccess) rc = B200TAG_E_CUDA;
+  }
+  cudaFree(d);
+  return rc;
+}
+
+int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count, double tagsize, double fx, double fy,
+                                        double cx, double cy, b200tag_pose *out) {
+  if (count < 0 || (count > 0 && (!dets || !out)) || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
+  if (count == 0) return 0;
+  const size_t db = sizeof(b200tag_detection) * static_cast<size_t>(count), pb = sizeof(b200tag_pose) * static_cast<size_t>(count);
+  uint8_t *d = nullptr;
+  if (cudaMalloc(&d, db + pb) != cudaSuccess) {
+    cudaGetLastError();
+    return B200TAG_E_NO_DEVICE;
+  }
+  int rc = 0;
+  const PoseLaunch pl{reinterpret_cast<const b200tag_detection *>(d), reinterpret_cast<b200tag_pose *>(d + db), nullptr,
+                      0, static_cast<uint32_t>(count), tagsize, fx, fy, cx, cy};
+  if (cudaMemcpy(d, dets, db, cudaMemcpyHostToDevice) != cudaSuccess) rc = B200TAG_E_CUDA;
+  if (!rc) {
+    launch_pose(pl, 1, nullptr, nullptr);
+    if (cudaGetLastError() != cudaSuccess || cudaMemcpy(out, d + db, pb, cudaMemcpyDeviceToHost) != cudaSuccess) rc = B200TAG_E_CUDA;
   }
   cudaFree(d);
   return rc;

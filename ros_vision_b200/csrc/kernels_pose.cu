@@ -1,0 +1,147 @@
+// The pose step on the device (b200tag_set_pose_estimation): libapriltag's estimate_tag_pose for every raw detection of
+// the batch, appended to the detection graph behind k_decode.  One warp per detection.  The homography start and the
+// orthogonal iteration run on every lane with the same values, reading the per-detection constants from shared memory;
+// lane 0 sets up the frame of the second-minimum search there, and the lanes split that search's grid.  The arithmetic is
+// pose_core.h's, the same the host functions in pose.cc run.
+//
+// A pose depends only on its own record, so computing it before the host's reconcile gives the pose of every
+// detection that survives it.
+#include <cuda_runtime.h>
+
+#include "dev_types.h"
+#include "kernels.h"
+#include "pose_core.h"
+
+namespace b200tag {
+
+namespace {
+
+using namespace pose;
+
+constexpr int kPoseWarps = 4;  // warps per CTA
+constexpr unsigned kFull = 0xffffffffu;
+
+struct PoseShared {
+  OiConsts oi;              // what every step of the orthogonal iteration reads
+  SecondMinFrame S;         // the frame and error quartic of the second-minimum search
+  b200tag_detection det;    // the record, read once from mapped host memory
+  M3 R1;                    // the first minimum, while the search runs
+  V3 t1;
+  double err1;
+  b200tag_pose out;
+};
+
+// Step 3's search, split over the lanes: round k evaluates dE/dt at grid points 1 + 32k + lane, a ballot of the
+// sign changes starts a bisection on each lane that holds one, and the refined minima are taken in grid order so that
+// the first of equal errors wins, as in the host's serial loop.  Returns the number of distinct minima found.  Not
+// inlined: register allocation of the search apart from the orthogonal iteration's keeps both free of spills.
+__device__ __noinline__ int search_second_minimum(const SecondMinFrame &S, int lane, double *best_beta) {
+  double carry_t = grid_t(0);
+  double carry_d = S.q.dnum(carry_t);
+  double best_err = HUGE_VAL;
+  int n_minima = 0;
+  *best_beta = 0;
+  for (int base = 1; base <= kGrid; base += 32) {
+    const int g = base + lane;
+    double tt = 0, d = 0;
+    if (g <= kGrid) {
+      tt = grid_t(g);
+      d = S.q.dnum(tt);
+    }
+    double prev_t = __shfl_up_sync(kFull, tt, 1), prev_d = __shfl_up_sync(kFull, d, 1);
+    if (lane == 0) {
+      prev_t = carry_t;
+      prev_d = carry_d;
+    }
+    bool found = false;
+    double beta = 0, e = 0;
+    if (g <= kGrid && prev_d < 0 && d >= 0) {  // derivative goes from negative to positive: a minimum in between
+      const double tmin = bisect_minimum(S.q, prev_t, tt);
+      found = distinct_minimum(S, tmin, &beta);
+      if (found) e = S.q.eval(tmin);
+    }
+    for (unsigned m = __ballot_sync(kFull, found); m; m &= m - 1) {
+      const int src = __ffs(m) - 1;
+      const double eb = __shfl_sync(kFull, e, src), bb = __shfl_sync(kFull, beta, src);
+      n_minima++;
+      if (eb < best_err) {
+        best_err = eb;
+        *best_beta = bb;
+      }
+    }
+    carry_t = __shfl_sync(kFull, tt, 31);
+    carry_d = __shfl_sync(kFull, d, 31);
+  }
+  return n_minima;
+}
+
+// b200tag_estimate_pose for one record, by one warp.
+__device__ void estimate_pose_warp(const b200tag_detection *rec, const PoseLaunch &L, PoseShared &sh, int lane, b200tag_pose *dst) {
+  static_assert(sizeof(b200tag_detection) % 8 == 0 && sizeof(b200tag_detection) / 8 <= 32, "record copy");
+  static_assert(sizeof(b200tag_pose) % 8 == 0 && sizeof(b200tag_pose) / 8 <= 32, "pose copy");
+  if (lane < static_cast<int>(sizeof(b200tag_detection) / 8))
+    reinterpret_cast<double *>(&sh.det)[lane] = reinterpret_cast<const double *>(rec)[lane];
+  __syncwarp();
+  int ok = 0;
+  if (lane == 0) {
+    V3 v[4], p[4];
+    rays_and_corners(sh.det, L.tagsize, L.fx, L.fy, L.cx, L.cy, v, p);
+    ok = oi_prepare(v, p, &sh.oi);
+  }
+  ok = __shfl_sync(kFull, ok, 0);
+  __syncwarp();
+  {
+    M3 R1;
+    V3 t1;
+    pose_from_homography(sh.det.H, L.tagsize, L.fx, L.fy, L.cx, L.cy, &R1, &t1);
+    const double err1 = ok ? orthogonal_iteration(sh.oi, 50, &R1, &t1) : HUGE_VAL;
+    int has = 0;
+    if (lane == 0) {
+      sh.R1 = R1;
+      sh.t1 = t1;
+      sh.err1 = err1;
+      has = second_minimum_frame(sh.oi.v, sh.oi.p, R1, t1, &sh.S);
+    }
+    ok |= __shfl_sync(kFull, has, 0) << 1;
+    __syncwarp();
+  }
+  M3 R2{};
+  V3 t2{{0, 0, 0}};
+  double err2 = HUGE_VAL, beta;
+  if ((ok & 2) && search_second_minimum(sh.S, lane, &beta) == 1) {
+    R2 = second_minimum_rotation(sh.S, beta);
+    if (ok & 1) err2 = orthogonal_iteration(sh.oi, 50, &R2, &t2);
+  }
+  if (lane == 0) choose_pose(sh.R1, sh.t1, sh.err1, R2, t2, err2, &sh.out);
+  __syncwarp();
+  if (lane < static_cast<int>(sizeof(b200tag_pose) / 8))
+    reinterpret_cast<double *>(dst)[lane] = reinterpret_cast<const double *>(&sh.out)[lane];
+  __syncwarp();  // sh is reused by this warp's next record
+}
+
+// blockIdx.y = frame; the warps of a frame's CTAs walk that frame's detections, as many as its counter says.
+__global__ void __launch_bounds__(kPoseWarps * 32) k_pose(PoseLaunch L) {
+  __shared__ PoseShared sh[kPoseWarps];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const size_t frame = blockIdx.y;
+  const uint32_t n = L.counters ? min(L.counters[frame].num_detections, L.stride) : L.count;
+  const b200tag_detection *recs = L.dets + frame * L.stride;
+  b200tag_pose *out = L.out + frame * L.stride;
+  for (uint32_t i = blockIdx.x * kPoseWarps + w; i < n; i += gridDim.x * kPoseWarps)
+    estimate_pose_warp(recs + i, L, sh[w], lane, out + i);
+}
+
+}  // namespace
+
+int launch_pose(const PoseLaunch &L, int frames, cudaStream_t s, KernelTimer *kt) {
+  if (kt) kt->begin("pose", s);
+  // a frame of a batch has a handful of tags: 8 warps each, the rest loop; up to four frames (the single-frame latency
+  // path, a cluttered 4K scene has ~100 tags): 128 warps each, one pass.  A list without counters is one frame.
+  unsigned ctas = static_cast<unsigned>(frames) <= 4 ? 32u : 2u;
+  if (!L.counters) ctas = static_cast<unsigned>((L.count + kPoseWarps - 1) / kPoseWarps);
+  if (ctas > 0) k_pose<<<dim3(ctas, static_cast<unsigned>(frames)), kPoseWarps * 32, 0, s>>>(L);
+  if (kt) kt->end(s);
+  return 1;
+}
+
+}  // namespace b200tag

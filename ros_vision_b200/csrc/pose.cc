@@ -1,311 +1,62 @@
 // Tag pose from a detection: the step the node runs right after the hot path
 // (reference: src/apriltags_cuda/src/apriltags_cuda_detector.cu:425-462 calls libapriltag's
-// estimate_tag_pose(&info_, &pose) per detection; SURVEY.md section 8 row f3).
-//
-// libapriltag (github.com/cgpadwick/apriltag tag 3.3.0) is not vendored in the reference tree, so this is
-// a restatement of the published algorithm its apriltag_pose.c implements -- PARITY UNPINNED against
-// libapriltag itself; checked against ground-truth poses and an independent numpy restatement
-// (tests/test_pose.py):
-//   1. initial pose from the homography (homography_to_pose + polar decomposition),
-//   2. orthogonal iteration (Lu, Hager, Mjolsness 2000) for 50 steps,
-//   3. the second local minimum of the object-space error (Schweighofer & Pinz 2006): rotate into the frame
-//      where the ambiguity is a rotation about the y axis, minimise the quartic-over-(1+t^2)^2 error in
-//      t = tan(beta / 2), refine that candidate by orthogonal iteration too,
-//   4. return the pose with the smaller object-space error.
-// Host code: a handful of 3x3 operations per detection.
+// estimate_tag_pose(&info_, &pose) per detection; SURVEY.md section 8 row f3).  The arithmetic is in pose_core.h,
+// which the device kernel (kernels_pose.cu) shares; here it runs serially, one detection and one grid point at a time.
 #include <algorithm>
 #include <cmath>
-#include <cstring>
+#include <vector>
 
 #include "../../include/b200tag.h"
+#include "pose_core.h"
+
+namespace b200tag {
+
+void locate_from_poses(const b200tag_detection *dets, const b200tag_pose *poses, int count, const double *rotation,
+                       const double *offset, b200tag_tag_position *out) {
+  static const double kEye[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, kZero[3] = {0, 0, 0};
+  const double *Rx = rotation ? rotation : kEye, *ox = offset ? offset : kZero;
+  for (int i = 0; i < count; i++) {
+    const b200tag_pose &pose = poses[i];
+    b200tag_tag_position &o = out[i];
+    o.index = i;
+    o.id = dets[i].id;
+    for (int k = 0; k < 3; k++) o.camera[k] = pose.t[k];
+    for (int r = 0; r < 3; r++) o.robot[r] = Rx[3 * r] * pose.t[0] + Rx[3 * r + 1] * pose.t[1] + Rx[3 * r + 2] * pose.t[2] + ox[r];
+    o.distance = std::sqrt(pose.t[0] * pose.t[0] + pose.t[1] * pose.t[1] + pose.t[2] * pose.t[2]);
+    o.err = pose.err;
+  }
+  std::stable_sort(out, out + count, [](const b200tag_tag_position &a, const b200tag_tag_position &b) { return a.distance < b.distance; });
+}
+
+}  // namespace b200tag
+
+using namespace b200tag::pose;
 
 namespace {
 
-struct M3 {
-  double a[9];
-  double &operator()(int r, int c) { return a[r * 3 + c]; }
-  double operator()(int r, int c) const { return a[r * 3 + c]; }
-};
-struct V3 {
-  double v[3];
-};
-
-M3 ident() { return M3{{1, 0, 0, 0, 1, 0, 0, 0, 1}}; }
-M3 mul(const M3 &A, const M3 &B) {
-  M3 C{};
-  for (int i = 0; i < 3; i++)
-    for (int j = 0; j < 3; j++) C(i, j) = A(i, 0) * B(0, j) + A(i, 1) * B(1, j) + A(i, 2) * B(2, j);
-  return C;
-}
-M3 transpose(const M3 &A) {
-  M3 T{};
-  for (int i = 0; i < 3; i++)
-    for (int j = 0; j < 3; j++) T(i, j) = A(j, i);
-  return T;
-}
-V3 mul(const M3 &A, const V3 &x) {
-  return V3{{A(0, 0) * x.v[0] + A(0, 1) * x.v[1] + A(0, 2) * x.v[2], A(1, 0) * x.v[0] + A(1, 1) * x.v[1] + A(1, 2) * x.v[2],
-             A(2, 0) * x.v[0] + A(2, 1) * x.v[1] + A(2, 2) * x.v[2]}};
-}
-V3 add(const V3 &a, const V3 &b) { return V3{{a.v[0] + b.v[0], a.v[1] + b.v[1], a.v[2] + b.v[2]}}; }
-V3 sub(const V3 &a, const V3 &b) { return V3{{a.v[0] - b.v[0], a.v[1] - b.v[1], a.v[2] - b.v[2]}}; }
-V3 scale(const V3 &a, double s) { return V3{{a.v[0] * s, a.v[1] * s, a.v[2] * s}}; }
-double dot(const V3 &a, const V3 &b) { return a.v[0] * b.v[0] + a.v[1] * b.v[1] + a.v[2] * b.v[2]; }
-V3 cross(const V3 &a, const V3 &b) {
-  return V3{{a.v[1] * b.v[2] - a.v[2] * b.v[1], a.v[2] * b.v[0] - a.v[0] * b.v[2], a.v[0] * b.v[1] - a.v[1] * b.v[0]}};
-}
-M3 sub(const M3 &A, const M3 &B) {
-  M3 C{};
-  for (int i = 0; i < 9; i++) C.a[i] = A.a[i] - B.a[i];
-  return C;
-}
-double det3(const M3 &A) {
-  return A(0, 0) * (A(1, 1) * A(2, 2) - A(1, 2) * A(2, 1)) - A(0, 1) * (A(1, 0) * A(2, 2) - A(1, 2) * A(2, 0)) +
-         A(0, 2) * (A(1, 0) * A(2, 1) - A(1, 1) * A(2, 0));
-}
-bool inverse(const M3 &A, M3 *out) {
-  const double d = det3(A);
-  if (!(std::fabs(d) > 1e-300)) return false;
-  M3 I{};
-  I(0, 0) = (A(1, 1) * A(2, 2) - A(1, 2) * A(2, 1)) / d;
-  I(0, 1) = (A(0, 2) * A(2, 1) - A(0, 1) * A(2, 2)) / d;
-  I(0, 2) = (A(0, 1) * A(1, 2) - A(0, 2) * A(1, 1)) / d;
-  I(1, 0) = (A(1, 2) * A(2, 0) - A(1, 0) * A(2, 2)) / d;
-  I(1, 1) = (A(0, 0) * A(2, 2) - A(0, 2) * A(2, 0)) / d;
-  I(1, 2) = (A(0, 2) * A(1, 0) - A(0, 0) * A(1, 2)) / d;
-  I(2, 0) = (A(1, 0) * A(2, 1) - A(1, 1) * A(2, 0)) / d;
-  I(2, 1) = (A(0, 1) * A(2, 0) - A(0, 0) * A(2, 1)) / d;
-  I(2, 2) = (A(0, 0) * A(1, 1) - A(0, 1) * A(1, 0)) / d;
-  *out = I;
-  return true;
-}
-
-// One-sided Jacobi SVD of a 3x3 matrix: A = U diag(s) V^T.  Only U V^T is used by the callers.
-void svd3(const M3 &A, M3 *U, M3 *V) {
-  M3 W = A;  // columns are rotated until mutually orthogonal: W = A V
-  M3 Vm = ident();
-  for (int sweep = 0; sweep < 60; sweep++) {
-    double off = 0;
-    for (int p = 0; p < 2; p++) {
-      for (int q = p + 1; q < 3; q++) {
-        double alpha = 0, beta = 0, gamma = 0;
-        for (int i = 0; i < 3; i++) {
-          alpha += W(i, p) * W(i, p);
-          beta += W(i, q) * W(i, q);
-          gamma += W(i, p) * W(i, q);
-        }
-        off = std::fmax(off, std::fabs(gamma) / std::sqrt(alpha * beta + 1e-300));
-        if (std::fabs(gamma) < 1e-300) continue;
-        const double zeta = (beta - alpha) / (2 * gamma);
-        const double t = (zeta >= 0 ? 1.0 : -1.0) / (std::fabs(zeta) + std::sqrt(1 + zeta * zeta));
-        const double c = 1 / std::sqrt(1 + t * t), s = c * t;
-        for (int i = 0; i < 3; i++) {
-          const double wp = W(i, p), wq = W(i, q);
-          W(i, p) = c * wp - s * wq;
-          W(i, q) = s * wp + c * wq;
-          const double vp = Vm(i, p), vq = Vm(i, q);
-          Vm(i, p) = c * vp - s * vq;
-          Vm(i, q) = s * vp + c * vq;
-        }
-      }
-    }
-    if (off < 1e-15) break;
-  }
-  // U = W with normalised columns; a (near) zero column is replaced by the cross product of the other two
-  M3 Um{};
-  double n[3];
-  for (int j = 0; j < 3; j++) n[j] = std::sqrt(W(0, j) * W(0, j) + W(1, j) * W(1, j) + W(2, j) * W(2, j));
-  const double nmax = std::fmax(n[0], std::fmax(n[1], n[2]));
-  int small = -1;
-  for (int j = 0; j < 3; j++) {
-    if (n[j] > 1e-12 * nmax && n[j] > 0) {
-      for (int i = 0; i < 3; i++) Um(i, j) = W(i, j) / n[j];
-    } else {
-      small = j;
-    }
-  }
-  if (small >= 0) {
-    const int a = (small + 1) % 3, b = (small + 2) % 3;
-    const V3 ca{{Um(0, a), Um(1, a), Um(2, a)}}, cb{{Um(0, b), Um(1, b), Um(2, b)}};
-    const V3 cc = cross(ca, cb);
-    for (int i = 0; i < 3; i++) Um(i, small) = cc.v[i];
-  }
-  *U = Um;
-  *V = Vm;
-}
-
-M3 outer_over_norm(const V3 &v) {  // v v^T / (v^T v)
-  M3 F{};
-  const double d = dot(v, v);
-  for (int i = 0; i < 3; i++)
-    for (int j = 0; j < 3; j++) F(i, j) = v.v[i] * v.v[j] / d;
-  return F;
-}
-
-// Lu-Hager-Mjolsness orthogonal iteration; returns the object-space error of the final (R, t).
-double orthogonal_iteration(const V3 *v, const V3 *p, int n, int steps, M3 *R, V3 *t) {
-  V3 p_mean{{0, 0, 0}};
-  for (int i = 0; i < n; i++) p_mean = add(p_mean, scale(p[i], 1.0 / n));
-  V3 p_res[4];
-  M3 F[4], avgF{};
-  for (int i = 0; i < n; i++) {
-    p_res[i] = sub(p[i], p_mean);
-    F[i] = outer_over_norm(v[i]);
-    for (int k = 0; k < 9; k++) avgF.a[k] += F[i].a[k] / n;
-  }
-  M3 M1inv;
-  if (!inverse(sub(ident(), avgF), &M1inv)) return HUGE_VAL;
-  double err = HUGE_VAL;
-  for (int it = 0; it < steps; it++) {
-    V3 M2{{0, 0, 0}};
-    for (int j = 0; j < n; j++) M2 = add(M2, scale(mul(sub(F[j], ident()), mul(*R, p[j])), 1.0 / n));
-    *t = mul(M1inv, M2);
-    V3 q[4], q_mean{{0, 0, 0}};
-    for (int j = 0; j < n; j++) {
-      q[j] = mul(F[j], add(mul(*R, p[j]), *t));
-      q_mean = add(q_mean, scale(q[j], 1.0 / n));
-    }
-    M3 M3m{};
-    for (int j = 0; j < n; j++) {
-      const V3 d = sub(q[j], q_mean);
-      for (int r = 0; r < 3; r++)
-        for (int c = 0; c < 3; c++) M3m(r, c) += d.v[r] * p_res[j].v[c];
-    }
-    M3 U, V;
-    svd3(M3m, &U, &V);
-    *R = mul(U, transpose(V));
-    if (det3(*R) < 0) {
-      (*R)(0, 2) = -(*R)(0, 2);
-      (*R)(1, 2) = -(*R)(1, 2);
-      (*R)(2, 2) = -(*R)(2, 2);
-    }
-    err = 0;
-    for (int j = 0; j < n; j++) {
-      const V3 e = mul(sub(ident(), F[j]), add(mul(*R, p[j]), *t));
-      err += dot(e, e);
-    }
-  }
-  return err;
-}
-
-// homography_to_pose (libapriltag common/homography.c) + the estimate_pose_for_tag_homography wrapper.
-void pose_from_homography(const double *H, double tagsize, double fx, double fy, double cx, double cy, M3 *R, V3 *t) {
-  const double nfx = -fx;  // the wrapper passes -fx and flips the y and z axes afterwards
-  double R20 = H[6], R21 = H[7], TZ = H[8];
-  double R00 = (H[0] - cx * R20) / nfx, R01 = (H[1] - cx * R21) / nfx, TX = (H[2] - cx * TZ) / nfx;
-  double R10 = (H[3] - cy * R20) / fy, R11 = (H[4] - cy * R21) / fy, TY = (H[5] - cy * TZ) / fy;
-  const double l1 = std::sqrt(R00 * R00 + R10 * R10 + R20 * R20), l2 = std::sqrt(R01 * R01 + R11 * R11 + R21 * R21);
-  double s = 1.0 / std::sqrt(l1 * l2);
-  if (TZ > 0) s = -s;  // tag in front of a camera looking down -z
-  R20 *= s; R21 *= s; TZ *= s; R00 *= s; R01 *= s; TX *= s; R10 *= s; R11 *= s; TY *= s;
-  const double R02 = R10 * R21 - R20 * R11, R12 = R20 * R01 - R00 * R21, R22 = R00 * R11 - R10 * R01;
-  M3 Rm{{R00, R01, R02, R10, R11, R12, R20, R21, R22}};
-  M3 U, V;
-  svd3(Rm, &U, &V);
-  Rm = mul(U, transpose(V));  // polar decomposition: closest rotation
-  const double sc = tagsize / 2.0;
-  // fix = diag(1, -1, -1): camera looking down +z with y down
-  *R = M3{{Rm(0, 0), Rm(0, 1), Rm(0, 2), -Rm(1, 0), -Rm(1, 1), -Rm(1, 2), -Rm(2, 0), -Rm(2, 1), -Rm(2, 2)}};
-  *t = V3{{TX * sc, -TY * sc, -TZ * sc}};
-}
-
-// Object-space error as a function of the rotation beta about the y axis of the transformed frame, in
-// t = tan(beta / 2): E(t) = (a0 + a1 t + a2 t^2 + a3 t^3 + a4 t^4) / (1 + t^2)^2.
-struct Quartic {
-  double a[5];
-  double eval(double t) const {
-    const double num = a[0] + t * (a[1] + t * (a[2] + t * (a[3] + t * a[4])));
-    const double d = 1 + t * t;
-    return num / (d * d);
-  }
-  // numerator of dE/dt times (1 + t^2)^3
-  double dnum(double t) const {
-    return a[1] + t * ((2 * a[2] - 4 * a[0]) + t * ((3 * a[3] - 3 * a[1]) + t * ((4 * a[4] - 2 * a[2]) - t * a[3])));
-  }
-};
-
-// Schweighofer-Pinz second minimum.  Returns false when there is no distinct second minimum.
-bool second_minimum(const V3 *v, const V3 *p, int n, const M3 &R, const V3 &t, M3 *R2) {
-  const double tn = std::sqrt(dot(t, t));
-  if (!(tn > 0)) return false;
-  const V3 rt3 = scale(t, 1.0 / tn);
-  const V3 ex{{1, 0, 0}};
-  V3 rt1 = sub(ex, scale(rt3, dot(ex, rt3)));
-  const double n1 = std::sqrt(dot(rt1, rt1));
-  if (!(n1 > 1e-12)) return false;
-  rt1 = scale(rt1, 1.0 / n1);
-  const V3 rt2 = cross(rt3, rt1);
-  const M3 Rt{{rt1.v[0], rt1.v[1], rt1.v[2], rt2.v[0], rt2.v[1], rt2.v[2], rt3.v[0], rt3.v[1], rt3.v[2]}};
-  const M3 R1p = mul(Rt, R);
-  double r31 = R1p(2, 0), r32 = R1p(2, 1);
-  double hyp = std::sqrt(r31 * r31 + r32 * r32);
-  if (hyp < 1e-100) { r31 = 1; r32 = 0; hyp = 1; }
-  const M3 Rz{{r31 / hyp, -r32 / hyp, 0, r32 / hyp, r31 / hyp, 0, 0, 0, 1}};
-  const M3 Rtrans = mul(R1p, Rz);
-  const double sin_gamma = -Rtrans(0, 1), cos_gamma = Rtrans(1, 1);
-  const M3 Rgamma{{cos_gamma, -sin_gamma, 0, sin_gamma, cos_gamma, 0, 0, 0, 1}};
-  const double sin_beta = -Rtrans(2, 0), cos_beta = Rtrans(2, 2);
-  const double beta0 = std::atan2(sin_beta, cos_beta);
-
-  V3 vt[4], pt[4];
-  M3 Ft[4], avgF{};
-  const M3 RzT = transpose(Rz);
-  for (int i = 0; i < n; i++) {
-    vt[i] = mul(Rt, v[i]);
-    pt[i] = mul(RzT, p[i]);
-    Ft[i] = outer_over_norm(vt[i]);
-    for (int k = 0; k < 9; k++) avgF.a[k] += Ft[i].a[k] / n;
-  }
-  M3 G;
-  if (!inverse(sub(ident(), avgF), &G)) return false;
-  for (int k = 0; k < 9; k++) G.a[k] /= n;
-  // R_beta = (I + t M1 + t^2 M2) / (1 + t^2)
-  const M3 Mk[3] = {ident(), M3{{0, 0, 2, 0, 0, 0, -2, 0, 0}}, M3{{-1, 0, 0, 0, 1, 0, 0, 0, -1}}};
-  V3 b[3];
-  for (int k = 0; k < 3; k++) {
-    V3 acc{{0, 0, 0}};
-    for (int i = 0; i < n; i++) acc = add(acc, mul(sub(Ft[i], ident()), mul(Rgamma, mul(Mk[k], pt[i]))));
-    b[k] = mul(G, acc);
-  }
-  Quartic q{{0, 0, 0, 0, 0}};
-  for (int i = 0; i < n; i++) {
-    V3 c[3];
-    for (int k = 0; k < 3; k++) c[k] = mul(sub(ident(), Ft[i]), add(mul(Rgamma, mul(Mk[k], pt[i])), b[k]));
-    q.a[0] += dot(c[0], c[0]);
-    q.a[1] += 2 * dot(c[0], c[1]);
-    q.a[2] += dot(c[1], c[1]) + 2 * dot(c[0], c[2]);
-    q.a[3] += 2 * dot(c[1], c[2]);
-    q.a[4] += dot(c[2], c[2]);
-  }
-  // stationary points of E over beta in (-pi, pi): sign changes of dE/dt on a fine grid, refined by bisection
-  const int kGrid = 1440;
-  const double kPi = 3.14159265358979323846;
+// Step 3: the second minimum's rotation, when there is exactly one other minimum (libapriltag's rule).
+bool second_minimum(const V3 *v, const V3 *p, const M3 &R, const V3 &t, M3 *R2) {
+  SecondMinFrame S;
+  if (!second_minimum_frame(v, p, R, t, &S)) return false;
   double best_beta = 0, best_err = HUGE_VAL;
   int n_minima = 0;
-  double prev_t = std::tan((-kPi + 1e-9) / 2), prev_d = q.dnum(prev_t);
+  double prev_t = grid_t(0), prev_d = S.q.dnum(prev_t);
   for (int g = 1; g <= kGrid; g++) {
-    const double beta = -kPi + (2 * kPi) * g / kGrid - (g == kGrid ? 1e-9 : 0);
-    const double tt = std::tan(beta / 2), d = q.dnum(tt);
+    const double tt = grid_t(g), d = S.q.dnum(tt);
     if (prev_d < 0 && d >= 0) {  // derivative goes from negative to positive: a minimum in between
-      double lo = prev_t, hi = tt;
-      for (int it = 0; it < 80; it++) {
-        const double mid = 0.5 * (lo + hi);
-        if (q.dnum(mid) < 0) lo = mid; else hi = mid;
-      }
-      const double tmin = 0.5 * (lo + hi), bmin = 2 * std::atan(tmin);
-      if (std::fabs(bmin - beta0) > 0.1) {  // a different minimum than the one we started from
+      const double tmin = bisect_minimum(S.q, prev_t, tt);
+      double bmin;
+      if (distinct_minimum(S, tmin, &bmin)) {
         n_minima++;
-        const double e = q.eval(tmin);
+        const double e = S.q.eval(tmin);
         if (e < best_err) { best_err = e; best_beta = bmin; }
       }
     }
     prev_t = tt;
     prev_d = d;
   }
-  if (n_minima != 1) return false;  // libapriltag only accepts a unique second minimum
-  const double cb = std::cos(best_beta), sb = std::sin(best_beta);
-  const M3 Rbeta{{cb, 0, sb, 0, 1, 0, -sb, 0, cb}};
-  *R2 = mul(mul(mul(transpose(Rt), Rgamma), Rbeta), RzT);
+  if (n_minima != 1) return false;
+  *R2 = second_minimum_rotation(S, best_beta);
   return true;
 }
 
@@ -316,23 +67,19 @@ extern "C" {
 int b200tag_estimate_pose(const b200tag_detection *det, double tagsize, double fx, double fy, double cx, double cy,
                           b200tag_pose *out) {
   if (!det || !out || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
-  const double sc = tagsize / 2.0;
-  const V3 p[4] = {{{-sc, sc, 0}}, {{sc, sc, 0}}, {{sc, -sc, 0}}, {{-sc, -sc, 0}}};
-  V3 v[4];
-  for (int i = 0; i < 4; i++) v[i] = V3{{(det->p[i][0] - cx) / fx, (det->p[i][1] - cy) / fy, 1}};
+  V3 v[4], p[4];
+  rays_and_corners(*det, tagsize, fx, fy, cx, cy, v, p);
+  OiConsts c;
+  const bool ok = oi_prepare(v, p, &c);
   M3 R1;
   V3 t1;
   pose_from_homography(det->H, tagsize, fx, fy, cx, cy, &R1, &t1);
-  const double err1 = orthogonal_iteration(v, p, 4, 50, &R1, &t1);
-  M3 R2;
+  const double err1 = ok ? orthogonal_iteration(c, 50, &R1, &t1) : HUGE_VAL;
+  M3 R2{};
   double err2 = HUGE_VAL;
   V3 t2{{0, 0, 0}};
-  if (second_minimum(v, p, 4, R1, t1, &R2)) err2 = orthogonal_iteration(v, p, 4, 50, &R2, &t2);
-  const bool first = err1 <= err2;
-  std::memcpy(out->R, (first ? R1 : R2).a, sizeof(out->R));
-  std::memcpy(out->t, (first ? t1 : t2).v, sizeof(out->t));
-  out->err = first ? err1 : err2;
-  out->err_other = first ? err2 : err1;
+  if (second_minimum(v, p, R1, t1, &R2) && ok) err2 = orthogonal_iteration(c, 50, &R2, &t2);
+  choose_pose(R1, t1, err1, R2, t2, err2, out);
   return 0;
 }
 
@@ -347,20 +94,9 @@ int b200tag_estimate_poses(const b200tag_detection *dets, int count, double tags
 int b200tag_locate_tags(const b200tag_detection *dets, int count, double tagsize, double fx, double fy, double cx,
                         double cy, const double *rotation, const double *offset, b200tag_tag_position *out) {
   if (count < 0 || (count > 0 && (!dets || !out))) return B200TAG_E_INVALID;
-  static const double kEye[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, kZero[3] = {0, 0, 0};
-  const double *Rx = rotation ? rotation : kEye, *ox = offset ? offset : kZero;
-  for (int i = 0; i < count; i++) {
-    b200tag_pose pose;
-    if (int rc = b200tag_estimate_pose(dets + i, tagsize, fx, fy, cx, cy, &pose)) return rc;
-    b200tag_tag_position &o = out[i];
-    o.index = i;
-    o.id = dets[i].id;
-    for (int k = 0; k < 3; k++) o.camera[k] = pose.t[k];
-    for (int r = 0; r < 3; r++) o.robot[r] = Rx[3 * r] * pose.t[0] + Rx[3 * r + 1] * pose.t[1] + Rx[3 * r + 2] * pose.t[2] + ox[r];
-    o.distance = std::sqrt(pose.t[0] * pose.t[0] + pose.t[1] * pose.t[1] + pose.t[2] * pose.t[2]);
-    o.err = pose.err;
-  }
-  std::stable_sort(out, out + count, [](const b200tag_tag_position &a, const b200tag_tag_position &b) { return a.distance < b.distance; });
+  std::vector<b200tag_pose> poses(static_cast<size_t>(count));
+  if (int rc = b200tag_estimate_poses(dets, count, tagsize, fx, fy, cx, cy, poses.data())) return rc;
+  b200tag::locate_from_poses(dets, poses.data(), count, rotation, offset, out);
   return 0;
 }
 

@@ -1,0 +1,398 @@
+// Arithmetic of the pose step (b200tag_estimate_pose), shared by the host functions in pose.cc and the device kernel in
+// kernels_pose.cu.  libapriltag (github.com/cgpadwick/apriltag tag 3.3.0) is not vendored in the reference tree, so
+// this is a restatement of the published algorithm its apriltag_pose.c implements -- PARITY UNPINNED against
+// libapriltag itself; checked against ground-truth poses and an independent numpy restatement (tests/test_pose.py):
+//   1. initial pose from the homography (homography_to_pose + polar decomposition),
+//   2. orthogonal iteration (Lu, Hager, Mjolsness 2000) for 50 steps,
+//   3. the second local minimum of the object-space error (Schweighofer & Pinz 2006): rotate into the frame
+//      where the ambiguity is a rotation about the y axis, minimise the quartic-over-(1+t^2)^2 error in
+//      t = tan(beta / 2), refine that candidate by orthogonal iteration too,
+//   4. return the pose with the smaller object-space error.
+//
+// One source for both sides keeps them in step: the library is built with -ffp-contract=off for the host and
+// -fmad=false for the device, and steps 1 and 2 use only + - * /, sqrt, fabs and fmax, so the first local minimum
+// comes out bit-identical on host and device.  Only step 3 calls tan / atan / atan2 / sin / cos, where glibc and
+// libdevice may differ by an ulp.
+#ifndef B200TAG_POSE_CORE_H_
+#define B200TAG_POSE_CORE_H_
+
+#include <cmath>
+#include <cstdint>
+#include <cstring>
+
+#include "../../include/b200tag.h"
+
+#ifdef __CUDACC__
+#define POSE_HD __host__ __device__ inline
+#define POSE_UNROLL _Pragma("unroll")
+#else
+#define POSE_HD inline
+#define POSE_UNROLL
+#endif
+
+namespace b200tag {
+namespace pose {
+
+struct M3 {
+  double a[9];
+  POSE_HD double &operator()(int r, int c) { return a[r * 3 + c]; }
+  POSE_HD double operator()(int r, int c) const { return a[r * 3 + c]; }
+};
+struct V3 {
+  double v[3];
+};
+
+POSE_HD M3 ident() { return M3{{1, 0, 0, 0, 1, 0, 0, 0, 1}}; }
+POSE_HD M3 mul(const M3 &A, const M3 &B) {
+  M3 C{};
+  POSE_UNROLL for (int i = 0; i < 3; i++)
+    POSE_UNROLL for (int j = 0; j < 3; j++) C(i, j) = A(i, 0) * B(0, j) + A(i, 1) * B(1, j) + A(i, 2) * B(2, j);
+  return C;
+}
+POSE_HD M3 transpose(const M3 &A) {
+  M3 T{};
+  POSE_UNROLL for (int i = 0; i < 3; i++)
+    POSE_UNROLL for (int j = 0; j < 3; j++) T(i, j) = A(j, i);
+  return T;
+}
+POSE_HD V3 mul(const M3 &A, const V3 &x) {
+  return V3{{A(0, 0) * x.v[0] + A(0, 1) * x.v[1] + A(0, 2) * x.v[2], A(1, 0) * x.v[0] + A(1, 1) * x.v[1] + A(1, 2) * x.v[2],
+             A(2, 0) * x.v[0] + A(2, 1) * x.v[1] + A(2, 2) * x.v[2]}};
+}
+POSE_HD V3 add(const V3 &a, const V3 &b) { return V3{{a.v[0] + b.v[0], a.v[1] + b.v[1], a.v[2] + b.v[2]}}; }
+POSE_HD V3 sub(const V3 &a, const V3 &b) { return V3{{a.v[0] - b.v[0], a.v[1] - b.v[1], a.v[2] - b.v[2]}}; }
+POSE_HD V3 scale(const V3 &a, double s) { return V3{{a.v[0] * s, a.v[1] * s, a.v[2] * s}}; }
+POSE_HD double dot(const V3 &a, const V3 &b) { return a.v[0] * b.v[0] + a.v[1] * b.v[1] + a.v[2] * b.v[2]; }
+POSE_HD V3 cross(const V3 &a, const V3 &b) {
+  return V3{{a.v[1] * b.v[2] - a.v[2] * b.v[1], a.v[2] * b.v[0] - a.v[0] * b.v[2], a.v[0] * b.v[1] - a.v[1] * b.v[0]}};
+}
+POSE_HD M3 sub(const M3 &A, const M3 &B) {
+  M3 C{};
+  POSE_UNROLL for (int i = 0; i < 9; i++) C.a[i] = A.a[i] - B.a[i];
+  return C;
+}
+POSE_HD double det3(const M3 &A) {
+  return A(0, 0) * (A(1, 1) * A(2, 2) - A(1, 2) * A(2, 1)) - A(0, 1) * (A(1, 0) * A(2, 2) - A(1, 2) * A(2, 0)) +
+         A(0, 2) * (A(1, 0) * A(2, 1) - A(1, 1) * A(2, 0));
+}
+POSE_HD bool inverse(const M3 &A, M3 *out) {
+  const double d = det3(A);
+  if (!(fabs(d) > 1e-300)) return false;
+  M3 I{};
+  I(0, 0) = (A(1, 1) * A(2, 2) - A(1, 2) * A(2, 1)) / d;
+  I(0, 1) = (A(0, 2) * A(2, 1) - A(0, 1) * A(2, 2)) / d;
+  I(0, 2) = (A(0, 1) * A(1, 2) - A(0, 2) * A(1, 1)) / d;
+  I(1, 0) = (A(1, 2) * A(2, 0) - A(1, 0) * A(2, 2)) / d;
+  I(1, 1) = (A(0, 0) * A(2, 2) - A(0, 2) * A(2, 0)) / d;
+  I(1, 2) = (A(0, 2) * A(1, 0) - A(0, 0) * A(1, 2)) / d;
+  I(2, 0) = (A(1, 0) * A(2, 1) - A(1, 1) * A(2, 0)) / d;
+  I(2, 1) = (A(0, 1) * A(2, 0) - A(0, 0) * A(2, 1)) / d;
+  I(2, 2) = (A(0, 0) * A(1, 1) - A(0, 1) * A(1, 0)) / d;
+  *out = I;
+  return true;
+}
+
+// One-sided Jacobi SVD of a 3x3 matrix: A = U diag(s) V^T.  Only U V^T is used by the callers.
+POSE_HD void svd3(const M3 &A, M3 *U, M3 *V) {
+  M3 W = A;  // columns are rotated until mutually orthogonal: W = A V
+  M3 Vm = ident();
+  for (int sweep = 0; sweep < 60; sweep++) {
+    double off = 0;
+    POSE_UNROLL for (int p = 0; p < 2; p++) {
+      POSE_UNROLL for (int q = p + 1; q < 3; q++) {
+        double alpha = 0, beta = 0, gamma = 0;
+        POSE_UNROLL for (int i = 0; i < 3; i++) {
+          alpha += W(i, p) * W(i, p);
+          beta += W(i, q) * W(i, q);
+          gamma += W(i, p) * W(i, q);
+        }
+        off = fmax(off, fabs(gamma) / sqrt(alpha * beta + 1e-300));
+        if (fabs(gamma) < 1e-300) continue;
+        const double zeta = (beta - alpha) / (2 * gamma);
+        const double t = (zeta >= 0 ? 1.0 : -1.0) / (fabs(zeta) + sqrt(1 + zeta * zeta));
+        const double c = 1 / sqrt(1 + t * t), s = c * t;
+        POSE_UNROLL for (int i = 0; i < 3; i++) {
+          const double wp = W(i, p), wq = W(i, q);
+          W(i, p) = c * wp - s * wq;
+          W(i, q) = s * wp + c * wq;
+          const double vp = Vm(i, p), vq = Vm(i, q);
+          Vm(i, p) = c * vp - s * vq;
+          Vm(i, q) = s * vp + c * vq;
+        }
+      }
+    }
+    if (off < 1e-15) break;
+  }
+  // U = W with normalised columns; a (near) zero column is replaced by the cross product of the other two
+  M3 Um{};
+  double n[3];
+  POSE_UNROLL for (int j = 0; j < 3; j++) n[j] = sqrt(W(0, j) * W(0, j) + W(1, j) * W(1, j) + W(2, j) * W(2, j));
+  const double nmax = fmax(n[0], fmax(n[1], n[2]));
+  int small = -1;
+  POSE_UNROLL for (int j = 0; j < 3; j++) {
+    if (n[j] > 1e-12 * nmax && n[j] > 0) {
+      POSE_UNROLL for (int i = 0; i < 3; i++) Um(i, j) = W(i, j) / n[j];
+    } else {
+      small = j;
+    }
+  }
+  // the replaced column, spelled out per case so that no matrix is indexed with a run-time value
+  POSE_UNROLL for (int j = 0; j < 3; j++) {
+    if (small == j) {
+      const int a = (j + 1) % 3, b = (j + 2) % 3;
+      const V3 ca{{Um(0, a), Um(1, a), Um(2, a)}}, cb{{Um(0, b), Um(1, b), Um(2, b)}};
+      const V3 cc = cross(ca, cb);
+      POSE_UNROLL for (int i = 0; i < 3; i++) Um(i, j) = cc.v[i];
+    }
+  }
+  *U = Um;
+  *V = Vm;
+}
+
+POSE_HD M3 outer_over_norm(const V3 &v) {  // v v^T / (v^T v)
+  M3 F{};
+  const double d = dot(v, v);
+  POSE_UNROLL for (int i = 0; i < 3; i++)
+    POSE_UNROLL for (int j = 0; j < 3; j++) F(i, j) = v.v[i] * v.v[j] / d;
+  return F;
+}
+
+POSE_HD bool same_bits(double a, double b) {
+#ifdef __CUDA_ARCH__
+  return __double_as_longlong(a) == __double_as_longlong(b);
+#else
+  int64_t x, y;
+  memcpy(&x, &a, sizeof(x));
+  memcpy(&y, &b, sizeof(y));
+  return x == y;
+#endif
+}
+
+// What the orthogonal iteration reads on every step for one detection: its four image rays v, the tag corners p,
+// p minus their mean, F = v v^T / v^T v and (I - mean F)^-1.  The device kernel keeps it in shared memory.
+struct OiConsts {
+  V3 v[4], p[4], p_res[4];
+  M3 F[4];
+  M3 M1inv;
+};
+
+// Fills `c` from v and p (4 points each); false when I - mean(F) cannot be inverted.
+POSE_HD bool oi_prepare(const V3 *v, const V3 *p, OiConsts *c) {
+  const int n = 4;
+  V3 p_mean{{0, 0, 0}};
+  POSE_UNROLL for (int i = 0; i < n; i++) p_mean = add(p_mean, scale(p[i], 1.0 / n));
+  M3 avgF{};
+  POSE_UNROLL for (int i = 0; i < n; i++) {
+    c->v[i] = v[i];
+    c->p[i] = p[i];
+    c->p_res[i] = sub(p[i], p_mean);
+    c->F[i] = outer_over_norm(v[i]);
+    POSE_UNROLL for (int k = 0; k < 9; k++) avgF.a[k] += c->F[i].a[k] / n;
+  }
+  return inverse(sub(ident(), avgF), &c->M1inv);
+}
+
+// Lu-Hager-Mjolsness orthogonal iteration from *R; returns the object-space error of the final (R, t).  A step that
+// gives back the rotation it started from, bit for bit, gives back the same t and error too, and so does every later
+// step: the iteration stops there with the result of all `steps` steps.
+POSE_HD double orthogonal_iteration(const OiConsts &c, int steps, M3 *R, V3 *t) {
+  const int n = 4;
+  double err = HUGE_VAL;
+  for (int it = 0; it < steps; it++) {
+    V3 M2{{0, 0, 0}};
+    POSE_UNROLL for (int j = 0; j < n; j++) M2 = add(M2, scale(mul(sub(c.F[j], ident()), mul(*R, c.p[j])), 1.0 / n));
+    *t = mul(c.M1inv, M2);
+    V3 q[4], q_mean{{0, 0, 0}};
+    POSE_UNROLL for (int j = 0; j < n; j++) {
+      q[j] = mul(c.F[j], add(mul(*R, c.p[j]), *t));
+      q_mean = add(q_mean, scale(q[j], 1.0 / n));
+    }
+    M3 M3m{};
+    POSE_UNROLL for (int j = 0; j < n; j++) {
+      const V3 d = sub(q[j], q_mean);
+      POSE_UNROLL for (int r = 0; r < 3; r++)
+        POSE_UNROLL for (int k = 0; k < 3; k++) M3m(r, k) += d.v[r] * c.p_res[j].v[k];
+    }
+    M3 U, V;
+    svd3(M3m, &U, &V);
+    M3 Rn = mul(U, transpose(V));
+    if (det3(Rn) < 0) {
+      Rn(0, 2) = -Rn(0, 2);
+      Rn(1, 2) = -Rn(1, 2);
+      Rn(2, 2) = -Rn(2, 2);
+    }
+    bool same = true;
+    POSE_UNROLL for (int k = 0; k < 9; k++) same = same && same_bits(Rn.a[k], R->a[k]);
+    *R = Rn;
+    err = 0;
+    POSE_UNROLL for (int j = 0; j < n; j++) {
+      const V3 e = mul(sub(ident(), c.F[j]), add(mul(*R, c.p[j]), *t));
+      err += dot(e, e);
+    }
+    if (same) break;
+  }
+  return err;
+}
+
+// homography_to_pose (libapriltag common/homography.c) + the estimate_pose_for_tag_homography wrapper.
+POSE_HD void pose_from_homography(const double *H, double tagsize, double fx, double fy, double cx, double cy, M3 *R, V3 *t) {
+  const double nfx = -fx;  // the wrapper passes -fx and flips the y and z axes afterwards
+  double R20 = H[6], R21 = H[7], TZ = H[8];
+  double R00 = (H[0] - cx * R20) / nfx, R01 = (H[1] - cx * R21) / nfx, TX = (H[2] - cx * TZ) / nfx;
+  double R10 = (H[3] - cy * R20) / fy, R11 = (H[4] - cy * R21) / fy, TY = (H[5] - cy * TZ) / fy;
+  const double l1 = sqrt(R00 * R00 + R10 * R10 + R20 * R20), l2 = sqrt(R01 * R01 + R11 * R11 + R21 * R21);
+  double s = 1.0 / sqrt(l1 * l2);
+  if (TZ > 0) s = -s;  // tag in front of a camera looking down -z
+  R20 *= s; R21 *= s; TZ *= s; R00 *= s; R01 *= s; TX *= s; R10 *= s; R11 *= s; TY *= s;
+  const double R02 = R10 * R21 - R20 * R11, R12 = R20 * R01 - R00 * R21, R22 = R00 * R11 - R10 * R01;
+  M3 Rm{{R00, R01, R02, R10, R11, R12, R20, R21, R22}};
+  M3 U, V;
+  svd3(Rm, &U, &V);
+  Rm = mul(U, transpose(V));  // polar decomposition: closest rotation
+  const double sc = tagsize / 2.0;
+  // fix = diag(1, -1, -1): camera looking down +z with y down
+  *R = M3{{Rm(0, 0), Rm(0, 1), Rm(0, 2), -Rm(1, 0), -Rm(1, 1), -Rm(1, 2), -Rm(2, 0), -Rm(2, 1), -Rm(2, 2)}};
+  *t = V3{{TX * sc, -TY * sc, -TZ * sc}};
+}
+
+// Rays through the detection's corners and the tag's corners in its own frame (step 1's inputs).
+POSE_HD void rays_and_corners(const b200tag_detection &det, double tagsize, double fx, double fy, double cx, double cy, V3 *v, V3 *p) {
+  const double sc = tagsize / 2.0;
+  p[0] = V3{{-sc, sc, 0}}; p[1] = V3{{sc, sc, 0}}; p[2] = V3{{sc, -sc, 0}}; p[3] = V3{{-sc, -sc, 0}};
+  POSE_UNROLL for (int i = 0; i < 4; i++) v[i] = V3{{(det.p[i][0] - cx) / fx, (det.p[i][1] - cy) / fy, 1}};
+}
+
+// Object-space error as a function of the rotation beta about the y axis of the transformed frame, in
+// t = tan(beta / 2): E(t) = (a0 + a1 t + a2 t^2 + a3 t^3 + a4 t^4) / (1 + t^2)^2.
+struct Quartic {
+  double a[5];
+  POSE_HD double eval(double t) const {
+    const double num = a[0] + t * (a[1] + t * (a[2] + t * (a[3] + t * a[4])));
+    const double d = 1 + t * t;
+    return num / (d * d);
+  }
+  // numerator of dE/dt times (1 + t^2)^3
+  POSE_HD double dnum(double t) const {
+    return a[1] + t * ((2 * a[2] - 4 * a[0]) + t * ((3 * a[3] - 3 * a[1]) + t * ((4 * a[4] - 2 * a[2]) - t * a[3])));
+  }
+};
+
+// The rotated frame of the Schweighofer-Pinz search and the error quartic in it.
+struct SecondMinFrame {
+  M3 Rt, Rgamma, RzT;
+  double beta0;  // beta of the pose the search started from
+  Quartic q;
+};
+
+// Step 3 up to the search: false when the pose has no distinct second minimum to look for.
+POSE_HD bool second_minimum_frame(const V3 *v, const V3 *p, const M3 &R, const V3 &t, SecondMinFrame *S) {
+  const int n = 4;
+  const double tn = sqrt(dot(t, t));
+  if (!(tn > 0)) return false;
+  const V3 rt3 = scale(t, 1.0 / tn);
+  const V3 ex{{1, 0, 0}};
+  V3 rt1 = sub(ex, scale(rt3, dot(ex, rt3)));
+  const double n1 = sqrt(dot(rt1, rt1));
+  if (!(n1 > 1e-12)) return false;
+  rt1 = scale(rt1, 1.0 / n1);
+  const V3 rt2 = cross(rt3, rt1);
+  const M3 Rt{{rt1.v[0], rt1.v[1], rt1.v[2], rt2.v[0], rt2.v[1], rt2.v[2], rt3.v[0], rt3.v[1], rt3.v[2]}};
+  const M3 R1p = mul(Rt, R);
+  double r31 = R1p(2, 0), r32 = R1p(2, 1);
+  double hyp = sqrt(r31 * r31 + r32 * r32);
+  if (hyp < 1e-100) { r31 = 1; r32 = 0; hyp = 1; }
+  const M3 Rz{{r31 / hyp, -r32 / hyp, 0, r32 / hyp, r31 / hyp, 0, 0, 0, 1}};
+  const M3 Rtrans = mul(R1p, Rz);
+  const double sin_gamma = -Rtrans(0, 1), cos_gamma = Rtrans(1, 1);
+  const M3 Rgamma{{cos_gamma, -sin_gamma, 0, sin_gamma, cos_gamma, 0, 0, 0, 1}};
+  const double sin_beta = -Rtrans(2, 0), cos_beta = Rtrans(2, 2);
+  S->beta0 = atan2(sin_beta, cos_beta);
+
+  V3 vt[4], pt[4];
+  M3 Ft[4], avgF{};
+  const M3 RzT = transpose(Rz);
+  POSE_UNROLL for (int i = 0; i < n; i++) {
+    vt[i] = mul(Rt, v[i]);
+    pt[i] = mul(RzT, p[i]);
+    Ft[i] = outer_over_norm(vt[i]);
+    POSE_UNROLL for (int k = 0; k < 9; k++) avgF.a[k] += Ft[i].a[k] / n;
+  }
+  M3 G;
+  if (!inverse(sub(ident(), avgF), &G)) return false;
+  POSE_UNROLL for (int k = 0; k < 9; k++) G.a[k] /= n;
+  // R_beta = (I + t M1 + t^2 M2) / (1 + t^2)
+  const M3 Mk[3] = {ident(), M3{{0, 0, 2, 0, 0, 0, -2, 0, 0}}, M3{{-1, 0, 0, 0, 1, 0, 0, 0, -1}}};
+  V3 b[3];
+  POSE_UNROLL for (int k = 0; k < 3; k++) {
+    V3 acc{{0, 0, 0}};
+    POSE_UNROLL for (int i = 0; i < n; i++) acc = add(acc, mul(sub(Ft[i], ident()), mul(Rgamma, mul(Mk[k], pt[i]))));
+    b[k] = mul(G, acc);
+  }
+  Quartic q{{0, 0, 0, 0, 0}};
+  POSE_UNROLL for (int i = 0; i < n; i++) {
+    V3 c[3];
+    POSE_UNROLL for (int k = 0; k < 3; k++) c[k] = mul(sub(ident(), Ft[i]), add(mul(Rgamma, mul(Mk[k], pt[i])), b[k]));
+    q.a[0] += dot(c[0], c[0]);
+    q.a[1] += 2 * dot(c[0], c[1]);
+    q.a[2] += dot(c[1], c[1]) + 2 * dot(c[0], c[2]);
+    q.a[3] += 2 * dot(c[1], c[2]);
+    q.a[4] += dot(c[2], c[2]);
+  }
+  S->Rt = Rt;
+  S->Rgamma = Rgamma;
+  S->RzT = RzT;
+  S->q = q;
+  return true;
+}
+
+// The search for stationary points of E over beta in (-pi, pi): the sign of dE/dt at grid points g = 0..kGrid, a
+// minimum wherever it goes from negative to non-negative, refined by bisection.
+constexpr int kGrid = 1440;
+constexpr double kPi = 3.14159265358979323846;
+
+POSE_HD double grid_t(int g) {  // t = tan(beta / 2) at grid point g; the ends stay 1e-9 inside (-pi, pi)
+  if (g == 0) return tan((-kPi + 1e-9) / 2);
+  const double beta = -kPi + (2 * kPi) * g / kGrid - (g == kGrid ? 1e-9 : 0);
+  return tan(beta / 2);
+}
+
+POSE_HD double bisect_minimum(const Quartic &q, double lo, double hi) {
+  for (int it = 0; it < 80; it++) {
+    const double mid = 0.5 * (lo + hi);
+    if (q.dnum(mid) < 0) lo = mid; else hi = mid;
+  }
+  return 0.5 * (lo + hi);
+}
+
+// A refined minimum counts when it is a different one than the search started from: then *beta is its angle.
+POSE_HD bool distinct_minimum(const SecondMinFrame &S, double tmin, double *beta) {
+  *beta = 2 * atan(tmin);
+  return fabs(*beta - S.beta0) > 0.1;
+}
+
+// The rotation of the second minimum, back in the camera frame.
+POSE_HD M3 second_minimum_rotation(const SecondMinFrame &S, double beta) {
+  const double cb = cos(beta), sb = sin(beta);
+  const M3 Rbeta{{cb, 0, sb, 0, 1, 0, -sb, 0, cb}};
+  return mul(mul(mul(transpose(S.Rt), S.Rgamma), Rbeta), S.RzT);
+}
+
+// The better of the two minima into `out` (b200tag_estimate_pose's choice).
+POSE_HD void choose_pose(const M3 &R1, const V3 &t1, double err1, const M3 &R2, const V3 &t2, double err2, b200tag_pose *out) {
+  const bool first = err1 <= err2;
+  POSE_UNROLL for (int k = 0; k < 9; k++) out->R[k] = first ? R1.a[k] : R2.a[k];
+  POSE_UNROLL for (int k = 0; k < 3; k++) out->t[k] = first ? t1.v[k] : t2.v[k];
+  out->err = first ? err1 : err2;
+  out->err_other = first ? err2 : err1;
+}
+
+}  // namespace pose
+
+// Host, pose.cc: the node's records from poses already estimated (robot frame, distance, closest first), the step
+// b200tag_locate_tags and b200tag_tag_positions share.  poses[i] belongs to dets[i].
+void locate_from_poses(const b200tag_detection *dets, const b200tag_pose *poses, int count, const double *rotation,
+                       const double *offset, b200tag_tag_position *out);
+
+}  // namespace b200tag
+
+#endif  // B200TAG_POSE_CORE_H_

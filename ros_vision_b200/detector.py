@@ -145,6 +145,12 @@ def load_library():
     L.b200tag_last_error.restype = C.c_char_p
     L.b200tag_estimate_poses.argtypes = [vp, i32] + [C.c_double] * 5 + [vp]
     L.b200tag_locate_tags.argtypes = [vp, i32] + [C.c_double] * 5 + [vp, vp, vp]
+    L.b200tag_set_pose_estimation.argtypes = [vp] + [C.c_double] * 5 + [vp, vp]
+    L.b200tag_poses.argtypes = [vp, i32, C.POINTER(i32)]
+    L.b200tag_poses.restype = vp
+    L.b200tag_tag_positions.argtypes = [vp, i32, C.POINTER(i32)]
+    L.b200tag_tag_positions.restype = vp
+    L.b200tag_debug_estimate_poses_device.argtypes = [vp, i32] + [C.c_double] * 5 + [vp]
     L.b200tag_version.restype = i32
     _lib = L
     return L
@@ -201,6 +207,27 @@ def locate_tags(detections: np.ndarray, tagsize: float, fx: float, fy: float, cx
     if rc:
         raise B200TagError(f"b200tag_locate_tags: {lib.b200tag_error_string(rc).decode()}")
     return out
+
+
+def estimate_poses_device(detections: np.ndarray, tagsize: float, fx: float, fy: float, cx: float, cy: float) -> np.ndarray:
+    """Test hook: estimate_poses computed by the device pose kernel (the one GpuDetector.SetPoseEstimation enables) on
+    the current CUDA device."""
+    lib = load_library()
+    dets = np.ascontiguousarray(detections, dtype=DETECTION_DT)
+    out = np.zeros(len(dets), dtype=POSE_DT)
+    rc = lib.b200tag_debug_estimate_poses_device(dets.ctypes.data_as(C.c_void_p) if len(dets) else None, len(dets), float(tagsize),
+                                                 float(fx), float(fy), float(cx), float(cy),
+                                                 out.ctypes.data_as(C.c_void_p) if len(dets) else None)
+    if rc:
+        raise B200TagError(f"b200tag_debug_estimate_poses_device: {lib.b200tag_error_string(rc).decode()}")
+    return out
+
+
+def _records(ptr, n, dtype) -> np.ndarray:
+    if not ptr or n == 0:
+        return np.zeros((0,), dtype=dtype)
+    buf = (C.c_char * (dtype.itemsize * n)).from_address(ptr)
+    return np.frombuffer(buf, dtype=dtype, count=n).copy()
 
 
 class PinnedBuffer:
@@ -397,6 +424,27 @@ class GpuDetector:
             return np.zeros((0,), dtype=QUAD_DT)
         buf = (C.c_char * (QUAD_DT.itemsize * n.value)).from_address(p)
         return np.frombuffer(buf, dtype=QUAD_DT, count=n.value).copy()
+
+    def SetPoseEstimation(self, tagsize, fx, fy, cx, cy, rotation=None, offset=None) -> None:
+        """The node's pose step on the GPU: from the next Detect on, a kernel at the end of the detection graph estimates
+        every detection's pose (Poses) and its robot-frame record (TagPositions), with the arguments of locate_tags.
+        tagsize = 0 turns it off."""
+        rot = None if rotation is None else np.ascontiguousarray(rotation, dtype=np.float64).reshape(9)
+        off = None if offset is None else np.ascontiguousarray(offset, dtype=np.float64).reshape(3)
+        self._check(self._lib.b200tag_set_pose_estimation(self._h, float(tagsize), float(fx), float(fy), float(cx), float(cy),
+                                                          None if rot is None else rot.ctypes.data_as(C.c_void_p),
+                                                          None if off is None else off.ctypes.data_as(C.c_void_p)),
+                    "b200tag_set_pose_estimation")
+
+    def Poses(self, frame: int = 0) -> np.ndarray:
+        """POSE_DT records parallel to Detections(frame); empty when the last call ran without the pose step."""
+        n = C.c_int()
+        return _records(self._lib.b200tag_poses(self._h, frame, C.byref(n)), n.value, POSE_DT)
+
+    def TagPositions(self, frame: int = 0) -> np.ndarray:
+        """TAG_POSITION_DT records of frame `frame`, closest first, as locate_tags(Detections(frame), ...) returns them."""
+        n = C.c_int()
+        return _records(self._lib.b200tag_tag_positions(self._h, frame, C.byref(n)), n.value, TAG_POSITION_DT)
 
     def ReinitializeDetections(self) -> None:
         """apriltag_gpu.cu:202-220 frees and re-creates the zarray; results here are plain arrays."""

@@ -1,0 +1,153 @@
+#!/usr/bin/env python3
+"""What the device pose step (GpuDetector.SetPoseEstimation) costs, on config 2 (bench.py's workload:
+synth.config_frame(2, i), 1280x800 YUYV, 1-6 tags per frame), in one run on one GPU:
+
+  * device-resident frames/s of 128-frame batches with the pose step off and on, alternating in the same run;
+  * single-frame latency (pinned host frame in -> detections and poses out), p50, off and on, alternating;
+  * the `pose` kernel's device time per 128-frame batch (b200tag_profile_device);
+  * the host time of b200tag_locate_tags on the same detections, on one CPU core of the same machine.
+
+Prints one JSON record, and writes it to --out when given.  Needs a CUDA device."""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+TAGSIZE = 0.1651
+FX, FY, CX, CY = 905.5, 907.9, 640.0, 400.0
+ROTATION = [[0, 0, 1], [-1, 0, 0], [0, -1, 0]]
+OFFSET = [0.1, -0.2, 0.5]
+BATCH, UNIQUE = 128, 16
+
+
+def gpu_identity():
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"],
+                             capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.TimeoutExpired):
+        out = ""
+    return out
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--rounds", type=int, default=6, help="alternations of the off / on measurements")
+    ap.add_argument("--steps", type=int, default=40, help="128-frame batches per throughput measurement")
+    ap.add_argument("--latency-iters", type=int, default=400, help="single frames per latency measurement")
+    ap.add_argument("--out", help="also write the JSON to this file (e.g. profiles/pose_r03.json)")
+    args = ap.parse_args()
+
+    import torch
+    from ros_vision_b200 import detector as D, synth
+    frames = [np.ascontiguousarray(synth.config_frame(2, i)[0]).reshape(-1) for i in range(UNIQUE)]
+    host_batch = np.stack([frames[i % UNIQUE] for i in range(BATCH)])
+    dev_batch = torch.from_numpy(host_batch).cuda()
+    ptr = dev_batch.data_ptr()
+
+    def detector(pose, max_batch):
+        d = D.GpuDetector(1280, 800, "yuyv", quad_decimate=2, max_batch=max_batch)
+        if pose:
+            d.SetPoseEstimation(TAGSIZE, FX, FY, CX, CY, rotation=ROTATION, offset=OFFSET)
+        return d
+
+    # throughput: 128-frame device-resident batches, off and on alternating
+    big = {False: detector(False, BATCH), True: detector(True, BATCH)}
+    for d in big.values():
+        for _ in range(5):
+            d.DetectDevice(ptr, BATCH)
+    fps = {False: [], True: []}
+    for _ in range(args.rounds):
+        for pose in (False, True):
+            d = big[pose]
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            for _ in range(args.steps):
+                d.DetectDevice(ptr, BATCH)
+            fps[pose].append(BATCH * args.steps / (time.perf_counter() - t0))
+    dets_per_batch = sum(len(big[True].Detections(f)) for f in range(BATCH))
+    raw_per_batch = sum(int(big[True].FrameInfo(f).num_detections) for f in range(BATCH))
+
+    # the pose kernel's device time per batch
+    prof = big[True].ProfileDevice(ptr, BATCH, iters=20)
+    pose_ms = [ms for name, ms in prof if name == "pose"]
+    total_ms = sum(ms for _, ms in prof)
+
+    # single-frame latency from a pinned host frame, off and on alternating over the 16 frames
+    one = {False: detector(False, 1), True: detector(True, 1)}
+    pins = []
+    for f in frames:
+        pb = D.PinnedBuffer(f.size)
+        pb.array[:] = f
+        pins.append(pb)
+    lat = {False: [], True: []}
+    for d in one.values():
+        for pb in pins:
+            d.DetectPointers([pb.ptr])
+    for i in range(args.latency_iters):
+        pb = pins[i % UNIQUE]
+        for pose in ((False, True) if i % 2 == 0 else (True, False)):
+            t0 = time.perf_counter()
+            one[pose].DetectPointers([pb.ptr])
+            lat[pose].append((time.perf_counter() - t0) * 1e6)
+
+    # host locate_tags on the same detections, one core
+    per_frame_dets = []
+    for pb_i in range(UNIQUE):
+        one[False].DetectPointers([pins[pb_i].ptr])
+        per_frame_dets.append(one[False].Detections(0))
+    cpu = sorted(os.sched_getaffinity(0))[0]
+    saved = os.sched_getaffinity(0)
+    os.sched_setaffinity(0, {cpu})
+    host_us = []
+    try:
+        for dets in per_frame_dets:
+            D.locate_tags(dets, TAGSIZE, FX, FY, CX, CY, ROTATION, OFFSET)
+            reps = []
+            for _ in range(20):
+                t0 = time.perf_counter()
+                D.locate_tags(dets, TAGSIZE, FX, FY, CX, CY, ROTATION, OFFSET)
+                reps.append((time.perf_counter() - t0) * 1e6)
+            host_us.append(float(np.median(reps)))
+    finally:
+        os.sched_setaffinity(0, saved)
+    n_dets = [len(d) for d in per_frame_dets]
+
+    p50 = {k: float(np.percentile(v, 50)) for k, v in lat.items()}
+    host_frame_p50 = float(np.median(host_us))
+    res = {
+        "gpu": gpu_identity(),
+        "torch_device": torch.cuda.get_device_name(0),
+        "workload": "config2: 1280x800 YUYV, synth.config_frame(2, 0..15) tiled to 128-frame batches, tag36h11, decimate 2",
+        "batch_frames_per_s": {"pose_off": fps[False], "pose_on": fps[True],
+                               "median_off": float(np.median(fps[False])), "median_on": float(np.median(fps[True])),
+                               "ratio_on_over_off": float(np.median(fps[True]) / np.median(fps[False]))},
+        "detections_per_batch": dets_per_batch, "raw_detections_per_batch": raw_per_batch,
+        "pose_kernel_ms_per_batch": pose_ms[0] if pose_ms else None,
+        "all_kernels_ms_per_batch_serial": total_ms,
+        "single_frame_latency_us": {"p50_off": p50[False], "p50_on": p50[True], "p90_off": float(np.percentile(lat[False], 90)),
+                                    "p90_on": float(np.percentile(lat[True], 90)), "iters": args.latency_iters},
+        "host_locate_tags_us_per_frame": {"per_frame": host_us, "detections": n_dets, "median": host_frame_p50,
+                                          "us_per_detection": float(sum(host_us) / max(1, sum(n_dets))), "cpu": cpu},
+        "targets": {"batch_ratio_at_least_0.95": bool(np.median(fps[True]) >= 0.95 * np.median(fps[False])),
+                    "p50_on_below_p50_off_plus_host_pose": bool(p50[True] < p50[False] + host_frame_p50)},
+    }
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            json.dump(res, f, indent=1)
+    print(json.dumps(res, indent=1))
+    for d in list(big.values()) + list(one.values()):
+        d.close()
+    for pb in pins:
+        pb.close()
+
+
+if __name__ == "__main__":
+    main()
