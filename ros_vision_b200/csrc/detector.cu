@@ -73,7 +73,6 @@ struct NativeJpeg {
   bool init = false;
   std::vector<JpegParsed> parsed;
   bool last_native = false;    // the last MJPG batch went through this decoder (else nvJPEG)
-  int launches = 0;            // kernels of the last decode
   const uint32_t *d_proven = nullptr;  // per frame of the last batch: decoded by the parallel kernels
   bool last_parallel = false;
 };
@@ -378,16 +377,16 @@ int record_sequence(b200tag_detector *det, const void *device_images, size_t str
     p.gray_stride = p.in_stride;
   }
   CK(cudaMemsetAsync(p.counters, 0, sizeof(Counters) * count, det->stream));
-  int launches = 0;
-  launches += launch_frontend(p, count, det->stream, kt);
-  launches += launch_blobs(p, count, det->stream, kt, kt ? nullptr : &det->side);  // per-kernel timing runs serially
-  launches += launch_decode(p, count, det->stream, kt);
+  Launcher ln{det->stream, kt};
+  launch_frontend(p, count, ln);
+  launch_blobs(p, count, ln, kt ? nullptr : &det->side);  // per-kernel timing runs serially
+  launch_decode(p, count, ln);
   if (det->pose.tagsize > 0) {
     const auto &ps = det->pose;
     const PoseLaunch pl{det->d_dets_alias, det->d_poses_alias, p.counters, p.det_cap, 0, ps.tagsize, ps.fx, ps.fy, ps.cx, ps.cy};
-    launches += launch_pose(pl, count, det->stream, kt);
+    launch_pose(pl, count, ln);
   }
-  *launches_out = launches;
+  *launches_out = ln.count;
   CK(cudaMemcpyAsync(det->h_counters, p.counters, sizeof(Counters) * count, cudaMemcpyDeviceToHost, det->stream));
   return 0;
 }
@@ -1065,7 +1064,7 @@ static int mjpg_native(b200tag_detector *det, const uint8_t *const *jpegs, const
   // B200TAG_MJPG_DECODER=sequential keeps every frame on the warp-per-frame kernel (tests / comparison)
   const char *which = getenv("B200TAG_MJPG_DECODER");
   if (which && std::string(which) == "sequential") any_parallel = false;
-  J.launches = launch_jpeg_decode(jb, any_parallel, det->stream);
+  launch_jpeg_decode(jb, any_parallel, det->stream);
   J.d_proven = jb.proven;
   J.last_parallel = any_parallel;
   CK(cudaGetLastError());
@@ -1476,7 +1475,8 @@ int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count
                       0, static_cast<uint32_t>(count), tagsize, fx, fy, cx, cy};
   if (cudaMemcpy(d, dets, db, cudaMemcpyHostToDevice) != cudaSuccess) rc = B200TAG_E_CUDA;
   if (!rc) {
-    launch_pose(pl, 1, nullptr, nullptr);
+    Launcher ln{nullptr, nullptr};
+    launch_pose(pl, 1, ln);
     if (cudaGetLastError() != cudaSuccess || cudaMemcpy(out, d + db, pb, cudaMemcpyDeviceToHost) != cudaSuccess) rc = B200TAG_E_CUDA;
   }
   cudaFree(d);

@@ -4,7 +4,6 @@
 
 #include <cuda_runtime.h>
 
-#include <cstdlib>
 #include <string>
 #include <vector>
 
@@ -20,7 +19,6 @@ struct KernelTimer {
   };
   std::vector<Span> spans;
   size_t cursor = 0;
-  bool recording = false;
   void begin(const char *name, cudaStream_t s) {
     if (cursor == spans.size()) {
       Span sp{name, nullptr, nullptr};
@@ -51,23 +49,30 @@ struct SideStreams {
   cudaEvent_t fork = nullptr, join[3] = {nullptr, nullptr, nullptr};
 };
 
-// Measurement switches (bit mask in the environment variable B200TAG_EXP, read once): select another variant of a
-// kernel so that both can be timed in one run (tools/exp_kernels.py).  Unset = the production variants.
-//    1: k_scatter with one point in flight per thread (production: 4)      32: ... with 8
-//    2: k_boundary with the uncapped point list and a 512-entry CTA-local table (9 CTAs per SM; production: 16)
-//    4: k_boundary with the capped list and a 512-entry table (12 CTAs per SM)
-//    8: k_ccl_final without the 32-register cap (6 CTAs per SM; production: 8)
-//   64: k_select at 5 instead of 8 CTAs per SM, grid sized for 4 per SM
-//  512: the shared-memory tile blur for filter lengths 3, 5, 7 (production: k_blur_strip)
-inline int exp_flags() {
-  static const int f = [] { const char *e = getenv("B200TAG_EXP"); return e ? atoi(e) : 0; }();
-  return f;
-}
+// The main stream of a launch sequence, the optional timer, and the number of kernels launched so far
+// (b200tag_kernels_per_batch).
+struct Launcher {
+  cudaStream_t s;
+  KernelTimer *kt;
+  int count = 0;
+  // One kernel, timed as span `name` on s -- also when `launch` puts it on a side stream.
+  template <class F>
+  void timed(const char *name, F &&launch) {
+    if (kt) kt->begin(name, s);
+    launch();
+    if (kt) kt->end(s);
+    count++;
+  }
+  template <class F>
+  void untimed(F &&launch) {
+    launch();
+    count++;
+  }
+};
 
-// Each returns the number of kernels it launched.
-int launch_frontend(const FrameParams &p, int frames, cudaStream_t s, KernelTimer *kt);
-int launch_blobs(const FrameParams &p, int frames, cudaStream_t s, KernelTimer *kt, const SideStreams *side);
-int launch_decode(const FrameParams &p, int frames, cudaStream_t s, KernelTimer *kt);
+void launch_frontend(const FrameParams &p, int frames, Launcher &ln);
+void launch_blobs(const FrameParams &p, int frames, Launcher &ln, const SideStreams *side);
+void launch_decode(const FrameParams &p, int frames, Launcher &ln);
 size_t ccl_tiles_per_frame(int w, int h);  // CCL tiles of one frame and the capacity of a tile's root list
 size_t ccl_root_cap();
 void launch_hash_clear(const FrameParams &p, int frames, cudaStream_t s);
@@ -81,12 +86,12 @@ struct PoseLaunch {
   uint32_t stride, count;
   double tagsize, fx, fy, cx, cy;
 };
-int launch_pose(const PoseLaunch &L, int frames, cudaStream_t s, KernelTimer *kt);
+void launch_pose(const PoseLaunch &L, int frames, Launcher &ln);
 
 // JPEG luminance planes of a batch (jpeg.h): the parallel kernels for streams without restart markers, the sequential
-// warp-per-frame kernel for the rest.  Returns the number of kernels launched.
+// warp-per-frame kernel for the rest.
 struct JpegBatch;
-int launch_jpeg_decode(const JpegBatch &B, bool any_parallel, cudaStream_t s);
+void launch_jpeg_decode(const JpegBatch &B, bool any_parallel, cudaStream_t s);
 
 }  // namespace b200tag
 

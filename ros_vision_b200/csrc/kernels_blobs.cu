@@ -54,8 +54,7 @@ __device__ __forceinline__ bool select_blob(const FrameParams &p, uint32_t count
 // points and run at the top of the fit kernels.
 // (a latency kernel -- two barriers and one round of atomics per trip: eight CTAs per SM and a grid that fills them
 //  once, so that every CTA makes as few trips as possible)
-template <int MIN_CTAS>
-__global__ void __launch_bounds__(256, MIN_CTAS) k_select(FrameParams p) {
+__global__ void __launch_bounds__(256, 8) k_select(FrameParams p) {
   __shared__ uint32_t s_warp[8][6];  // per-warp totals: occupied, candidates, small, points, medium, huge
   __shared__ unsigned long long s_base;
   __shared__ uint32_t s_pbase, s_mbase, s_lbase, s_hbase;
@@ -192,8 +191,8 @@ __global__ void __launch_bounds__(256, MIN_CTAS) k_select(FrameParams p) {
 // U points per thread and trip: the chain point -> slot_off[slot] -> store is two dependent memory round trips, and with
 // one point per thread the kernel ran at the latency of that chain (0.082 ms per 128 config-2 frames, 53 % of the HBM
 // peak); U independent chains per thread hide it.
-template <int U>
 __global__ void __launch_bounds__(256) k_scatter(FrameParams p) {
+  constexpr int U = 4;
   const int frame = blockIdx.y;
   const Counters *ctr = p.counters + frame;
   const uint32_t np = min(ctr->num_points, p.point_cap);
@@ -1480,21 +1479,13 @@ void launch_blobs_init(cudaStream_t s) {
   }
 }
 
-int launch_blobs(const FrameParams &p, int frames, cudaStream_t s, KernelTimer *kt, const SideStreams *side) {
-  if (kt) kt->begin("select", s);
-  if (exp_flags() & 64) k_select<1><<<dim3(max(1u, min(16u, cdivu(148u * 4u, frames))), frames), 256, 0, s>>>(p);
-  else k_select<8><<<dim3(max(1u, min(16u, 148u * 8u / static_cast<unsigned>(frames))), frames), 256, 0, s>>>(p);
-  if (kt) kt->end(s);
-  if (kt) kt->begin("scatter", s);
-  if (exp_flags() & 1) k_scatter<1><<<dim3(max(8u, min(592u, cdivu(4736u, frames))), frames), 256, 0, s>>>(p);
-  else if (exp_flags() & 32) k_scatter<8><<<dim3(max(8u, min(592u, cdivu(4736u, frames))), frames), 256, 0, s>>>(p);
-  else k_scatter<4><<<dim3(max(8u, min(592u, cdivu(4736u, frames))), frames), 256, 0, s>>>(p);
-  if (kt) kt->end(s);
-  int launches = 6;
+void launch_blobs(const FrameParams &p, int frames, Launcher &ln, const SideStreams *side) {
+  const cudaStream_t s = ln.s;
+  ln.timed("select", [&] { k_select<<<dim3(max(1u, min(16u, 148u * 8u / static_cast<unsigned>(frames))), frames), 256, 0, s>>>(p); });
+  ln.timed("scatter", [&] { k_scatter<<<dim3(max(8u, min(592u, cdivu(4736u, frames))), frames), 256, 0, s>>>(p); });
   if (p.clusters) {  // debug stage only (keep_stages)
-    k_cluster_extents<<<dim3(max(8u, min(592u, cdivu(4736u, frames))), frames), 256, 0, s>>>(p);
-    k_cluster_finish<<<dim3(16, frames), 256, 0, s>>>(p);
-    launches += 2;
+    ln.untimed([&] { k_cluster_extents<<<dim3(max(8u, min(592u, cdivu(4736u, frames))), frames), 256, 0, s>>>(p); });
+    ln.untimed([&] { k_cluster_finish<<<dim3(16, frames), 256, 0, s>>>(p); });
   }
   // The three tiers are independent and each is latency bound at modest occupancy: with side streams they run
   // concurrently (largest blobs first), so their tails overlap; the per-kernel timing mode runs them serially.
@@ -1507,41 +1498,34 @@ int launch_blobs(const FrameParams &p, int frames, cudaStream_t s, KernelTimer *
     cudaStreamWaitEvent(s_medium, side->fork, 0);
     cudaStreamWaitEvent(s_huge, side->fork, 0);
   }
-  if (kt) kt->begin("fit_huge", s);
-  {
+  ln.timed("fit_huge", [&] {
     const dim3 g(max(1u, min(148u, cdivu(592u, frames))), frames);
     if (p.keep_stages) K_FIT_HUGE(true)<<<g, kHugeThreads, sizeof(HugeShared), s_huge>>>(p, 2);
     else K_FIT_HUGE(false)<<<g, kHugeThreads, sizeof(HugeShared), s_huge>>>(p, 2);
-  }
-  if (kt) kt->end(s);
-  if (kt) kt->begin("fit_large", s);
+  });
   // (the shared-memory prefix moments keep Mx, My, W as 32-bit words: kSortCap points of weight <= 361 must not reach
   //  2^32, which holds for quad images up to 1451 pixels a side -- larger frames take the 256-thread kernel)
   const bool lf32_ok = static_cast<uint64_t>(kSortCap) * 361u * (2u * static_cast<uint32_t>(max(p.w, p.h)) + 1u) < (1ull << 32);
-  if (frames <= kLowLatencyFrames && lf32_ok) {
-    const dim3 g(max(1u, min(148u, cdivu(592u, frames))), frames);
-    if (p.keep_stages) K_FIT_LARGE512(true)<<<g, kHugeThreads, sizeof(Large512Shared), s_large>>>(p, 1);
-    else K_FIT_LARGE512(false)<<<g, kHugeThreads, sizeof(Large512Shared), s_large>>>(p, 1);
-  } else {
-    const dim3 g(max(3u, min(444u, cdivu(1776u, frames))), frames);
-    if (p.keep_stages) K_FIT_LARGE(true)<<<g, kLargeThreads, sizeof(LargeShared), s_large>>>(p, 1);
-    else K_FIT_LARGE(false)<<<g, kLargeThreads, sizeof(LargeShared), s_large>>>(p, 1);
-  }
-  if (kt) kt->end(s);
-  if (kt) kt->begin("fit_medium", s);
-  {
-    const dim3 g(max(4u, min(740u, cdivu(2960u, frames))), frames);
+  ln.timed("fit_large", [&] {
+    if (frames <= kLowLatencyFrames && lf32_ok) {
+      const dim3 g(max(1u, min(148u, cdivu(592u, frames))), frames);
+      if (p.keep_stages) K_FIT_LARGE512(true)<<<g, kHugeThreads, sizeof(Large512Shared), s_large>>>(p, 1);
+      else K_FIT_LARGE512(false)<<<g, kHugeThreads, sizeof(Large512Shared), s_large>>>(p, 1);
+    } else {
+      const dim3 g(max(3u, min(444u, cdivu(1776u, frames))), frames);
+      if (p.keep_stages) K_FIT_LARGE(true)<<<g, kLargeThreads, sizeof(LargeShared), s_large>>>(p, 1);
+      else K_FIT_LARGE(false)<<<g, kLargeThreads, sizeof(LargeShared), s_large>>>(p, 1);
+    }
+  });
+  const dim3 g(max(4u, min(740u, cdivu(2960u, frames))), frames);
+  ln.timed("fit_medium", [&] {
     if (p.keep_stages) K_FIT_MEDIUM(true)<<<g, 128, sizeof(MediumShared), s_medium>>>(p, 0);
     else K_FIT_MEDIUM(false)<<<g, 128, sizeof(MediumShared), s_medium>>>(p, 0);
-  }
-  if (kt) kt->end(s);
-  if (kt) kt->begin("fit_small", s);
-  {
-    const dim3 g(max(4u, min(740u, cdivu(2960u, frames))), frames);
+  });
+  ln.timed("fit_small", [&] {
     if (p.keep_stages) k_fit_small<true><<<g, kSmallWarps * 32, sizeof(SmallWarpShared) * kSmallWarps, s>>>(p);
     else k_fit_small<false><<<g, kSmallWarps * 32, sizeof(SmallWarpShared) * kSmallWarps, s>>>(p);
-  }
-  if (kt) kt->end(s);
+  });
   if (fork) {
     cudaEventRecord(side->join[0], s_large);
     cudaEventRecord(side->join[1], s_medium);
@@ -1550,10 +1534,7 @@ int launch_blobs(const FrameParams &p, int frames, cudaStream_t s, KernelTimer *
     cudaStreamWaitEvent(s, side->join[1], 0);
     cudaStreamWaitEvent(s, side->join[2], 0);
   }
-  if (kt) kt->begin("quads", s);
-  k_quads<<<dim3(max(2u, min(592u, cdivu(2368u, frames))), frames), kQuadWarps * 32, 0, s>>>(p);
-  if (kt) kt->end(s);
-  return launches + 1;
+  ln.timed("quads", [&] { k_quads<<<dim3(max(2u, min(592u, cdivu(2368u, frames))), frames), kQuadWarps * 32, 0, s>>>(p); });
 }
 
 }  // namespace b200tag

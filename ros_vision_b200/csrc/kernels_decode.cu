@@ -547,15 +547,14 @@ __global__ void __launch_bounds__(32 * WARPS) k_decode(FrameParams p) {
   }
 }
 
-int launch_decode(const FrameParams &p, int frames, cudaStream_t s, KernelTimer *kt) {
-  if (kt) kt->begin("decode", s);
+void launch_decode(const FrameParams &p, int frames, Launcher &ln) {
   // batches: one warp per CTA, about 2400 CTAs in total (a frame has ~100 candidate quads); up to four frames: four
   // warps per quad, all 148 SMs
   const unsigned per_frame = static_cast<unsigned>(frames) >= 16 ? (2368u + frames - 1) / frames : 148u;
-  if (frames <= 4) k_decode<4><<<dim3(148u, frames), 128, 0, s>>>(p);
-  else k_decode<1><<<dim3(per_frame < 8u ? 8u : per_frame, frames), 32, 0, s>>>(p);
-  if (kt) kt->end(s);
-  return 1;
+  ln.timed("decode", [&] {
+    if (frames <= 4) k_decode<4><<<dim3(148u, frames), 128, 0, ln.s>>>(p);
+    else k_decode<1><<<dim3(per_frame < 8u ? 8u : per_frame, frames), 32, 0, ln.s>>>(p);
+  });
 }
 
 }  // namespace b200tag

@@ -11,7 +11,6 @@
 // here is a contraction; the bound is HBM/L2 bandwidth and atomics latency.
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 #include "dev_types.h"
 #include "kernels.h"
@@ -226,13 +225,12 @@ __global__ void __launch_bounds__(256) k_pre_bgr_dec1(FrameParams p) {
 // rest copied), rows first then columns.  One CTA = 64x128 output pixels (64x32: 0.066 ms per 16 config-3 frames, 64x128: 0.061).  The input tile with its halo is staged in
 // shared memory with 4-byte loads (the halo is rounded up to a multiple of 4 columns so every word is aligned); both
 // passes work on words: a thread filters 4 neighbouring pixels from the bytes it has in registers (row pass) or from
-// aligned word loads of the rows above and below (column pass) and stores one word.  KSZ = filter length as a
-// compile-time constant (3, 5, 7: quad_sigma up to 1.9), or 0 to take it from the parameters.
+// aligned word loads of the rows above and below (column pass) and stores one word.  Runs the filter lengths that
+// k_blur_strip does not take.
 constexpr int kBlurTW = 64, kBlurTH = 128;  // (the host caps the filter radius at 15: detector.cu blur_kernel)
-template <int KSZ>
 __global__ void __launch_bounds__(256) k_blur(FrameParams p) {
   extern __shared__ __align__(16) uint8_t s_blur[];
-  const int ksz = KSZ ? KSZ : p.blur_ksz, r = ksz >> 1, r4 = (r + 3) & ~3;
+  const int ksz = p.blur_ksz, r = ksz >> 1, r4 = (r + 3) & ~3;
   const int sw = kBlurTW + 2 * r4, sh = kBlurTH + 2 * r;   // staged input tile, sw a multiple of 4
   uint8_t *s_in = s_blur;                                   // [sh][sw]
   uint8_t *s_row = s_blur + sh * sw;                        // [sh][kBlurTW]: row-filtered
@@ -253,9 +251,6 @@ __global__ void __launch_bounds__(256) k_blur(FrameParams p) {
     }
   }
   __syncthreads();
-  uint32_t kk[KSZ ? KSZ : 32];
-#pragma unroll
-  for (int j = 0; j < (KSZ ? KSZ : 32); j++) kk[j] = j < ksz ? p.blur_k[j] : 0u;
   // row pass: thread = 4 pixels of a staged row (16 words per row, 16 rows per sweep)
   const int q = threadIdx.x & 15, rsub = threadIdx.x >> 4;
   for (int yy = rsub; yy < sh; yy += 16) {
@@ -267,12 +262,7 @@ __global__ void __launch_bounds__(256) k_blur(FrameParams p) {
       uint32_t v = row[px];
       if (gx >= r && gx < p.w - ksz + r) {
         uint32_t acc = 0;
-        if constexpr (KSZ != 0) {
-#pragma unroll
-          for (int j = 0; j < KSZ; j++) acc += kk[j] * row[px - r + j];
-        } else {
-          for (int j = 0; j < ksz; j++) acc += static_cast<uint32_t>(p.blur_k[j]) * row[px - r + j];
-        }
+        for (int j = 0; j < ksz; j++) acc += static_cast<uint32_t>(p.blur_k[j]) * row[px - r + j];
         v = (acc >> 8) & 0xff;
       }
       out |= v << (8 * px);
@@ -287,17 +277,9 @@ __global__ void __launch_bounds__(256) k_blur(FrameParams p) {
     uint32_t out = reinterpret_cast<const uint32_t *>(s_row + (yy + r) * kBlurTW)[q];
     if (gy >= r && gy < p.h - ksz + r) {
       uint32_t a0 = 0, a1 = 0, a2 = 0, a3 = 0;
-      if constexpr (KSZ != 0) {
-#pragma unroll
-        for (int j = 0; j < KSZ; j++) {
-          const uint32_t wv = reinterpret_cast<const uint32_t *>(s_row + (yy + j) * kBlurTW)[q];
-          a0 += kk[j] * (wv & 0xff); a1 += kk[j] * ((wv >> 8) & 0xff); a2 += kk[j] * ((wv >> 16) & 0xff); a3 += kk[j] * (wv >> 24);
-        }
-      } else {
-        for (int j = 0; j < ksz; j++) {
-          const uint32_t wv = reinterpret_cast<const uint32_t *>(s_row + (yy + j) * kBlurTW)[q], kj = p.blur_k[j];
-          a0 += kj * (wv & 0xff); a1 += kj * ((wv >> 8) & 0xff); a2 += kj * ((wv >> 16) & 0xff); a3 += kj * (wv >> 24);
-        }
+      for (int j = 0; j < ksz; j++) {
+        const uint32_t wv = reinterpret_cast<const uint32_t *>(s_row + (yy + j) * kBlurTW)[q], kj = p.blur_k[j];
+        a0 += kj * (wv & 0xff); a1 += kj * ((wv >> 8) & 0xff); a2 += kj * ((wv >> 16) & 0xff); a3 += kj * (wv >> 24);
       }
       out = ((a0 >> 8) & 0xff) | (((a1 >> 8) & 0xff) << 8) | (((a2 >> 8) & 0xff) << 16) | (((a3 >> 8) & 0xff) << 24);
     }
@@ -476,7 +458,6 @@ __global__ void __launch_bounds__(128) k_tile_minmax(FrameParams p) {
 constexpr int kCclTW = 32;  // tile width: one 32-bit run mask per row and colour
 constexpr int kCclTH = 64;  // tile height
 constexpr int kCclThreads = 128;
-constexpr int kCclWarps = kCclThreads / 32;
 static_assert(kCclThreads == 2 * kCclTH, "one thread per (row, colour)");
 static_assert(kCclThreads == (kCclTW / 4) * (kCclTH / 4), "one thread per 4x4 threshold tile of the CCL tile");
 
@@ -556,8 +537,7 @@ constexpr uint32_t kCclRootCap = 2 * kCclTW + 2 * kCclTH;
 // (tried: a run's first link to the row above as ONE atomicMin on the run's own word -- it still is its own root unless a
 //  run below has linked it already, and any smaller index of the other component keeps the forest valid -- instead of two
 //  finds and the atomicMin: correct, but the links to non-roots make the later finds longer, 0.269 -> 0.298 ms)
-template <int MIN_CTAS>
-__global__ void __launch_bounds__(kCclThreads, MIN_CTAS) k_ccl_local(FrameParams p) {
+__global__ void __launch_bounds__(kCclThreads, 16) k_ccl_local(FrameParams p) {
   __shared__ uint32_t s_mask[2][kCclTH];  // [0] black, [1] white
   // parent links; from phase (C) on a ROOT's word also carries its counters above the index (kParBits):
   // [10:0] parent | [22:11] pixels of the component (<= 2048) | [30:23] runs of it that touch the tile border (<= 192)
@@ -573,7 +553,7 @@ __global__ void __launch_bounds__(kCclThreads, MIN_CTAS) k_ccl_local(FrameParams
   uint8_t *th = p.thresh + frame * n;
   uint32_t *labels = p.labels + frame * n;
   uint32_t *sizes = p.sizes + frame * n;
-  const int tid = threadIdx.x, lane = tid & 31;
+  const int tid = threadIdx.x;
 
   {  // (T)
     const int tlx = tid & 7, tly = tid >> 3;
@@ -890,8 +870,8 @@ __global__ void __launch_bounds__(256) k_ccl_handoff(FrameParams p, uint32_t til
 constexpr int kFinThreads = 256;
 constexpr int kFinPasses = kCclTW * kCclTH / 4 / kFinThreads;
 constexpr uint32_t kFinUnused = 0xffffffffu, kFinNeeded = 0xfffffffeu;
-template <int MIN_CTAS>
-__global__ void __launch_bounds__(kFinThreads, MIN_CTAS) k_ccl_final(FrameParams p) {
+// (8 CTAs per SM caps it at 32 registers; uncapped it ran at 6 CTAs per SM: 0.111 against 0.097 ms per 128 config-2 frames)
+__global__ void __launch_bounds__(kFinThreads, 8) k_ccl_final(FrameParams p) {
   __shared__ uint32_t s_out[kCclTW * kCclTH];
   __shared__ uint16_t s_list[kCclTW * kCclTH];
   __shared__ uint32_t s_nlist;
@@ -969,7 +949,7 @@ __global__ void __launch_bounds__(kFinThreads, MIN_CTAS) k_ccl_final(FrameParams
 // ---------------------------------------------------------------------------------------------
 // K6: boundary points, grouped by blob pair.
 //
-// One CTA = one 64x8 (or 64x16) pixel tile (halo staged in shared memory as label | big | colour).
+// One CTA = one 64x8 pixel tile (halo staged in shared memory as label | big | colour).
 //   (1) per pixel: which of the 4 directions emit a point (apriltag_gpu.cu:276-357); the points
 //       are compacted into a shared-memory list, so everything after this runs with full warps;
 //   (2) per point: blob-pair key -> entry of a CTA-local hash table, local rank by one
@@ -1012,21 +992,21 @@ __device__ uint32_t hash_insert(const FrameParams &p, unsigned long long *keys, 
 }
 
 // staged cell = label word: [27:0] label | [28] big enough | [30:29] colour class (0 black, 1 white, 2 gray)
-// TH = tile height (16 or 8 rows); 16 threads per row.
-// CAP = points of the tile that phases (2)-(4) take in one go.  A tile can emit up to four points per pixel, thresholded
-// sensor noise emits 0.75, long one-pixel stripes 2: the list buffers hold CAP = 2 points per pixel and a tile with more
-// goes through (2)-(4) in several rounds, each with a fresh CTA-local table (ranks stay consistent: every round adds its
-// counts to the global table before its records are written).  Half the list memory = 12 instead of 9 CTAs per SM.
+constexpr int kBpTH = 8;                 // tile height; 16 threads per row
+constexpr int kBpThreads = kBpTH * 16;
+// kBpMaxPts = points of the tile that phases (2)-(4) take in one go.  A tile can emit up to four points per pixel,
+// thresholded sensor noise emits 0.75, long one-pixel stripes 2: the list buffers hold 2 points per pixel and a tile with
+// more goes through (2)-(4) in several rounds, each with a fresh CTA-local table (ranks stay consistent: every round adds
+// its counts to the global table before its records are written).  Half the list memory = 12 instead of 9 CTAs per SM.
+constexpr int kBpMaxPts = 1024;
+static_assert(kBpMaxPts <= kBpTW * kBpTH * 4 && kBpMaxPts % 32 == 0, "list capacity");
+constexpr int kBpLHBits = 8;
+constexpr uint32_t kBpLH = 1u << kBpLHBits;  // local blob-pair table (power of two, <= 1024: 10-bit entry index in s_loc)
+static_assert(kBpLH <= 1024, "local table size");
 // SMALL_ROUNDS: the test variant that takes 96 points per round (B200TAG_TEST_SMALL_CHUNKS), its own instantiation so
 // that the production kernel compares against a compile-time capacity.
-template <int TH, int CAP, int LHBITS, bool SMALL_ROUNDS>
-__global__ void __launch_bounds__(TH * 16) k_boundary(FrameParams p) {
-  constexpr int kBpTH = TH, kBpThreads = TH * 16;
-  constexpr int kBpMaxPts = CAP;
-  static_assert(CAP <= kBpTW * TH * 4 && CAP % 32 == 0, "list capacity");
-  constexpr uint32_t kBpLH = 1u << LHBITS;  // local blob-pair table (power of two, <= 1024: 10-bit entry index in s_loc)
-  constexpr int kBpLHBits = LHBITS;
-  static_assert(kBpLH <= 1024 && (kBpLH & (kBpLH - 1)) == 0, "local table size");
+template <bool SMALL_ROUNDS>
+__global__ void __launch_bounds__(kBpThreads) k_boundary(FrameParams p) {
   __shared__ uint32_t s_cell[kBpTH + 1][kBpTW + 2];
   __shared__ uint16_t s_pts[kBpMaxPts];             // [12:3] pixel of the tile | [2:1] dir | [0] black_to_white
   __shared__ uint32_t s_loc[kBpMaxPts];             // [9:0] local entry | [31:10] rank among the tile's points of that entry
@@ -1034,7 +1014,7 @@ __global__ void __launch_bounds__(TH * 16) k_boundary(FrameParams p) {
   __shared__ __align__(16) uint32_t s_lcnt[kBpLH];            // points of the entry in this tile; after (3): base rank
   __shared__ uint16_t s_used[kBpLH];                // entries in use, in claim order: (3) runs over these, densely
   __shared__ uint32_t s_nused;
-  __shared__ uint32_t s_npts, s_gbase, s_half;
+  __shared__ uint32_t s_npts, s_gbase;
   __shared__ uint32_t s_rowm[kBpTH + 1][3][2];      // white / black / big masks of a staged row, two 32-bit halves
   __shared__ uint8_t s_halo[kBpTH + 1][2];          // the same three bits for the left / right halo column
   __shared__ unsigned long long s_emit[kBpTH][4], s_b2w[kBpTH][4];
@@ -1145,7 +1125,8 @@ __global__ void __launch_bounds__(TH * 16) k_boundary(FrameParams p) {
     }
     s_emit[ry][d] = emit;
     s_b2w[ry][d] = b2w;
-    // exclusive prefix of the popcounts over the 64 (row, direction) words: two warps, then a fix-up
+    // exclusive prefix of the popcounts over the 32 (row, direction) words: one warp
+    static_assert(kBpTH * 4 == 32, "one warp per (row, direction) word");
     const uint32_t cnt = static_cast<uint32_t>(__popcll(emit));
     uint32_t incl = cnt;
 #pragma unroll
@@ -1154,21 +1135,15 @@ __global__ void __launch_bounds__(TH * 16) k_boundary(FrameParams p) {
       if (lane >= o) incl += t;
     }
     s_ebase[ry][d] = incl - cnt;
-    if (tid == 31) s_half = incl;
-    if (tid == kBpTH * 4 - 1) s_npts = incl;  // (with two warps: the second half only; completed below)
-  }
-  if constexpr (kBpTH * 4 > 32) {
-    __syncthreads();
-    if (tid >= 32 && tid < kBpTH * 4) s_ebase[tid >> 2][tid & 3] += s_half;
-    if (tid == 0) s_npts += s_half;
+    if (tid == 31) s_npts = incl;
   }
   __syncthreads();
   const uint32_t npts = s_npts;
   if (npts == 0) return;
   if (tid == 0) s_gbase = atomicAdd(&ctr->num_points, npts);
-  constexpr uint32_t cap = SMALL_ROUNDS ? 96u : static_cast<uint32_t>(CAP);
+  constexpr uint32_t cap = SMALL_ROUNDS ? 96u : static_cast<uint32_t>(kBpMaxPts);
   const bool one_round = npts <= cap;  // (CTA-uniform)
-  for (uint32_t c0 = 0; c0 < npts; c0 += cap) {  // one round unless the tile has more than CAP points
+  for (uint32_t c0 = 0; c0 < npts; c0 += cap) {  // one round unless the tile has more than kBpMaxPts points
     if (c0 > 0) {
       __syncthreads();  // the previous round's records are written: list and table are free again
       clear_table();
@@ -1281,94 +1256,54 @@ __global__ void k_hash_clear(FrameParams p, int frames) {
 // ---------------------------------------------------------------------------------------------
 static inline unsigned cdiv(unsigned a, unsigned b) { return (a + b - 1) / b; }
 
-int launch_frontend(const FrameParams &p, int frames, cudaStream_t s, KernelTimer *kt) {
-  int launches = 0;
+void launch_frontend(const FrameParams &p, int frames, Launcher &ln) {
+  const cudaStream_t s = ln.s;
   const dim3 tgrid(cdiv(p.tiles_x, 128), p.tiles_y, frames);
   if (p.fmt == B200TAG_FMT_YUYV && p.f == 2 && !p.blur_ksz) {
-    if (kt) kt->begin("pre_yuyv_dec2", s);
-    k_pre_yuyv_dec2<<<tgrid, 128, 0, s>>>(p);
-    if (kt) kt->end(s);
-    launches++;
+    ln.timed("pre_yuyv_dec2", [&] { k_pre_yuyv_dec2<<<tgrid, 128, 0, s>>>(p); });
   } else if (p.fmt == B200TAG_FMT_BGR8 && p.f == 2 && !p.blur_ksz && (reinterpret_cast<uintptr_t>(p.in) | p.in_stride) % 8 == 0) {
-    if (kt) kt->begin("pre_bgr_dec2", s);
-    k_pre_bgr_dec2<<<tgrid, 128, 0, s>>>(p);
-    if (kt) kt->end(s);
-    launches++;
+    ln.timed("pre_bgr_dec2", [&] { k_pre_bgr_dec2<<<tgrid, 128, 0, s>>>(p); });
   } else if (p.fmt == B200TAG_FMT_GRAY8 && p.f == 2 && !p.blur_ksz && (reinterpret_cast<uintptr_t>(p.in) | p.in_stride) % 8 == 0) {
-    if (kt) kt->begin("pre_gray_dec2", s);
-    k_pre_gray_dec2<<<tgrid, 128, 0, s>>>(p);
-    if (kt) kt->end(s);
-    launches++;
+    ln.timed("pre_gray_dec2", [&] { k_pre_gray_dec2<<<tgrid, 128, 0, s>>>(p); });
   } else {
     const bool vec_bgr = (p.fmt == B200TAG_FMT_BGR8 && p.f == 1 && (static_cast<size_t>(p.W) * p.H) % 16 == 0 && p.in_stride % 16 == 0);
     if (vec_bgr) {
-      if (kt) kt->begin("pre_bgr_dec1", s);
       const size_t groups = static_cast<size_t>(p.W) * p.H / 16;
-      k_pre_bgr_dec1<<<dim3(cdiv(static_cast<unsigned>(groups), 256), frames), 256, 0, s>>>(p);
-      if (kt) kt->end(s);
-      launches++;
+      ln.timed("pre_bgr_dec1", [&] { k_pre_bgr_dec1<<<dim3(cdiv(static_cast<unsigned>(groups), 256), frames), 256, 0, s>>>(p); });
     } else {
-      if (kt) kt->begin("pre_generic", s);
-      k_pre_generic<<<tgrid, 128, 0, s>>>(p, p.blur_ksz ? 0 : 1);
-      if (kt) kt->end(s);
-      launches++;
+      ln.timed("pre_generic", [&] { k_pre_generic<<<tgrid, 128, 0, s>>>(p, p.blur_ksz ? 0 : 1); });
     }
     if (p.blur_ksz) {
-      if (kt) kt->begin("blur", s);
       const int r = p.blur_ksz >> 1, r4 = (r + 3) & ~3;
       const size_t smem = static_cast<size_t>(kBlurTH + 2 * r) * (kBlurTW + 2 * r4) + static_cast<size_t>(kBlurTH + 2 * r) * kBlurTW;
       const dim3 bgrid(cdiv(p.w, kBlurTW), cdiv(p.h, kBlurTH), frames);
       // (the quad image is word aligned: its width is a multiple of 4 and so is every frame's size)
       const dim3 sgrid(cdiv(p.w / 4, 32), cdiv(p.h, 4 * kBlurRows), frames);
-      const bool strip = !(exp_flags() & 512);
-      switch (p.blur_ksz) {
-        case 3: if (strip) k_blur_strip<3><<<sgrid, 128, 0, s>>>(p); else k_blur<3><<<bgrid, 256, smem, s>>>(p); break;
-        case 5: if (strip) k_blur_strip<5><<<sgrid, 128, 0, s>>>(p); else k_blur<5><<<bgrid, 256, smem, s>>>(p); break;
-        case 7: if (strip) k_blur_strip<7><<<sgrid, 128, 0, s>>>(p); else k_blur<7><<<bgrid, 256, smem, s>>>(p); break;
-        default: k_blur<0><<<bgrid, 256, smem, s>>>(p); break;
-      }
-      if (kt) kt->end(s);
-      launches++;
+      ln.timed("blur", [&] {
+        switch (p.blur_ksz) {
+          case 3: k_blur_strip<3><<<sgrid, 128, 0, s>>>(p); break;
+          case 5: k_blur_strip<5><<<sgrid, 128, 0, s>>>(p); break;
+          case 7: k_blur_strip<7><<<sgrid, 128, 0, s>>>(p); break;
+          default: k_blur<<<bgrid, 256, smem, s>>>(p); break;
+        }
+      });
     }
-    const bool minmax_done = p.blur_ksz >= 3 && p.blur_ksz <= 7 && !(exp_flags() & 512);  // k_blur_strip writes the tile min/max itself
-    if ((p.blur_ksz || vec_bgr) && !minmax_done) {
-      if (kt) kt->begin("tile_minmax", s);
-      k_tile_minmax<<<tgrid, 128, 0, s>>>(p);
-      if (kt) kt->end(s);
-      launches++;
-    }
+    const bool minmax_done = p.blur_ksz >= 3 && p.blur_ksz <= 7;  // k_blur_strip writes the tile min/max itself
+    if ((p.blur_ksz || vec_bgr) && !minmax_done) ln.timed("tile_minmax", [&] { k_tile_minmax<<<tgrid, 128, 0, s>>>(p); });
   }
   const dim3 cgrid(cdiv(p.w, kCclTW), cdiv(p.h, kCclTH), frames);
-  if (kt) kt->begin("ccl_local", s);
-  k_ccl_local<16><<<cgrid, kCclThreads, 0, s>>>(p);
-  if (kt) kt->end(s);
-  if (kt) kt->begin("ccl_merge", s);
-  if (frames <= 4) k_ccl_merge<true><<<cgrid, kCclMergeThreads, 0, s>>>(p);   // single-frame latency: see gfind_halving
-  else k_ccl_merge<false><<<cgrid, kCclMergeThreads, 0, s>>>(p);
-  if (kt) kt->end(s);
-  if (kt) kt->begin("ccl_handoff", s);
-  k_ccl_handoff<32><<<dim3(cdiv(cgrid.x * cgrid.y, 8), frames), 256, 0, s>>>(p, cgrid.x * cgrid.y);
-  if (kt) kt->end(s);
-  if (kt) kt->begin("ccl_final", s);
-  if (exp_flags() & 8) k_ccl_final<1><<<cgrid, kFinThreads, 0, s>>>(p);
-  else k_ccl_final<8><<<cgrid, kFinThreads, 0, s>>>(p);
-  if (kt) kt->end(s);
-  launches += 4;
-
-  if (kt) kt->begin("boundary", s);
-  {  // tile height: 16 rows (256 threads) or 8 rows (128 threads, half the shared memory: more CTAs per SM)
-    // (measured on config 2, 128 frames: 0.384 ms with 16 rows, 0.363 ms with 8; B200TAG_BP_TH=16 selects the former)
-    static const int th = [] { const char *e = getenv("B200TAG_BP_TH"); return (e && atoi(e) == 16) ? 16 : 8; }();
-    const dim3 g8(cdiv(p.w, kBpTW), cdiv(p.h, 8), frames);
-    if (th == 8 && (p.test_flags & B200TAG_TEST_SMALL_CHUNKS)) k_boundary<8, 1024, 8, true><<<g8, 128, 0, s>>>(p);
-    else if (th == 8 && (exp_flags() & 2)) k_boundary<8, 2048, 9, false><<<g8, 128, 0, s>>>(p);
-    else if (th == 8 && (exp_flags() & 4)) k_boundary<8, 1024, 9, false><<<g8, 128, 0, s>>>(p);
-    else if (th == 8) k_boundary<8, 1024, 8, false><<<g8, 128, 0, s>>>(p);
-    else k_boundary<16, 4096, 10, false><<<dim3(cdiv(p.w, kBpTW), cdiv(p.h, 16), frames), 256, 0, s>>>(p);
-  }
-  if (kt) kt->end(s);
-  launches++;
-  return launches;
+  ln.timed("ccl_local", [&] { k_ccl_local<<<cgrid, kCclThreads, 0, s>>>(p); });
+  ln.timed("ccl_merge", [&] {
+    if (frames <= 4) k_ccl_merge<true><<<cgrid, kCclMergeThreads, 0, s>>>(p);   // single-frame latency: see gfind_halving
+    else k_ccl_merge<false><<<cgrid, kCclMergeThreads, 0, s>>>(p);
+  });
+  ln.timed("ccl_handoff", [&] { k_ccl_handoff<32><<<dim3(cdiv(cgrid.x * cgrid.y, 8), frames), 256, 0, s>>>(p, cgrid.x * cgrid.y); });
+  ln.timed("ccl_final", [&] { k_ccl_final<<<cgrid, kFinThreads, 0, s>>>(p); });
+  ln.timed("boundary", [&] {
+    const dim3 g(cdiv(p.w, kBpTW), cdiv(p.h, kBpTH), frames);
+    if (p.test_flags & B200TAG_TEST_SMALL_CHUNKS) k_boundary<true><<<g, kBpThreads, 0, s>>>(p);
+    else k_boundary<false><<<g, kBpThreads, 0, s>>>(p);
+  });
 }
 
 size_t ccl_tiles_per_frame(int w, int h) { return static_cast<size_t>(cdiv(w, kCclTW)) * cdiv(h, kCclTH); }

@@ -707,11 +707,9 @@ __global__ void __launch_bounds__(kIdctBlocks * 8) k_jpeg_idct(JpegBatch B) {
 
 }  // namespace
 
-// Returns the number of kernels launched.  Frames whose parallel decode did not reach its fixed point within
-// kJpegSyncRounds rounds (or whose restart markers do not add up) are decoded by the sequential warp-per-frame kernel
-// at the end.
-int launch_jpeg_decode(const JpegBatch &B, bool any_parallel, cudaStream_t s) {
-  int launches = 0;
+// Frames whose parallel decode did not reach its fixed point within kJpegSyncRounds rounds (or whose restart markers do
+// not add up) are decoded by the sequential warp-per-frame kernel at the end.
+void launch_jpeg_decode(const JpegBatch &B, bool any_parallel, cudaStream_t s) {
   if (any_parallel) {
     cudaMemsetAsync(B.changed, 0, sizeof(uint32_t) * kJpegSyncRounds * B.count, s);
     const dim3 gch((B.max_chunks + 255) / 256, B.count);
@@ -722,16 +720,12 @@ int launch_jpeg_decode(const JpegBatch &B, bool any_parallel, cudaStream_t s) {
     for (int r = 0; r < kJpegSyncRounds; r++) k_jpeg_sync<<<gsub, kSyncThreads, 0, s>>>(B, r);
     k_jpeg_blockscan<<<B.count, 1024, 0, s>>>(B);
     k_jpeg_write<<<gsub, kSyncThreads, 0, s>>>(B);
-    if (B.max_intervals) {
+    if (B.max_intervals)
       k_jpeg_write_rst<<<dim3((B.max_intervals + kSyncThreads - 1) / kSyncThreads, B.count), kSyncThreads, 0, s>>>(B);
-      launches++;
-    }
     k_jpeg_dcscan<<<B.count, 1024, 0, s>>>(B);
     k_jpeg_idct<<<dim3((B.max_luma_blocks + kIdctBlocks - 1) / kIdctBlocks, B.count), kIdctBlocks * 8, 0, s>>>(B);
-    launches += 7 + kJpegSyncRounds;
   }
   k_jpeg_luma<<<B.count, 32, 0, s>>>(B.raw, B.frames, B.tables, B.out, B.out_stride, any_parallel ? B.proven : nullptr);
-  return launches + 1;
 }
 
 }  // namespace b200tag

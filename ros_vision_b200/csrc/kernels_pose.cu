@@ -133,15 +133,14 @@ __global__ void __launch_bounds__(kPoseWarps * 32) k_pose(PoseLaunch L) {
 
 }  // namespace
 
-int launch_pose(const PoseLaunch &L, int frames, cudaStream_t s, KernelTimer *kt) {
-  if (kt) kt->begin("pose", s);
+void launch_pose(const PoseLaunch &L, int frames, Launcher &ln) {
   // a frame of a batch has a handful of tags: 8 warps each, the rest loop; up to four frames (the single-frame latency
   // path, a cluttered 4K scene has ~100 tags): 128 warps each, one pass.  A list without counters is one frame.
   unsigned ctas = static_cast<unsigned>(frames) <= 4 ? 32u : 2u;
   if (!L.counters) ctas = static_cast<unsigned>((L.count + kPoseWarps - 1) / kPoseWarps);
-  if (ctas > 0) k_pose<<<dim3(ctas, static_cast<unsigned>(frames)), kPoseWarps * 32, 0, s>>>(L);
-  if (kt) kt->end(s);
-  return 1;
+  ln.timed("pose", [&] {
+    if (ctas > 0) k_pose<<<dim3(ctas, static_cast<unsigned>(frames)), kPoseWarps * 32, 0, ln.s>>>(L);
+  });
 }
 
 }  // namespace b200tag
