@@ -294,6 +294,18 @@ int b200tag_estimate_pose(const b200tag_detection *det, double tagsize, double f
 int b200tag_estimate_poses(const b200tag_detection *dets, int count, double tagsize, double fx, double fy, double cx,
                            double cy, b200tag_pose *out);
 
+/* Pose methods.  ORTHOGONAL_ITERATION is the algorithm above (libapriltag's estimate_tag_pose, the default
+ * everywhere).  IPPE is Infinitesimal Plane-based Pose Estimation (Collins & Bartoli 2014) for a square tag, the two
+ * candidates OpenCV's solvePnPGeneric(..., SOLVEPNP_IPPE_SQUARE) returns: closed form from the homography of the
+ * detection's corners p (not H), without iteration.  It solves the image-plane problem rather than minimising the
+ * object-space error, so with pixel noise its pose differs from OI's by about the pose's own uncertainty.  The returned
+ * candidate is the one with the smaller object-space error, and err / err_other are object-space errors as for OI.
+ * A quad for which no candidate can be formed gives R = I, t = 0 and err = err_other = HUGE_VAL. */
+enum { B200TAG_POSE_ORTHOGONAL_ITERATION = 0, B200TAG_POSE_IPPE = 1 };
+/* b200tag_estimate_poses with IPPE; the same arguments and checks. */
+int b200tag_estimate_poses_ippe(const b200tag_detection *dets, int count, double tagsize, double fx, double fy, double cx,
+                                double cy, b200tag_pose *out);
+
 /* The rest of the node's per-frame step (apriltags_cuda_detector.cu:421-462,595-599): every detection's pose, the tag
  * position in the camera frame (the pose's t), in the robot frame (rotation * t + offset, transformCameraToRobot) and
  * its Euclidean distance from the camera; the records come back closest first, as the node publishes them (ties
@@ -318,6 +330,11 @@ int b200tag_locate_tags(const b200tag_detection *dets, int count, double tagsize
  * fy are non-zero.  Takes effect from the next detect call; adds one kernel to b200tag_kernels_per_batch. */
 int b200tag_set_pose_estimation(b200tag_detector *det, double tagsize, double fx, double fy, double cx, double cy,
                                 const double *rotation, const double *offset);
+/* The method the device pose step runs from the next detect call: B200TAG_POSE_ORTHOGONAL_ITERATION (the default) or
+ * B200TAG_POSE_IPPE, whose poses are bit-identical to b200tag_estimate_poses_ippe's.  Independent of
+ * b200tag_set_pose_estimation, which alone turns the step on and off.  B200TAG_E_INVALID (state unchanged) for any
+ * other value. */
+int b200tag_set_pose_method(b200tag_detector *det, int method);
 /* Poses of frame `frame` of the last call, parallel to b200tag_detections(det, frame): element i is the pose of
  * detection i.  NULL and *count = 0 when the last call ran without the pose step.  Owned by the detector, valid until
  * the next detect call. */
@@ -328,6 +345,9 @@ const b200tag_tag_position *b200tag_tag_positions(const b200tag_detector *det, i
  * results as b200tag_estimate_poses. */
 int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count, double tagsize, double fx, double fy,
                                         double cx, double cy, b200tag_pose *out);
+/* The same for the device IPPE kernel; results as b200tag_estimate_poses_ippe. */
+int b200tag_debug_estimate_poses_ippe_device(const b200tag_detection *dets, int count, double tagsize, double fx,
+                                             double fy, double cx, double cy, b200tag_pose *out);
 
 /* Pinned host staging memory, so b200tag_detect* can overlap H2D with compute. */
 void *b200tag_alloc_pinned(size_t bytes);

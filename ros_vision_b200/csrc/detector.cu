@@ -121,6 +121,7 @@ struct b200tag_detector {
   struct PoseSettings {
     double tagsize = 0, fx = 0, fy = 0, cx = 0, cy = 0;
     double rotation[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, offset[3] = {0, 0, 0};
+    int method = B200TAG_POSE_ORTHOGONAL_ITERATION;  // b200tag_set_pose_method
   };
   PoseSettings pose, last_pose;                // current; what the last enqueue ran with
   b200tag_pose *h_poses = nullptr;             // pinned + mapped, parallel to h_dets; allocated when first turned on
@@ -383,7 +384,8 @@ int record_sequence(b200tag_detector *det, const void *device_images, size_t str
   launch_decode(p, count, ln);
   if (det->pose.tagsize > 0) {
     const auto &ps = det->pose;
-    const PoseLaunch pl{det->d_dets_alias, det->d_poses_alias, p.counters, p.det_cap, 0, ps.tagsize, ps.fx, ps.fy, ps.cx, ps.cy};
+    const PoseLaunch pl{det->d_dets_alias, det->d_poses_alias, p.counters, p.det_cap, 0, ps.tagsize, ps.fx, ps.fy, ps.cx, ps.cy,
+                        ps.method};
     launch_pose(pl, count, ln);
   }
   *launches_out = ln.count;
@@ -1382,6 +1384,14 @@ int b200tag_set_pose_estimation(b200tag_detector *det, double tagsize, double fx
   return 0;
 }
 
+int b200tag_set_pose_method(b200tag_detector *det, int method) {
+  if (!det || (method != B200TAG_POSE_ORTHOGONAL_ITERATION && method != B200TAG_POSE_IPPE)) return B200TAG_E_INVALID;
+  DeviceGuard on_device(det->device);
+  drop_graphs(det);  // the kernel is baked into the captured launches
+  det->pose.method = method;
+  return 0;
+}
+
 int b200tag_set_distortion(b200tag_detector *det, double k1, double k2, double p1, double p2, double k3) {
   if (!det) return B200TAG_E_INVALID;
   DeviceGuard on_device(det->device);
@@ -1460,8 +1470,13 @@ int b200tag_debug_math(int op, const float *a, const float *b, float *out, int n
   return rc;
 }
 
-int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count, double tagsize, double fx, double fy,
-                                        double cx, double cy, b200tag_pose *out) {
+}  // extern "C"
+
+namespace {
+
+// The test hooks' common part: the pose kernel of `method` on caller records, through device copies of them.
+int estimate_poses_device(int method, const b200tag_detection *dets, int count, double tagsize, double fx, double fy,
+                          double cx, double cy, b200tag_pose *out) {
   if (count < 0 || (count > 0 && (!dets || !out)) || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
   if (count == 0) return 0;
   const size_t db = sizeof(b200tag_detection) * static_cast<size_t>(count), pb = sizeof(b200tag_pose) * static_cast<size_t>(count);
@@ -1472,7 +1487,7 @@ int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count
   }
   int rc = 0;
   const PoseLaunch pl{reinterpret_cast<const b200tag_detection *>(d), reinterpret_cast<b200tag_pose *>(d + db), nullptr,
-                      0, static_cast<uint32_t>(count), tagsize, fx, fy, cx, cy};
+                      0, static_cast<uint32_t>(count), tagsize, fx, fy, cx, cy, method};
   if (cudaMemcpy(d, dets, db, cudaMemcpyHostToDevice) != cudaSuccess) rc = B200TAG_E_CUDA;
   if (!rc) {
     Launcher ln{nullptr, nullptr};
@@ -1481,6 +1496,20 @@ int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count
   }
   cudaFree(d);
   return rc;
+}
+
+}  // namespace
+
+extern "C" {
+
+int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count, double tagsize, double fx, double fy,
+                                        double cx, double cy, b200tag_pose *out) {
+  return estimate_poses_device(B200TAG_POSE_ORTHOGONAL_ITERATION, dets, count, tagsize, fx, fy, cx, cy, out);
+}
+
+int b200tag_debug_estimate_poses_ippe_device(const b200tag_detection *dets, int count, double tagsize, double fx,
+                                             double fy, double cx, double cy, b200tag_pose *out) {
+  return estimate_poses_device(B200TAG_POSE_IPPE, dets, count, tagsize, fx, fy, cx, cy, out);
 }
 
 int b200tag_kernels_per_batch(const b200tag_detector *det) { return det ? det->kernels_per_batch : 0; }

@@ -78,13 +78,15 @@ size_t ccl_root_cap();
 void launch_hash_clear(const FrameParams &p, int frames, cudaStream_t s);
 void launch_blobs_init(cudaStream_t s);
 
-// The pose step (kernels_pose.cu): b200tag_estimate_pose of every raw detection, poses parallel to the records.
+// The pose step (kernels_pose.cu): b200tag_estimate_pose (k_pose) or the IPPE pose (k_pose_ippe) of every raw
+// detection, poses parallel to the records.
 struct PoseLaunch {
   const b200tag_detection *dets;  // frame f's records start at dets + f * stride
   b200tag_pose *out;              // the same layout
   const Counters *counters;       // per-frame record counts; null: one list of `count` records
   uint32_t stride, count;
   double tagsize, fx, fy, cx, cy;
+  int method;                     // B200TAG_POSE_*
 };
 void launch_pose(const PoseLaunch &L, int frames, Launcher &ln);
 

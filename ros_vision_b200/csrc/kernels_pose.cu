@@ -2,11 +2,14 @@
 // the batch, appended to the detection graph behind k_decode.  One warp per detection.  The homography start and the
 // orthogonal iteration run on every lane with the same values, reading the per-detection constants from shared memory;
 // lane 0 sets up the frame of the second-minimum search there, and the lanes split that search's grid.  The arithmetic is
-// pose_core.h's, the same the host functions in pose.cc run.
+// pose_core.h's, the same the host functions in pose.cc run.  With b200tag_set_pose_method(B200TAG_POSE_IPPE) the step
+// is k_pose_ippe instead: the closed-form IPPE pose, one thread per detection.
 //
 // A pose depends only on its own record, so computing it before the host's reconcile gives the pose of every
 // detection that survives it.
 #include <cuda_runtime.h>
+
+#include <cstddef>
 
 #include "dev_types.h"
 #include "kernels.h"
@@ -131,9 +134,48 @@ __global__ void __launch_bounds__(kPoseWarps * 32) k_pose(PoseLaunch L) {
     estimate_pose_warp(recs + i, L, sh[w], lane, out + i);
 }
 
+constexpr int kIppeThreads = 128;  // threads per CTA of k_pose_ippe
+static_assert(offsetof(b200tag_detection, p) % 16 == 0 && sizeof(b200tag_detection) % 16 == 0, "corner loads");
+static_assert(sizeof(b200tag_pose) % 16 == 0, "pose stores");
+
+// The IPPE pose (B200TAG_POSE_IPPE) of every raw detection: one thread per record, blockIdx.y = frame, as many records
+// as the frame's counter holds.  A thread reads only the record's four corners from the mapped detection buffer and
+// writes the pose to the same index of the mapped pose buffer; the arithmetic is ippe_pose, which the host's
+// b200tag_estimate_poses_ippe runs too.
+__global__ void __launch_bounds__(kIppeThreads) k_pose_ippe(PoseLaunch L) {
+  const size_t frame = blockIdx.y;
+  const uint32_t n = L.counters ? min(L.counters[frame].num_detections, L.stride) : L.count;
+  const b200tag_detection *recs = L.dets + frame * L.stride;
+  b200tag_pose *out = L.out + frame * L.stride;
+  for (uint32_t i = blockIdx.x * kIppeThreads + threadIdx.x; i < n; i += gridDim.x * kIppeThreads) {
+    const double2 *src = reinterpret_cast<const double2 *>(recs[i].p);
+    double px[4][2];
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+      const double2 c = src[k];
+      px[k][0] = c.x;
+      px[k][1] = c.y;
+    }
+    b200tag_pose pose;
+    ippe_pose(px, L.tagsize, L.fx, L.fy, L.cx, L.cy, &pose);
+    const double2 *from = reinterpret_cast<const double2 *>(&pose);
+    double2 *dst = reinterpret_cast<double2 *>(out + i);
+#pragma unroll
+    for (int k = 0; k < static_cast<int>(sizeof(b200tag_pose) / 16); k++) dst[k] = from[k];
+  }
+}
+
 }  // namespace
 
 void launch_pose(const PoseLaunch &L, int frames, Launcher &ln) {
+  if (L.method == B200TAG_POSE_IPPE) {
+    // one thread per record, all of a frame's records in one pass up to 1024 of them; CTAs past a frame's count exit
+    const unsigned ctas = L.counters ? min((L.stride + kIppeThreads - 1) / kIppeThreads, 8u) : (L.count + kIppeThreads - 1) / kIppeThreads;
+    ln.timed("pose_ippe", [&] {
+      if (ctas > 0) k_pose_ippe<<<dim3(ctas, static_cast<unsigned>(frames)), kIppeThreads, 0, ln.s>>>(L);
+    });
+    return;
+  }
   // a frame of a batch has a handful of tags: 8 warps each, the rest loop; up to four frames (the single-frame latency
   // path, a cluttered 4K scene has ~100 tags): 128 warps each, one pass.  A list without counters is one frame.
   unsigned ctas = static_cast<unsigned>(frames) <= 4 ? 32u : 2u;

@@ -91,6 +91,14 @@ int b200tag_estimate_poses(const b200tag_detection *dets, int count, double tags
   return 0;
 }
 
+int b200tag_estimate_poses_ippe(const b200tag_detection *dets, int count, double tagsize, double fx, double fy, double cx,
+                                double cy, b200tag_pose *out) {
+  if (count < 0 || (count > 0 && (!dets || !out))) return B200TAG_E_INVALID;
+  if (count > 0 && (!(tagsize > 0) || fx == 0 || fy == 0)) return B200TAG_E_INVALID;
+  for (int i = 0; i < count; i++) ippe_pose(dets[i].p, tagsize, fx, fy, cx, cy, out + i);
+  return 0;
+}
+
 int b200tag_locate_tags(const b200tag_detection *dets, int count, double tagsize, double fx, double fy, double cx,
                         double cy, const double *rotation, const double *offset, b200tag_tag_position *out) {
   if (count < 0 || (count > 0 && (!dets || !out))) return B200TAG_E_INVALID;

@@ -13,6 +13,9 @@
 // -fmad=false for the device, and steps 1 and 2 use only + - * /, sqrt, fabs and fmax, so the first local minimum
 // comes out bit-identical on host and device.  Only step 3 calls tan / atan / atan2 / sin / cos, where glibc and
 // libdevice may differ by an ulp.
+//
+// The second method, IPPE (ippe_pose, at the end), is closed form and uses only + - * /, sqrt, fabs and fmax: its
+// poses are bit-identical on host and device.
 #ifndef B200TAG_POSE_CORE_H_
 #define B200TAG_POSE_CORE_H_
 
@@ -255,11 +258,14 @@ POSE_HD void pose_from_homography(const double *H, double tagsize, double fx, do
   *t = V3{{TX * sc, -TY * sc, -TZ * sc}};
 }
 
-// Rays through the detection's corners and the tag's corners in its own frame (step 1's inputs).
-POSE_HD void rays_and_corners(const b200tag_detection &det, double tagsize, double fx, double fy, double cx, double cy, V3 *v, V3 *p) {
+// Rays through the four image corners `px` and the tag's corners in its own frame (step 1's inputs).
+POSE_HD void rays_and_corners(const double (*px)[2], double tagsize, double fx, double fy, double cx, double cy, V3 *v, V3 *p) {
   const double sc = tagsize / 2.0;
   p[0] = V3{{-sc, sc, 0}}; p[1] = V3{{sc, sc, 0}}; p[2] = V3{{sc, -sc, 0}}; p[3] = V3{{-sc, -sc, 0}};
-  POSE_UNROLL for (int i = 0; i < 4; i++) v[i] = V3{{(det.p[i][0] - cx) / fx, (det.p[i][1] - cy) / fy, 1}};
+  POSE_UNROLL for (int i = 0; i < 4; i++) v[i] = V3{{(px[i][0] - cx) / fx, (px[i][1] - cy) / fy, 1}};
+}
+POSE_HD void rays_and_corners(const b200tag_detection &det, double tagsize, double fx, double fy, double cx, double cy, V3 *v, V3 *p) {
+  rays_and_corners(det.p, tagsize, fx, fy, cx, cy, v, p);
 }
 
 // Object-space error as a function of the rotation beta about the y axis of the transformed frame, in
@@ -384,6 +390,121 @@ POSE_HD void choose_pose(const M3 &R1, const V3 &t1, double err1, const M3 &R2, 
   POSE_UNROLL for (int k = 0; k < 3; k++) out->t[k] = first ? t1.v[k] : t2.v[k];
   out->err = first ? err1 : err2;
   out->err_other = first ? err2 : err1;
+}
+
+// ---- IPPE (b200tag_estimate_poses_ippe, B200TAG_POSE_IPPE) ----
+// Infinitesimal Plane-based Pose Estimation (Collins & Bartoli 2014) of a square tag, the two candidates OpenCV's
+// solvePnPGeneric(..., SOLVEPNP_IPPE_SQUARE) returns: the homography from the tag plane to normalised image points, its
+// Jacobian at the tag centre, two rotations from the Jacobian in closed form and a least-squares translation for each.
+// Only + - * /, sqrt, fabs and fmax: no iteration and no libm transcendental, so host and device agree bit for bit.
+
+// Homography H (row-major, H22 = 1) from the tag plane to the normalised image points u[0..3] of the tag corners
+// (-s, s), (s, s), (s, -s), (-s, -s): Heckbert's square-to-quad mapping of the unit square, (X, Y) on the tag being
+// ((X + s) / 2s, (s - Y) / 2s) on the square.  False when the quad has no such mapping.
+POSE_HD bool square_homography(const V3 *u, double s, double *H) {
+  const double x0 = u[0].v[0], y0 = u[0].v[1], x1 = u[1].v[0], y1 = u[1].v[1];
+  const double x2 = u[2].v[0], y2 = u[2].v[1], x3 = u[3].v[0], y3 = u[3].v[1];
+  const double sx = x0 - x1 + x2 - x3, sy = y0 - y1 + y2 - y3;
+  const double dx1 = x1 - x2, dx2 = x3 - x2, dy1 = y1 - y2, dy2 = y3 - y2;
+  const double den = dx1 * dy2 - dx2 * dy1;
+  if (!(fabs(den) > 0)) return false;
+  const double g = (sx * dy2 - dx2 * sy) / den, h = (dx1 * sy - sx * dy1) / den;
+  const double a = x1 - x0 + g * x1, b = x3 - x0 + h * x3, d = y1 - y0 + g * y1, e = y3 - y0 + h * y3;
+  const double w = 0.5 * (g + h) + 1;  // homogeneous weight of the tag centre
+  if (!(fabs(w) > 0)) return false;
+  const double k = 0.5 / (s * w);
+  H[0] = a * k; H[1] = -b * k; H[2] = (0.5 * (a + b) + x0) / w;
+  H[3] = d * k; H[4] = -e * k; H[5] = (0.5 * (d + e) + y0) / w;
+  H[6] = g * k; H[7] = -h * k; H[8] = 1;
+  return true;
+}
+
+// The two IPPE rotations from H.  (p, q) is the image of the tag centre, J the Jacobian of H there, Rv the rotation
+// taking e_z to (p, q, 1) / |(p, q, 1)| (Rodrigues' formula about e_z x v, with (1 - cos) / sin^2 = 1 / (n (n + 1))
+// so that p = q = 0 gives the identity), A = B^-1 J and gamma its larger singular value.  False when B cannot be
+// inverted or gamma is not positive.
+POSE_HD bool ippe_rotations(const double *H, M3 *R) {
+  const double p = H[2], q = H[5];
+  const double J00 = H[0] - H[6] * p, J01 = H[1] - H[7] * p, J10 = H[3] - H[6] * q, J11 = H[4] - H[7] * q;
+  const double n = sqrt(p * p + q * q + 1), w = 1 / (n * (n + 1));
+  const M3 Rv{{1 - p * p * w, -p * q * w, p / n, -p * q * w, 1 - q * q * w, q / n, -p / n, -q / n, 1 / n}};
+  const double B00 = Rv(0, 0) - p * Rv(2, 0), B01 = Rv(0, 1) - p * Rv(2, 1);
+  const double B10 = Rv(1, 0) - q * Rv(2, 0), B11 = Rv(1, 1) - q * Rv(2, 1);
+  const double detB = B00 * B11 - B01 * B10;
+  if (!(fabs(detB) > 0)) return false;
+  const double A00 = (B11 * J00 - B01 * J10) / detB, A01 = (B11 * J01 - B01 * J11) / detB;
+  const double A10 = (B00 * J10 - B10 * J00) / detB, A11 = (B00 * J11 - B10 * J01) / detB;
+  const double a = A00 * A00 + A10 * A10, b = A00 * A01 + A10 * A11, c = A01 * A01 + A11 * A11;
+  const double gamma = sqrt(0.5 * (a + c + sqrt((a - c) * (a - c) + 4 * b * b)));
+  if (!(gamma > 0)) return false;
+  const double r00 = A00 / gamma, r01 = A01 / gamma, r10 = A10 / gamma, r11 = A11 / gamma;
+  const double b0 = sqrt(fmax(0.0, 1 - r00 * r00 - r10 * r10));
+  double b1 = sqrt(fmax(0.0, 1 - r01 * r01 - r11 * r11));
+  if (r00 * r01 + r10 * r11 > 0) b1 = -b1;
+  POSE_UNROLL for (int k = 0; k < 2; k++) {
+    const double sg = k == 0 ? 1.0 : -1.0;
+    const V3 c1{{r00, r10, sg * b0}}, c2{{r01, r11, sg * b1}}, c3 = cross(c1, c2);
+    R[k] = mul(Rv, M3{{c1.v[0], c2.v[0], c3.v[0], c1.v[1], c2.v[1], c3.v[1], c1.v[2], c2.v[2], c3.v[2]}});
+  }
+  return true;
+}
+
+// The t minimising the image-plane residuals of R's corners, linearised: for every corner, [1, 0, -u_x] t =
+// u_x (R p)_z - (R p)_x and [0, 1, -u_y] t = u_y (R p)_z - (R p)_y, solved through the 3x3 normal equations (whose
+// matrix does not depend on R).  False when the corners coincide.
+POSE_HD bool ippe_translation(const V3 *u, const V3 *p, const M3 &R, V3 *t) {
+  double N02 = 0, N12 = 0, N22 = 0, r0 = 0, r1 = 0, r2 = 0;  // N00 = N11 = 4, N01 = 0
+  POSE_UNROLL for (int i = 0; i < 4; i++) {
+    const V3 rp = mul(R, p[i]);
+    const double ux = u[i].v[0], uy = u[i].v[1];
+    const double bx = ux * rp.v[2] - rp.v[0], by = uy * rp.v[2] - rp.v[1];
+    N02 -= ux;
+    N12 -= uy;
+    N22 += ux * ux + uy * uy;
+    r0 += bx;
+    r1 += by;
+    r2 -= ux * bx + uy * by;
+  }
+  const double det = 16 * N22 - 4 * N12 * N12 - 4 * N02 * N02;
+  if (!(fabs(det) > 0)) return false;
+  // the adjugate of N (symmetric)
+  const double S00 = 4 * N22 - N12 * N12, S01 = N02 * N12, S02 = -4 * N02, S11 = 4 * N22 - N02 * N02, S12 = -4 * N12, S22 = 16;
+  *t = V3{{(S00 * r0 + S01 * r1 + S02 * r2) / det, (S01 * r0 + S11 * r1 + S12 * r2) / det, (S02 * r0 + S12 * r1 + S22 * r2) / det}};
+  return true;
+}
+
+// Object-space error sum |(I - F_j)(R p_j + t)|^2 with F_j = v_j v_j^T / v_j^T v_j, as orthogonal_iteration scores.
+POSE_HD double object_space_error(const V3 *v, const V3 *p, const M3 &R, const V3 &t) {
+  double err = 0;
+  POSE_UNROLL for (int j = 0; j < 4; j++) {
+    const V3 e = mul(sub(ident(), outer_over_norm(v[j])), add(mul(R, p[j]), t));
+    err += dot(e, e);
+  }
+  return err;
+}
+
+// IPPE pose of a tag whose corners are at image points px[0..3]: the candidate with the smaller object-space error,
+// the other's error in err_other.  A quad for which a candidate cannot be formed gives R = I, t = 0 and both errors
+// HUGE_VAL.
+POSE_HD void ippe_pose(const double (*px)[2], double tagsize, double fx, double fy, double cx, double cy, b200tag_pose *out) {
+  V3 v[4], p[4];
+  rays_and_corners(px, tagsize, fx, fy, cx, cy, v, p);
+  double H[9];
+  M3 R[2];
+  V3 t[2];
+  double err[2] = {HUGE_VAL, HUGE_VAL};
+  bool ok = square_homography(v, tagsize / 2.0, H) && ippe_rotations(H, R);
+  POSE_UNROLL for (int k = 0; k < 2; k++) {
+    ok = ok && ippe_translation(v, p, R[k], &t[k]);
+    if (ok) err[k] = object_space_error(v, p, R[k], t[k]);
+  }
+  if (!(err[0] < HUGE_VAL && err[1] < HUGE_VAL)) {  // also catches a NaN from overflowing intermediates
+    const M3 I = ident();
+    const V3 z{{0, 0, 0}};
+    choose_pose(I, z, HUGE_VAL, I, z, HUGE_VAL, out);
+    return;
+  }
+  choose_pose(R[0], t[0], err[0], R[1], t[1], err[1], out);
 }
 
 }  // namespace pose

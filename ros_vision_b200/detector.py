@@ -82,6 +82,7 @@ _STAGE_DTYPES = {
 POSE_DT = np.dtype([("R", "<f8", (3, 3)), ("t", "<f8", (3,)), ("err", "<f8"), ("err_other", "<f8")])
 TAG_POSITION_DT = np.dtype([("index", "<i4"), ("id", "<i4"), ("camera", "<f8", (3,)), ("robot", "<f8", (3,)),
                             ("distance", "<f8"), ("err", "<f8")])  # b200tag_tag_position
+POSE_METHODS = {"oi": 0, "ippe": 1}  # B200TAG_POSE_ORTHOGONAL_ITERATION, B200TAG_POSE_IPPE
 
 _lib = None
 
@@ -151,6 +152,9 @@ def load_library():
     L.b200tag_tag_positions.argtypes = [vp, i32, C.POINTER(i32)]
     L.b200tag_tag_positions.restype = vp
     L.b200tag_debug_estimate_poses_device.argtypes = [vp, i32] + [C.c_double] * 5 + [vp]
+    L.b200tag_estimate_poses_ippe.argtypes = [vp, i32] + [C.c_double] * 5 + [vp]
+    L.b200tag_debug_estimate_poses_ippe_device.argtypes = [vp, i32] + [C.c_double] * 5 + [vp]
+    L.b200tag_set_pose_method.argtypes = [vp, i32]
     L.b200tag_version.restype = i32
     _lib = L
     return L
@@ -176,17 +180,27 @@ def jpeg_model_decode(jpeg: bytes, width: int, height: int):
     return out, rounds.value
 
 
-def estimate_poses(detections: np.ndarray, tagsize: float, fx: float, fy: float, cx: float, cy: float) -> np.ndarray:
+def _pose_method(method: str) -> int:
+    if method not in POSE_METHODS:
+        raise ValueError(f"unknown pose method {method!r}: expected one of {sorted(POSE_METHODS)}")
+    return POSE_METHODS[method]
+
+
+def estimate_poses(detections: np.ndarray, tagsize: float, fx: float, fy: float, cx: float, cy: float,
+                   method: str = "oi") -> np.ndarray:
     """estimate_tag_pose for every detection (the node's step after Detect, apriltags_cuda_detector.cu:425-462):
-    returns POSE_DT records (R, t in the camera frame, object-space error).  Pure host math in libb200tag.so."""
+    returns POSE_DT records (R, t in the camera frame, object-space error).  Pure host math in libb200tag.so.
+    method="ippe" computes the closed-form IPPE pose instead (b200tag_estimate_poses_ippe, OpenCV's SOLVEPNP_IPPE_SQUARE
+    candidates, the one with the smaller object-space error returned)."""
     lib = load_library()
+    fn = {0: "b200tag_estimate_poses", 1: "b200tag_estimate_poses_ippe"}[_pose_method(method)]
     dets = np.ascontiguousarray(detections, dtype=DETECTION_DT)
     out = np.zeros(len(dets), dtype=POSE_DT)
     if len(dets):
-        rc = lib.b200tag_estimate_poses(dets.ctypes.data_as(C.c_void_p), len(dets), float(tagsize), float(fx), float(fy),
-                                        float(cx), float(cy), out.ctypes.data_as(C.c_void_p))
+        rc = getattr(lib, fn)(dets.ctypes.data_as(C.c_void_p), len(dets), float(tagsize), float(fx), float(fy),
+                              float(cx), float(cy), out.ctypes.data_as(C.c_void_p))
         if rc:
-            raise B200TagError(f"b200tag_estimate_poses: {lib.b200tag_error_string(rc).decode()}")
+            raise B200TagError(f"{fn}: {lib.b200tag_error_string(rc).decode()}")
     return out
 
 
@@ -209,17 +223,18 @@ def locate_tags(detections: np.ndarray, tagsize: float, fx: float, fy: float, cx
     return out
 
 
-def estimate_poses_device(detections: np.ndarray, tagsize: float, fx: float, fy: float, cx: float, cy: float) -> np.ndarray:
-    """Test hook: estimate_poses computed by the device pose kernel (the one GpuDetector.SetPoseEstimation enables) on
-    the current CUDA device."""
+def estimate_poses_device(detections: np.ndarray, tagsize: float, fx: float, fy: float, cx: float, cy: float,
+                          method: str = "oi") -> np.ndarray:
+    """Test hook: estimate_poses computed by the device pose kernel of `method` (the one GpuDetector.SetPoseEstimation
+    enables) on the current CUDA device."""
     lib = load_library()
+    fn = {0: "b200tag_debug_estimate_poses_device", 1: "b200tag_debug_estimate_poses_ippe_device"}[_pose_method(method)]
     dets = np.ascontiguousarray(detections, dtype=DETECTION_DT)
     out = np.zeros(len(dets), dtype=POSE_DT)
-    rc = lib.b200tag_debug_estimate_poses_device(dets.ctypes.data_as(C.c_void_p) if len(dets) else None, len(dets), float(tagsize),
-                                                 float(fx), float(fy), float(cx), float(cy),
-                                                 out.ctypes.data_as(C.c_void_p) if len(dets) else None)
+    rc = getattr(lib, fn)(dets.ctypes.data_as(C.c_void_p) if len(dets) else None, len(dets), float(tagsize),
+                          float(fx), float(fy), float(cx), float(cy), out.ctypes.data_as(C.c_void_p) if len(dets) else None)
     if rc:
-        raise B200TagError(f"b200tag_debug_estimate_poses_device: {lib.b200tag_error_string(rc).decode()}")
+        raise B200TagError(f"{fn}: {lib.b200tag_error_string(rc).decode()}")
     return out
 
 
@@ -425,16 +440,19 @@ class GpuDetector:
         buf = (C.c_char * (QUAD_DT.itemsize * n.value)).from_address(p)
         return np.frombuffer(buf, dtype=QUAD_DT, count=n.value).copy()
 
-    def SetPoseEstimation(self, tagsize, fx, fy, cx, cy, rotation=None, offset=None) -> None:
+    def SetPoseEstimation(self, tagsize, fx, fy, cx, cy, rotation=None, offset=None, method="oi") -> None:
         """The node's pose step on the GPU: from the next Detect on, a kernel at the end of the detection graph estimates
         every detection's pose (Poses) and its robot-frame record (TagPositions), with the arguments of locate_tags.
-        tagsize = 0 turns it off."""
+        tagsize = 0 turns it off.  method="ippe" runs the closed-form IPPE pose (estimate_poses(..., method="ippe"))
+        instead of libapriltag's orthogonal iteration."""
+        m = _pose_method(method)
         rot = None if rotation is None else np.ascontiguousarray(rotation, dtype=np.float64).reshape(9)
         off = None if offset is None else np.ascontiguousarray(offset, dtype=np.float64).reshape(3)
         self._check(self._lib.b200tag_set_pose_estimation(self._h, float(tagsize), float(fx), float(fy), float(cx), float(cy),
                                                           None if rot is None else rot.ctypes.data_as(C.c_void_p),
                                                           None if off is None else off.ctypes.data_as(C.c_void_p)),
                     "b200tag_set_pose_estimation")
+        self._check(self._lib.b200tag_set_pose_method(self._h, m), "b200tag_set_pose_method")
 
     def Poses(self, frame: int = 0) -> np.ndarray:
         """POSE_DT records parallel to Detections(frame); empty when the last call ran without the pose step."""

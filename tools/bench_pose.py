@@ -7,6 +7,10 @@ synth.config_frame(2, i), 1280x800 YUYV, 1-6 tags per frame), in one run on one 
   * the `pose` kernel's device time per 128-frame batch (b200tag_profile_device);
   * the host time of b200tag_locate_tags on the same detections, on one CPU core of the same machine.
 
+--method ippe measures the IPPE method instead (SetPoseEstimation(..., method="ippe"), the `pose_ippe` kernel), and the
+host leg times estimate_poses(..., method="ippe") against estimate_poses with the default method on the same
+detections.
+
 Prints one JSON record, and writes it to --out when given.  Needs a CUDA device."""
 import argparse
 import json
@@ -41,6 +45,7 @@ def main():
     ap.add_argument("--rounds", type=int, default=6, help="alternations of the off / on measurements")
     ap.add_argument("--steps", type=int, default=40, help="128-frame batches per throughput measurement")
     ap.add_argument("--latency-iters", type=int, default=400, help="single frames per latency measurement")
+    ap.add_argument("--method", choices=("oi", "ippe"), default="oi", help="pose method of the device step")
     ap.add_argument("--out", help="also write the JSON to this file (e.g. profiles/pose_r03.json)")
     args = ap.parse_args()
 
@@ -54,7 +59,7 @@ def main():
     def detector(pose, max_batch):
         d = D.GpuDetector(1280, 800, "yuyv", quad_decimate=2, max_batch=max_batch)
         if pose:
-            d.SetPoseEstimation(TAGSIZE, FX, FY, CX, CY, rotation=ROTATION, offset=OFFSET)
+            d.SetPoseEstimation(TAGSIZE, FX, FY, CX, CY, rotation=ROTATION, offset=OFFSET, method=args.method)
         return d
 
     # throughput: 128-frame device-resident batches, off and on alternating
@@ -76,7 +81,8 @@ def main():
 
     # the pose kernel's device time per batch
     prof = big[True].ProfileDevice(ptr, BATCH, iters=20)
-    pose_ms = [ms for name, ms in prof if name == "pose"]
+    kernel = "pose" if args.method == "oi" else "pose_ippe"
+    pose_ms = [ms for name, ms in prof if name == kernel]
     total_ms = sum(ms for _, ms in prof)
 
     # single-frame latency from a pinned host frame, off and on alternating over the 16 frames
@@ -97,46 +103,63 @@ def main():
             one[pose].DetectPointers([pb.ptr])
             lat[pose].append((time.perf_counter() - t0) * 1e6)
 
-    # host locate_tags on the same detections, one core
+    # the host step on the same detections, one core: the median of 20 calls per frame
     per_frame_dets = []
     for pb_i in range(UNIQUE):
         one[False].DetectPointers([pins[pb_i].ptr])
         per_frame_dets.append(one[False].Detections(0))
+    n_dets = [len(d) for d in per_frame_dets]
     cpu = sorted(os.sched_getaffinity(0))[0]
     saved = os.sched_getaffinity(0)
-    os.sched_setaffinity(0, {cpu})
-    host_us = []
-    try:
-        for dets in per_frame_dets:
-            D.locate_tags(dets, TAGSIZE, FX, FY, CX, CY, ROTATION, OFFSET)
-            reps = []
-            for _ in range(20):
-                t0 = time.perf_counter()
-                D.locate_tags(dets, TAGSIZE, FX, FY, CX, CY, ROTATION, OFFSET)
-                reps.append((time.perf_counter() - t0) * 1e6)
-            host_us.append(float(np.median(reps)))
-    finally:
-        os.sched_setaffinity(0, saved)
-    n_dets = [len(d) for d in per_frame_dets]
+
+    def host_leg(step):
+        os.sched_setaffinity(0, {cpu})
+        host_us = []
+        try:
+            for dets in per_frame_dets:
+                step(dets)
+                reps = []
+                for _ in range(20):
+                    t0 = time.perf_counter()
+                    step(dets)
+                    reps.append((time.perf_counter() - t0) * 1e6)
+                host_us.append(float(np.median(reps)))
+        finally:
+            os.sched_setaffinity(0, saved)
+        return {"per_frame": host_us, "detections": n_dets, "median": float(np.median(host_us)),
+                "us_per_detection": float(sum(host_us) / max(1, sum(n_dets))), "cpu": cpu}
 
     p50 = {k: float(np.percentile(v, 50)) for k, v in lat.items()}
-    host_frame_p50 = float(np.median(host_us))
+    ratio = float(np.median(fps[True]) / np.median(fps[False]))
+    if args.method == "oi":
+        host = {"host_locate_tags_us_per_frame": host_leg(lambda d: D.locate_tags(d, TAGSIZE, FX, FY, CX, CY, ROTATION, OFFSET))}
+        host_frame_p50 = host["host_locate_tags_us_per_frame"]["median"]
+        targets = {"batch_ratio_at_least_0.95": bool(ratio >= 0.95),
+                   "p50_on_below_p50_off_plus_host_pose": bool(p50[True] < p50[False] + host_frame_p50)}
+    else:
+        host = {"host_estimate_poses_ippe_us_per_frame": host_leg(lambda d: D.estimate_poses(d, TAGSIZE, FX, FY, CX, CY, method="ippe")),
+                "host_estimate_poses_oi_us_per_frame": host_leg(lambda d: D.estimate_poses(d, TAGSIZE, FX, FY, CX, CY))}
+        ippe_us = host["host_estimate_poses_ippe_us_per_frame"]["us_per_detection"]
+        oi_us = host["host_estimate_poses_oi_us_per_frame"]["us_per_detection"]
+        targets = {"batch_ratio_at_least_0.95": bool(ratio >= 0.95),
+                   "p50_on_at_most_p50_off_plus_20us": bool(p50[True] <= p50[False] + 20),
+                   "pose_kernel_at_most_0.05ms_per_batch": bool(pose_ms and pose_ms[0] <= 0.05),
+                   "host_ippe_at_least_10x_cheaper_than_host_oi": bool(10 * ippe_us <= oi_us)}
     res = {
+        "method": args.method,
         "gpu": gpu_identity(),
         "torch_device": torch.cuda.get_device_name(0),
         "workload": "config2: 1280x800 YUYV, synth.config_frame(2, 0..15) tiled to 128-frame batches, tag36h11, decimate 2",
         "batch_frames_per_s": {"pose_off": fps[False], "pose_on": fps[True],
                                "median_off": float(np.median(fps[False])), "median_on": float(np.median(fps[True])),
-                               "ratio_on_over_off": float(np.median(fps[True]) / np.median(fps[False]))},
+                               "ratio_on_over_off": ratio},
         "detections_per_batch": dets_per_batch, "raw_detections_per_batch": raw_per_batch,
         "pose_kernel_ms_per_batch": pose_ms[0] if pose_ms else None,
         "all_kernels_ms_per_batch_serial": total_ms,
         "single_frame_latency_us": {"p50_off": p50[False], "p50_on": p50[True], "p90_off": float(np.percentile(lat[False], 90)),
                                     "p90_on": float(np.percentile(lat[True], 90)), "iters": args.latency_iters},
-        "host_locate_tags_us_per_frame": {"per_frame": host_us, "detections": n_dets, "median": host_frame_p50,
-                                          "us_per_detection": float(sum(host_us) / max(1, sum(n_dets))), "cpu": cpu},
-        "targets": {"batch_ratio_at_least_0.95": bool(np.median(fps[True]) >= 0.95 * np.median(fps[False])),
-                    "p50_on_below_p50_off_plus_host_pose": bool(p50[True] < p50[False] + host_frame_p50)},
+        **host,
+        "targets": targets,
     }
     if args.out:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
