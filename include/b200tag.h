@@ -349,6 +349,70 @@ int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count
 int b200tag_debug_estimate_poses_ippe_device(const b200tag_detection *dets, int count, double tagsize, double fx,
                                              double fy, double cx, double cy, b200tag_pose *out);
 
+/* Field pose from every visible layout tag (a multi-tag solve): one camera pose per frame, fitted to the corners of all
+ * tags of a field layout in view by least-squares pixel reprojection error.
+ *
+ * Tag frame: the one of b200tag_pose.  Detection corner p[i] is tag point P_i = (-s, s, 0), (s, s, 0), (s, -s, 0),
+ * (-s, -s, 0), s = tagsize / 2; x points right and y down as the tag is read, z into the tag, so an upright tag seen
+ * head-on has R = I.
+ *
+ * Layout: b200tag_field_tag places one tag's frame in the field, X_field = R * X_tag + t (R row-major, a rotation).
+ * Every layout tag has the pose step's tagsize.
+ *
+ * Which detections take part: per layout (family, id) at most one, the one reconcile prefers (lower hamming, then the
+ * larger decision_margin, then the smaller corners in reconcile's order).  Reconcile only removes the loser of a pair,
+ * so that detection survives it: a raw device list and the reconciled list give the same pose.  A tag whose IPPE pose
+ * cannot be formed is left out.  Correspondences are ordered by layout index, then corner 0..3.
+ *
+ * Solve: both IPPE candidates of every used tag, composed with its layout entry, are seeds, scored by the summed
+ * squared pixel error over all corners (a seed putting any corner at Z <= 0 scores HUGE_VAL); the best is refined by
+ * Levenberg-Marquardt on that error (pinhole model, Cayley rotation update, at most 20 iterations).  With exactly one
+ * tag both candidates are refined and the better returned.  Only + - * /, sqrt, fabs and fmax, with every sum taken in
+ * one fixed order, so host and device results are bit-identical. */
+typedef struct b200tag_field_tag {
+  int32_t family, id;  /* index into the detector's families, tag id */
+  double R[9];         /* row-major: X_field = R * X_tag + t */
+  double t[3];
+} b200tag_field_tag;
+
+typedef struct b200tag_field_pose {
+  int32_t num_tags;     /* layout tags the solve used */
+  int32_t iterations;   /* Levenberg-Marquardt iterations run (accepted and rejected steps) */
+  int32_t reserved[2];
+  double camera_R[9];   /* the camera in the field: X_field = camera_R * X_cam + camera_t */
+  double camera_t[3];
+  double robot_R[9];    /* the robot in the field, through the extrinsics X_robot = rotation * X_cam + offset:
+                           robot_R = camera_R * rotation^T, robot_t = camera_t - robot_R * offset */
+  double robot_t[3];
+  double rms;           /* RMS pixel reprojection error over the corners used; HUGE_VAL when no seed has every corner
+                           in front of the camera */
+  double rms_other;     /* one tag only: the same for the other IPPE candidate after the same refinement; else HUGE_VAL */
+} b200tag_field_pose;   /* num_tags == 0 (no usable layout tag): R = I, t = 0, rms = rms_other = HUGE_VAL */
+
+#define B200TAG_MAX_FIELD_TAGS 1024
+
+/* One frame on the host.  `dets` as b200tag_detections or a raw list; rotation / offset may be NULL (identity / zero).
+ * B200TAG_E_INVALID for bad arguments (tagsize > 0, fx, fy non-zero) or a bad layout: NULL with nlayout > 0, more than
+ * B200TAG_MAX_FIELD_TAGS tags, a duplicate (family, id), R not a rotation within 1e-6 (R R^T = I, det R > 0), a
+ * non-finite value. */
+int b200tag_estimate_field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout,
+                                double tagsize, double fx, double fy, double cx, double cy, const double *rotation,
+                                const double *offset, b200tag_field_pose *out);
+/* The same solve on the device, inside every detect call, one kernel after the pose step: from the next detect call,
+ * whenever the pose step is on (b200tag_set_pose_estimation, with either method) and the layout is not empty, with the
+ * pose step's tagsize, intrinsics and extrinsics.  count == 0 turns it off.  The layout is copied to the device on the
+ * detector's stream (a batch in flight keeps the old one).  Besides the checks of b200tag_estimate_field_pose,
+ * B200TAG_E_INVALID for a family outside the detector's families or an id outside the family's codes; the state is
+ * unchanged on any error.  Adds one kernel to b200tag_kernels_per_batch while it runs. */
+int b200tag_set_field_layout(b200tag_detector *det, const b200tag_field_tag *layout, int count);
+/* The field pose of frame `frame` of the last call; NULL when that call ran without the step.  Owned by the detector,
+ * valid until the next detect call. */
+const b200tag_field_pose *b200tag_field_pose_get(const b200tag_detector *det, int frame);
+/* Test hook: the device kernel on one caller-supplied (raw) list; arguments and result as b200tag_estimate_field_pose. */
+int b200tag_debug_estimate_field_pose_device(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
+                                             int nlayout, double tagsize, double fx, double fy, double cx, double cy,
+                                             const double *rotation, const double *offset, b200tag_field_pose *out);
+
 /* Pinned host staging memory, so b200tag_detect* can overlap H2D with compute. */
 void *b200tag_alloc_pinned(size_t bytes);
 /* Write-combined pinned memory: for buffers the CPU (or a capture driver) only ever WRITES, such as a camera ring

@@ -128,6 +128,17 @@ struct b200tag_detector {
   b200tag_pose *d_poses_alias = nullptr;
   std::vector<std::vector<b200tag_pose>> poses;                   // parallel to dets
   std::vector<std::vector<b200tag_tag_position>> positions;       // closest first
+  std::vector<uint32_t> family_ncodes;                            // codes per family, for the layout checks
+  // the field pose step (b200tag_set_field_layout): on while the pose step is on and field_n > 0
+  int field_n = 0;
+  bool last_field = false;                     // the last enqueue ran the step
+  b200tag_field_tag *d_field_layout = nullptr; // device, B200TAG_MAX_FIELD_TAGS entries; allocated when first set
+  pose::FieldKey *d_field_keys = nullptr;      // device, the layout's sorted keys
+  void *d_field_scratch = nullptr;             // device, per frame field_scratch_stride pose::FieldTagData
+  uint32_t field_scratch_stride = 0;
+  b200tag_field_pose *h_field = nullptr;       // pinned + mapped, max_batch entries
+  b200tag_field_pose *d_field_alias = nullptr;
+  std::vector<b200tag_field_pose> field_poses; // per frame of the last call
 };
 
 namespace b200tag {
@@ -356,6 +367,7 @@ int finish_impl(b200tag_detector *det) {
       det->poses[f].clear();
       det->positions[f].clear();
     }
+    if (det->last_field) det->field_poses[f] = det->h_field[f];
     det->quads_valid[f] = false;
     if (c.status) rc = B200TAG_E_OVERFLOW;
   }
@@ -387,6 +399,14 @@ int record_sequence(b200tag_detector *det, const void *device_images, size_t str
     const PoseLaunch pl{det->d_dets_alias, det->d_poses_alias, p.counters, p.det_cap, 0, ps.tagsize, ps.fx, ps.fy, ps.cx, ps.cy,
                         ps.method};
     launch_pose(pl, count, ln);
+    if (det->field_n > 0) {
+      FieldLaunch fl{det->d_dets_alias, p.counters, p.det_cap, 0, det->d_field_layout, det->d_field_keys, det->field_n,
+                     static_cast<pose::FieldTagData *>(det->d_field_scratch), det->field_scratch_stride,
+                     ps.tagsize, ps.fx, ps.fy, ps.cx, ps.cy, {}, {}, det->d_field_alias};
+      memcpy(fl.rotation, ps.rotation, sizeof(fl.rotation));
+      memcpy(fl.offset, ps.offset, sizeof(fl.offset));
+      launch_field_pose(fl, count, ln);
+    }
   }
   *launches_out = ln.count;
   CK(cudaMemcpyAsync(det->h_counters, p.counters, sizeof(Counters) * count, cudaMemcpyDeviceToHost, det->stream));
@@ -435,6 +455,7 @@ int enqueue_impl(b200tag_detector *det, const void *device_images, size_t stride
   det->kernels_per_batch = launches;
   CK(cudaGetLastError());
   det->last_pose = det->pose;
+  det->last_field = det->pose.tagsize > 0 && det->field_n > 0;
   det->last_count = count;
   det->pending = true;
   return 0;
@@ -540,6 +561,8 @@ int install_families(b200tag_detector *det, const b200tag_family *fams, int n) {
     min_wb = std::min(min_wb, f.width_at_border);
     total_codes += f.ncodes;
   }
+  det->family_ncodes.clear();
+  for (int i = 0; i < n; i++) det->family_ncodes.push_back(fams[i].ncodes);
   if (normal && reversed) {  // apriltag_detect.cu:108: exactly one border polarity across the families
     det->err = "tag families with normal and with reversed borders cannot be mixed (apriltag_detect.cu:108)";
     return B200TAG_E_INVALID;
@@ -760,6 +783,7 @@ int b200tag_create_families(const b200tag_config *cfg, const b200tag_family *fam
   det->dets.resize(B);
   det->poses.resize(B);
   det->positions.resize(B);
+  det->field_poses.resize(B);
   det->quads.resize(B);
   det->quads_valid.assign(B, false);
   memset(det->h_counters, 0, sizeof(Counters) * B);
@@ -796,6 +820,10 @@ void b200tag_destroy(b200tag_detector *det) {
   if (det->h_counters) cudaFreeHost(det->h_counters);
   if (det->h_dets) cudaFreeHost(det->h_dets);
   if (det->h_poses) cudaFreeHost(det->h_poses);
+  if (det->d_field_layout) cudaFree(det->d_field_layout);
+  if (det->d_field_keys) cudaFree(det->d_field_keys);
+  if (det->d_field_scratch) cudaFree(det->d_field_scratch);
+  if (det->h_field) cudaFreeHost(det->h_field);
   delete det;
 }
 
@@ -1223,6 +1251,11 @@ const b200tag_pose *b200tag_poses(const b200tag_detector *det, int frame, int *c
   return det->poses[frame].data();
 }
 
+const b200tag_field_pose *b200tag_field_pose_get(const b200tag_detector *det, int frame) {
+  if (!det || frame < 0 || frame >= det->last_count || det->pending || !det->last_field) return nullptr;
+  return &det->field_poses[frame];
+}
+
 const b200tag_tag_position *b200tag_tag_positions(const b200tag_detector *det, int frame, int *count) {
   if (count) *count = 0;
   if (!det || frame < 0 || frame >= det->last_count || det->pending || !(det->last_pose.tagsize > 0)) return nullptr;
@@ -1384,6 +1417,49 @@ int b200tag_set_pose_estimation(b200tag_detector *det, double tagsize, double fx
   return 0;
 }
 
+int b200tag_set_field_layout(b200tag_detector *det, const b200tag_field_tag *layout, int count) {
+  if (!det) return B200TAG_E_INVALID;
+  std::vector<pose::FieldKey> keys(static_cast<size_t>(std::max(count, 0)));
+  if (!field_layout_keys(layout, count, det->family_ncodes.data(), static_cast<int>(det->family_ncodes.size()), keys.data())) {
+    det->err = "invalid field layout";
+    return B200TAG_E_INVALID;
+  }
+  DeviceGuard on_device(det->device);
+  if (count > 0 && !det->h_field) {
+    const size_t B = static_cast<size_t>(det->cfg.max_batch);
+    const uint32_t stride = std::min<uint32_t>(det->fp.det_cap, B200TAG_MAX_FIELD_TAGS);
+    void *dl = nullptr, *dk = nullptr, *ds = nullptr;
+    b200tag_field_pose *h = nullptr, *d = nullptr;
+    const bool ok = cudaMalloc(&dl, sizeof(b200tag_field_tag) * B200TAG_MAX_FIELD_TAGS) == cudaSuccess &&
+                    cudaMalloc(&dk, sizeof(pose::FieldKey) * B200TAG_MAX_FIELD_TAGS) == cudaSuccess &&
+                    cudaMalloc(&ds, field_tag_bytes() * stride * B) == cudaSuccess &&
+                    cudaHostAlloc(reinterpret_cast<void **>(&h), sizeof(b200tag_field_pose) * B, cudaHostAllocMapped) == cudaSuccess &&
+                    cudaHostGetDevicePointer(reinterpret_cast<void **>(&d), h, 0) == cudaSuccess;
+    if (!ok) {
+      cudaGetLastError();
+      cudaFree(dl);
+      cudaFree(dk);
+      cudaFree(ds);
+      if (h) cudaFreeHost(h);
+      det->err = "allocating the field pose buffers failed";
+      return B200TAG_E_CUDA;
+    }
+    det->d_field_layout = static_cast<b200tag_field_tag *>(dl);
+    det->d_field_keys = static_cast<pose::FieldKey *>(dk);
+    det->d_field_scratch = ds;
+    det->field_scratch_stride = stride;
+    det->h_field = h;
+    det->d_field_alias = d;
+  }
+  if (count > 0) {  // stream-ordered: a batch in flight reads the old layout to its end
+    CK(cudaMemcpyAsync(det->d_field_layout, layout, sizeof(b200tag_field_tag) * count, cudaMemcpyHostToDevice, det->stream));
+    CK(cudaMemcpyAsync(det->d_field_keys, keys.data(), sizeof(pose::FieldKey) * count, cudaMemcpyHostToDevice, det->stream));
+  }
+  drop_graphs(det);  // the layout size is baked into the captured launches
+  det->field_n = count;
+  return 0;
+}
+
 int b200tag_set_pose_method(b200tag_detector *det, int method) {
   if (!det || (method != B200TAG_POSE_ORTHOGONAL_ITERATION && method != B200TAG_POSE_IPPE)) return B200TAG_E_INVALID;
   DeviceGuard on_device(det->device);
@@ -1510,6 +1586,42 @@ int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count
 int b200tag_debug_estimate_poses_ippe_device(const b200tag_detection *dets, int count, double tagsize, double fx,
                                              double fy, double cx, double cy, b200tag_pose *out) {
   return estimate_poses_device(B200TAG_POSE_IPPE, dets, count, tagsize, fx, fy, cx, cy, out);
+}
+
+int b200tag_debug_estimate_field_pose_device(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
+                                             int nlayout, double tagsize, double fx, double fy, double cx, double cy,
+                                             const double *rotation, const double *offset, b200tag_field_pose *out) {
+  if (count < 0 || (count > 0 && !dets) || !out || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
+  std::vector<pose::FieldKey> keys(static_cast<size_t>(std::max(nlayout, 0)));
+  if (!field_layout_keys(layout, nlayout, nullptr, 0, keys.data())) return B200TAG_E_INVALID;
+  const size_t db = sizeof(b200tag_detection) * static_cast<size_t>(count), lb = sizeof(b200tag_field_tag) * nlayout,
+               kb = sizeof(pose::FieldKey) * nlayout, sb = field_tag_bytes() * std::max(count, 1);
+  const size_t o_l = align_up(db, 256), o_k = align_up(o_l + lb, 256), o_s = align_up(o_k + kb, 256), o_o = align_up(o_s + sb, 256);
+  uint8_t *d = nullptr;
+  if (cudaMalloc(&d, o_o + sizeof(b200tag_field_pose)) != cudaSuccess) {
+    cudaGetLastError();
+    return B200TAG_E_NO_DEVICE;
+  }
+  static const double kEye[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, kZero[3] = {0, 0, 0};
+  FieldLaunch fl{reinterpret_cast<const b200tag_detection *>(d), nullptr, 0, static_cast<uint32_t>(count),
+                 reinterpret_cast<const b200tag_field_tag *>(d + o_l), reinterpret_cast<const pose::FieldKey *>(d + o_k), nlayout,
+                 reinterpret_cast<pose::FieldTagData *>(d + o_s), 0, tagsize, fx, fy, cx, cy, {}, {},
+                 reinterpret_cast<b200tag_field_pose *>(d + o_o)};
+  memcpy(fl.rotation, rotation ? rotation : kEye, sizeof(fl.rotation));
+  memcpy(fl.offset, offset ? offset : kZero, sizeof(fl.offset));
+  int rc = 0;
+  if ((db && cudaMemcpy(d, dets, db, cudaMemcpyHostToDevice) != cudaSuccess) ||
+      (lb && cudaMemcpy(d + o_l, layout, lb, cudaMemcpyHostToDevice) != cudaSuccess) ||
+      (kb && cudaMemcpy(d + o_k, keys.data(), kb, cudaMemcpyHostToDevice) != cudaSuccess))
+    rc = B200TAG_E_CUDA;
+  if (!rc) {
+    Launcher ln{nullptr, nullptr};
+    launch_field_pose(fl, 1, ln);
+    if (cudaGetLastError() != cudaSuccess || cudaMemcpy(out, d + o_o, sizeof(*out), cudaMemcpyDeviceToHost) != cudaSuccess)
+      rc = B200TAG_E_CUDA;
+  }
+  cudaFree(d);
+  return rc;
 }
 
 int b200tag_kernels_per_batch(const b200tag_detector *det) { return det ? det->kernels_per_batch : 0; }

@@ -90,6 +90,27 @@ struct PoseLaunch {
 };
 void launch_pose(const PoseLaunch &L, int frames, Launcher &ln);
 
+// The field pose step (kernels_pose.cu, k_field_pose): one b200tag_field_pose per frame from the frame's raw records.
+namespace pose {
+struct FieldKey;
+struct FieldTagData;
+}  // namespace pose
+struct FieldLaunch {
+  const b200tag_detection *dets;     // frame f's records start at dets + f * stride
+  const Counters *counters;          // per-frame record counts; null: one list of `count` records
+  uint32_t stride, count;
+  const b200tag_field_tag *layout;   // device copies of the layout and its sorted keys
+  const pose::FieldKey *keys;
+  int nlayout;
+  pose::FieldTagData *scratch;       // frame f's used tags start at scratch + f * scratch_stride
+  uint32_t scratch_stride;           // >= min(records, nlayout) of any frame
+  double tagsize, fx, fy, cx, cy;
+  double rotation[9], offset[3];
+  b200tag_field_pose *out;           // one per frame
+};
+void launch_field_pose(const FieldLaunch &L, int frames, Launcher &ln);
+size_t field_tag_bytes();            // sizeof(pose::FieldTagData)
+
 // JPEG luminance planes of a batch (jpeg.h): the parallel kernels for streams without restart markers, the sequential
 // warp-per-frame kernel for the rest.
 struct JpegBatch;

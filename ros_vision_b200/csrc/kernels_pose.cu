@@ -165,7 +165,122 @@ __global__ void __launch_bounds__(kIppeThreads) k_pose_ippe(PoseLaunch L) {
   }
 }
 
+// The sum of v over the warp by the xor tree of pose_core.h (field_slot_tree): every lane ends with the same bits.
+__device__ double warp_sum(double v) {
+#pragma unroll
+  for (int m = kFieldSlots / 2; m >= 1; m >>= 1) v = v + __shfl_xor_sync(kFull, v, m);
+  return v;
+}
+
+// The field pose (b200tag_set_field_layout) of every frame: one warp per frame, blockIdx.x = frame, reading the frame's
+// raw records from the mapped detection buffer, as many as its counter holds.  The lanes look the records up in the
+// layout and keep, per layout tag, the record reconcile prefers; in layout order they write each used tag's corners and
+// seeds to the frame's scratch, and then run field_solve with correspondence k on lane k % 32 and the 6x6 solve on every
+// lane.  The arithmetic is pose_core.h's, the same b200tag_estimate_field_pose runs on the host.
+__global__ void __launch_bounds__(32) k_field_pose(FieldLaunch L) {
+  __shared__ int cnt[B200TAG_MAX_FIELD_TAGS], sel[B200TAG_MAX_FIELD_TAGS];
+  __shared__ int dup;
+  const int lane = threadIdx.x;
+  const size_t frame = blockIdx.x;
+  const uint32_t n = L.counters ? min(L.counters[frame].num_detections, L.stride) : L.count;
+  const b200tag_detection *recs = L.dets + frame * L.stride;
+  FieldTagData *tags = L.scratch + frame * L.scratch_stride;
+  for (int i = lane; i < L.nlayout; i += 32) cnt[i] = 0;
+  if (lane == 0) dup = 0;
+  __syncwarp();
+  for (uint32_t i = lane; i < n; i += 32) {
+    const int li = field_lookup(L.keys, L.nlayout, recs[i].family, recs[i].id);
+    if (li >= 0) {
+      if (atomicAdd(&cnt[li], 1) > 0) dup = 1;
+      sel[li] = static_cast<int>(i);
+    }
+  }
+  __syncwarp();
+  if (dup) {  // a layout tag seen more than once: the preferred record, the lowest index of identical ones
+    for (uint32_t i = lane; i < n; i += 32) {
+      const int32_t fam = recs[i].family, id = recs[i].id;
+      const int li = field_lookup(L.keys, L.nlayout, fam, id);
+      if (li < 0 || cnt[li] < 2) continue;
+      bool wins = true;
+      for (uint32_t k = 0; k < n && wins; k++) {
+        if (k == i || recs[k].family != fam || recs[k].id != id) continue;
+        wins = !field_prefers(recs[k], recs[i]) && (k > i || field_prefers(recs[i], recs[k]));
+      }
+      if (wins) sel[li] = static_cast<int>(i);
+    }
+    __syncwarp();
+  }
+  // the used tags in layout order; a tag whose IPPE candidates cannot be formed is left out
+  const FieldCamera cam{L.fx, L.fy, L.cx, L.cy};
+  const unsigned below = (1u << lane) - 1;
+  int used = 0;
+  for (int base = 0; base < L.nlayout; base += 32) {
+    const int li = base + lane;
+    const bool has = li < L.nlayout && cnt[li] > 0;
+    const unsigned hm = __ballot_sync(kFull, has);
+    bool ok = false;
+    if (has) {
+      const double2 *src = reinterpret_cast<const double2 *>(recs[sel[li]].p);
+      double px[4][2];
+#pragma unroll
+      for (int k = 0; k < 4; k++) {
+        const double2 c = src[k];
+        px[k][0] = c.x;
+        px[k][1] = c.y;
+      }
+      ok = field_tag_data(L.layout[li], px, L.tagsize, cam, &tags[used + __popc(hm & below)]);
+    }
+    const unsigned om = __ballot_sync(kFull, ok);
+    __syncwarp();
+    for (unsigned m = om; om != hm && m; m &= m - 1) {  // move the formed tags down over the others, in order
+      const int l = __ffs(m) - 1;
+      const double *from = reinterpret_cast<const double *>(&tags[used + __popc(hm & ((1u << l) - 1))]);
+      double *to = reinterpret_cast<double *>(&tags[used + __popc(om & ((1u << l) - 1))]);
+      static_assert(sizeof(FieldTagData) % 8 == 0, "tag copy");
+      if (from != to)
+        for (int w = lane; w < static_cast<int>(sizeof(FieldTagData) / 8); w += 32) to[w] = from[w];
+      __syncwarp();
+    }
+    used += __popc(om);
+  }
+  b200tag_field_pose res;
+  if (used == 0) {
+    field_empty(&res);
+  } else {
+    const int ncorr = 4 * used;
+    auto cost = [&](const M3 &R, const V3 &t) {
+      double acc = 0;
+      for (int k = lane; k < ncorr; k += 32) {
+        const FieldTagData &g = tags[k >> 2];
+        V3 Y, P;
+        double ru, rv;
+        acc += field_corner_cost(g.px[k & 3][0], g.px[k & 3][1], g.X[k & 3], R, t, cam, &Y, &P, &ru, &rv);
+      }
+      return warp_sum(acc);
+    };
+    auto sum = [&](const M3 &R, const V3 &t, double *S) {
+      double acc[kFieldSums];
+#pragma unroll
+      for (int j = 0; j < kFieldSums; j++) acc[j] = 0;
+      for (int k = lane; k < ncorr; k += 32) {
+        const FieldTagData &g = tags[k >> 2];
+        field_corner_terms(g.px[k & 3][0], g.px[k & 3][1], g.X[k & 3], R, t, cam, acc);
+      }
+#pragma unroll
+      for (int j = 0; j < kFieldSums; j++) S[j] = warp_sum(acc[j]);
+    };
+    field_solve(tags, used, cost, sum, L.rotation, L.offset, &res);
+  }
+  if (lane == 0) L.out[frame] = res;
+}
+
 }  // namespace
+
+size_t field_tag_bytes() { return sizeof(FieldTagData); }
+
+void launch_field_pose(const FieldLaunch &L, int frames, Launcher &ln) {
+  ln.timed("field_pose", [&] { k_field_pose<<<static_cast<unsigned>(frames), 32, 0, ln.s>>>(L); });
+}
 
 void launch_pose(const PoseLaunch &L, int frames, Launcher &ln) {
   if (L.method == B200TAG_POSE_IPPE) {

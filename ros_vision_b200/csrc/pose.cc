@@ -28,6 +28,30 @@ void locate_from_poses(const b200tag_detection *dets, const b200tag_pose *poses,
   std::stable_sort(out, out + count, [](const b200tag_tag_position &a, const b200tag_tag_position &b) { return a.distance < b.distance; });
 }
 
+bool field_layout_keys(const b200tag_field_tag *layout, int nlayout, const uint32_t *ncodes, int nfamilies, pose::FieldKey *keys) {
+  if (nlayout < 0 || nlayout > B200TAG_MAX_FIELD_TAGS || (nlayout > 0 && !layout)) return false;
+  for (int i = 0; i < nlayout; i++) {
+    const b200tag_field_tag &L = layout[i];
+    if (ncodes && (L.family < 0 || L.family >= nfamilies || L.id < 0 || static_cast<uint32_t>(L.id) >= ncodes[L.family]))
+      return false;
+    for (double x : L.R) if (!std::isfinite(x)) return false;
+    for (double x : L.t) if (!std::isfinite(x)) return false;
+    for (int r = 0; r < 3; r++)
+      for (int c = 0; c < 3; c++) {
+        const double d = L.R[3 * r] * L.R[3 * c] + L.R[3 * r + 1] * L.R[3 * c + 1] + L.R[3 * r + 2] * L.R[3 * c + 2];
+        if (!(std::fabs(d - (r == c ? 1.0 : 0.0)) <= 1e-6)) return false;
+      }
+    pose::M3 R;
+    for (int k = 0; k < 9; k++) R.a[k] = L.R[k];
+    if (!(pose::det3(R) > 0)) return false;
+    keys[i] = pose::FieldKey{L.family, L.id, i, 0};
+  }
+  std::sort(keys, keys + nlayout, [](const pose::FieldKey &a, const pose::FieldKey &b) { return pose::key_less(a.family, a.id, b.family, b.id); });
+  for (int i = 1; i < nlayout; i++)
+    if (keys[i].family == keys[i - 1].family && keys[i].id == keys[i - 1].id) return false;
+  return true;
+}
+
 }  // namespace b200tag
 
 using namespace b200tag::pose;
@@ -105,6 +129,56 @@ int b200tag_locate_tags(const b200tag_detection *dets, int count, double tagsize
   std::vector<b200tag_pose> poses(static_cast<size_t>(count));
   if (int rc = b200tag_estimate_poses(dets, count, tagsize, fx, fy, cx, cy, poses.data())) return rc;
   b200tag::locate_from_poses(dets, poses.data(), count, rotation, offset, out);
+  return 0;
+}
+
+int b200tag_estimate_field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout,
+                                double tagsize, double fx, double fy, double cx, double cy, const double *rotation,
+                                const double *offset, b200tag_field_pose *out) {
+  if (count < 0 || (count > 0 && !dets) || !out || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
+  std::vector<FieldKey> keys(static_cast<size_t>(std::max(nlayout, 0)));
+  if (!b200tag::field_layout_keys(layout, nlayout, nullptr, 0, keys.data())) return B200TAG_E_INVALID;
+  static const double kEye[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, kZero[3] = {0, 0, 0};
+  const double *Rx = rotation ? rotation : kEye, *ox = offset ? offset : kZero;
+  // the detection reconcile prefers, per layout tag
+  std::vector<int> sel(static_cast<size_t>(nlayout), -1);
+  for (int i = 0; i < count; i++) {
+    const int L = field_lookup(keys.data(), nlayout, dets[i].family, dets[i].id);
+    if (L >= 0 && (sel[L] < 0 || field_prefers(dets[i], dets[sel[L]]))) sel[L] = i;
+  }
+  const FieldCamera cam{fx, fy, cx, cy};
+  std::vector<FieldTagData> tags;
+  for (int L = 0; L < nlayout; L++) {
+    FieldTagData d;
+    if (sel[L] >= 0 && field_tag_data(layout[L], dets[sel[L]].p, tagsize, cam, &d)) tags.push_back(d);
+  }
+  const int ntags = static_cast<int>(tags.size());
+  if (ntags == 0) {
+    field_empty(out);
+    return 0;
+  }
+  const int ncorr = 4 * ntags;
+  auto cost = [&](const M3 &R, const V3 &t) {
+    double slot[kFieldSlots][1] = {};
+    for (int k = 0; k < ncorr; k++) {
+      const FieldTagData &g = tags[k >> 2];
+      V3 Y, P;
+      double ru, rv;
+      slot[k % kFieldSlots][0] += field_corner_cost(g.px[k & 3][0], g.px[k & 3][1], g.X[k & 3], R, t, cam, &Y, &P, &ru, &rv);
+    }
+    double total;
+    field_slot_tree<1>(slot, &total);
+    return total;
+  };
+  auto sum = [&](const M3 &R, const V3 &t, double *S) {
+    double slot[kFieldSlots][kFieldSums] = {};
+    for (int k = 0; k < ncorr; k++) {
+      const FieldTagData &g = tags[k >> 2];
+      field_corner_terms(g.px[k & 3][0], g.px[k & 3][1], g.X[k & 3], R, t, cam, slot[k % kFieldSlots]);
+    }
+    field_slot_tree<kFieldSums>(slot, S);
+  };
+  field_solve(tags.data(), ntags, cost, sum, Rx, ox, out);
   return 0;
 }
 

@@ -15,7 +15,8 @@
 // libdevice may differ by an ulp.
 //
 // The second method, IPPE (ippe_pose, at the end), is closed form and uses only + - * /, sqrt, fabs and fmax: its
-// poses are bit-identical on host and device.
+// poses are bit-identical on host and device.  So is the field pose (field_solve, at the end): the same operations, and
+// every sum over correspondences taken in one order on both sides.
 #ifndef B200TAG_POSE_CORE_H_
 #define B200TAG_POSE_CORE_H_
 
@@ -27,9 +28,11 @@
 
 #ifdef __CUDACC__
 #define POSE_HD __host__ __device__ inline
+#define POSE_HD_CALL __host__ __device__ inline __noinline__  // a call of its own: keeps the caller's registers free of spills
 #define POSE_UNROLL _Pragma("unroll")
 #else
 #define POSE_HD inline
+#define POSE_HD_CALL inline
 #define POSE_UNROLL
 #endif
 
@@ -483,22 +486,30 @@ POSE_HD double object_space_error(const V3 *v, const V3 *p, const M3 &R, const V
   return err;
 }
 
+// Both IPPE candidates of the tag with rays v and corners p (rays_and_corners) and their object-space errors; false
+// when a candidate cannot be formed (an error is not below HUGE_VAL, which also catches a NaN from overflowing
+// intermediates).
+POSE_HD bool ippe_candidates(const V3 *v, const V3 *p, double tagsize, M3 *R, V3 *t, double *err) {
+  double H[9];
+  err[0] = err[1] = HUGE_VAL;
+  bool ok = square_homography(v, tagsize / 2.0, H) && ippe_rotations(H, R);
+  POSE_UNROLL for (int k = 0; k < 2; k++) {
+    ok = ok && ippe_translation(v, p, R[k], &t[k]);
+    if (ok) err[k] = object_space_error(v, p, R[k], t[k]);
+  }
+  return err[0] < HUGE_VAL && err[1] < HUGE_VAL;
+}
+
 // IPPE pose of a tag whose corners are at image points px[0..3]: the candidate with the smaller object-space error,
 // the other's error in err_other.  A quad for which a candidate cannot be formed gives R = I, t = 0 and both errors
 // HUGE_VAL.
 POSE_HD void ippe_pose(const double (*px)[2], double tagsize, double fx, double fy, double cx, double cy, b200tag_pose *out) {
   V3 v[4], p[4];
   rays_and_corners(px, tagsize, fx, fy, cx, cy, v, p);
-  double H[9];
   M3 R[2];
   V3 t[2];
-  double err[2] = {HUGE_VAL, HUGE_VAL};
-  bool ok = square_homography(v, tagsize / 2.0, H) && ippe_rotations(H, R);
-  POSE_UNROLL for (int k = 0; k < 2; k++) {
-    ok = ok && ippe_translation(v, p, R[k], &t[k]);
-    if (ok) err[k] = object_space_error(v, p, R[k], t[k]);
-  }
-  if (!(err[0] < HUGE_VAL && err[1] < HUGE_VAL)) {  // also catches a NaN from overflowing intermediates
+  double err[2];
+  if (!ippe_candidates(v, p, tagsize, R, t, err)) {
     const M3 I = ident();
     const V3 z{{0, 0, 0}};
     choose_pose(I, z, HUGE_VAL, I, z, HUGE_VAL, out);
@@ -507,12 +518,297 @@ POSE_HD void ippe_pose(const double (*px)[2], double tagsize, double fx, double 
   choose_pose(R[0], t[0], err[0], R[1], t[1], err[1], out);
 }
 
+// ---- Field pose (b200tag_estimate_field_pose, b200tag_set_field_layout) ----
+// One camera-from-field pose (R, t: X_cam = R X_field + t) fitted to the corners of every layout tag in view.  The
+// caller selects the detections (field_lookup, field_prefers) and fills one FieldTagData per used tag, in layout order;
+// field_solve does the rest.  Every sum over correspondences is taken in one order: correspondence k (tag k / 4, corner
+// k % 4) adds into slot k % kFieldSlots in increasing k, and the slots are combined by the xor tree of field_slot_tree.
+// The device runs a slot per lane and the tree with __shfl_xor_sync, the host loops; IEEE addition is commutative, so
+// every lane and the host hold the same bits.
+
+constexpr int kFieldSlots = 32;
+constexpr int kFieldSums = 28;      // cost, J^T r (6), the upper triangle of J^T J (21)
+constexpr int kFieldMaxIterations = 20;
+
+// Layout lookup: (family, id) -> layout index, sorted by (family, id).
+struct FieldKey {
+  int32_t family, id, index, pad;
+};
+POSE_HD bool key_less(int32_t f0, int32_t i0, int32_t f1, int32_t i1) { return f0 != f1 ? f0 < f1 : i0 < i1; }
+POSE_HD int field_lookup(const FieldKey *keys, int n, int32_t family, int32_t id) {
+  int lo = 0, hi = n;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (key_less(keys[mid].family, keys[mid].id, family, id)) lo = mid + 1; else hi = mid;
+  }
+  return lo < n && keys[lo].family == family && keys[lo].id == id ? keys[lo].index : -1;
+}
+
+// True when reconcile() prefers detection a to b: lower hamming, then larger decision_margin, then the smaller corner
+// coordinates in p order.  False for a tie, which needs identical corners -- and the solve reads nothing else.
+POSE_HD bool field_prefers(const b200tag_detection &a, const b200tag_detection &b) {
+  double qa[10], qb[10];
+  qa[0] = a.hamming; qb[0] = b.hamming;
+  qa[1] = -a.decision_margin; qb[1] = -b.decision_margin;
+  POSE_UNROLL for (int i = 0; i < 4; i++) {
+    qa[2 + 2 * i] = a.p[i][0]; qb[2 + 2 * i] = b.p[i][0];
+    qa[3 + 2 * i] = a.p[i][1]; qb[3 + 2 * i] = b.p[i][1];
+  }
+  POSE_UNROLL for (int k = 0; k < 10; k++) {
+    if (qa[k] < qb[k]) return true;
+    if (qb[k] < qa[k]) return false;
+  }
+  return false;
+}
+
+// What the solve reads of one used tag: its image corners, the same corners in the field, and its two seeds (each IPPE
+// candidate composed with the layout entry into a camera-from-field pose).
+struct FieldTagData {
+  double px[4][2];
+  V3 X[4];
+  M3 R[2];
+  V3 t[2];
+};
+
+struct FieldCamera {
+  double fx, fy, cx, cy;
+};
+
+// Fills *d for the layout tag L seen at image corners px; false when its IPPE candidates cannot be formed.
+POSE_HD bool field_tag_data(const b200tag_field_tag &L, const double (*px)[2], double tagsize, const FieldCamera &cam,
+                            FieldTagData *d) {
+  V3 v[4], p[4];
+  rays_and_corners(px, tagsize, cam.fx, cam.fy, cam.cx, cam.cy, v, p);
+  M3 R[2];
+  V3 t[2];
+  double err[2];
+  if (!ippe_candidates(v, p, tagsize, R, t, err)) return false;
+  M3 Lr;
+  POSE_UNROLL for (int k = 0; k < 9; k++) Lr.a[k] = L.R[k];
+  const V3 Lt{{L.t[0], L.t[1], L.t[2]}};
+  const M3 LrT = transpose(Lr);
+  POSE_UNROLL for (int i = 0; i < 4; i++) {
+    d->px[i][0] = px[i][0];
+    d->px[i][1] = px[i][1];
+    d->X[i] = add(mul(Lr, p[i]), Lt);
+  }
+  // X_cam = Rc (Lr^T (X_field - Lt)) + tc
+  POSE_UNROLL for (int k = 0; k < 2; k++) {
+    const M3 Rf = mul(R[k], LrT);
+    d->R[k] = Rf;
+    d->t[k] = sub(t[k], mul(Rf, Lt));
+  }
+  return true;
+}
+
+// Squared pixel error of one correspondence (image point u, v; field point X) at pose (R, t), HUGE_VAL when the point
+// is not in front of the camera.  *Y = R X, *P = R X + t for field_corner_terms.
+POSE_HD double field_corner_cost(double u, double v, const V3 &X, const M3 &R, const V3 &t, const FieldCamera &cam, V3 *Y,
+                                 V3 *P, double *ru, double *rv) {
+  *Y = mul(R, X);
+  *P = add(*Y, t);
+  if (!(P->v[2] > 0)) return HUGE_VAL;
+  const double iz = 1 / P->v[2];
+  *ru = cam.fx * (P->v[0] * iz) + cam.cx - u;
+  *rv = cam.fy * (P->v[1] * iz) + cam.cy - v;
+  return *ru * *ru + *rv * *rv;
+}
+
+// Adds one correspondence's cost, J^T r and J^T J into acc[kFieldSums].  J is the Jacobian of the residual for the update
+// R <- cayley(c) R, t <- t + dt at c = 0, dt = 0: d(R X + t)/dc = -2 [R X]x.
+POSE_HD void field_corner_terms(double u, double v, const V3 &X, const M3 &R, const V3 &t, const FieldCamera &cam, double *acc) {
+  V3 Y, P;
+  double ru = 0, rv = 0;
+  const double e = field_corner_cost(u, v, X, R, t, cam, &Y, &P, &ru, &rv);
+  acc[0] += e;
+  if (!(e < HUGE_VAL)) return;
+  const double iz = 1 / P.v[2];
+  const V3 du{{cam.fx * iz, 0, -cam.fx * (P.v[0] * iz) * iz}}, dv{{0, cam.fy * iz, -cam.fy * (P.v[1] * iz) * iz}};
+  const V3 cu = cross(Y, du), cv = cross(Y, dv);
+  const double Ju[6] = {2 * cu.v[0], 2 * cu.v[1], 2 * cu.v[2], du.v[0], du.v[1], du.v[2]};
+  const double Jv[6] = {2 * cv.v[0], 2 * cv.v[1], 2 * cv.v[2], dv.v[0], dv.v[1], dv.v[2]};
+  POSE_UNROLL for (int i = 0; i < 6; i++) acc[1 + i] += Ju[i] * ru + Jv[i] * rv;
+  int o = 7;
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = i; j < 6; j++) acc[o++] += Ju[i] * Ju[j] + Jv[i] * Jv[j];
+}
+
+// The host's form of the slot tree: slot[l] += slot[l + m] for m = 16, 8, 4, 2, 1; the total ends in slot[0].  A warp
+// computes the same with lane l adding lane l ^ m.
+template <int K>
+inline void field_slot_tree(double (*slot)[K], double *out) {
+  for (int m = kFieldSlots / 2; m >= 1; m >>= 1)
+    for (int l = 0; l < m; l++)
+      for (int j = 0; j < K; j++) slot[l][j] = slot[l][j] + slot[l + m][j];
+  for (int j = 0; j < K; j++) out[j] = slot[0][j];
+}
+
+// Solves (J^T J + lambda diag(J^T J)) d = -J^T r from the sums S by Cholesky; false when the matrix is not positive
+// definite.
+POSE_HD_CALL bool field_step(const double *S, double lambda, double *d) {
+  double A[6][6];
+  int o = 7;
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = i; j < 6; j++) A[i][j] = A[j][i] = S[o++];
+  POSE_UNROLL for (int i = 0; i < 6; i++) A[i][i] = A[i][i] + lambda * A[i][i];
+  double Lm[6][6] = {};
+  POSE_UNROLL for (int j = 0; j < 6; j++) {
+    double s = A[j][j];
+    POSE_UNROLL for (int k = 0; k < j; k++) s -= Lm[j][k] * Lm[j][k];
+    if (!(s > 0)) return false;
+    Lm[j][j] = sqrt(s);
+    POSE_UNROLL for (int i = j + 1; i < 6; i++) {
+      double r = A[i][j];
+      POSE_UNROLL for (int k = 0; k < j; k++) r -= Lm[i][k] * Lm[j][k];
+      Lm[i][j] = r / Lm[j][j];
+    }
+  }
+  double y[6];
+  POSE_UNROLL for (int i = 0; i < 6; i++) {
+    double r = -S[1 + i];
+    POSE_UNROLL for (int k = 0; k < i; k++) r -= Lm[i][k] * y[k];
+    y[i] = r / Lm[i][i];
+  }
+  POSE_UNROLL for (int i = 5; i >= 0; i--) {
+    double r = y[i];
+    POSE_UNROLL for (int k = i + 1; k < 6; k++) r -= Lm[k][i] * d[k];
+    d[i] = r / Lm[i][i];
+  }
+  return true;
+}
+
+// R <- cayley(d[0..2]) R, t <- t + d[3..5]; cayley(c) = ((1 - c.c) I + 2 c c^T + 2 [c]x) / (1 + c.c) is a rotation and
+// needs no trigonometry.
+POSE_HD void field_update(const M3 &R, const V3 &t, const double *d, M3 *Rn, V3 *tn) {
+  const double a = d[0], b = d[1], c = d[2];
+  const double n2 = a * a + b * b + c * c, s = 1 / (1 + n2), w = 1 - n2;
+  const M3 C{{(w + 2 * a * a) * s, 2 * (a * b - c) * s, 2 * (a * c + b) * s,
+              2 * (a * b + c) * s, (w + 2 * b * b) * s, 2 * (b * c - a) * s,
+              2 * (a * c - b) * s, 2 * (b * c + a) * s, (w + 2 * c * c) * s}};
+  *Rn = mul(C, R);
+  *tn = V3{{t.v[0] + d[3], t.v[1] + d[4], t.v[2] + d[5]}};
+}
+
+// Levenberg-Marquardt from (*R, *t).  sum(R, t, S) fills S[kFieldSums] with the reduced sums at (R, t).  A step is
+// accepted when it lowers the cost (lambda / 10), else rejected (lambda * 10).  The iteration stops after a step of at
+// most 1e-10 in every parameter (Cayley vector, metres), accepted or not; after an accepted step that lowers the cost
+// by at most 1e-12 of itself; when lambda exceeds 1e8; or after kFieldMaxIterations.
+// Returns the final cost; *iterations counts accepted and rejected steps.
+template <class SumFn>
+POSE_HD double field_refine(SumFn &sum, M3 *R, V3 *t, int *iterations) {
+  double S[kFieldSums];
+  sum(*R, *t, S);
+  double cost = S[0];
+  int it = 0;
+  if (cost < HUGE_VAL) {
+    double lambda = 1e-3;
+    while (it < kFieldMaxIterations) {
+      it++;
+      double d[6];
+      if (field_step(S, lambda, d)) {
+        M3 Rn;
+        V3 tn;
+        field_update(*R, *t, d, &Rn, &tn);
+        double Sn[kFieldSums];
+        sum(Rn, tn, Sn);
+        bool small = true;
+        POSE_UNROLL for (int j = 0; j < 6; j++) small = small && fabs(d[j]) <= 1e-10;
+        if (Sn[0] < cost) {
+          small = small || cost - Sn[0] <= 1e-12 * cost;
+          *R = Rn;
+          *t = tn;
+          cost = Sn[0];
+          POSE_UNROLL for (int j = 0; j < kFieldSums; j++) S[j] = Sn[j];
+          lambda = lambda * 0.1;
+          if (small) break;
+          continue;
+        }
+        if (small) break;  // a step this small that does not lower the cost: the minimum, to rounding
+      }
+      lambda = lambda * 10;
+      if (lambda > 1e8) break;
+    }
+  }
+  *iterations = it;
+  return cost;
+}
+
+POSE_HD void field_empty(b200tag_field_pose *out) {
+  out->num_tags = 0;
+  out->iterations = 0;
+  out->reserved[0] = out->reserved[1] = 0;
+  POSE_UNROLL for (int k = 0; k < 9; k++) out->camera_R[k] = out->robot_R[k] = (k % 4 == 0) ? 1.0 : 0.0;
+  POSE_UNROLL for (int k = 0; k < 3; k++) out->camera_t[k] = out->robot_t[k] = 0;
+  out->rms = out->rms_other = HUGE_VAL;
+}
+
+// The record of camera-from-field pose (R, t): the camera and the robot in the field.
+POSE_HD void field_result(const M3 &R, const V3 &t, double cost, double cost_other, int ntags, int iterations,
+                          const double *rotation, const double *offset, b200tag_field_pose *out) {
+  const M3 Rc = transpose(R);
+  const V3 tc = scale(mul(Rc, t), -1.0);
+  M3 Rx, Rr;
+  POSE_UNROLL for (int k = 0; k < 9; k++) Rx.a[k] = rotation[k];
+  Rr = mul(Rc, transpose(Rx));
+  const V3 tr = sub(tc, mul(Rr, V3{{offset[0], offset[1], offset[2]}}));
+  out->num_tags = ntags;
+  out->iterations = iterations;
+  out->reserved[0] = out->reserved[1] = 0;
+  POSE_UNROLL for (int k = 0; k < 9; k++) {
+    out->camera_R[k] = Rc.a[k];
+    out->robot_R[k] = Rr.a[k];
+  }
+  POSE_UNROLL for (int k = 0; k < 3; k++) {
+    out->camera_t[k] = tc.v[k];
+    out->robot_t[k] = tr.v[k];
+  }
+  const double n = 4.0 * ntags;
+  out->rms = sqrt(cost / n);
+  out->rms_other = cost_other < HUGE_VAL ? sqrt(cost_other / n) : HUGE_VAL;
+}
+
+// The solve over `ntags` used tags (ntags >= 1).  cost(R, t) returns the reduced seed score, sum(R, t, S) the reduced
+// sums of field_refine.  Seeds are scored in tag order, candidate 0 before 1, and the first best wins; with one tag
+// both candidates are refined, the lower cost returned (candidate 0 on a tie) and the other reported in rms_other.
+template <class CostFn, class SumFn>
+POSE_HD void field_solve(const FieldTagData *tags, int ntags, CostFn &cost, SumFn &sum, const double *rotation,
+                         const double *offset, b200tag_field_pose *out) {
+  if (ntags == 1) {
+    M3 R0 = tags[0].R[0], R1 = tags[0].R[1];
+    V3 t0 = tags[0].t[0], t1 = tags[0].t[1];
+    int it0 = 0, it1 = 0;
+    const double c0 = field_refine(sum, &R0, &t0, &it0);
+    const double c1 = field_refine(sum, &R1, &t1, &it1);
+    if (c1 < c0) field_result(R1, t1, c1, c0, 1, it1, rotation, offset, out);
+    else field_result(R0, t0, c0, c1, 1, it0, rotation, offset, out);
+    return;
+  }
+  int best = 0;
+  double best_cost = HUGE_VAL;
+  for (int s = 0; s < 2 * ntags; s++) {
+    const double c = cost(tags[s >> 1].R[s & 1], tags[s >> 1].t[s & 1]);
+    if (c < best_cost) {
+      best_cost = c;
+      best = s;
+    }
+  }
+  M3 R = tags[best >> 1].R[best & 1];
+  V3 t = tags[best >> 1].t[best & 1];
+  int it = 0;
+  const double c = field_refine(sum, &R, &t, &it);
+  field_result(R, t, c, HUGE_VAL, ntags, it, rotation, offset, out);
+}
+
 }  // namespace pose
 
 // Host, pose.cc: the node's records from poses already estimated (robot frame, distance, closest first), the step
 // b200tag_locate_tags and b200tag_tag_positions share.  poses[i] belongs to dets[i].
 void locate_from_poses(const b200tag_detection *dets, const b200tag_pose *poses, int count, const double *rotation,
                        const double *offset, b200tag_tag_position *out);
+
+// Host, pose.cc: the checks of b200tag_estimate_field_pose on a layout, plus, when `ncodes` is given, family < nfamilies
+// and id < ncodes[family].  On success fills `keys` (nlayout entries, sorted) and returns true.
+bool field_layout_keys(const b200tag_field_tag *layout, int nlayout, const uint32_t *ncodes, int nfamilies, pose::FieldKey *keys);
 
 }  // namespace b200tag
 

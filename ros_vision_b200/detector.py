@@ -83,6 +83,10 @@ POSE_DT = np.dtype([("R", "<f8", (3, 3)), ("t", "<f8", (3,)), ("err", "<f8"), ("
 TAG_POSITION_DT = np.dtype([("index", "<i4"), ("id", "<i4"), ("camera", "<f8", (3,)), ("robot", "<f8", (3,)),
                             ("distance", "<f8"), ("err", "<f8")])  # b200tag_tag_position
 POSE_METHODS = {"oi": 0, "ippe": 1}  # B200TAG_POSE_ORTHOGONAL_ITERATION, B200TAG_POSE_IPPE
+FIELD_TAG_DT = np.dtype([("family", "<i4"), ("id", "<i4"), ("R", "<f8", (3, 3)), ("t", "<f8", (3,))])  # b200tag_field_tag
+FIELD_POSE_DT = np.dtype([("num_tags", "<i4"), ("iterations", "<i4"), ("reserved", "<i4", (2,)), ("camera_R", "<f8", (3, 3)),
+                          ("camera_t", "<f8", (3,)), ("robot_R", "<f8", (3, 3)), ("robot_t", "<f8", (3,)), ("rms", "<f8"),
+                          ("rms_other", "<f8")])  # b200tag_field_pose
 
 _lib = None
 
@@ -155,6 +159,11 @@ def load_library():
     L.b200tag_estimate_poses_ippe.argtypes = [vp, i32] + [C.c_double] * 5 + [vp]
     L.b200tag_debug_estimate_poses_ippe_device.argtypes = [vp, i32] + [C.c_double] * 5 + [vp]
     L.b200tag_set_pose_method.argtypes = [vp, i32]
+    L.b200tag_estimate_field_pose.argtypes = [vp, i32, vp, i32] + [C.c_double] * 5 + [vp, vp, vp]
+    L.b200tag_debug_estimate_field_pose_device.argtypes = [vp, i32, vp, i32] + [C.c_double] * 5 + [vp, vp, vp]
+    L.b200tag_set_field_layout.argtypes = [vp, vp, i32]
+    L.b200tag_field_pose_get.argtypes = [vp, i32]
+    L.b200tag_field_pose_get.restype = vp
     L.b200tag_version.restype = i32
     _lib = L
     return L
@@ -236,6 +245,37 @@ def estimate_poses_device(detections: np.ndarray, tagsize: float, fx: float, fy:
     if rc:
         raise B200TagError(f"{fn}: {lib.b200tag_error_string(rc).decode()}")
     return out
+
+
+def _field_call(fn, detections, layout, tagsize, fx, fy, cx, cy, rotation, offset) -> np.ndarray:
+    lib = load_library()
+    dets = np.ascontiguousarray(detections, dtype=DETECTION_DT)
+    lay = np.ascontiguousarray(np.zeros(0, dtype=FIELD_TAG_DT) if layout is None else layout, dtype=FIELD_TAG_DT)
+    rot = None if rotation is None else np.ascontiguousarray(rotation, dtype=np.float64).reshape(9)
+    off = None if offset is None else np.ascontiguousarray(offset, dtype=np.float64).reshape(3)
+    out = np.zeros(1, dtype=FIELD_POSE_DT)
+    rc = getattr(lib, fn)(dets.ctypes.data_as(C.c_void_p) if len(dets) else None, len(dets),
+                          lay.ctypes.data_as(C.c_void_p) if len(lay) else None, len(lay), float(tagsize), float(fx),
+                          float(fy), float(cx), float(cy), None if rot is None else rot.ctypes.data_as(C.c_void_p),
+                          None if off is None else off.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p))
+    if rc:
+        raise B200TagError(f"{fn}: {lib.b200tag_error_string(rc).decode()}")
+    return out[0]
+
+
+def estimate_field_pose(detections: np.ndarray, layout: np.ndarray, tagsize: float, fx: float, fy: float, cx: float,
+                        cy: float, rotation=None, offset=None) -> np.ndarray:
+    """One camera (and robot) pose in the field from every detection of a layout tag (b200tag_estimate_field_pose): a
+    FIELD_POSE_DT record.  `layout` holds FIELD_TAG_DT records (X_field = R X_tag + t); `detections` may be reconciled
+    or raw.  rotation / offset are the camera's extrinsics, as for locate_tags.  Pure host math in libb200tag.so."""
+    return _field_call("b200tag_estimate_field_pose", detections, layout, tagsize, fx, fy, cx, cy, rotation, offset)
+
+
+def estimate_field_pose_device(detections: np.ndarray, layout: np.ndarray, tagsize: float, fx: float, fy: float,
+                               cx: float, cy: float, rotation=None, offset=None) -> np.ndarray:
+    """Test hook: estimate_field_pose computed by the device kernel GpuDetector.SetFieldLayout enables."""
+    return _field_call("b200tag_debug_estimate_field_pose_device", detections, layout, tagsize, fx, fy, cx, cy, rotation,
+                       offset)
 
 
 def _records(ptr, n, dtype) -> np.ndarray:
@@ -463,6 +503,20 @@ class GpuDetector:
         """TAG_POSITION_DT records of frame `frame`, closest first, as locate_tags(Detections(frame), ...) returns them."""
         n = C.c_int()
         return _records(self._lib.b200tag_tag_positions(self._h, frame, C.byref(n)), n.value, TAG_POSITION_DT)
+
+    def SetFieldLayout(self, layout) -> None:
+        """From the next Detect on, while the pose step is on, one field pose per frame from every visible tag of
+        `layout` (FIELD_TAG_DT records, e.g. field_layout.from_wpilib), with SetPoseEstimation's tagsize, intrinsics and
+        extrinsics (FieldPose).  None or an empty layout turns it off."""
+        lay = np.ascontiguousarray(np.zeros(0, dtype=FIELD_TAG_DT) if layout is None else layout, dtype=FIELD_TAG_DT)
+        self._check(self._lib.b200tag_set_field_layout(self._h, lay.ctypes.data_as(C.c_void_p) if len(lay) else None,
+                                                       len(lay)), "b200tag_set_field_layout")
+
+    def FieldPose(self, frame: int = 0):
+        """The FIELD_POSE_DT record of frame `frame`, as estimate_field_pose(Detections(frame), ...) returns it; None when
+        the last call ran without the field step."""
+        p = self._lib.b200tag_field_pose_get(self._h, frame)
+        return None if not p else _records(p, 1, FIELD_POSE_DT)[0]
 
     def ReinitializeDetections(self) -> None:
         """apriltag_gpu.cu:202-220 frees and re-creates the zarray; results here are plain arrays."""

@@ -211,6 +211,39 @@ def make_scene(width: int, height: int, seed: int, n_tags: int, side_range=(60.0
     return Scene(gray, tags)
 
 
+def field_scene(width: int, height: int, layout, tagsize: float, camera_R, camera_t, fx: float, fy: float, cx: float,
+                cy: float, seed: int, noise_sigma: float = 2.0, family: str = "tag36h11", background: float = 128.0,
+                white: float = 230.0, black: float = 25.0, ss: int = 4) -> Scene:
+    """A gray frame of the tags of a field layout (detector.FIELD_TAG_DT records, X_field = R X_tag + t) seen by a
+    pinhole camera placed in the field by X_field = camera_R X_cam + camera_t.  Each tag's black-border corners are
+    projected; the tags lying fully in front of the camera and inside the frame are rendered, farthest first.  TagPose
+    corners (-1,-1), (1,-1), (1,1), (-1,1) are the tag points (-s,-s), (s,-s), (s,s), (-s,s), s = tagsize / 2.  Returns the
+    Scene: the frame and the rendered tags with their true corners."""
+    rng = np.random.default_rng(seed)
+    Rc = np.asarray(camera_R, dtype=np.float64).reshape(3, 3)
+    tc = np.asarray(camera_t, dtype=np.float64).reshape(3)
+    s = tagsize / 2.0
+    P = np.array([[-s, -s, 0.0], [s, -s, 0.0], [s, s, 0.0], [-s, s, 0.0]])
+    visible = []
+    for rec in np.asarray(layout):
+        X = P @ np.asarray(rec["R"], dtype=np.float64).reshape(3, 3).T + np.asarray(rec["t"], dtype=np.float64)
+        cam = (X - tc) @ Rc  # Rc^T (X - tc), row by row
+        if not (cam[:, 2] > 1e-6).all():
+            continue
+        px = np.stack([fx * cam[:, 0] / cam[:, 2] + cx, fy * cam[:, 1] / cam[:, 2] + cy], axis=1)
+        if (px[:, 0] < 0).any() or (px[:, 0] > width).any() or (px[:, 1] < 0).any() or (px[:, 1] > height).any():
+            continue
+        visible.append((float(cam[:, 2].mean()), TagPose(int(rec["id"]), px, family)))
+    img = np.full((height, width), float(background), dtype=np.float64)
+    visible.sort(key=lambda v: -v[0])
+    for _, pose in visible:
+        render_tag(img, pose, white, black, ss)
+    if noise_sigma > 0:
+        img = img + rng.normal(0.0, noise_sigma, size=img.shape)
+    gray = np.clip(np.floor(img + 0.5), 0, 255).astype(np.uint8)
+    return Scene(gray, [v[1] for v in visible])
+
+
 # --- frame format packers -------------------------------------------------
 
 def gray_to_yuyv(gray: np.ndarray) -> np.ndarray:

@@ -11,6 +11,14 @@ synth.config_frame(2, i), 1280x800 YUYV, 1-6 tags per frame), in one run on one 
 host leg times estimate_poses(..., method="ippe") against estimate_poses with the default method on the same
 detections.
 
+--field measures the field pose step (GpuDetector.SetFieldLayout, the `field_pose` kernel) on top of IPPE:
+  * frames/s of 128-frame batches and single-frame p50 for three arms alternating in the same run: pose off, IPPE on,
+    IPPE + field (a layout holding every tag36h11 id, so every detection takes part);
+  * the `field_pose` kernel's device time per 128-frame batch on two workloads: config-2 frames with that all-ids
+    layout (geometry that fits no frame, so Levenberg-Marquardt runs to its cap: the worst case), and synth.field_scene
+    frames of one 6-tag layout seen from 16 robot poses (consistent geometry);
+  * the host estimate_field_pose per field_scene frame on one CPU core.
+
 Prints one JSON record, and writes it to --out when given.  Needs a CUDA device."""
 import argparse
 import json
@@ -46,8 +54,11 @@ def main():
     ap.add_argument("--steps", type=int, default=40, help="128-frame batches per throughput measurement")
     ap.add_argument("--latency-iters", type=int, default=400, help="single frames per latency measurement")
     ap.add_argument("--method", choices=("oi", "ippe"), default="oi", help="pose method of the device step")
+    ap.add_argument("--field", action="store_true", help="measure the field pose step (IPPE + SetFieldLayout)")
     ap.add_argument("--out", help="also write the JSON to this file (e.g. profiles/pose_r03.json)")
     args = ap.parse_args()
+    if args.field:
+        return field_main(args)
 
     import torch
     from ros_vision_b200 import detector as D, synth
@@ -167,6 +178,165 @@ def main():
             json.dump(res, f, indent=1)
     print(json.dumps(res, indent=1))
     for d in list(big.values()) + list(one.values()):
+        d.close()
+    for pb in pins:
+        pb.close()
+
+
+def all_ids_layout(D, seed=1):
+    """Every tag36h11 id at a random field pose."""
+    from ros_vision_b200.field_layout import quaternion_matrix
+    rng = np.random.default_rng(seed)
+    lay = np.zeros(587, dtype=D.FIELD_TAG_DT)
+    lay["id"] = np.arange(587)
+    for i in range(587):
+        lay["R"][i] = quaternion_matrix(*rng.normal(size=4))
+        lay["t"][i] = rng.uniform(-8, 8, size=3)
+    return lay
+
+
+def field_frames(D, synth, n):
+    """One layout of 6 tags 1.5-4 m in front of a nominal robot pose, and `n` field_scene frames (YUYV) from robot poses
+    within 0.3 m / 5 deg of it."""
+    rng = np.random.default_rng(6)
+    R0 = np.array(ROTATION, dtype=np.float64)
+    lay = np.zeros(6, dtype=D.FIELD_TAG_DT)
+    lay["id"] = rng.choice(587, 6, replace=False)
+    for j in range(6):
+        z = rng.uniform(1.5, 4.0)
+        a = rng.uniform(-0.4, 0.4, size=3)
+        Rx = np.array([[1, 0, 0], [0, np.cos(a[0]), -np.sin(a[0])], [0, np.sin(a[0]), np.cos(a[0])]])
+        Ry = np.array([[np.cos(a[1]), 0, np.sin(a[1])], [0, 1, 0], [-np.sin(a[1]), 0, np.cos(a[1])]])
+        lay["R"][j] = R0 @ Ry @ Rx
+        lay["t"][j] = R0 @ np.array([rng.uniform(-0.3, 0.3) * z, rng.uniform(-0.2, 0.2) * z, z]) + [0, 0, 0.6]
+    frames = []
+    for i in range(n):
+        yaw = np.radians(rng.uniform(-5, 5))
+        Rz = np.array([[np.cos(yaw), -np.sin(yaw), 0], [np.sin(yaw), np.cos(yaw), 0], [0, 0, 1]])
+        t = np.array([rng.uniform(-0.3, 0.3), rng.uniform(-0.3, 0.3), 0.6])
+        sc = synth.field_scene(1280, 800, lay, TAGSIZE, Rz @ R0, t, FX, FY, CX, CY, seed=i, noise_sigma=4.0)
+        frames.append(np.ascontiguousarray(synth.gray_to_yuyv(sc.gray)).reshape(-1))
+    return lay, frames
+
+
+def field_main(args):
+    import torch
+    from ros_vision_b200 import detector as D, synth
+    arms = ("pose_off", "ippe", "ippe_field")
+    lay_all = all_ids_layout(D)
+    frames = [np.ascontiguousarray(synth.config_frame(2, i)[0]).reshape(-1) for i in range(UNIQUE)]
+    dev_batch = torch.from_numpy(np.stack([frames[i % UNIQUE] for i in range(BATCH)])).cuda()
+    ptr = dev_batch.data_ptr()
+    fs_lay, fs_frames = field_frames(D, synth, UNIQUE)
+    fs_batch = torch.from_numpy(np.stack([fs_frames[i % UNIQUE] for i in range(BATCH)])).cuda()
+
+    def detector(arm, max_batch, lay=lay_all):
+        d = D.GpuDetector(1280, 800, "yuyv", quad_decimate=2, max_batch=max_batch)
+        if arm != "pose_off":
+            d.SetPoseEstimation(TAGSIZE, FX, FY, CX, CY, rotation=ROTATION, offset=OFFSET, method="ippe")
+        if arm == "ippe_field":
+            d.SetFieldLayout(lay)
+        return d
+
+    big = {a: detector(a, BATCH) for a in arms}
+    for d in big.values():
+        for _ in range(5):
+            d.DetectDevice(ptr, BATCH)
+    fps = {a: [] for a in arms}
+    for _ in range(args.rounds):
+        for a in arms:
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            for _ in range(args.steps):
+                big[a].DetectDevice(ptr, BATCH)
+            fps[a].append(BATCH * args.steps / (time.perf_counter() - t0))
+    kpb = {a: big[a].kernels_per_batch() for a in arms}
+    raw_per_batch = sum(int(big["ippe_field"].FrameInfo(f).num_detections) for f in range(BATCH))
+    used_cfg2 = [int(big["ippe_field"].FieldPose(f)["num_tags"]) for f in range(BATCH)]
+    iters_cfg2 = [int(big["ippe_field"].FieldPose(f)["iterations"]) for f in range(BATCH)]
+
+    def kernel_ms(det, p):
+        prof = det.ProfileDevice(p, BATCH, iters=20)
+        return [ms for name, ms in prof if name == "field_pose"][0]
+
+    worst_ms = kernel_ms(big["ippe_field"], ptr)
+    fs_det = detector("ippe_field", BATCH, fs_lay)
+    fs_det.DetectDevice(fs_batch.data_ptr(), BATCH)
+    fs_used = [int(fs_det.FieldPose(f)["num_tags"]) for f in range(BATCH)]
+    fs_iters = [int(fs_det.FieldPose(f)["iterations"]) for f in range(BATCH)]
+    fs_ms = kernel_ms(fs_det, fs_batch.data_ptr())
+
+    # single-frame latency from a pinned host frame, the three arms in rotating order
+    one = {a: detector(a, 1) for a in arms}
+    pins = []
+    for f in frames:
+        pb = D.PinnedBuffer(f.size)
+        pb.array[:] = f
+        pins.append(pb)
+    for d in one.values():
+        for pb in pins:
+            d.DetectPointers([pb.ptr])
+    lat = {a: [] for a in arms}
+    for i in range(args.latency_iters):
+        pb = pins[i % UNIQUE]
+        for k in range(3):
+            a = arms[(i + k) % 3]
+            t0 = time.perf_counter()
+            one[a].DetectPointers([pb.ptr])
+            lat[a].append((time.perf_counter() - t0) * 1e6)
+
+    # the host solve on the field_scene frames' detections, one core: the median of 20 calls per frame
+    fs_one = detector("ippe", 1)
+    per_frame = []
+    for f in fs_frames:
+        fs_one.Detect(f)
+        per_frame.append(fs_one.Detections(0))
+    cpu = sorted(os.sched_getaffinity(0))[0]
+    saved = os.sched_getaffinity(0)
+    host_us = []
+    os.sched_setaffinity(0, {cpu})
+    try:
+        for dets in per_frame:
+            reps = []
+            for _ in range(21):
+                t0 = time.perf_counter()
+                D.estimate_field_pose(dets, fs_lay, TAGSIZE, FX, FY, CX, CY, ROTATION, OFFSET)
+                reps.append((time.perf_counter() - t0) * 1e6)
+            host_us.append(float(np.median(reps[1:])))
+    finally:
+        os.sched_setaffinity(0, saved)
+
+    med = {a: float(np.median(fps[a])) for a in arms}
+    p50 = {a: float(np.percentile(lat[a], 50)) for a in arms}
+    ratio = med["ippe_field"] / med["pose_off"]
+    res = {
+        "mode": "field",
+        "gpu": gpu_identity(),
+        "torch_device": torch.cuda.get_device_name(0),
+        "workload": "config2: 1280x800 YUYV, synth.config_frame(2, 0..15) tiled to 128-frame batches, tag36h11, decimate 2; "
+                    "field arm: layout with all 587 tag36h11 ids at random field poses",
+        "batch_frames_per_s": {"rounds": fps, "median": med, "ratio_ippe_field_over_off": ratio,
+                               "ratio_ippe_field_over_ippe": med["ippe_field"] / med["ippe"]},
+        "kernels_per_batch": kpb,
+        "single_frame_latency_us": {"p50": p50, "p90": {a: float(np.percentile(lat[a], 90)) for a in arms},
+                                    "iters": args.latency_iters},
+        "field_pose_kernel_ms_per_batch": {
+            "config2_all_ids_layout": worst_ms, "config2_raw_detections_per_batch": raw_per_batch,
+            "config2_tags_used_per_batch": sum(used_cfg2), "config2_max_iterations": max(iters_cfg2),
+            "field_scene": fs_ms, "field_scene_tags_used_per_batch": sum(fs_used),
+            "field_scene_iterations_median": float(np.median(fs_iters))},
+        "host_estimate_field_pose_us_per_frame": {"per_frame": host_us, "median": float(np.median(host_us)),
+                                                  "tags": [int(len(d)) for d in per_frame], "cpu": cpu},
+        "targets": {"batch_ratio_at_least_0.95": bool(ratio >= 0.95),
+                    "p50_field_at_most_p50_ippe_plus_40us": bool(p50["ippe_field"] <= p50["ippe"] + 40),
+                    "field_kernel_worst_at_most_0.1ms_per_batch": bool(worst_ms <= 0.1)},
+    }
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            json.dump(res, f, indent=1)
+    print(json.dumps(res, indent=1))
+    for d in list(big.values()) + list(one.values()) + [fs_det, fs_one]:
         d.close()
     for pb in pins:
         pb.close()
