@@ -413,6 +413,55 @@ int b200tag_debug_estimate_field_pose_device(const b200tag_detection *dets, int 
                                              int nlayout, double tagsize, double fx, double fy, double cx, double cy,
                                              const double *rotation, const double *offset, b200tag_field_pose *out);
 
+/* Lens distortion in the pose step.  The functions above assume a pinhole camera, but detection corners (p, c, H) are
+ * in raw, distorted pixels: the decoder undistorts its edge samples and re-distorts the refined corners.  These
+ * variants first map each corner to the ideal pinhole image through the exact inverse of the 5-coefficient
+ * Brown-Conrady model of OpenCV's projectPoints (and of the decoder's re-distortion), `dist` = {k1, k2, p1, p2, k3}:
+ *   x' = x (1 + k1 r^2 + k2 r^4 + k3 r^6) + 2 p1 x y + p2 (r^2 + 2 x^2),
+ *   y' = y (1 + k1 r^2 + k2 r^4 + k3 r^6) + p1 (r^2 + 2 y^2) + 2 p2 x y,
+ * in normalised coordinates ((u - cx) / fx, (v - cy) / fy).  This is not b200tag_undistort, the reference's UnDistort,
+ * whose tangential term inverts that model only when p2 = 0.  The inverse is Newton's method from the distorted point,
+ * stopped after a step of at most 1e-14 (normalised) in both coordinates; a point fails when that takes more than 20
+ * steps, when the Jacobian's determinant is not positive at some step (past the fold of a strong barrel model), or when
+ * the result re-distorts more than 1e-9 (normalised) away from the input.  Only + - * / and fabs, so host and device
+ * results are bit-identical.
+ *
+ * dist == NULL or all five coefficients zero means no undistortion step at all: results are bit-identical to the
+ * functions without distortion.  A non-finite coefficient gives B200TAG_E_INVALID. */
+
+/* out[i] = the ideal pixel seen at distorted pixel in[i] (in == out is allowed); NaN, NaN for a point that fails.  With
+ * no distortion, out = in. */
+int b200tag_undistort_points(const double (*in)[2], int n, double fx, double fy, double cx, double cy, const double *dist,
+                             double (*out)[2]);
+/* b200tag_estimate_poses (method B200TAG_POSE_ORTHOGONAL_ITERATION) or b200tag_estimate_poses_ippe
+ * (B200TAG_POSE_IPPE) on the undistorted detections: IPPE reads the undistorted corners; OI also reads H, rebuilt from
+ * them (H maps the tag's (-1, 1), (1, 1), (1, -1), (-1, -1) to p[0..3], c = H (0, 0)).  A detection with a corner that
+ * fails, and for OI one whose undistorted corners have no homography, gets R = I, t = 0, err = err_other = HUGE_VAL.
+ * B200TAG_E_INVALID for another method and as the functions without distortion. */
+int b200tag_estimate_poses_distorted(const b200tag_detection *dets, int count, int method, double tagsize, double fx,
+                                     double fy, double cx, double cy, const double *dist, b200tag_pose *out);
+/* b200tag_estimate_field_pose with distortion.  The detections are selected on their raw records as without it; then
+ * the chosen detection's corners are undistorted, and a tag with a corner that fails is left out.  The solve minimises
+ * the pixel error in the ideal (undistorted) image, and rms / rms_other are measured there. */
+int b200tag_estimate_field_pose_distorted(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
+                                          int nlayout, double tagsize, double fx, double fy, double cx, double cy,
+                                          const double *dist, const double *rotation, const double *offset,
+                                          b200tag_field_pose *out);
+/* The device pose step (both methods) and field pose step use these coefficients from the next detect call, as the
+ * functions above do; NULL or all zero turns the correction off.  Independent of b200tag_set_pose_estimation and
+ * b200tag_set_pose_method.  Adds no kernel.  B200TAG_E_INVALID (state unchanged) for a non-finite coefficient. */
+int b200tag_set_pose_distortion(b200tag_detector *det, const double *dist);
+/* Test hooks: the device kernels on caller-supplied records, with distortion; arguments and results as
+ * b200tag_estimate_poses_distorted and b200tag_estimate_field_pose_distorted. */
+int b200tag_debug_estimate_poses_distorted_device(int method, const b200tag_detection *dets, int count, double tagsize,
+                                                  double fx, double fy, double cx, double cy, const double *dist,
+                                                  b200tag_pose *out);
+int b200tag_debug_estimate_field_pose_distorted_device(const b200tag_detection *dets, int count,
+                                                       const b200tag_field_tag *layout, int nlayout, double tagsize,
+                                                       double fx, double fy, double cx, double cy, const double *dist,
+                                                       const double *rotation, const double *offset,
+                                                       b200tag_field_pose *out);
+
 /* Pinned host staging memory, so b200tag_detect* can overlap H2D with compute. */
 void *b200tag_alloc_pinned(size_t bytes);
 /* Write-combined pinned memory: for buffers the CPU (or a capture driver) only ever WRITES, such as a camera ring

@@ -122,6 +122,7 @@ struct b200tag_detector {
     double tagsize = 0, fx = 0, fy = 0, cx = 0, cy = 0;
     double rotation[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, offset[3] = {0, 0, 0};
     int method = B200TAG_POSE_ORTHOGONAL_ITERATION;  // b200tag_set_pose_method
+    double dist[5] = {0, 0, 0, 0, 0};                 // b200tag_set_pose_distortion; all zero: none
   };
   PoseSettings pose, last_pose;                // current; what the last enqueue ran with
   b200tag_pose *h_poses = nullptr;             // pinned + mapped, parallel to h_dets; allocated when first turned on
@@ -396,15 +397,17 @@ int record_sequence(b200tag_detector *det, const void *device_images, size_t str
   launch_decode(p, count, ln);
   if (det->pose.tagsize > 0) {
     const auto &ps = det->pose;
-    const PoseLaunch pl{det->d_dets_alias, det->d_poses_alias, p.counters, p.det_cap, 0, ps.tagsize, ps.fx, ps.fy, ps.cx, ps.cy,
-                        ps.method};
+    PoseLaunch pl{det->d_dets_alias, det->d_poses_alias, p.counters, p.det_cap, 0, ps.tagsize, ps.fx, ps.fy, ps.cx, ps.cy,
+                  ps.method, {}};
+    memcpy(pl.dist, ps.dist, sizeof(pl.dist));
     launch_pose(pl, count, ln);
     if (det->field_n > 0) {
       FieldLaunch fl{det->d_dets_alias, p.counters, p.det_cap, 0, det->d_field_layout, det->d_field_keys, det->field_n,
                      static_cast<pose::FieldTagData *>(det->d_field_scratch), det->field_scratch_stride,
-                     ps.tagsize, ps.fx, ps.fy, ps.cx, ps.cy, {}, {}, det->d_field_alias};
+                     ps.tagsize, ps.fx, ps.fy, ps.cx, ps.cy, {}, {}, det->d_field_alias, {}};
       memcpy(fl.rotation, ps.rotation, sizeof(fl.rotation));
       memcpy(fl.offset, ps.offset, sizeof(fl.offset));
+      memcpy(fl.dist, ps.dist, sizeof(fl.dist));
       launch_field_pose(fl, count, ln);
     }
   }
@@ -1468,6 +1471,17 @@ int b200tag_set_pose_method(b200tag_detector *det, int method) {
   return 0;
 }
 
+int b200tag_set_pose_distortion(b200tag_detector *det, const double *dist) {
+  bool active;
+  pose::Distortion D;
+  if (!det || !read_distortion(dist, &active, &D)) return B200TAG_E_INVALID;
+  DeviceGuard on_device(det->device);
+  drop_graphs(det);  // the kernel variant and the coefficients are baked into the captured launches
+  const double c[5] = {D.k1, D.k2, D.p1, D.p2, D.k3};
+  memcpy(det->pose.dist, c, sizeof(c));
+  return 0;
+}
+
 int b200tag_set_distortion(b200tag_detector *det, double k1, double k2, double p1, double p2, double k3) {
   if (!det) return B200TAG_E_INVALID;
   DeviceGuard on_device(det->device);
@@ -1552,8 +1566,12 @@ namespace {
 
 // The test hooks' common part: the pose kernel of `method` on caller records, through device copies of them.
 int estimate_poses_device(int method, const b200tag_detection *dets, int count, double tagsize, double fx, double fy,
-                          double cx, double cy, b200tag_pose *out) {
+                          double cx, double cy, const double *dist, b200tag_pose *out) {
+  bool active;
+  pose::Distortion D;
   if (count < 0 || (count > 0 && (!dets || !out)) || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
+  if ((method != B200TAG_POSE_ORTHOGONAL_ITERATION && method != B200TAG_POSE_IPPE) || !read_distortion(dist, &active, &D))
+    return B200TAG_E_INVALID;
   if (count == 0) return 0;
   const size_t db = sizeof(b200tag_detection) * static_cast<size_t>(count), pb = sizeof(b200tag_pose) * static_cast<size_t>(count);
   uint8_t *d = nullptr;
@@ -1563,7 +1581,7 @@ int estimate_poses_device(int method, const b200tag_detection *dets, int count, 
   }
   int rc = 0;
   const PoseLaunch pl{reinterpret_cast<const b200tag_detection *>(d), reinterpret_cast<b200tag_pose *>(d + db), nullptr,
-                      0, static_cast<uint32_t>(count), tagsize, fx, fy, cx, cy, method};
+                      0, static_cast<uint32_t>(count), tagsize, fx, fy, cx, cy, method, {D.k1, D.k2, D.p1, D.p2, D.k3}};
   if (cudaMemcpy(d, dets, db, cudaMemcpyHostToDevice) != cudaSuccess) rc = B200TAG_E_CUDA;
   if (!rc) {
     Launcher ln{nullptr, nullptr};
@@ -1580,18 +1598,36 @@ extern "C" {
 
 int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count, double tagsize, double fx, double fy,
                                         double cx, double cy, b200tag_pose *out) {
-  return estimate_poses_device(B200TAG_POSE_ORTHOGONAL_ITERATION, dets, count, tagsize, fx, fy, cx, cy, out);
+  return estimate_poses_device(B200TAG_POSE_ORTHOGONAL_ITERATION, dets, count, tagsize, fx, fy, cx, cy, nullptr, out);
 }
 
 int b200tag_debug_estimate_poses_ippe_device(const b200tag_detection *dets, int count, double tagsize, double fx,
                                              double fy, double cx, double cy, b200tag_pose *out) {
-  return estimate_poses_device(B200TAG_POSE_IPPE, dets, count, tagsize, fx, fy, cx, cy, out);
+  return estimate_poses_device(B200TAG_POSE_IPPE, dets, count, tagsize, fx, fy, cx, cy, nullptr, out);
+}
+
+int b200tag_debug_estimate_poses_distorted_device(int method, const b200tag_detection *dets, int count, double tagsize,
+                                                  double fx, double fy, double cx, double cy, const double *dist,
+                                                  b200tag_pose *out) {
+  return estimate_poses_device(method, dets, count, tagsize, fx, fy, cx, cy, dist, out);
 }
 
 int b200tag_debug_estimate_field_pose_device(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
                                              int nlayout, double tagsize, double fx, double fy, double cx, double cy,
                                              const double *rotation, const double *offset, b200tag_field_pose *out) {
+  return b200tag_debug_estimate_field_pose_distorted_device(dets, count, layout, nlayout, tagsize, fx, fy, cx, cy, nullptr,
+                                                            rotation, offset, out);
+}
+
+int b200tag_debug_estimate_field_pose_distorted_device(const b200tag_detection *dets, int count,
+                                                       const b200tag_field_tag *layout, int nlayout, double tagsize,
+                                                       double fx, double fy, double cx, double cy, const double *dist,
+                                                       const double *rotation, const double *offset,
+                                                       b200tag_field_pose *out) {
+  bool active;
+  pose::Distortion D;
   if (count < 0 || (count > 0 && !dets) || !out || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
+  if (!read_distortion(dist, &active, &D)) return B200TAG_E_INVALID;
   std::vector<pose::FieldKey> keys(static_cast<size_t>(std::max(nlayout, 0)));
   if (!field_layout_keys(layout, nlayout, nullptr, 0, keys.data())) return B200TAG_E_INVALID;
   const size_t db = sizeof(b200tag_detection) * static_cast<size_t>(count), lb = sizeof(b200tag_field_tag) * nlayout,
@@ -1606,7 +1642,7 @@ int b200tag_debug_estimate_field_pose_device(const b200tag_detection *dets, int 
   FieldLaunch fl{reinterpret_cast<const b200tag_detection *>(d), nullptr, 0, static_cast<uint32_t>(count),
                  reinterpret_cast<const b200tag_field_tag *>(d + o_l), reinterpret_cast<const pose::FieldKey *>(d + o_k), nlayout,
                  reinterpret_cast<pose::FieldTagData *>(d + o_s), 0, tagsize, fx, fy, cx, cy, {}, {},
-                 reinterpret_cast<b200tag_field_pose *>(d + o_o)};
+                 reinterpret_cast<b200tag_field_pose *>(d + o_o), {D.k1, D.k2, D.p1, D.p2, D.k3}};
   memcpy(fl.rotation, rotation ? rotation : kEye, sizeof(fl.rotation));
   memcpy(fl.offset, offset ? offset : kZero, sizeof(fl.offset));
   int rc = 0;

@@ -87,6 +87,7 @@ struct PoseLaunch {
   uint32_t stride, count;
   double tagsize, fx, fy, cx, cy;
   int method;                     // B200TAG_POSE_*
+  double dist[5];                 // {k1, k2, p1, p2, k3} of b200tag_set_pose_distortion; all zero: no undistortion step
 };
 void launch_pose(const PoseLaunch &L, int frames, Launcher &ln);
 
@@ -107,8 +108,14 @@ struct FieldLaunch {
   double tagsize, fx, fy, cx, cy;
   double rotation[9], offset[3];
   b200tag_field_pose *out;           // one per frame
+  double dist[5];                    // as PoseLaunch::dist
 };
 void launch_field_pose(const FieldLaunch &L, int frames, Launcher &ln);
+// True when `dist` ({k1, k2, p1, p2, k3}) has a non-zero coefficient: the launches then choose the kernels' variants
+// with the undistortion step.
+inline bool has_distortion(const double *dist) {
+  return dist[0] != 0 || dist[1] != 0 || dist[2] != 0 || dist[3] != 0 || dist[4] != 0;
+}
 size_t field_tag_bytes();            // sizeof(pose::FieldTagData)
 
 // JPEG luminance planes of a batch (jpeg.h): the parallel kernels for streams without restart markers, the sequential

@@ -3,7 +3,9 @@
 // orthogonal iteration run on every lane with the same values, reading the per-detection constants from shared memory;
 // lane 0 sets up the frame of the second-minimum search there, and the lanes split that search's grid.  The arithmetic is
 // pose_core.h's, the same the host functions in pose.cc run.  With b200tag_set_pose_method(B200TAG_POSE_IPPE) the step
-// is k_pose_ippe instead: the closed-form IPPE pose, one thread per detection.
+// is k_pose_ippe instead: the closed-form IPPE pose, one thread per detection.  With b200tag_set_pose_distortion each
+// kernel's variant with kDistorted = true runs: it undistorts the corners first (pose_core.h's undistort_point); the
+// variant without compiles to the kernel without the step.
 //
 // A pose depends only on its own record, so computing it before the host's reconcile gives the pose of every
 // detection that survives it.
@@ -78,13 +80,37 @@ __device__ __noinline__ int search_second_minimum(const SecondMinFrame &S, int l
   return n_minima;
 }
 
-// b200tag_estimate_pose for one record, by one warp.
+__device__ Distortion lens(const double *dist) { return Distortion{dist[0], dist[1], dist[2], dist[3], dist[4]}; }
+
+__device__ void copy_pose_out(const PoseShared &sh, int lane, b200tag_pose *dst) {
+  static_assert(sizeof(b200tag_pose) % 8 == 0 && sizeof(b200tag_pose) / 8 <= 32, "pose copy");
+  if (lane < static_cast<int>(sizeof(b200tag_pose) / 8))
+    reinterpret_cast<double *>(dst)[lane] = reinterpret_cast<const double *>(&sh.out)[lane];
+  __syncwarp();  // sh is reused by this warp's next record
+}
+
+// b200tag_estimate_pose for one record, by one warp; with kDistorted, of the record undistort_record makes of it (lanes
+// 0-3 undistort a corner each, lane 0 rebuilds H), or pose_failure's record when that fails.
+template <bool kDistorted>
 __device__ void estimate_pose_warp(const b200tag_detection *rec, const PoseLaunch &L, PoseShared &sh, int lane, b200tag_pose *dst) {
   static_assert(sizeof(b200tag_detection) % 8 == 0 && sizeof(b200tag_detection) / 8 <= 32, "record copy");
-  static_assert(sizeof(b200tag_pose) % 8 == 0 && sizeof(b200tag_pose) / 8 <= 32, "pose copy");
   if (lane < static_cast<int>(sizeof(b200tag_detection) / 8))
     reinterpret_cast<double *>(&sh.det)[lane] = reinterpret_cast<const double *>(rec)[lane];
   __syncwarp();
+  if (kDistorted) {
+    int fine = 1;
+    if (lane < 4) fine = undistort_point(sh.det.p[lane], L.fx, L.fy, L.cx, L.cy, lens(L.dist), sh.det.p[lane]);
+    fine = __all_sync(kFull, fine);
+    __syncwarp();
+    if (lane == 0 && fine) fine = record_homography(&sh.det);
+    if (!__shfl_sync(kFull, fine, 0)) {
+      if (lane == 0) pose_failure(&sh.out);
+      __syncwarp();
+      copy_pose_out(sh, lane, dst);
+      return;
+    }
+    __syncwarp();
+  }
   int ok = 0;
   if (lane == 0) {
     V3 v[4], p[4];
@@ -117,12 +143,11 @@ __device__ void estimate_pose_warp(const b200tag_detection *rec, const PoseLaunc
   }
   if (lane == 0) choose_pose(sh.R1, sh.t1, sh.err1, R2, t2, err2, &sh.out);
   __syncwarp();
-  if (lane < static_cast<int>(sizeof(b200tag_pose) / 8))
-    reinterpret_cast<double *>(dst)[lane] = reinterpret_cast<const double *>(&sh.out)[lane];
-  __syncwarp();  // sh is reused by this warp's next record
+  copy_pose_out(sh, lane, dst);
 }
 
 // blockIdx.y = frame; the warps of a frame's CTAs walk that frame's detections, as many as its counter says.
+template <bool kDistorted>
 __global__ void __launch_bounds__(kPoseWarps * 32) k_pose(PoseLaunch L) {
   __shared__ PoseShared sh[kPoseWarps];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -131,7 +156,7 @@ __global__ void __launch_bounds__(kPoseWarps * 32) k_pose(PoseLaunch L) {
   const b200tag_detection *recs = L.dets + frame * L.stride;
   b200tag_pose *out = L.out + frame * L.stride;
   for (uint32_t i = blockIdx.x * kPoseWarps + w; i < n; i += gridDim.x * kPoseWarps)
-    estimate_pose_warp(recs + i, L, sh[w], lane, out + i);
+    estimate_pose_warp<kDistorted>(recs + i, L, sh[w], lane, out + i);
 }
 
 constexpr int kIppeThreads = 128;  // threads per CTA of k_pose_ippe
@@ -141,7 +166,9 @@ static_assert(sizeof(b200tag_pose) % 16 == 0, "pose stores");
 // The IPPE pose (B200TAG_POSE_IPPE) of every raw detection: one thread per record, blockIdx.y = frame, as many records
 // as the frame's counter holds.  A thread reads only the record's four corners from the mapped detection buffer and
 // writes the pose to the same index of the mapped pose buffer; the arithmetic is ippe_pose, which the host's
-// b200tag_estimate_poses_ippe runs too.
+// b200tag_estimate_poses_ippe runs too.  With kDistorted the thread undistorts the four corners first, one after the
+// other, as b200tag_estimate_poses_distorted does.
+template <bool kDistorted>
 __global__ void __launch_bounds__(kIppeThreads) k_pose_ippe(PoseLaunch L) {
   const size_t frame = blockIdx.y;
   const uint32_t n = L.counters ? min(L.counters[frame].num_detections, L.stride) : L.count;
@@ -157,7 +184,10 @@ __global__ void __launch_bounds__(kIppeThreads) k_pose_ippe(PoseLaunch L) {
       px[k][1] = c.y;
     }
     b200tag_pose pose;
-    ippe_pose(px, L.tagsize, L.fx, L.fy, L.cx, L.cy, &pose);
+    if (!kDistorted || undistort_corners(px, L.fx, L.fy, L.cx, L.cy, lens(L.dist), px))
+      ippe_pose(px, L.tagsize, L.fx, L.fy, L.cx, L.cy, &pose);
+    else
+      pose_failure(&pose);
     const double2 *from = reinterpret_cast<const double2 *>(&pose);
     double2 *dst = reinterpret_cast<double2 *>(out + i);
 #pragma unroll
@@ -176,7 +206,9 @@ __device__ double warp_sum(double v) {
 // raw records from the mapped detection buffer, as many as its counter holds.  The lanes look the records up in the
 // layout and keep, per layout tag, the record reconcile prefers; in layout order they write each used tag's corners and
 // seeds to the frame's scratch, and then run field_solve with correspondence k on lane k % 32 and the 6x6 solve on every
-// lane.  The arithmetic is pose_core.h's, the same b200tag_estimate_field_pose runs on the host.
+// lane.  The arithmetic is pose_core.h's, the same b200tag_estimate_field_pose runs on the host.  With kDistorted the
+// lane that owns a used layout tag undistorts its chosen record's corners first and leaves the tag out when one fails.
+template <bool kDistorted>
 __global__ void __launch_bounds__(32) k_field_pose(FieldLaunch L) {
   __shared__ int cnt[B200TAG_MAX_FIELD_TAGS], sel[B200TAG_MAX_FIELD_TAGS];
   __shared__ int dup;
@@ -228,7 +260,8 @@ __global__ void __launch_bounds__(32) k_field_pose(FieldLaunch L) {
         px[k][0] = c.x;
         px[k][1] = c.y;
       }
-      ok = field_tag_data(L.layout[li], px, L.tagsize, cam, &tags[used + __popc(hm & below)]);
+      ok = (!kDistorted || undistort_corners(px, L.fx, L.fy, L.cx, L.cy, lens(L.dist), px)) &&
+           field_tag_data(L.layout[li], px, L.tagsize, cam, &tags[used + __popc(hm & below)]);
     }
     const unsigned om = __ballot_sync(kFull, ok);
     __syncwarp();
@@ -279,15 +312,17 @@ __global__ void __launch_bounds__(32) k_field_pose(FieldLaunch L) {
 size_t field_tag_bytes() { return sizeof(FieldTagData); }
 
 void launch_field_pose(const FieldLaunch &L, int frames, Launcher &ln) {
-  ln.timed("field_pose", [&] { k_field_pose<<<static_cast<unsigned>(frames), 32, 0, ln.s>>>(L); });
+  const auto kernel = has_distortion(L.dist) ? k_field_pose<true> : k_field_pose<false>;
+  ln.timed("field_pose", [&] { kernel<<<static_cast<unsigned>(frames), 32, 0, ln.s>>>(L); });
 }
 
 void launch_pose(const PoseLaunch &L, int frames, Launcher &ln) {
   if (L.method == B200TAG_POSE_IPPE) {
     // one thread per record, all of a frame's records in one pass up to 1024 of them; CTAs past a frame's count exit
     const unsigned ctas = L.counters ? min((L.stride + kIppeThreads - 1) / kIppeThreads, 8u) : (L.count + kIppeThreads - 1) / kIppeThreads;
+    const auto kernel = has_distortion(L.dist) ? k_pose_ippe<true> : k_pose_ippe<false>;
     ln.timed("pose_ippe", [&] {
-      if (ctas > 0) k_pose_ippe<<<dim3(ctas, static_cast<unsigned>(frames)), kIppeThreads, 0, ln.s>>>(L);
+      if (ctas > 0) kernel<<<dim3(ctas, static_cast<unsigned>(frames)), kIppeThreads, 0, ln.s>>>(L);
     });
     return;
   }
@@ -295,8 +330,9 @@ void launch_pose(const PoseLaunch &L, int frames, Launcher &ln) {
   // path, a cluttered 4K scene has ~100 tags): 128 warps each, one pass.  A list without counters is one frame.
   unsigned ctas = static_cast<unsigned>(frames) <= 4 ? 32u : 2u;
   if (!L.counters) ctas = static_cast<unsigned>((L.count + kPoseWarps - 1) / kPoseWarps);
+  const auto kernel = has_distortion(L.dist) ? k_pose<true> : k_pose<false>;
   ln.timed("pose", [&] {
-    if (ctas > 0) k_pose<<<dim3(ctas, static_cast<unsigned>(frames)), kPoseWarps * 32, 0, ln.s>>>(L);
+    if (ctas > 0) kernel<<<dim3(ctas, static_cast<unsigned>(frames)), kPoseWarps * 32, 0, ln.s>>>(L);
   });
 }
 

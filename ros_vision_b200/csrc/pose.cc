@@ -52,6 +52,18 @@ bool field_layout_keys(const b200tag_field_tag *layout, int nlayout, const uint3
   return true;
 }
 
+bool read_distortion(const double *dist, bool *active, pose::Distortion *D) {
+  *active = false;
+  *D = pose::Distortion{0, 0, 0, 0, 0};
+  if (!dist) return true;
+  for (int k = 0; k < 5; k++) {
+    if (!std::isfinite(dist[k])) return false;
+    *active = *active || dist[k] != 0;
+  }
+  *D = pose::Distortion{dist[0], dist[1], dist[2], dist[3], dist[4]};
+  return true;
+}
+
 }  // namespace b200tag
 
 using namespace b200tag::pose;
@@ -132,9 +144,14 @@ int b200tag_locate_tags(const b200tag_detection *dets, int count, double tagsize
   return 0;
 }
 
-int b200tag_estimate_field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout,
-                                double tagsize, double fx, double fy, double cx, double cy, const double *rotation,
-                                const double *offset, b200tag_field_pose *out) {
+}  // extern "C"
+
+namespace {
+
+// b200tag_estimate_field_pose(_distorted); `lens` null: no undistortion step.
+int field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout, double tagsize,
+               double fx, double fy, double cx, double cy, const Distortion *lens, const double *rotation,
+               const double *offset, b200tag_field_pose *out) {
   if (count < 0 || (count > 0 && !dets) || !out || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
   std::vector<FieldKey> keys(static_cast<size_t>(std::max(nlayout, 0)));
   if (!b200tag::field_layout_keys(layout, nlayout, nullptr, 0, keys.data())) return B200TAG_E_INVALID;
@@ -149,8 +166,13 @@ int b200tag_estimate_field_pose(const b200tag_detection *dets, int count, const 
   const FieldCamera cam{fx, fy, cx, cy};
   std::vector<FieldTagData> tags;
   for (int L = 0; L < nlayout; L++) {
+    if (sel[L] < 0) continue;
+    // only the chosen record's corners are undistorted; one that fails leaves the tag out
+    double px[4][2];
+    if (!lens) memcpy(px, dets[sel[L]].p, sizeof(px));
+    else if (!undistort_corners(dets[sel[L]].p, fx, fy, cx, cy, *lens, px)) continue;
     FieldTagData d;
-    if (sel[L] >= 0 && field_tag_data(layout[L], dets[sel[L]].p, tagsize, cam, &d)) tags.push_back(d);
+    if (field_tag_data(layout[L], px, tagsize, cam, &d)) tags.push_back(d);
   }
   const int ntags = static_cast<int>(tags.size());
   if (ntags == 0) {
@@ -180,6 +202,68 @@ int b200tag_estimate_field_pose(const b200tag_detection *dets, int count, const 
   };
   field_solve(tags.data(), ntags, cost, sum, Rx, ox, out);
   return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int b200tag_estimate_field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout,
+                                double tagsize, double fx, double fy, double cx, double cy, const double *rotation,
+                                const double *offset, b200tag_field_pose *out) {
+  return field_pose(dets, count, layout, nlayout, tagsize, fx, fy, cx, cy, nullptr, rotation, offset, out);
+}
+
+int b200tag_undistort_points(const double (*in)[2], int n, double fx, double fy, double cx, double cy, const double *dist,
+                             double (*out)[2]) {
+  bool active;
+  Distortion D;
+  if (n < 0 || (n > 0 && (!in || !out)) || fx == 0 || fy == 0 || !b200tag::read_distortion(dist, &active, &D))
+    return B200TAG_E_INVALID;
+  for (int i = 0; i < n; i++) {
+    if (!active) {
+      out[i][0] = in[i][0];
+      out[i][1] = in[i][1];
+    } else if (!undistort_point(in[i], fx, fy, cx, cy, D, out[i])) {
+      out[i][0] = out[i][1] = NAN;
+    }
+  }
+  return 0;
+}
+
+int b200tag_estimate_poses_distorted(const b200tag_detection *dets, int count, int method, double tagsize, double fx,
+                                     double fy, double cx, double cy, const double *dist, b200tag_pose *out) {
+  bool active;
+  Distortion D;
+  if ((method != B200TAG_POSE_ORTHOGONAL_ITERATION && method != B200TAG_POSE_IPPE) || !b200tag::read_distortion(dist, &active, &D))
+    return B200TAG_E_INVALID;
+  const bool ippe = method == B200TAG_POSE_IPPE;
+  if (!active)
+    return ippe ? b200tag_estimate_poses_ippe(dets, count, tagsize, fx, fy, cx, cy, out)
+                : b200tag_estimate_poses(dets, count, tagsize, fx, fy, cx, cy, out);
+  if (count < 0 || (count > 0 && (!dets || !out))) return B200TAG_E_INVALID;
+  if (count > 0 && (!(tagsize > 0) || fx == 0 || fy == 0)) return B200TAG_E_INVALID;
+  for (int i = 0; i < count; i++) {
+    b200tag_detection rec = dets[i];
+    if (ippe) {
+      if (undistort_corners(rec.p, fx, fy, cx, cy, D, rec.p)) ippe_pose(rec.p, tagsize, fx, fy, cx, cy, out + i);
+      else pose_failure(out + i);
+    } else {
+      if (undistort_record(&rec, fx, fy, cx, cy, D)) b200tag_estimate_pose(&rec, tagsize, fx, fy, cx, cy, out + i);
+      else pose_failure(out + i);
+    }
+  }
+  return 0;
+}
+
+int b200tag_estimate_field_pose_distorted(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
+                                          int nlayout, double tagsize, double fx, double fy, double cx, double cy,
+                                          const double *dist, const double *rotation, const double *offset,
+                                          b200tag_field_pose *out) {
+  bool active;
+  Distortion D;
+  if (!b200tag::read_distortion(dist, &active, &D)) return B200TAG_E_INVALID;
+  return field_pose(dets, count, layout, nlayout, tagsize, fx, fy, cx, cy, active ? &D : nullptr, rotation, offset, out);
 }
 
 }  // extern "C"

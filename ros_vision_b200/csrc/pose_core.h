@@ -16,7 +16,8 @@
 //
 // The second method, IPPE (ippe_pose, at the end), is closed form and uses only + - * /, sqrt, fabs and fmax: its
 // poses are bit-identical on host and device.  So is the field pose (field_solve, at the end): the same operations, and
-// every sum over correspondences taken in one order on both sides.
+// every sum over correspondences taken in one order on both sides.  So is the exact inverse of the lens distortion model
+// (undistort_point, after IPPE) that corrects the detections' corners before either pose.
 #ifndef B200TAG_POSE_CORE_H_
 #define B200TAG_POSE_CORE_H_
 
@@ -500,9 +501,15 @@ POSE_HD bool ippe_candidates(const V3 *v, const V3 *p, double tagsize, M3 *R, V3
   return err[0] < HUGE_VAL && err[1] < HUGE_VAL;
 }
 
+// The record of a tag without a pose: R = I, t = 0 and both errors HUGE_VAL.
+POSE_HD void pose_failure(b200tag_pose *out) {
+  const M3 I = ident();
+  const V3 z{{0, 0, 0}};
+  choose_pose(I, z, HUGE_VAL, I, z, HUGE_VAL, out);
+}
+
 // IPPE pose of a tag whose corners are at image points px[0..3]: the candidate with the smaller object-space error,
-// the other's error in err_other.  A quad for which a candidate cannot be formed gives R = I, t = 0 and both errors
-// HUGE_VAL.
+// the other's error in err_other.  A quad for which a candidate cannot be formed gives pose_failure's record.
 POSE_HD void ippe_pose(const double (*px)[2], double tagsize, double fx, double fy, double cx, double cy, b200tag_pose *out) {
   V3 v[4], p[4];
   rays_and_corners(px, tagsize, fx, fy, cx, cy, v, p);
@@ -510,12 +517,90 @@ POSE_HD void ippe_pose(const double (*px)[2], double tagsize, double fx, double 
   V3 t[2];
   double err[2];
   if (!ippe_candidates(v, p, tagsize, R, t, err)) {
-    const M3 I = ident();
-    const V3 z{{0, 0, 0}};
-    choose_pose(I, z, HUGE_VAL, I, z, HUGE_VAL, out);
+    pose_failure(out);
     return;
   }
   choose_pose(R[0], t[0], err[0], R[1], t[1], err[1], out);
+}
+
+// ---- Lens distortion (b200tag_undistort_points, b200tag_set_pose_distortion) ----
+// The 5-coefficient Brown-Conrady model of OpenCV's projectPoints and of the decoder's redistort(): a pinhole point at
+// normalised (x, y) = ((u - cx) / fx, (v - cy) / fy) is seen at
+//   x' = x (1 + k1 r^2 + k2 r^4 + k3 r^6) + 2 p1 x y + p2 (r^2 + 2 x^2)
+//   y' = y (1 + k1 r^2 + k2 r^4 + k3 r^6) + p1 (r^2 + 2 y^2) + 2 p2 x y,   r^2 = x^2 + y^2.
+// The pose step inverts it exactly (not with the reference's UnDistort, whose tangential term differs when p2 != 0) by
+// Newton's method on the 2x2 system.  Only + - * / and fabs, so host and device agree bit for bit.
+
+struct Distortion {
+  double k1, k2, p1, p2, k3;
+};
+
+constexpr int kUndistortMaxIterations = 20;
+
+// The model at normalised (x, y): the distorted point and the Jacobian (symmetric, j01 = j10).
+POSE_HD void distort_normalised(const Distortion &D, double x, double y, double *xd, double *yd, double *j00, double *j01,
+                                double *j11) {
+  const double r2 = x * x + y * y;
+  const double radial = 1 + r2 * (D.k1 + r2 * (D.k2 + r2 * D.k3));
+  const double dr = 2 * (D.k1 + r2 * (2 * D.k2 + r2 * (3 * D.k3)));  // 2 d(radial)/d(r^2)
+  *xd = x * radial + 2 * D.p1 * x * y + D.p2 * (r2 + 2 * x * x);
+  *yd = y * radial + D.p1 * (r2 + 2 * y * y) + 2 * D.p2 * x * y;
+  *j00 = radial + x * x * dr + 2 * D.p1 * y + 6 * D.p2 * x;
+  *j01 = x * y * dr + 2 * D.p1 * x + 2 * D.p2 * y;
+  *j11 = radial + y * y * dr + 6 * D.p1 * y + 2 * D.p2 * x;
+}
+
+// The ideal pixel out[] seen at distorted pixel in[] (in == out is allowed).  Newton's method from the distorted point,
+// stopped after a step of at most 1e-14 in both normalised coordinates; false when that takes more than
+// kUndistortMaxIterations steps, when the Jacobian's determinant is not positive at some step (past the fold of a strong
+// barrel model, where the model is not invertible), or when the result re-distorts more than 1e-9 (normalised) away.
+POSE_HD bool undistort_point(const double *in, double fx, double fy, double cx, double cy, const Distortion &D, double *out) {
+  const double xd = (in[0] - cx) / fx, yd = (in[1] - cy) / fy;
+  double x = xd, y = yd, fxd, fyd, j00, j01, j11;
+  bool done = false;
+  for (int it = 0; it < kUndistortMaxIterations && !done; it++) {
+    distort_normalised(D, x, y, &fxd, &fyd, &j00, &j01, &j11);
+    const double det = j00 * j11 - j01 * j01;
+    if (!(det > 0)) return false;
+    const double ex = xd - fxd, ey = yd - fyd;
+    const double dx = (j11 * ex - j01 * ey) / det, dy = (j00 * ey - j01 * ex) / det;
+    x = x + dx;
+    y = y + dy;
+    done = fabs(dx) <= 1e-14 && fabs(dy) <= 1e-14;
+  }
+  if (!done) return false;
+  distort_normalised(D, x, y, &fxd, &fyd, &j00, &j01, &j11);
+  if (!(fabs(fxd - xd) <= 1e-9 && fabs(fyd - yd) <= 1e-9)) return false;
+  out[0] = fx * x + cx;
+  out[1] = fy * y + cy;
+  return true;
+}
+
+// undistort_point on four corners; false when any fails.
+POSE_HD bool undistort_corners(const double (*in)[2], double fx, double fy, double cx, double cy, const Distortion &D,
+                               double (*out)[2]) {
+  bool ok = true;
+  POSE_UNROLL for (int i = 0; i < 4; i++) ok = undistort_point(in[i], fx, fy, cx, cy, D, out[i]) && ok;
+  return ok;
+}
+
+// Rebuilds det->H and det->c from det->p in the decoder's convention: H maps the tag's (-1, 1), (1, 1), (1, -1),
+// (-1, -1) to p[0..3] (H22 = 1), c = H (0, 0).  False when the corners have no such homography.
+POSE_HD bool record_homography(b200tag_detection *det) {
+  V3 u[4];
+  POSE_UNROLL for (int i = 0; i < 4; i++) u[i] = V3{{det->p[i][0], det->p[i][1], 1}};
+  double H[9];
+  if (!square_homography(u, 1.0, H)) return false;
+  POSE_UNROLL for (int k = 0; k < 9; k++) det->H[k] = H[k];
+  det->c[0] = H[2];
+  det->c[1] = H[5];
+  return true;
+}
+
+// A detection as a pinhole camera would have recorded it: corners undistorted, H and c rebuilt from them.  False when a
+// corner cannot be undistorted or the corners have no homography.
+POSE_HD bool undistort_record(b200tag_detection *det, double fx, double fy, double cx, double cy, const Distortion &D) {
+  return undistort_corners(det->p, fx, fy, cx, cy, D, det->p) && record_homography(det);
 }
 
 // ---- Field pose (b200tag_estimate_field_pose, b200tag_set_field_layout) ----
@@ -809,6 +894,10 @@ void locate_from_poses(const b200tag_detection *dets, const b200tag_pose *poses,
 // Host, pose.cc: the checks of b200tag_estimate_field_pose on a layout, plus, when `ncodes` is given, family < nfamilies
 // and id < ncodes[family].  On success fills `keys` (nlayout entries, sorted) and returns true.
 bool field_layout_keys(const b200tag_field_tag *layout, int nlayout, const uint32_t *ncodes, int nfamilies, pose::FieldKey *keys);
+
+// Host, pose.cc: the check of a `dist` argument ({k1, k2, p1, p2, k3} or NULL): false when a coefficient is not finite.
+// *active is true when a coefficient is non-zero; only then is there an undistortion step, and *D holds the model.
+bool read_distortion(const double *dist, bool *active, pose::Distortion *D);
 
 }  // namespace b200tag
 

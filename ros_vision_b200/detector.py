@@ -164,6 +164,12 @@ def load_library():
     L.b200tag_set_field_layout.argtypes = [vp, vp, i32]
     L.b200tag_field_pose_get.argtypes = [vp, i32]
     L.b200tag_field_pose_get.restype = vp
+    L.b200tag_undistort_points.argtypes = [vp, i32] + [C.c_double] * 4 + [vp, vp]
+    L.b200tag_estimate_poses_distorted.argtypes = [vp, i32, i32] + [C.c_double] * 5 + [vp, vp]
+    L.b200tag_debug_estimate_poses_distorted_device.argtypes = [i32, vp, i32] + [C.c_double] * 5 + [vp, vp]
+    L.b200tag_estimate_field_pose_distorted.argtypes = [vp, i32, vp, i32] + [C.c_double] * 5 + [vp, vp, vp, vp]
+    L.b200tag_debug_estimate_field_pose_distorted_device.argtypes = [vp, i32, vp, i32] + [C.c_double] * 5 + [vp, vp, vp, vp]
+    L.b200tag_set_pose_distortion.argtypes = [vp, vp]
     L.b200tag_version.restype = i32
     _lib = L
     return L
@@ -195,19 +201,55 @@ def _pose_method(method: str) -> int:
     return POSE_METHODS[method]
 
 
+def _distortion(distortion):
+    """The `dist` argument of the C ABI: None, or 5 float64 coefficients (k1, k2, p1, p2, k3)."""
+    if distortion is None:
+        return None
+    d = np.ascontiguousarray(distortion, dtype=np.float64).reshape(-1)
+    if d.size != 5:
+        raise ValueError(f"distortion needs 5 coefficients (k1, k2, p1, p2, k3), got {d.size}")
+    return d
+
+
+def _ptr(a):
+    return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def undistort_points(points, fx: float, fy: float, cx: float, cy: float, distortion) -> np.ndarray:
+    """Ideal pinhole pixels of distorted pixels `points` (..., 2) under the 5-coefficient Brown-Conrady model
+    `distortion` = (k1, k2, p1, p2, k3) of OpenCV's projectPoints, inverted exactly (b200tag_undistort_points); NaN where
+    a point cannot be undistorted (past the fold of a strong barrel model)."""
+    lib = load_library()
+    pts = np.ascontiguousarray(points, dtype=np.float64)
+    flat = pts.reshape(-1, 2)
+    out = np.zeros_like(flat)
+    rc = lib.b200tag_undistort_points(_ptr(flat) if len(flat) else None, len(flat), float(fx), float(fy), float(cx),
+                                      float(cy), _ptr(_distortion(distortion)), _ptr(out) if len(flat) else None)
+    if rc:
+        raise B200TagError(f"b200tag_undistort_points: {lib.b200tag_error_string(rc).decode()}")
+    return out.reshape(pts.shape)
+
+
 def estimate_poses(detections: np.ndarray, tagsize: float, fx: float, fy: float, cx: float, cy: float,
-                   method: str = "oi") -> np.ndarray:
+                   method: str = "oi", distortion=None) -> np.ndarray:
     """estimate_tag_pose for every detection (the node's step after Detect, apriltags_cuda_detector.cu:425-462):
     returns POSE_DT records (R, t in the camera frame, object-space error).  Pure host math in libb200tag.so.
     method="ippe" computes the closed-form IPPE pose instead (b200tag_estimate_poses_ippe, OpenCV's SOLVEPNP_IPPE_SQUARE
-    candidates, the one with the smaller object-space error returned)."""
+    candidates, the one with the smaller object-space error returned).  With `distortion` = (k1, k2, p1, p2, k3) the
+    corners are undistorted first (b200tag_estimate_poses_distorted)."""
     lib = load_library()
-    fn = {0: "b200tag_estimate_poses", 1: "b200tag_estimate_poses_ippe"}[_pose_method(method)]
+    m = _pose_method(method)
+    dist = _distortion(distortion)
     dets = np.ascontiguousarray(detections, dtype=DETECTION_DT)
     out = np.zeros(len(dets), dtype=POSE_DT)
     if len(dets):
-        rc = getattr(lib, fn)(dets.ctypes.data_as(C.c_void_p), len(dets), float(tagsize), float(fx), float(fy),
-                              float(cx), float(cy), out.ctypes.data_as(C.c_void_p))
+        args = (float(tagsize), float(fx), float(fy), float(cx), float(cy))
+        if dist is None:
+            fn = {0: "b200tag_estimate_poses", 1: "b200tag_estimate_poses_ippe"}[m]
+            rc = getattr(lib, fn)(_ptr(dets), len(dets), *args, _ptr(out))
+        else:
+            fn = "b200tag_estimate_poses_distorted"
+            rc = lib.b200tag_estimate_poses_distorted(_ptr(dets), len(dets), m, *args, _ptr(dist), _ptr(out))
         if rc:
             raise B200TagError(f"{fn}: {lib.b200tag_error_string(rc).decode()}")
     return out
@@ -233,49 +275,62 @@ def locate_tags(detections: np.ndarray, tagsize: float, fx: float, fy: float, cx
 
 
 def estimate_poses_device(detections: np.ndarray, tagsize: float, fx: float, fy: float, cx: float, cy: float,
-                          method: str = "oi") -> np.ndarray:
+                          method: str = "oi", distortion=None) -> np.ndarray:
     """Test hook: estimate_poses computed by the device pose kernel of `method` (the one GpuDetector.SetPoseEstimation
     enables) on the current CUDA device."""
     lib = load_library()
-    fn = {0: "b200tag_debug_estimate_poses_device", 1: "b200tag_debug_estimate_poses_ippe_device"}[_pose_method(method)]
+    m = _pose_method(method)
+    dist = _distortion(distortion)
     dets = np.ascontiguousarray(detections, dtype=DETECTION_DT)
     out = np.zeros(len(dets), dtype=POSE_DT)
-    rc = getattr(lib, fn)(dets.ctypes.data_as(C.c_void_p) if len(dets) else None, len(dets), float(tagsize),
-                          float(fx), float(fy), float(cx), float(cy), out.ctypes.data_as(C.c_void_p) if len(dets) else None)
+    args = (_ptr(dets) if len(dets) else None, len(dets), float(tagsize), float(fx), float(fy), float(cx), float(cy))
+    if dist is None:
+        fn = {0: "b200tag_debug_estimate_poses_device", 1: "b200tag_debug_estimate_poses_ippe_device"}[m]
+        rc = getattr(lib, fn)(*args, _ptr(out) if len(dets) else None)
+    else:
+        fn = "b200tag_debug_estimate_poses_distorted_device"
+        rc = lib.b200tag_debug_estimate_poses_distorted_device(m, *args, _ptr(dist), _ptr(out) if len(dets) else None)
     if rc:
         raise B200TagError(f"{fn}: {lib.b200tag_error_string(rc).decode()}")
     return out
 
 
-def _field_call(fn, detections, layout, tagsize, fx, fy, cx, cy, rotation, offset) -> np.ndarray:
+def _field_call(fn, fn_distorted, detections, layout, tagsize, fx, fy, cx, cy, rotation, offset, distortion) -> np.ndarray:
     lib = load_library()
+    dist = _distortion(distortion)
     dets = np.ascontiguousarray(detections, dtype=DETECTION_DT)
     lay = np.ascontiguousarray(np.zeros(0, dtype=FIELD_TAG_DT) if layout is None else layout, dtype=FIELD_TAG_DT)
     rot = None if rotation is None else np.ascontiguousarray(rotation, dtype=np.float64).reshape(9)
     off = None if offset is None else np.ascontiguousarray(offset, dtype=np.float64).reshape(3)
     out = np.zeros(1, dtype=FIELD_POSE_DT)
-    rc = getattr(lib, fn)(dets.ctypes.data_as(C.c_void_p) if len(dets) else None, len(dets),
-                          lay.ctypes.data_as(C.c_void_p) if len(lay) else None, len(lay), float(tagsize), float(fx),
-                          float(fy), float(cx), float(cy), None if rot is None else rot.ctypes.data_as(C.c_void_p),
-                          None if off is None else off.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p))
+    args = [dets.ctypes.data_as(C.c_void_p) if len(dets) else None, len(dets),
+            lay.ctypes.data_as(C.c_void_p) if len(lay) else None, len(lay), float(tagsize), float(fx), float(fy),
+            float(cx), float(cy)]
+    if dist is not None:
+        fn = fn_distorted
+        args.append(_ptr(dist))
+    rc = getattr(lib, fn)(*args, _ptr(rot), _ptr(off), _ptr(out))
     if rc:
         raise B200TagError(f"{fn}: {lib.b200tag_error_string(rc).decode()}")
     return out[0]
 
 
 def estimate_field_pose(detections: np.ndarray, layout: np.ndarray, tagsize: float, fx: float, fy: float, cx: float,
-                        cy: float, rotation=None, offset=None) -> np.ndarray:
+                        cy: float, rotation=None, offset=None, distortion=None) -> np.ndarray:
     """One camera (and robot) pose in the field from every detection of a layout tag (b200tag_estimate_field_pose): a
     FIELD_POSE_DT record.  `layout` holds FIELD_TAG_DT records (X_field = R X_tag + t); `detections` may be reconciled
-    or raw.  rotation / offset are the camera's extrinsics, as for locate_tags.  Pure host math in libb200tag.so."""
-    return _field_call("b200tag_estimate_field_pose", detections, layout, tagsize, fx, fy, cx, cy, rotation, offset)
+    or raw.  rotation / offset are the camera's extrinsics, as for locate_tags.  With `distortion` = (k1, k2, p1, p2,
+    k3) the used tags' corners are undistorted first and rms is measured in the ideal image
+    (b200tag_estimate_field_pose_distorted).  Pure host math in libb200tag.so."""
+    return _field_call("b200tag_estimate_field_pose", "b200tag_estimate_field_pose_distorted", detections, layout, tagsize,
+                       fx, fy, cx, cy, rotation, offset, distortion)
 
 
 def estimate_field_pose_device(detections: np.ndarray, layout: np.ndarray, tagsize: float, fx: float, fy: float,
-                               cx: float, cy: float, rotation=None, offset=None) -> np.ndarray:
+                               cx: float, cy: float, rotation=None, offset=None, distortion=None) -> np.ndarray:
     """Test hook: estimate_field_pose computed by the device kernel GpuDetector.SetFieldLayout enables."""
-    return _field_call("b200tag_debug_estimate_field_pose_device", detections, layout, tagsize, fx, fy, cx, cy, rotation,
-                       offset)
+    return _field_call("b200tag_debug_estimate_field_pose_device", "b200tag_debug_estimate_field_pose_distorted_device",
+                       detections, layout, tagsize, fx, fy, cx, cy, rotation, offset, distortion)
 
 
 def _records(ptr, n, dtype) -> np.ndarray:
@@ -480,12 +535,14 @@ class GpuDetector:
         buf = (C.c_char * (QUAD_DT.itemsize * n.value)).from_address(p)
         return np.frombuffer(buf, dtype=QUAD_DT, count=n.value).copy()
 
-    def SetPoseEstimation(self, tagsize, fx, fy, cx, cy, rotation=None, offset=None, method="oi") -> None:
+    def SetPoseEstimation(self, tagsize, fx, fy, cx, cy, rotation=None, offset=None, method="oi", distortion=None) -> None:
         """The node's pose step on the GPU: from the next Detect on, a kernel at the end of the detection graph estimates
         every detection's pose (Poses) and its robot-frame record (TagPositions), with the arguments of locate_tags.
         tagsize = 0 turns it off.  method="ippe" runs the closed-form IPPE pose (estimate_poses(..., method="ippe"))
-        instead of libapriltag's orthogonal iteration."""
+        instead of libapriltag's orthogonal iteration.  `distortion` = (k1, k2, p1, p2, k3) undistorts the corners
+        before the pose and field pose steps, as estimate_poses(..., distortion=...) does; None turns that off."""
         m = _pose_method(method)
+        dist = _distortion(distortion)
         rot = None if rotation is None else np.ascontiguousarray(rotation, dtype=np.float64).reshape(9)
         off = None if offset is None else np.ascontiguousarray(offset, dtype=np.float64).reshape(3)
         self._check(self._lib.b200tag_set_pose_estimation(self._h, float(tagsize), float(fx), float(fy), float(cx), float(cy),
@@ -493,6 +550,7 @@ class GpuDetector:
                                                           None if off is None else off.ctypes.data_as(C.c_void_p)),
                     "b200tag_set_pose_estimation")
         self._check(self._lib.b200tag_set_pose_method(self._h, m), "b200tag_set_pose_method")
+        self._check(self._lib.b200tag_set_pose_distortion(self._h, _ptr(dist)), "b200tag_set_pose_distortion")
 
     def Poses(self, frame: int = 0) -> np.ndarray:
         """POSE_DT records parallel to Detections(frame); empty when the last call ran without the pose step."""

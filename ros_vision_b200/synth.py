@@ -83,8 +83,56 @@ def _invert3(H: np.ndarray) -> np.ndarray:
     return inv / det
 
 
-def render_tag(img: np.ndarray, pose: TagPose, white: float, black: float, ss: int = 4) -> None:
-    """Composite one tag into float image `img` (H, W) in place."""
+def distort_pixels(u, v, fx: float, fy: float, cx: float, cy: float, distortion):
+    """Where a pinhole camera's pixels (u, v) are seen through the 5-coefficient Brown-Conrady model `distortion` =
+    (k1, k2, p1, p2, k3) of OpenCV's projectPoints."""
+    k1, k2, p1, p2, k3 = [float(c) for c in distortion]
+    x = (np.asarray(u, dtype=np.float64) - cx) / fx
+    y = (np.asarray(v, dtype=np.float64) - cy) / fy
+    r2 = x * x + y * y
+    radial = 1.0 + r2 * (k1 + r2 * (k2 + r2 * k3))
+    xd = x * radial + 2.0 * p1 * x * y + p2 * (r2 + 2.0 * x * x)
+    yd = y * radial + p1 * (r2 + 2.0 * y * y) + 2.0 * p2 * x * y
+    return fx * xd + cx, fy * yd + cy
+
+
+def undistort_pixels(u, v, fx: float, fy: float, cx: float, cy: float, distortion):
+    """The exact inverse of distort_pixels, as the pose step computes it (b200tag_undistort_points): Newton's method from
+    the distorted point, at most 20 steps, down to a step of 1e-14 (normalised); NaN where it does not converge, where
+    the Jacobian's determinant is not positive or where the result does not re-distort to within 1e-9."""
+    k1, k2, p1, p2, k3 = [float(c) for c in distortion]
+    xd = (np.asarray(u, dtype=np.float64) - cx) / fx
+    yd = (np.asarray(v, dtype=np.float64) - cy) / fy
+    x, y = xd.copy(), yd.copy()
+    ok = np.ones(x.shape, dtype=bool)
+    done = np.zeros(x.shape, dtype=bool)
+    for _ in range(20):
+        r2 = x * x + y * y
+        radial = 1.0 + r2 * (k1 + r2 * (k2 + r2 * k3))
+        dr = 2.0 * (k1 + r2 * (2.0 * k2 + r2 * (3.0 * k3)))
+        ex = xd - (x * radial + 2.0 * p1 * x * y + p2 * (r2 + 2.0 * x * x))
+        ey = yd - (y * radial + p1 * (r2 + 2.0 * y * y) + 2.0 * p2 * x * y)
+        j00 = radial + x * x * dr + 2.0 * p1 * y + 6.0 * p2 * x
+        j01 = x * y * dr + 2.0 * p1 * x + 2.0 * p2 * y
+        j11 = radial + y * y * dr + 6.0 * p1 * y + 2.0 * p2 * x
+        det = j00 * j11 - j01 * j01
+        live = ok & ~done
+        ok &= ~live | (det > 0)
+        live &= ok
+        with np.errstate(divide="ignore", invalid="ignore"):
+            dx = np.where(live, (j11 * ex - j01 * ey) / det, 0.0)
+            dy = np.where(live, (j00 * ey - j01 * ex) / det, 0.0)
+        x, y = x + dx, y + dy
+        done |= live & (np.abs(dx) <= 1e-14) & (np.abs(dy) <= 1e-14)
+    rx, ry = distort_pixels(fx * x + cx, fy * y + cy, fx, fy, cx, cy, distortion)
+    ok &= done & (np.abs((rx - cx) / fx - xd) <= 1e-9) & (np.abs((ry - cy) / fy - yd) <= 1e-9)
+    return np.where(ok, fx * x + cx, np.nan), np.where(ok, fy * y + cy, np.nan)
+
+
+def render_tag(img: np.ndarray, pose: TagPose, white: float, black: float, ss: int = 4, lens=None) -> None:
+    """Composite one tag into float image `img` (H, W) in place.  With `lens` = (fx, fy, cx, cy, distortion) the corners
+    are those of the ideal pinhole image and the tag is rendered as the distorting lens shows it: every sample position
+    goes through undistort_pixels before the tag's inverse homography."""
     Himg, Wimg = img.shape
     tag_pts = [(-1.0, -1.0), (1.0, -1.0), (1.0, 1.0), (-1.0, 1.0)]
     H = solve_homography(tag_pts, [tuple(map(float, p)) for p in pose.corners])
@@ -94,11 +142,17 @@ def render_tag(img: np.ndarray, pose: TagPose, white: float, black: float, ss: i
     # outer extent of the quiet zone: +-1.25 in tag units for tag36h11
     q = 1.0 + cell
     outer = []
-    for x, y in [(-q, -q), (q, -q), (q, q), (-q, q)]:
+    # the quiet zone's outline; through a lens its edges curve, so they are sampled along their length
+    edge = [(-q, -q), (q, -q), (q, q), (-q, q)] if lens is None else \
+        [(a, b) for g in np.linspace(-q, q, 33) for a, b in ((g, -q), (g, q), (-q, g), (q, g))]
+    for x, y in edge:
         X = H[0, 0] * x + H[0, 1] * y + H[0, 2]
         Y = H[1, 0] * x + H[1, 1] * y + H[1, 2]
         Z = H[2, 0] * x + H[2, 1] * y + H[2, 2]
         outer.append((X / Z, Y / Z))
+    if lens is not None:
+        du, dv = distort_pixels([p[0] for p in outer], [p[1] for p in outer], *lens)
+        outer = list(zip(du.tolist(), dv.tolist()))
     xs = [p[0] for p in outer]
     ys = [p[1] for p in outer]
     x0 = max(0, int(math.floor(min(xs))) - 1)
@@ -114,10 +168,14 @@ def render_tag(img: np.ndarray, pose: TagPose, white: float, black: float, ss: i
     py = (y0 + np.arange(bh, dtype=np.float64))[:, None] + sub[None, :]
     PX = px.reshape(1, bw * ss)
     PY = py.reshape(bh * ss, 1)
+    if lens is not None:
+        PX, PY = undistort_pixels(*np.broadcast_arrays(PX, PY), *lens)
     Z = Hi[2, 0] * PX + Hi[2, 1] * PY + Hi[2, 2]
     TX = (Hi[0, 0] * PX + Hi[0, 1] * PY + Hi[0, 2]) / Z
     TY = (Hi[1, 0] * PX + Hi[1, 1] * PY + Hi[1, 2]) / Z
     inside = (TX >= -q) & (TX < q) & (TY >= -q) & (TY < q) & (Z > 0)
+    if lens is not None:  # samples past the lens model's fold are NaN, and outside
+        TX, TY = np.where(inside, TX, 0.0), np.where(inside, TY, 0.0)
     cx = np.floor((TX + q) / cell).astype(np.int64)
     cy = np.floor((TY + q) / cell).astype(np.int64)
     np.clip(cx, 0, fam["total_width"] - 1, out=cx)
@@ -213,17 +271,22 @@ def make_scene(width: int, height: int, seed: int, n_tags: int, side_range=(60.0
 
 def field_scene(width: int, height: int, layout, tagsize: float, camera_R, camera_t, fx: float, fy: float, cx: float,
                 cy: float, seed: int, noise_sigma: float = 2.0, family: str = "tag36h11", background: float = 128.0,
-                white: float = 230.0, black: float = 25.0, ss: int = 4) -> Scene:
+                white: float = 230.0, black: float = 25.0, ss: int = 4, distortion=None) -> Scene:
     """A gray frame of the tags of a field layout (detector.FIELD_TAG_DT records, X_field = R X_tag + t) seen by a
     pinhole camera placed in the field by X_field = camera_R X_cam + camera_t.  Each tag's black-border corners are
     projected; the tags lying fully in front of the camera and inside the frame are rendered, farthest first.  TagPose
     corners (-1,-1), (1,-1), (1,1), (-1,1) are the tag points (-s,-s), (s,-s), (s,s), (-s,s), s = tagsize / 2.  Returns the
-    Scene: the frame and the rendered tags with their true corners."""
+    Scene: the frame and the rendered tags with their true corners.
+
+    With `distortion` = (k1, k2, p1, p2, k3) the camera has that lens (distort_pixels): each pixel is rendered from the
+    point of the pinhole image undistort_pixels maps it to, the frame test applies to the distorted corners, and the
+    returned corners are the distorted projections."""
     rng = np.random.default_rng(seed)
     Rc = np.asarray(camera_R, dtype=np.float64).reshape(3, 3)
     tc = np.asarray(camera_t, dtype=np.float64).reshape(3)
     s = tagsize / 2.0
     P = np.array([[-s, -s, 0.0], [s, -s, 0.0], [s, s, 0.0], [-s, s, 0.0]])
+    lens = None if distortion is None else (fx, fy, cx, cy, tuple(float(c) for c in distortion))
     visible = []
     for rec in np.asarray(layout):
         X = P @ np.asarray(rec["R"], dtype=np.float64).reshape(3, 3).T + np.asarray(rec["t"], dtype=np.float64)
@@ -231,17 +294,23 @@ def field_scene(width: int, height: int, layout, tagsize: float, camera_R, camer
         if not (cam[:, 2] > 1e-6).all():
             continue
         px = np.stack([fx * cam[:, 0] / cam[:, 2] + cx, fy * cam[:, 1] / cam[:, 2] + cy], axis=1)
-        if (px[:, 0] < 0).any() or (px[:, 0] > width).any() or (px[:, 1] < 0).any() or (px[:, 1] > height).any():
+        seen = px
+        if lens is not None:
+            seen = np.stack(distort_pixels(px[:, 0], px[:, 1], *lens), axis=1)
+            back = np.stack(undistort_pixels(seen[:, 0], seen[:, 1], *lens), axis=1)
+            if not (np.abs(back - px) <= 1e-6).all():  # beyond the lens model's fold: not in view
+                continue
+        if (seen[:, 0] < 0).any() or (seen[:, 0] > width).any() or (seen[:, 1] < 0).any() or (seen[:, 1] > height).any():
             continue
-        visible.append((float(cam[:, 2].mean()), TagPose(int(rec["id"]), px, family)))
+        visible.append((float(cam[:, 2].mean()), TagPose(int(rec["id"]), px, family), TagPose(int(rec["id"]), seen, family)))
     img = np.full((height, width), float(background), dtype=np.float64)
     visible.sort(key=lambda v: -v[0])
-    for _, pose in visible:
-        render_tag(img, pose, white, black, ss)
+    for _, pose, _ in visible:
+        render_tag(img, pose, white, black, ss, lens)
     if noise_sigma > 0:
         img = img + rng.normal(0.0, noise_sigma, size=img.shape)
     gray = np.clip(np.floor(img + 0.5), 0, 255).astype(np.uint8)
-    return Scene(gray, [v[1] for v in visible])
+    return Scene(gray, [v[2] for v in visible])
 
 
 # --- frame format packers -------------------------------------------------

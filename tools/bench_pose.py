@@ -19,6 +19,14 @@ detections.
     frames of one 6-tag layout seen from 16 robot poses (consistent geometry);
   * the host estimate_field_pose per field_scene frame on one CPU core.
 
+--distortion K1,K2,P1,P2,K3 measures what the undistortion of the corners (SetPoseEstimation(..., distortion=...))
+adds to the arm chosen by the other options (OI, --method ippe, or --field on top of IPPE): two arms alternating in the
+same run, the pose step on without and with the coefficients, on the same config-2 workload:
+  * frames/s of 128-frame batches and kernels per batch;
+  * single-frame p50 and p90;
+  * the arm's kernel (`pose`, `pose_ippe` or `field_pose`) per 128-frame batch, from b200tag_profile_device, alternated
+    over rounds; for --field on the synth.field_scene frames of the field arm.
+
 Prints one JSON record, and writes it to --out when given.  Needs a CUDA device."""
 import argparse
 import json
@@ -55,8 +63,14 @@ def main():
     ap.add_argument("--latency-iters", type=int, default=400, help="single frames per latency measurement")
     ap.add_argument("--method", choices=("oi", "ippe"), default="oi", help="pose method of the device step")
     ap.add_argument("--field", action="store_true", help="measure the field pose step (IPPE + SetFieldLayout)")
+    ap.add_argument("--distortion", help="K1,K2,P1,P2,K3: measure the pose step with these lens coefficients against without")
     ap.add_argument("--out", help="also write the JSON to this file (e.g. profiles/pose_r03.json)")
     args = ap.parse_args()
+    if args.distortion:
+        dist = [float(v) for v in args.distortion.split(",")]
+        if len(dist) != 5:
+            ap.error("--distortion needs 5 coefficients")
+        return distortion_main(args, dist)
     if args.field:
         return field_main(args)
 
@@ -337,6 +351,104 @@ def field_main(args):
             json.dump(res, f, indent=1)
     print(json.dumps(res, indent=1))
     for d in list(big.values()) + list(one.values()) + [fs_det, fs_one]:
+        d.close()
+    for pb in pins:
+        pb.close()
+
+
+def distortion_main(args, dist):
+    import torch
+    from ros_vision_b200 import detector as D, synth
+    method = "ippe" if args.field else args.method
+    kernel = "field_pose" if args.field else {"oi": "pose", "ippe": "pose_ippe"}[method]
+    arms = ("plain", "distorted")
+    frames = [np.ascontiguousarray(synth.config_frame(2, i)[0]).reshape(-1) for i in range(UNIQUE)]
+    dev_batch = torch.from_numpy(np.stack([frames[i % UNIQUE] for i in range(BATCH)])).cuda()
+    ptr = dev_batch.data_ptr()
+    lay, kernel_ptr = None, ptr
+    if args.field:
+        lay, fs_frames = field_frames(D, synth, UNIQUE)
+        fs_batch = torch.from_numpy(np.stack([fs_frames[i % UNIQUE] for i in range(BATCH)])).cuda()
+        kernel_ptr = fs_batch.data_ptr()
+
+    def detector(arm, max_batch):
+        d = D.GpuDetector(1280, 800, "yuyv", quad_decimate=2, max_batch=max_batch)
+        d.SetPoseEstimation(TAGSIZE, FX, FY, CX, CY, rotation=ROTATION, offset=OFFSET, method=method,
+                            distortion=dist if arm == "distorted" else None)
+        if lay is not None:
+            d.SetFieldLayout(lay)
+        return d
+
+    big = {a: detector(a, BATCH) for a in arms}
+    for d in big.values():
+        for _ in range(5):
+            d.DetectDevice(ptr, BATCH)
+    fps = {a: [] for a in arms}
+    for _ in range(args.rounds):
+        for a in arms:
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            for _ in range(args.steps):
+                big[a].DetectDevice(ptr, BATCH)
+            fps[a].append(BATCH * args.steps / (time.perf_counter() - t0))
+    kpb = {a: big[a].kernels_per_batch() for a in arms}
+    failed = sum(int(np.isinf(big["distorted"].Poses(f)["err"]).sum()) for f in range(BATCH))
+
+    kms = {a: [] for a in arms}
+    for _ in range(3):
+        for a in arms:
+            kms[a].append([ms for name, ms in big[a].ProfileDevice(kernel_ptr, BATCH, iters=20) if name == kernel][0])
+
+    one = {a: detector(a, 1) for a in arms}
+    pins = []
+    for f in frames:
+        pb = D.PinnedBuffer(f.size)
+        pb.array[:] = f
+        pins.append(pb)
+    for d in one.values():
+        for pb in pins:
+            d.DetectPointers([pb.ptr])
+    lat = {a: [] for a in arms}
+    for i in range(args.latency_iters):
+        pb = pins[i % UNIQUE]
+        for a in (arms if i % 2 == 0 else arms[::-1]):
+            t0 = time.perf_counter()
+            one[a].DetectPointers([pb.ptr])
+            lat[a].append((time.perf_counter() - t0) * 1e6)
+
+    med = {a: float(np.median(fps[a])) for a in arms}
+    p50 = {a: float(np.percentile(lat[a], 50)) for a in arms}
+    kmed = {a: float(np.median(kms[a])) for a in arms}
+    kratio = kmed["distorted"] / kmed["plain"]
+    if args.field:
+        targets = {"field_pose_at_most_1.1x_without": bool(kratio <= 1.1)}
+    elif method == "oi":
+        targets = {"pose_at_most_1.05x_without": bool(kratio <= 1.05)}
+    else:
+        targets = {"pose_ippe_at_most_0.03ms_per_batch": bool(kmed["distorted"] <= 0.03),
+                   "p50_at_most_p50_without_plus_5us": bool(p50["distorted"] <= p50["plain"] + 5)}
+    res = {
+        "mode": "field" if args.field else method,
+        "distortion": dist,
+        "gpu": gpu_identity(),
+        "torch_device": torch.cuda.get_device_name(0),
+        "workload": "config2: 1280x800 YUYV, synth.config_frame(2, 0..15) tiled to 128-frame batches, tag36h11, decimate 2"
+                    + ("; field_pose kernel on synth.field_scene frames of one 6-tag layout (the --field workload)" if args.field else ""),
+        "batch_frames_per_s": {"rounds": fps, "median": med, "ratio_distorted_over_plain": med["distorted"] / med["plain"]},
+        "kernels_per_batch": kpb,
+        "failed_poses_per_batch_distorted": failed,
+        "kernel": kernel,
+        "kernel_ms_per_batch": {"rounds": kms, "median": kmed, "ratio_distorted_over_plain": kratio},
+        "single_frame_latency_us": {"p50": p50, "p90": {a: float(np.percentile(lat[a], 90)) for a in arms},
+                                    "iters": args.latency_iters},
+        "targets": targets,
+    }
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            json.dump(res, f, indent=1)
+    print(json.dumps(res, indent=1))
+    for d in list(big.values()) + list(one.values()):
         d.close()
     for pb in pins:
         pb.close()
