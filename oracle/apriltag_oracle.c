@@ -25,14 +25,15 @@ float orc_emul_atan2f(float y, float x) { return orc_cuda_atan2f(y, x); }
 float orc_emul_hypotf(float a, float b) { return orc_cuda_hypotf(a, b); }
 uint64_t orc_tag36h11_code(int id) { return orc_tag36h11_codes[id]; }
 
-/* Built-in families (libapriltag tagXXhYY_create(), apriltag_utils.cu:10-27): AprilTag 3 layouts, normal border. */
+/* Built-in families (libapriltag tagXXhYY_create(), apriltag_utils.cu:10-27): AprilTag 3 layouts, normal border,
+ * added with bits_corrected = 2 (apriltags_cuda_detector.cu:140). */
 static const orc_family k_families[ORC_NUM_FAMILIES] = {
     {"tag36h11", orc_tag36h11_NBITS, orc_tag36h11_NCODES, orc_tag36h11_WIDTH_AT_BORDER, orc_tag36h11_TOTAL_WIDTH, 0,
-     orc_tag36h11_MIN_HAMMING, orc_tag36h11_codes, orc_tag36h11_bit_x, orc_tag36h11_bit_y},
+     orc_tag36h11_MIN_HAMMING, orc_tag36h11_codes, orc_tag36h11_bit_x, orc_tag36h11_bit_y, 2},
     {"tag25h9", orc_tag25h9_NBITS, orc_tag25h9_NCODES, orc_tag25h9_WIDTH_AT_BORDER, orc_tag25h9_TOTAL_WIDTH, 0,
-     orc_tag25h9_MIN_HAMMING, orc_tag25h9_codes, orc_tag25h9_bit_x, orc_tag25h9_bit_y},
+     orc_tag25h9_MIN_HAMMING, orc_tag25h9_codes, orc_tag25h9_bit_x, orc_tag25h9_bit_y, 2},
     {"tag16h5", orc_tag16h5_NBITS, orc_tag16h5_NCODES, orc_tag16h5_WIDTH_AT_BORDER, orc_tag16h5_TOTAL_WIDTH, 0,
-     orc_tag16h5_MIN_HAMMING, orc_tag16h5_codes, orc_tag16h5_bit_x, orc_tag16h5_bit_y},
+     orc_tag16h5_MIN_HAMMING, orc_tag16h5_codes, orc_tag16h5_bit_x, orc_tag16h5_bit_y, 2},
 };
 const orc_family *orc_family_get(int index) { return (index >= 0 && index < ORC_NUM_FAMILIES) ? &k_families[index] : NULL; }
 int orc_family_index(const char *name) {
@@ -41,6 +42,24 @@ int orc_family_index(const char *name) {
   return -1;
 }
 static uint32_t family_mask_of(const orc_config *c) { return c->family_mask ? c->family_mask : 1u; }
+
+/* The families a configuration decodes, numbered as its detections number them: the caller's list, or the built-in
+ * families family_mask selects at their built-in index (a slot the mask leaves out is NULL). */
+int orc_i_family_slots(const orc_config *c) { return c->nfamilies > 0 ? c->nfamilies : ORC_NUM_FAMILIES; }
+const orc_family *orc_i_family(const orc_config *c, int slot) {
+  if (c->nfamilies > 0) return &c->families[slot];
+  return ((family_mask_of(c) >> slot) & 1u) ? &k_families[slot] : NULL;
+}
+/* Border polarities over the families in use (apriltag_gpu.cu:169-177). */
+void orc_i_border_polarities(const orc_config *c, int *normal_border, int *reversed_border) {
+  *normal_border = *reversed_border = 0;
+  for (int fi = 0; fi < orc_i_family_slots(c); fi++) {
+    const orc_family *fam = orc_i_family(c, fi);
+    if (!fam) continue;
+    *normal_border |= !fam->reversed_border;
+    *reversed_border |= fam->reversed_border != 0;
+  }
+}
 
 void orc_default_config(orc_config *c, int width, int height, int format) {
   memset(c, 0, sizeof(*c));
@@ -327,9 +346,8 @@ static float extents_dot(const orc_cluster *e) { /* line_fit_filter.h:51-58 */
 
 int orc_i_min_tag_width(const orc_config *c) { /* apriltag_gpu.cu:169-181: min over the families */
   int m = 1000000;
-  for (int f = 0; f < ORC_NUM_FAMILIES; f++)
-    if ((family_mask_of(c) >> f) & 1u)
-      if (k_families[f].width_at_border < m) m = k_families[f].width_at_border;
+  for (int f = 0; f < orc_i_family_slots(c); f++)
+    if (orc_i_family(c, f) && orc_i_family(c, f)->width_at_border < m) m = orc_i_family(c, f)->width_at_border;
   m = (int)((float)m / (float)c->quad_decimate);
   if (m < 3) m = 3;
   return m;
@@ -371,7 +389,8 @@ static void clusters_and_filter(const orc_config *c, orc_result *r) {
   const uint32_t min_px = (uint32_t)(c->min_cluster_pixels > 24 ? c->min_cluster_pixels : 24);
   const uint32_t max_px = (uint32_t)(4 * (r->w + r->h));
   const int tag_width = min_tag_width(c);
-  const int reversed_border = 0, normal_border = 1; /* tag36h11 */
+  int normal_border, reversed_border;
+  orc_i_border_polarities(c, &normal_border, &reversed_border);
   uint32_t sel = 0;
   for (int i = 0; i < nc; i++) {
     orc_cluster *e = &cl[i];
@@ -665,6 +684,8 @@ static void quad_corners(const orc_config *c, orc_result *r) {
   r->corners = (orc_quadcorners *)calloc((size_t)r->num_fitquads + 1, sizeof(orc_quadcorners));
   int n = 0;
   const int mtw = min_tag_width(c);
+  int normal_border, reversed_border;
+  orc_i_border_polarities(c, &normal_border, &reversed_border);
   for (int qi = 0; qi < r->num_fitquads; qi++) {
     const orc_fitquad *q = &r->fitquads[qi];
     if (!q->valid) continue;
@@ -673,7 +694,7 @@ static void quad_corners(const orc_config *c, orc_result *r) {
     qc.blob = q->blob;
     qc.rep0 = q->rep0;
     qc.rep1 = q->rep1;
-    qc.reversed_border = 0;
+    qc.reversed_border = reversed_border && !normal_border; /* one polarity across the families */
     double lines[4][4];
     for (int i = 0; i < 4; i++) {
       double err, mse;
@@ -975,13 +996,15 @@ static uint64_t rotate90(uint64_t w, int nbits) {
 }
 
 int orc_decode_codeword_family(const orc_family *fam, uint64_t rcode, int *hamming, int *rotation) {
-  /* quick_decode_codeword with maxhamming = 2: the hash table holds every code with <= 2 flipped bits; a minimum
-   * distance of 5 or more (rotations included) makes the hit unique, so a linear popcount scan returns the same
-   * (id, hamming). */
+  /* quick_decode_codeword: the first rotation with a code within max_hamming bits, and at that rotation the lowest
+   * id within reach.  The hit need not be unique: tag16h5 (minimum distance 5) at max_hamming 3 has words within 3
+   * bits of two codes.  libapriltag's hash table answers with the lowest id there too: quick_decode_init inserts the
+   * codes in id order, each with every word within max_hamming bits, and an insert only takes an empty slot, so on a
+   * word's probe chain the lowest id's entry comes first and the lookup returns it. */
   for (int ridx = 0; ridx < 4; ridx++) {
     for (int id = 0; id < fam->ncodes; id++) {
       const int d = __builtin_popcountll(rcode ^ fam->codes[id]);
-      if (d <= 2) {
+      if (d <= fam->max_hamming) {
         *hamming = d;
         *rotation = ridx;
         return id;
@@ -1105,7 +1128,7 @@ void orc_i_fill_detection(orc_detection *d, int family, int id, int hamming, flo
 }
 
 static void decode_quads(const orc_config *c, orc_result *r) {
-  r->detections = (orc_detection *)calloc((size_t)r->num_corners * ORC_NUM_FAMILIES + 1, sizeof(orc_detection));
+  r->detections = (orc_detection *)calloc((size_t)r->num_corners * orc_i_family_slots(c) + 1, sizeof(orc_detection));
   r->refined = (orc_quadcorners *)calloc((size_t)r->num_corners + 1, sizeof(orc_quadcorners));
   int nd = 0;
   for (int qi = 0; qi < r->num_corners; qi++) {
@@ -1128,10 +1151,9 @@ static void decode_quads(const orc_config *c, orc_result *r) {
                          Hm[2] * (Hm[3] * Hm[7] - Hm[4] * Hm[6]);
       if (!(fabs(det) > 1e-300)) continue;
     }
-    for (int fi = 0; fi < ORC_NUM_FAMILIES; fi++) { /* quad_decode_task: every family of the matching polarity */
-      if (!((family_mask_of(c) >> fi) & 1u)) continue;
-      const orc_family *fam = &k_families[fi];
-      if (fam->reversed_border != r->corners[qi].reversed_border) continue;
+    for (int fi = 0; fi < orc_i_family_slots(c); fi++) { /* quad_decode_task: every family of the matching polarity */
+      const orc_family *fam = orc_i_family(c, fi);
+      if (!fam || (fam->reversed_border != 0) != (r->corners[qi].reversed_border != 0)) continue;
       int id, hamming, rotation;
       const float margin = orc_i_quad_decode(c, fam, r->gray, r->W, r->H, Hm, &id, &hamming, &rotation);
       if (margin >= 0 && hamming < 255) {

@@ -15,9 +15,13 @@
  *   - decode / reconcile (quad_decode_index, reconcile_detections) live in the
  *     un-vendored libapriltag fork github.com/cgpadwick/apriltag tag 3.3.0
  *     (src/external/CMakeLists.txt:86-95); restated from the published AprilTag 3
- *     algorithm.  For hamming, decision_margin and H: PARITY UNPINNED (no reference
+ *     algorithm.  For decision_margin and H: PARITY UNPINNED (no reference
  *     test asserts them); ids and corners are pinned by gpu_detector_test.cu's
- *     known answers.
+ *     known answers.  The codeword lookup (id, hamming, rotation at max_hamming
+ *     0..3, lowest id when two codes are within reach), the rotation applied to H
+ *     and the corner order are pinned by a brute-force reference and rendered
+ *     ground truth (tests/test_decode_reference_cpu.py): every orientation,
+ *     0..4 flipped cells, reversed borders.
  */
 #ifndef APRILTAG_ORACLE_H_
 #define APRILTAG_ORACLE_H_
@@ -47,10 +51,15 @@ typedef struct {
   double k1, k2, p1, p2, k3;  /* DistCoeffs, apriltag_gpu.h:68-74 */
   int max_stage;          /* stop after this stage (ORC_STAGE_*), for timing/tests */
   uint32_t family_mask;   /* bit i = built-in family i (orc_family_get); 0 means tag36h11 only */
+  /* The caller's families, as b200tag_family lists them (codes, bit_x / bit_y, widths, reversed_border,
+   * max_hamming).  When nfamilies > 0 they replace family_mask and detections carry an index into this list. */
+  const struct orc_family *families;
+  int nfamilies;
 } orc_config;
 
-/* apriltag_family_t (libapriltag apriltag.h), the fields the detector reads. */
-typedef struct {
+/* apriltag_family_t (libapriltag apriltag.h), the fields the detector reads, and the bits_corrected the family was
+ * added with (apriltag_detector_add_family_bits). */
+typedef struct orc_family {
   const char *name;
   int nbits, ncodes;
   int width_at_border, total_width;
@@ -58,6 +67,7 @@ typedef struct {
   int h; /* minimum Hamming distance */
   const uint64_t *codes;
   const int32_t *bit_x, *bit_y;
+  int max_hamming; /* 0..3; the built-in families use 2 */
 } orc_family;
 #define ORC_NUM_FAMILIES 3 /* 0 tag36h11, 1 tag25h9, 2 tag16h5 */
 const orc_family *orc_family_get(int index);
@@ -184,7 +194,8 @@ int orc_undistort(double *u, double *v, const orc_config *cfg);
 void orc_redistort(double *x, double *y, const orc_config *cfg);
 int orc_homography_compute(const double corr[4][4], double H[9]);
 uint64_t orc_tag36h11_code(int id);
-/* quick-decode: returns id or -1; hamming/rotation via out params */
+/* quick-decode: returns id or -1; hamming/rotation via out params.  orc_decode_codeword is tag36h11 at
+ * max_hamming 2; orc_decode_codeword_family takes the family's own max_hamming. */
 int orc_decode_codeword(uint64_t rcode, int *hamming, int *rotation);
 int orc_decode_codeword_family(const orc_family *fam, uint64_t rcode, int *hamming, int *rotation);
 

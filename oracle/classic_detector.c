@@ -593,12 +593,8 @@ int orc_classic_detect(const orc_config *c, const uint8_t *gray, orc_detection *
   gradient_clusters(&m, &uf, thresh, w, h);
 
   /* fit_quads: family-derived limits (apriltag_quad_thresh.c) */
-  int normal_border = 0, reversed_border = 0;
-  for (int fi = 0; fi < ORC_NUM_FAMILIES; fi++) {
-    if (!(((c->family_mask ? c->family_mask : 1u) >> fi) & 1u)) continue;
-    normal_border |= !orc_family_get(fi)->reversed_border;
-    reversed_border |= orc_family_get(fi)->reversed_border;
-  }
+  int normal_border, reversed_border;
+  orc_i_border_polarities(c, &normal_border, &reversed_border);
   const int tag_width = orc_i_min_tag_width(c);
   struct quad *quads = (struct quad *)malloc(((size_t)m.n + 1) * sizeof(struct quad));
   int nq = 0;
@@ -620,7 +616,7 @@ int orc_classic_detect(const orc_config *c, const uint8_t *gray, orc_detection *
   if (nquads_out) *nquads_out = nq;
 
   /* quad_decode_task */
-  orc_detection *dets = (orc_detection *)malloc(((size_t)nq * ORC_NUM_FAMILIES + 1) * sizeof(orc_detection));
+  orc_detection *dets = (orc_detection *)malloc(((size_t)nq * orc_i_family_slots(c) + 1) * sizeof(orc_detection));
   int nd = 0;
   for (int qi = 0; qi < nq; qi++) {
     struct quad *q = &quads[qi];
@@ -637,10 +633,9 @@ int orc_classic_detect(const orc_config *c, const uint8_t *gray, orc_detection *
     const double det = Hm[0] * (Hm[4] * Hm[8] - Hm[5] * Hm[7]) - Hm[1] * (Hm[3] * Hm[8] - Hm[5] * Hm[6]) +
                        Hm[2] * (Hm[3] * Hm[7] - Hm[4] * Hm[6]);
     if (!(fabs(det) > 1e-300)) continue;
-    for (int fi = 0; fi < ORC_NUM_FAMILIES; fi++) {
-      if (!(((c->family_mask ? c->family_mask : 1u) >> fi) & 1u)) continue;
-      const orc_family *fam = orc_family_get(fi);
-      if (fam->reversed_border != q->reversed_border) continue;
+    for (int fi = 0; fi < orc_i_family_slots(c); fi++) {
+      const orc_family *fam = orc_i_family(c, fi);
+      if (!fam || (fam->reversed_border != 0) != (q->reversed_border != 0)) continue;
       int id, hamming, rotation;
       const float margin = orc_i_quad_decode(c, fam, gray, W, H, Hm, &id, &hamming, &rotation);
       if (margin >= 0 && hamming < 255) orc_i_fill_detection(&dets[nd++], fi, id, hamming, margin, rotation, Hm);

@@ -8,6 +8,9 @@ void orc_i_decimate(const uint8_t *gray, int W, int f, uint8_t *out, int w, int 
 void orc_i_gaussian_blur(uint8_t *im, int w, int h, float quad_sigma);
 void orc_i_threshold(const uint8_t *im, int w, int h, int min_white_black_diff, uint8_t *minmax_out, uint8_t *out);
 int orc_i_min_tag_width(const orc_config *c);
+int orc_i_family_slots(const orc_config *c);
+const orc_family *orc_i_family(const orc_config *c, int slot);
+void orc_i_border_polarities(const orc_config *c, int *normal_border, int *reversed_border);
 float orc_i_quad_decode(const orc_config *c, const orc_family *fam, const uint8_t *im, int W, int H, const double *Hm, int *id,
                         int *hamming, int *rotation);
 void orc_i_fill_detection(orc_detection *d, int family, int id, int hamming, float margin, int rotation, const double *Hm);

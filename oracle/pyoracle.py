@@ -27,7 +27,15 @@ class OrcConfig(C.Structure):
         ("max_line_fit_mse", C.c_float), ("min_white_black_diff", C.c_int),
         ("fx", C.c_double), ("cx", C.c_double), ("fy", C.c_double), ("cy", C.c_double),
         ("k1", C.c_double), ("k2", C.c_double), ("p1", C.c_double), ("p2", C.c_double), ("k3", C.c_double),
-        ("max_stage", C.c_int), ("family_mask", C.c_uint32),
+        ("max_stage", C.c_int), ("family_mask", C.c_uint32), ("families", C.c_void_p), ("nfamilies", C.c_int),
+    ]
+
+
+class OrcFamily(C.Structure):
+    _fields_ = [
+        ("name", C.c_char_p), ("nbits", C.c_int), ("ncodes", C.c_int), ("width_at_border", C.c_int),
+        ("total_width", C.c_int), ("reversed_border", C.c_int), ("h", C.c_int), ("codes", C.POINTER(C.c_uint64)),
+        ("bit_x", C.POINTER(C.c_int32)), ("bit_y", C.POINTER(C.c_int32)), ("max_hamming", C.c_int),
     ]
 
 
@@ -99,6 +107,10 @@ def lib():
         L.orc_tag36h11_code.restype = C.c_uint64
         L.orc_decode_codeword.argtypes = [C.c_uint64, C.POINTER(C.c_int), C.POINTER(C.c_int)]
         L.orc_decode_codeword.restype = C.c_int
+        L.orc_decode_codeword_family.argtypes = [C.POINTER(OrcFamily), C.c_uint64, C.POINTER(C.c_int), C.POINTER(C.c_int)]
+        L.orc_decode_codeword_family.restype = C.c_int
+        L.orc_family_get.argtypes = [C.c_int]
+        L.orc_family_get.restype = C.POINTER(OrcFamily)
         L.orc_classic_detect.argtypes = [C.POINTER(OrcConfig), C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_int)]
         L.orc_classic_detect.restype = C.c_int
         L.orc_family_index.argtypes = [C.c_char_p]
@@ -116,15 +128,56 @@ def family_mask(families) -> int:
     return sum(1 << FAMILY_NAMES.index(f) for f in families)
 
 
+def family_table(family) -> OrcFamily:
+    """An orc_family from a built-in name or from a dict in the layout GpuDetector takes (ros_vision_b200.tag_families
+    entries + optional "reversed_border", "max_hamming", "name").  The arrays it points to live on the returned object."""
+    if isinstance(family, str):
+        i = lib().orc_family_index(family.encode())
+        if i < 0:
+            raise ValueError(f"no built-in tag family {family!r}")
+        return lib().orc_family_get(i).contents
+    fam = OrcFamily()
+    fam._keep = (f"{family.get('name', 'custom')}".encode(), (C.c_uint64 * len(family["codes"]))(*family["codes"]),
+                 (C.c_int32 * family["nbits"])(*family["bit_x"]), (C.c_int32 * family["nbits"])(*family["bit_y"]))
+    fam.name, fam.codes, fam.bit_x, fam.bit_y = fam._keep
+    fam.nbits, fam.ncodes = family["nbits"], len(family["codes"])
+    fam.width_at_border, fam.total_width = family["width_at_border"], family["total_width"]
+    fam.reversed_border, fam.max_hamming = int(family.get("reversed_border", 0)), int(family.get("max_hamming", 2))
+    fam.h = int(family.get("min_hamming", 0))
+    return fam
+
+
+def decode_codeword(family, word: int, max_hamming: int):
+    """quick_decode_codeword of the oracle for `family` (name or dict) at `max_hamming`: (id, hamming, rotation) or
+    None."""
+    table = family_table(family)
+    fam = OrcFamily.from_buffer_copy(table)   # (the copy points into `table`'s arrays, alive until we return)
+    fam.max_hamming = int(max_hamming)
+    h, r = C.c_int(), C.c_int()
+    i = lib().orc_decode_codeword_family(C.byref(fam), C.c_uint64(word), C.byref(h), C.byref(r))
+    return None if i < 0 else (i, h.value, r.value)
+
+
 def make_config(width, height, fmt="yuyv", quad_decimate=2, quad_sigma=0.0, refine_edges=True, camera=None,
                 dist=None, max_stage=STAGE_DECODE, families=("tag36h11",), **qtp) -> OrcConfig:
+    """`families` as GpuDetector takes them: built-in names select the oracle's tables by family_mask (detections
+    carry the built-in index); a list with any dict becomes the configuration's own family list, in that order
+    (detections carry the index into it)."""
     cfg = OrcConfig()
     lib().orc_default_config(C.byref(cfg), width, height, FMT[fmt])
     cfg.quad_decimate = int(quad_decimate)
     cfg.quad_sigma = float(quad_sigma)
     cfg.refine_edges = int(bool(refine_edges))
     cfg.max_stage = max_stage
-    cfg.family_mask = family_mask(families)
+    if isinstance(families, (str, dict)):
+        families = [families]
+    if all(isinstance(f, str) for f in families):
+        cfg.family_mask = family_mask(families)
+    else:
+        tables = [family_table(f) for f in families]
+        arr = (OrcFamily * len(tables))(*tables)
+        cfg._keep = (tables, arr)
+        cfg.families, cfg.nfamilies = C.addressof(arr), len(tables)
     if camera is not None:
         cfg.fx, cfg.cx, cfg.fy, cfg.cy = camera
     if dist is not None:

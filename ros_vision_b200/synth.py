@@ -23,6 +23,7 @@ class TagPose:
     tag_id: int
     corners: np.ndarray  # (4,2) image positions of tag-frame (-1,-1),(1,-1),(1,1),(-1,1)
     family: str = "tag36h11"
+    flips: tuple = ()  # code bit indices drawn inverted (tag_pattern)
 
 
 @dataclass
@@ -31,16 +32,17 @@ class Scene:
     tags: list = field(default_factory=list)
 
 
-def tag_pattern(tag_id: int, family: str = "tag36h11") -> np.ndarray:
+def tag_pattern(tag_id: int, family: str = "tag36h11", flips=()) -> np.ndarray:
     """total_width x total_width cell image (1 = white) of tag `tag_id` of `family`, one-cell quiet zone included
-    (10 x 10 for tag36h11: black border 8 x 8, data 6 x 6)."""
+    (10 x 10 for tag36h11: black border 8 x 8, data 6 x 6).  Each entry i of `flips` draws code bit i (integer bit
+    nbits-1-i) inverted: a tag with bit errors."""
     fam = FAMILIES[family]
     tw, wb, nbits = fam["total_width"], fam["width_at_border"], fam["nbits"]
     pat = np.ones((tw, tw), dtype=np.float64)
     pat[1:1 + wb, 1:1 + wb] = 0.0
     code = fam["codes"][tag_id]
     for i in range(nbits):
-        bit = (code >> (nbits - 1 - i)) & 1
+        bit = ((code >> (nbits - 1 - i)) & 1) ^ (i in flips)
         # border cell (bx, by) in [0, width_at_border) sits at pattern cell (bx+1, by+1)
         pat[fam["bit_y"][i] + 1, fam["bit_x"][i] + 1] = float(bit)
     return pat
@@ -180,7 +182,7 @@ def render_tag(img: np.ndarray, pose: TagPose, white: float, black: float, ss: i
     cy = np.floor((TY + q) / cell).astype(np.int64)
     np.clip(cx, 0, fam["total_width"] - 1, out=cx)
     np.clip(cy, 0, fam["total_width"] - 1, out=cy)
-    pat = tag_pattern(pose.tag_id, pose.family)
+    pat = tag_pattern(pose.tag_id, pose.family, pose.flips)
     val = pat[cy, cx] * (white - black) + black
     val = np.where(inside, val, 0.0)
     cov = inside.astype(np.float64)
@@ -197,6 +199,12 @@ def random_pose(rng: np.random.Generator, tag_id: int, cx: float, cy: float, sid
     rot = math.radians(float(rng.uniform(-max_rot_deg, max_rot_deg)))
     tilt = math.radians(float(rng.uniform(0.0, max_tilt_deg)))
     axis = float(rng.uniform(0.0, 2.0 * math.pi))
+    return TagPose(tag_id, square_corners(cx, cy, side, rot, tilt, axis))
+
+
+def square_corners(cx: float, cy: float, side: float, rot: float, tilt: float, axis: float) -> np.ndarray:
+    """(4,2) image corners of a square of side `side` px centred at (cx, cy): turned in-plane by `rot`, then tilted by
+    `tilt` about the in-plane axis at angle `axis` (radians), seen by a pinhole of focal length 4 * side."""
     f = 4.0 * side  # focal length in px for the mini pinhole model
     ax, ay = math.cos(axis), math.sin(axis)
     c, s = math.cos(tilt), math.sin(tilt)
@@ -213,7 +221,7 @@ def random_pose(rng: np.random.Generator, tag_id: int, cx: float, cy: float, sid
         Y = R[1, 0] * x + R[1, 1] * y
         Zc = R[2, 0] * x + R[2, 1] * y + f
         corners.append((cx + f * X / Zc, cy + f * Y / Zc))
-    return TagPose(tag_id, np.array(corners, dtype=np.float64))
+    return np.array(corners, dtype=np.float64)
 
 
 def make_scene(width: int, height: int, seed: int, n_tags: int, side_range=(60.0, 300.0), ids=None,

@@ -154,9 +154,10 @@ def _dlt(src, dst):
 TAG_CORNERS = [(-1.0, 1.0), (1.0, 1.0), (1.0, -1.0), (-1.0, -1.0)]  # det->p[i] = H * (tcx, tcy), quad_decode_task
 
 
-def check_detection_geometry(dets):
+def check_detection_geometry(dets, max_hamming=2):
     """Checks that need no oracle (they pin H, c and p of a detection against each other and against independent
-    homography solvers): H is THE homography that maps the tag corners (+-1, +-1) to p; c = H (0, 0)."""
+    homography solvers): H is THE homography that maps the tag corners (+-1, +-1) to p; c = H (0, 0).  `max_hamming`:
+    the largest any of the detector's families corrects (2 unless a family table says otherwise)."""
     for d in dets:
         H = np.asarray(d["H"], dtype=np.float64).reshape(3, 3)
         assert H[2, 2] != 0 and np.isfinite(H).all()
@@ -179,7 +180,7 @@ def check_detection_geometry(dets):
             assert np.abs(Hn[2, :2] - cvH[2, :2]).max() <= H_REL_TOL * max(np.abs(cvH[2, :2]).max(), 1.0 / a), "H[2,:] vs cv2"
         except ImportError:
             pass
-        assert 0 <= int(d["hamming"]) <= 2 and float(d["decision_margin"]) >= 0.0
+        assert 0 <= int(d["hamming"]) <= max_hamming and float(d["decision_margin"]) >= 0.0
     ids = [int(x) for x in dets["id"]]
     assert ids == sorted(ids), "detections are sorted by id (apriltag_detect.cu:662)"
 
@@ -208,11 +209,14 @@ def compare_detections(det: D.GpuDetector, orc, frame=0):
     ref = orc.detections
     assert [int(x) for x in got["id"]] == [int(x) for x in ref["id"]], "tag ids"
     assert np.array_equal(got["hamming"], ref["hamming"]), "hamming"
+    families = getattr(det, "families", ["tag36h11"])
     if "family" in got.dtype.names and "family" in ref.dtype.names:
-        # the engine numbers the families as its caller listed them, the oracle by its built-in table
+        # the engine numbers the families as its caller listed them; the oracle by its built-in table when it was
+        # given names only, else by the caller's list too (pyoracle.make_config)
         from oracle.pyoracle import FAMILY_NAMES
-        mine = [f if isinstance(f, str) else f.get("name") for f in getattr(det, "families", ["tag36h11"])]
-        assert [mine[int(i)] for i in got["family"]] == [FAMILY_NAMES[int(i)] for i in ref["family"]], "tag family"
+        mine = [f if isinstance(f, str) else f.get("name") for f in families]
+        theirs = FAMILY_NAMES if all(isinstance(f, str) for f in families) else mine
+        assert [mine[int(i)] for i in got["family"]] == [theirs[int(i)] for i in ref["family"]], "tag family"
     if len(ref):
         assert np.abs(got["p"] - ref["p"]).max() <= CORNER_TOL_PX, "corners"
         assert np.abs(got["c"] - ref["c"]).max() <= CORNER_TOL_PX, "centres"
@@ -221,8 +225,9 @@ def compare_detections(det: D.GpuDetector, orc, frame=0):
         dp = np.abs(got["p"] - ref["p"]).reshape(len(ref), -1).max(axis=1)
         dm = np.abs(got["decision_margin"].astype(np.float64) - ref["decision_margin"].astype(np.float64))
         assert (dm <= margin_tolerance(dp)).all(), f"decision margin: diff {dm.tolist()} at corner diff {dp.tolist()}"
-    check_detection_geometry(got)
-    check_detection_geometry(ref)
+    max_hamming = max(2 if isinstance(f, str) else int(f.get("max_hamming", 2)) for f in families)
+    check_detection_geometry(got, max_hamming)
+    check_detection_geometry(ref, max_hamming)
     return got
 
 
