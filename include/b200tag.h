@@ -462,6 +462,76 @@ int b200tag_debug_estimate_field_pose_distorted_device(const b200tag_detection *
                                                        const double *rotation, const double *offset,
                                                        b200tag_field_pose *out);
 
+/* Pose covariance: how far to trust a tag pose or a field pose, for a pose estimator's measurement noise (WPILib's
+ * addVisionMeasurement standard deviations).
+ *
+ * Convention.  A pose (R, t) maps X_a -> R X_a + t into frame b.  Its covariance C is the 6x6 covariance of
+ * xi = (r, dt) with R_true = exp([r]x) R and t_true = t + dt, r and dt expressed in frame b, in the order
+ * (rx, ry, rz, tx, ty, tz), rad and m; row-major, exactly symmetric.  For a tag pose (b200tag_pose) b is the camera
+ * frame; for the field results (camera_R / camera_t and robot_R / robot_t) it is the field frame.  The standard
+ * deviations of a robot Pose2d (x, y, heading) are then sqrt(C[3][3]), sqrt(C[4][4]) and sqrt(C[2][2]) of the robot
+ * covariance.
+ *
+ * Noise model.  Every coordinate of every detected corner (b200tag_detection.p, raw pixels) carries independent
+ * zero-mean noise of standard deviation sigma px, a caller-supplied constant.
+ *
+ * The covariance is that of the pixel least-squares pose over the corners the step used (a tag's four corners, or
+ * every corner the field solve used), linearised at the returned pose:
+ *   C = sigma^2 (J^T J)^-1 (sum_i J_i^T A_i A_i^T J_i) (J^T J)^-1,
+ * J the Jacobian of the ideal-image (undistorted) projections with respect to xi, J_i corner i's 2x6 block of it, and
+ * A_i the 2x2 Jacobian of the undistortion at corner i in pixels: diag(fx, fy) (dx_d/dx_u)^-1 diag(1/fx, 1/fy).  The
+ * lens stretches a raw pixel's noise at the frame's edges (about 2.4x for a wide-angle lens), which A_i accounts for.
+ * Without distortion A_i = I and C = sigma^2 (J^T J)^-1.  C is computed for sigma = 1 and multiplied by sigma^2 last,
+ * so C(2 sigma) = 4 C(sigma) bit for bit.  Only + - * / and sqrt: host and device results are bit-identical.
+ *
+ * For the field pose, which minimises exactly this pixel error, this is the usual first-order covariance.  For a tag
+ * pose from OI or IPPE it is the first-order covariance of the pixel least-squares estimate at the returned pose, not
+ * of those estimators themselves; DESIGN.md section 9 lists how close they come in a Monte Carlo test.
+ *
+ * Failure: a failed pose record (err == HUGE_VAL), a corner that cannot be undistorted or is behind the camera, a J^T J
+ * that is not positive definite, or a field pose with num_tags == 0 gives all 36 entries HUGE_VAL. */
+typedef struct b200tag_covariance {
+  double C[36];
+} b200tag_covariance;
+typedef struct b200tag_field_covariance {
+  double camera[36];  /* of camera_R / camera_t */
+  double robot[36];   /* of robot_R / robot_t */
+} b200tag_field_covariance;
+/* out[i] = the covariance of poses[i], the pose of dets[i] estimated by either method (with `dist` as given to
+ * b200tag_estimate_poses_distorted).  `dist` as there: NULL or all zero means no distortion.  B200TAG_E_INVALID unless
+ * sigma is finite and > 0, and as b200tag_estimate_poses_distorted. */
+int b200tag_estimate_pose_covariances(const b200tag_detection *dets, const b200tag_pose *poses, int count, double tagsize,
+                                      double fx, double fy, double cx, double cy, const double *dist, double sigma,
+                                      b200tag_covariance *out);
+/* b200tag_estimate_field_pose_distorted (its pose, bit for bit) and the covariance of its camera and robot poses.  With
+ * one tag, the covariance is that of the returned candidate.  B200TAG_E_INVALID unless sigma is finite and > 0, and as
+ * b200tag_estimate_field_pose_distorted. */
+int b200tag_estimate_field_pose_covariance(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
+                                           int nlayout, double tagsize, double fx, double fy, double cx, double cy,
+                                           const double *dist, const double *rotation, const double *offset, double sigma,
+                                           b200tag_field_pose *out, b200tag_field_covariance *cov);
+/* The covariances on the device, from the next detect call: sigma > 0 turns them on, 0 off.  With the pose step on, a
+ * kernel after it computes every detection's covariance (one more kernel in b200tag_kernels_per_batch); with the field
+ * step on, the field kernel adds the field covariance (no kernel added).  Independent of the method, distortion and
+ * layout setters.  B200TAG_E_INVALID (state unchanged) for any other sigma.  Off, nothing changes: results, launches and
+ * allocations are those of a detector that never turned it on. */
+int b200tag_set_pose_covariance(b200tag_detector *det, double sigma);
+/* Covariances of frame `frame` of the last call, parallel to b200tag_poses; NULL and *count = 0 when the last call ran
+ * without them.  Owned by the detector, valid until the next detect call. */
+const b200tag_covariance *b200tag_pose_covariances(const b200tag_detector *det, int frame, int *count);
+/* The field covariance of frame `frame` of the last call, for b200tag_field_pose_get's pose; NULL when the last call
+ * ran without it. */
+const b200tag_field_covariance *b200tag_field_covariance_get(const b200tag_detector *det, int frame);
+/* Test hooks: the device kernels on caller-supplied records and a raw list; arguments and results as the host
+ * functions above. */
+int b200tag_debug_pose_covariances_device(const b200tag_detection *dets, const b200tag_pose *poses, int count,
+                                          double tagsize, double fx, double fy, double cx, double cy, const double *dist,
+                                          double sigma, b200tag_covariance *out);
+int b200tag_debug_field_pose_covariance_device(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
+                                               int nlayout, double tagsize, double fx, double fy, double cx, double cy,
+                                               const double *dist, const double *rotation, const double *offset,
+                                               double sigma, b200tag_field_pose *out, b200tag_field_covariance *cov);
+
 /* Pinned host staging memory, so b200tag_detect* can overlap H2D with compute. */
 void *b200tag_alloc_pinned(size_t bytes);
 /* Write-combined pinned memory: for buffers the CPU (or a capture driver) only ever WRITES, such as a camera ring

@@ -123,6 +123,7 @@ struct b200tag_detector {
     double rotation[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, offset[3] = {0, 0, 0};
     int method = B200TAG_POSE_ORTHOGONAL_ITERATION;  // b200tag_set_pose_method
     double dist[5] = {0, 0, 0, 0, 0};                 // b200tag_set_pose_distortion; all zero: none
+    double sigma = 0;                                 // b200tag_set_pose_covariance; 0: no covariances
   };
   PoseSettings pose, last_pose;                // current; what the last enqueue ran with
   b200tag_pose *h_poses = nullptr;             // pinned + mapped, parallel to h_dets; allocated when first turned on
@@ -140,6 +141,13 @@ struct b200tag_detector {
   b200tag_field_pose *h_field = nullptr;       // pinned + mapped, max_batch entries
   b200tag_field_pose *d_field_alias = nullptr;
   std::vector<b200tag_field_pose> field_poses; // per frame of the last call
+  // the covariances (b200tag_set_pose_covariance): pinned + mapped, allocated when first turned on
+  b200tag_covariance *h_cov = nullptr;         // parallel to h_dets
+  b200tag_covariance *d_cov_alias = nullptr;
+  b200tag_field_covariance *h_field_cov = nullptr;  // max_batch entries
+  b200tag_field_covariance *d_field_cov_alias = nullptr;
+  std::vector<std::vector<b200tag_covariance>> covs;  // parallel to dets
+  std::vector<b200tag_field_covariance> field_covs;   // per frame of the last call
 };
 
 namespace b200tag {
@@ -258,8 +266,15 @@ struct DetPose {
   b200tag_detection det;
   b200tag_pose pose;
 };
+// The same with the pose's covariance (b200tag_set_pose_covariance).
+struct DetPoseCov {
+  b200tag_detection det;
+  b200tag_pose pose;
+  b200tag_covariance cov;
+};
 const b200tag_detection &rec(const b200tag_detection &d) { return d; }
 const b200tag_detection &rec(const DetPose &d) { return d.det; }
+const b200tag_detection &rec(const DetPoseCov &d) { return d.det; }
 
 template <class T>
 void reconcile(std::vector<T> &v) {
@@ -348,7 +363,23 @@ int finish_impl(b200tag_detector *det) {
     const Counters &c = det->h_counters[f];
     const uint32_t nd = std::min(c.num_detections, det->fp.det_cap);
     const b200tag_detection *src = det->h_dets + static_cast<size_t>(f) * det->fp.det_cap;
-    if (det->last_pose.tagsize > 0) {
+    if (det->last_pose.tagsize > 0 && det->last_pose.sigma > 0) {
+      const size_t o = static_cast<size_t>(f) * det->fp.det_cap;
+      std::vector<DetPoseCov> all(nd);
+      for (uint32_t i = 0; i < nd; i++) all[i] = DetPoseCov{src[i], det->h_poses[o + i], det->h_cov[o + i]};
+      reconcile(all);
+      det->dets[f].resize(all.size());
+      det->poses[f].resize(all.size());
+      det->covs[f].resize(all.size());
+      for (size_t i = 0; i < all.size(); i++) {
+        det->dets[f][i] = all[i].det;
+        det->poses[f][i] = all[i].pose;
+        det->covs[f][i] = all[i].cov;
+      }
+      det->positions[f].resize(all.size());
+      locate_from_poses(det->dets[f].data(), det->poses[f].data(), static_cast<int>(all.size()), det->last_pose.rotation,
+                        det->last_pose.offset, det->positions[f].data());
+    } else if (det->last_pose.tagsize > 0) {
       const b200tag_pose *ps = det->h_poses + static_cast<size_t>(f) * det->fp.det_cap;
       std::vector<DetPose> both(nd);
       for (uint32_t i = 0; i < nd; i++) both[i] = DetPose{src[i], ps[i]};
@@ -369,6 +400,7 @@ int finish_impl(b200tag_detector *det) {
       det->positions[f].clear();
     }
     if (det->last_field) det->field_poses[f] = det->h_field[f];
+    if (det->last_field && det->last_pose.sigma > 0) det->field_covs[f] = det->h_field_cov[f];
     det->quads_valid[f] = false;
     if (c.status) rc = B200TAG_E_OVERFLOW;
   }
@@ -401,6 +433,7 @@ int record_sequence(b200tag_detector *det, const void *device_images, size_t str
                   ps.method, {}};
     memcpy(pl.dist, ps.dist, sizeof(pl.dist));
     launch_pose(pl, count, ln);
+    if (ps.sigma > 0) launch_pose_cov(pl, det->d_cov_alias, ps.sigma, count, ln);
     if (det->field_n > 0) {
       FieldLaunch fl{det->d_dets_alias, p.counters, p.det_cap, 0, det->d_field_layout, det->d_field_keys, det->field_n,
                      static_cast<pose::FieldTagData *>(det->d_field_scratch), det->field_scratch_stride,
@@ -408,6 +441,8 @@ int record_sequence(b200tag_detector *det, const void *device_images, size_t str
       memcpy(fl.rotation, ps.rotation, sizeof(fl.rotation));
       memcpy(fl.offset, ps.offset, sizeof(fl.offset));
       memcpy(fl.dist, ps.dist, sizeof(fl.dist));
+      fl.cov = det->d_field_cov_alias;
+      fl.sigma = ps.sigma;
       launch_field_pose(fl, count, ln);
     }
   }
@@ -787,6 +822,8 @@ int b200tag_create_families(const b200tag_config *cfg, const b200tag_family *fam
   det->poses.resize(B);
   det->positions.resize(B);
   det->field_poses.resize(B);
+  det->covs.resize(B);
+  det->field_covs.resize(B);
   det->quads.resize(B);
   det->quads_valid.assign(B, false);
   memset(det->h_counters, 0, sizeof(Counters) * B);
@@ -827,6 +864,8 @@ void b200tag_destroy(b200tag_detector *det) {
   if (det->d_field_keys) cudaFree(det->d_field_keys);
   if (det->d_field_scratch) cudaFree(det->d_field_scratch);
   if (det->h_field) cudaFreeHost(det->h_field);
+  if (det->h_cov) cudaFreeHost(det->h_cov);
+  if (det->h_field_cov) cudaFreeHost(det->h_field_cov);
   delete det;
 }
 
@@ -1259,6 +1298,21 @@ const b200tag_field_pose *b200tag_field_pose_get(const b200tag_detector *det, in
   return &det->field_poses[frame];
 }
 
+const b200tag_covariance *b200tag_pose_covariances(const b200tag_detector *det, int frame, int *count) {
+  if (count) *count = 0;
+  if (!det || frame < 0 || frame >= det->last_count || det->pending || !(det->last_pose.tagsize > 0) ||
+      !(det->last_pose.sigma > 0))
+    return nullptr;
+  if (count) *count = static_cast<int>(det->covs[frame].size());
+  return det->covs[frame].data();
+}
+
+const b200tag_field_covariance *b200tag_field_covariance_get(const b200tag_detector *det, int frame) {
+  if (!det || frame < 0 || frame >= det->last_count || det->pending || !det->last_field || !(det->last_pose.sigma > 0))
+    return nullptr;
+  return &det->field_covs[frame];
+}
+
 const b200tag_tag_position *b200tag_tag_positions(const b200tag_detector *det, int frame, int *count) {
   if (count) *count = 0;
   if (!det || frame < 0 || frame >= det->last_count || det->pending || !(det->last_pose.tagsize > 0)) return nullptr;
@@ -1482,6 +1536,34 @@ int b200tag_set_pose_distortion(b200tag_detector *det, const double *dist) {
   return 0;
 }
 
+int b200tag_set_pose_covariance(b200tag_detector *det, double sigma) {
+  if (!det || !(sigma == 0 || valid_sigma(sigma))) return B200TAG_E_INVALID;
+  DeviceGuard on_device(det->device);
+  if (sigma > 0 && !det->h_cov) {
+    const size_t B = static_cast<size_t>(det->cfg.max_batch);
+    b200tag_covariance *h = nullptr, *d = nullptr;
+    b200tag_field_covariance *hf = nullptr, *df = nullptr;
+    const bool ok = cudaHostAlloc(reinterpret_cast<void **>(&h), sizeof(b200tag_covariance) * det->fp.det_cap * B, cudaHostAllocMapped) == cudaSuccess &&
+                    cudaHostGetDevicePointer(reinterpret_cast<void **>(&d), h, 0) == cudaSuccess &&
+                    cudaHostAlloc(reinterpret_cast<void **>(&hf), sizeof(b200tag_field_covariance) * B, cudaHostAllocMapped) == cudaSuccess &&
+                    cudaHostGetDevicePointer(reinterpret_cast<void **>(&df), hf, 0) == cudaSuccess;
+    if (!ok) {
+      cudaGetLastError();
+      if (h) cudaFreeHost(h);
+      if (hf) cudaFreeHost(hf);
+      det->err = "allocating the covariance buffers failed";
+      return B200TAG_E_CUDA;
+    }
+    det->h_cov = h;
+    det->d_cov_alias = d;
+    det->h_field_cov = hf;
+    det->d_field_cov_alias = df;
+  }
+  drop_graphs(det);  // the kernels and sigma are baked into the captured launches
+  det->pose.sigma = sigma;
+  return 0;
+}
+
 int b200tag_set_distortion(b200tag_detector *det, double k1, double k2, double p1, double p2, double k3) {
   if (!det) return B200TAG_E_INVALID;
   DeviceGuard on_device(det->device);
@@ -1592,6 +1674,50 @@ int estimate_poses_device(int method, const b200tag_detection *dets, int count, 
   return rc;
 }
 
+// The field hook's common part: k_field_pose on one caller list; with sigma > 0 the variant with the covariance.
+int field_pose_device(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout,
+                      double tagsize, double fx, double fy, double cx, double cy, const double *dist,
+                      const double *rotation, const double *offset, double sigma, b200tag_field_pose *out,
+                      b200tag_field_covariance *cov) {
+  bool active;
+  pose::Distortion D;
+  if (count < 0 || (count > 0 && !dets) || !out || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
+  if (!read_distortion(dist, &active, &D)) return B200TAG_E_INVALID;
+  std::vector<pose::FieldKey> keys(static_cast<size_t>(std::max(nlayout, 0)));
+  if (!field_layout_keys(layout, nlayout, nullptr, 0, keys.data())) return B200TAG_E_INVALID;
+  const size_t db = sizeof(b200tag_detection) * static_cast<size_t>(count), lb = sizeof(b200tag_field_tag) * nlayout,
+               kb = sizeof(pose::FieldKey) * nlayout, sb = field_tag_bytes() * std::max(count, 1);
+  const size_t o_l = align_up(db, 256), o_k = align_up(o_l + lb, 256), o_s = align_up(o_k + kb, 256), o_o = align_up(o_s + sb, 256);
+  const size_t o_c = align_up(o_o + sizeof(b200tag_field_pose), 256);
+  uint8_t *d = nullptr;
+  if (cudaMalloc(&d, o_c + (cov ? sizeof(b200tag_field_covariance) : 0)) != cudaSuccess) {
+    cudaGetLastError();
+    return B200TAG_E_NO_DEVICE;
+  }
+  static const double kEye[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, kZero[3] = {0, 0, 0};
+  FieldLaunch fl{reinterpret_cast<const b200tag_detection *>(d), nullptr, 0, static_cast<uint32_t>(count),
+                 reinterpret_cast<const b200tag_field_tag *>(d + o_l), reinterpret_cast<const pose::FieldKey *>(d + o_k), nlayout,
+                 reinterpret_cast<pose::FieldTagData *>(d + o_s), 0, tagsize, fx, fy, cx, cy, {}, {},
+                 reinterpret_cast<b200tag_field_pose *>(d + o_o), {D.k1, D.k2, D.p1, D.p2, D.k3},
+                 cov ? reinterpret_cast<b200tag_field_covariance *>(d + o_c) : nullptr, cov ? sigma : 0};
+  memcpy(fl.rotation, rotation ? rotation : kEye, sizeof(fl.rotation));
+  memcpy(fl.offset, offset ? offset : kZero, sizeof(fl.offset));
+  int rc = 0;
+  if ((db && cudaMemcpy(d, dets, db, cudaMemcpyHostToDevice) != cudaSuccess) ||
+      (lb && cudaMemcpy(d + o_l, layout, lb, cudaMemcpyHostToDevice) != cudaSuccess) ||
+      (kb && cudaMemcpy(d + o_k, keys.data(), kb, cudaMemcpyHostToDevice) != cudaSuccess))
+    rc = B200TAG_E_CUDA;
+  if (!rc) {
+    Launcher ln{nullptr, nullptr};
+    launch_field_pose(fl, 1, ln);
+    if (cudaGetLastError() != cudaSuccess || cudaMemcpy(out, d + o_o, sizeof(*out), cudaMemcpyDeviceToHost) != cudaSuccess ||
+        (cov && cudaMemcpy(cov, d + o_c, sizeof(*cov), cudaMemcpyDeviceToHost) != cudaSuccess))
+      rc = B200TAG_E_CUDA;
+  }
+  cudaFree(d);
+  return rc;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1624,37 +1750,42 @@ int b200tag_debug_estimate_field_pose_distorted_device(const b200tag_detection *
                                                        double fx, double fy, double cx, double cy, const double *dist,
                                                        const double *rotation, const double *offset,
                                                        b200tag_field_pose *out) {
+  return field_pose_device(dets, count, layout, nlayout, tagsize, fx, fy, cx, cy, dist, rotation, offset, 0, out, nullptr);
+}
+
+int b200tag_debug_field_pose_covariance_device(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
+                                               int nlayout, double tagsize, double fx, double fy, double cx, double cy,
+                                               const double *dist, const double *rotation, const double *offset,
+                                               double sigma, b200tag_field_pose *out, b200tag_field_covariance *cov) {
+  if (!valid_sigma(sigma) || !cov) return B200TAG_E_INVALID;
+  return field_pose_device(dets, count, layout, nlayout, tagsize, fx, fy, cx, cy, dist, rotation, offset, sigma, out, cov);
+}
+
+int b200tag_debug_pose_covariances_device(const b200tag_detection *dets, const b200tag_pose *poses, int count,
+                                          double tagsize, double fx, double fy, double cx, double cy, const double *dist,
+                                          double sigma, b200tag_covariance *out) {
   bool active;
   pose::Distortion D;
-  if (count < 0 || (count > 0 && !dets) || !out || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
-  if (!read_distortion(dist, &active, &D)) return B200TAG_E_INVALID;
-  std::vector<pose::FieldKey> keys(static_cast<size_t>(std::max(nlayout, 0)));
-  if (!field_layout_keys(layout, nlayout, nullptr, 0, keys.data())) return B200TAG_E_INVALID;
-  const size_t db = sizeof(b200tag_detection) * static_cast<size_t>(count), lb = sizeof(b200tag_field_tag) * nlayout,
-               kb = sizeof(pose::FieldKey) * nlayout, sb = field_tag_bytes() * std::max(count, 1);
-  const size_t o_l = align_up(db, 256), o_k = align_up(o_l + lb, 256), o_s = align_up(o_k + kb, 256), o_o = align_up(o_s + sb, 256);
+  if (!valid_sigma(sigma) || !read_distortion(dist, &active, &D)) return B200TAG_E_INVALID;
+  if (count < 0 || (count > 0 && (!dets || !poses || !out))) return B200TAG_E_INVALID;
+  if (count > 0 && (!(tagsize > 0) || fx == 0 || fy == 0)) return B200TAG_E_INVALID;
+  if (count == 0) return 0;
+  const size_t db = sizeof(b200tag_detection) * static_cast<size_t>(count), pb = sizeof(b200tag_pose) * static_cast<size_t>(count),
+               cb = sizeof(b200tag_covariance) * static_cast<size_t>(count);
   uint8_t *d = nullptr;
-  if (cudaMalloc(&d, o_o + sizeof(b200tag_field_pose)) != cudaSuccess) {
+  if (cudaMalloc(&d, db + pb + cb) != cudaSuccess) {
     cudaGetLastError();
     return B200TAG_E_NO_DEVICE;
   }
-  static const double kEye[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, kZero[3] = {0, 0, 0};
-  FieldLaunch fl{reinterpret_cast<const b200tag_detection *>(d), nullptr, 0, static_cast<uint32_t>(count),
-                 reinterpret_cast<const b200tag_field_tag *>(d + o_l), reinterpret_cast<const pose::FieldKey *>(d + o_k), nlayout,
-                 reinterpret_cast<pose::FieldTagData *>(d + o_s), 0, tagsize, fx, fy, cx, cy, {}, {},
-                 reinterpret_cast<b200tag_field_pose *>(d + o_o), {D.k1, D.k2, D.p1, D.p2, D.k3}};
-  memcpy(fl.rotation, rotation ? rotation : kEye, sizeof(fl.rotation));
-  memcpy(fl.offset, offset ? offset : kZero, sizeof(fl.offset));
   int rc = 0;
-  if ((db && cudaMemcpy(d, dets, db, cudaMemcpyHostToDevice) != cudaSuccess) ||
-      (lb && cudaMemcpy(d + o_l, layout, lb, cudaMemcpyHostToDevice) != cudaSuccess) ||
-      (kb && cudaMemcpy(d + o_k, keys.data(), kb, cudaMemcpyHostToDevice) != cudaSuccess))
+  const PoseLaunch pl{reinterpret_cast<const b200tag_detection *>(d), reinterpret_cast<b200tag_pose *>(d + db), nullptr,
+                      0, static_cast<uint32_t>(count), tagsize, fx, fy, cx, cy, B200TAG_POSE_IPPE, {D.k1, D.k2, D.p1, D.p2, D.k3}};
+  if (cudaMemcpy(d, dets, db, cudaMemcpyHostToDevice) != cudaSuccess || cudaMemcpy(d + db, poses, pb, cudaMemcpyHostToDevice) != cudaSuccess)
     rc = B200TAG_E_CUDA;
   if (!rc) {
     Launcher ln{nullptr, nullptr};
-    launch_field_pose(fl, 1, ln);
-    if (cudaGetLastError() != cudaSuccess || cudaMemcpy(out, d + o_o, sizeof(*out), cudaMemcpyDeviceToHost) != cudaSuccess)
-      rc = B200TAG_E_CUDA;
+    launch_pose_cov(pl, reinterpret_cast<b200tag_covariance *>(d + db + pb), sigma, 1, ln);
+    if (cudaGetLastError() != cudaSuccess || cudaMemcpy(out, d + db + pb, cb, cudaMemcpyDeviceToHost) != cudaSuccess) rc = B200TAG_E_CUDA;
   }
   cudaFree(d);
   return rc;

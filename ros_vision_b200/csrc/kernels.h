@@ -90,6 +90,9 @@ struct PoseLaunch {
   double dist[5];                 // {k1, k2, p1, p2, k3} of b200tag_set_pose_distortion; all zero: no undistortion step
 };
 void launch_pose(const PoseLaunch &L, int frames, Launcher &ln);
+// b200tag_set_pose_covariance: k_pose_cov after launch_pose(L), the covariances of L.out's poses into `cov` (L.out's
+// layout) at sigma > 0.
+void launch_pose_cov(const PoseLaunch &L, b200tag_covariance *cov, double sigma, int frames, Launcher &ln);
 
 // The field pose step (kernels_pose.cu, k_field_pose): one b200tag_field_pose per frame from the frame's raw records.
 namespace pose {
@@ -109,6 +112,8 @@ struct FieldLaunch {
   double rotation[9], offset[3];
   b200tag_field_pose *out;           // one per frame
   double dist[5];                    // as PoseLaunch::dist
+  b200tag_field_covariance *cov;     // one per frame; written by the variant with covariance (sigma > 0)
+  double sigma;
 };
 void launch_field_pose(const FieldLaunch &L, int frames, Launcher &ln);
 // True when `dist` ({k1, k2, p1, p2, k3}) has a non-zero coefficient: the launches then choose the kernels' variants

@@ -5,7 +5,8 @@
 // pose_core.h's, the same the host functions in pose.cc run.  With b200tag_set_pose_method(B200TAG_POSE_IPPE) the step
 // is k_pose_ippe instead: the closed-form IPPE pose, one thread per detection.  With b200tag_set_pose_distortion each
 // kernel's variant with kDistorted = true runs: it undistorts the corners first (pose_core.h's undistort_point); the
-// variant without compiles to the kernel without the step.
+// variant without compiles to the kernel without the step.  With b200tag_set_pose_covariance, k_pose_cov runs behind
+// either pose kernel and writes every pose's covariance.
 //
 // A pose depends only on its own record, so computing it before the host's reconcile gives the pose of every
 // detection that survives it.
@@ -195,11 +196,72 @@ __global__ void __launch_bounds__(kIppeThreads) k_pose_ippe(PoseLaunch L) {
   }
 }
 
+// The covariance (b200tag_set_pose_covariance) of every raw detection's pose, behind k_pose or k_pose_ippe: one thread
+// per record, laid out as k_pose_ippe.  A thread reads the record's corners and its pose from the mapped buffers and
+// writes the 36 entries to the same index of the mapped covariance buffer; the arithmetic is tag_covariance, which the
+// host's b200tag_estimate_pose_covariances runs too.  kDistorted: through the lens of b200tag_set_pose_distortion.
+template <bool kDistorted>
+__global__ void __launch_bounds__(kIppeThreads) k_pose_cov(PoseLaunch L, b200tag_covariance *cov, double sigma) {
+  static_assert(sizeof(b200tag_covariance) % 16 == 0, "covariance stores");
+  const size_t frame = blockIdx.y;
+  const uint32_t n = L.counters ? min(L.counters[frame].num_detections, L.stride) : L.count;
+  const b200tag_detection *recs = L.dets + frame * L.stride;
+  const b200tag_pose *poses = L.out + frame * L.stride;
+  b200tag_covariance *out = cov + frame * L.stride;
+  const FieldCamera cam{L.fx, L.fy, L.cx, L.cy};
+  const Distortion D = lens(L.dist);
+  for (uint32_t i = blockIdx.x * kIppeThreads + threadIdx.x; i < n; i += gridDim.x * kIppeThreads) {
+    const double2 *src = reinterpret_cast<const double2 *>(recs[i].p);
+    double px[4][2];
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+      const double2 c = src[k];
+      px[k][0] = c.x;
+      px[k][1] = c.y;
+    }
+    b200tag_pose pose;
+    const double2 *ps = reinterpret_cast<const double2 *>(poses + i);
+#pragma unroll
+    for (int k = 0; k < static_cast<int>(sizeof(b200tag_pose) / 16); k++) reinterpret_cast<double2 *>(&pose)[k] = ps[k];
+    b200tag_covariance c;
+    tag_covariance(px, pose, L.tagsize, cam, kDistorted ? &D : nullptr, sigma, c.C);
+    double2 *dst = reinterpret_cast<double2 *>(out + i);
+#pragma unroll
+    for (int k = 0; k < static_cast<int>(sizeof(b200tag_covariance) / 16); k++) dst[k] = reinterpret_cast<const double2 *>(&c)[k];
+  }
+}
+
 // The sum of v over the warp by the xor tree of pose_core.h (field_slot_tree): every lane ends with the same bits.
 __device__ double warp_sum(double v) {
 #pragma unroll
   for (int m = kFieldSlots / 2; m >= 1; m >>= 1) v = v + __shfl_xor_sync(kFull, v, m);
   return v;
+}
+
+// The field covariance of result `res` over the frame's `used` tags (k_field_pose with kCov): correspondence k on lane
+// k % 32, the sums by warp_sum, then field_covariance on every lane; the lanes write the result between them.  Not
+// inlined, so the solve's register allocation is that of the kernel without it.
+template <bool kDistorted>
+__device__ __noinline__ void field_covariance_warp(const FieldTagData *tags, int used, const b200tag_field_pose &res,
+                                                   const FieldLaunch &L, int lane, b200tag_field_covariance *dst) {
+  constexpr int kSums = kDistorted ? kCovSums : 22;  // without distortion B is not summed
+  M3 R;
+  V3 t;
+  field_cov_pose(res, &R, &t);
+  const FieldCamera cam{L.fx, L.fy, L.cx, L.cy};
+  const Distortion D = lens(L.dist);
+  double acc[kCovSums];
+#pragma unroll
+  for (int j = 0; j < kCovSums; j++) acc[j] = 0;
+  for (int k = lane; k < 4 * used; k += 32) field_cov_corner_terms(tags[k >> 2], k & 3, R, t, cam, kDistorted ? &D : nullptr, acc);
+  double S[kCovSums];
+#pragma unroll
+  for (int j = 0; j < kCovSums; j++) S[j] = j < kSums ? warp_sum(acc[j]) : 0.0;
+  b200tag_field_covariance out;
+  field_covariance(S, kDistorted, res, L.offset, L.sigma, &out);
+  static_assert(sizeof(b200tag_field_covariance) / 8 <= 96, "covariance copy");
+  for (int w = lane; w < static_cast<int>(sizeof(b200tag_field_covariance) / 8); w += 32)
+    reinterpret_cast<double *>(dst)[w] = reinterpret_cast<const double *>(&out)[w];
 }
 
 // The field pose (b200tag_set_field_layout) of every frame: one warp per frame, blockIdx.x = frame, reading the frame's
@@ -208,7 +270,9 @@ __device__ double warp_sum(double v) {
 // seeds to the frame's scratch, and then run field_solve with correspondence k on lane k % 32 and the 6x6 solve on every
 // lane.  The arithmetic is pose_core.h's, the same b200tag_estimate_field_pose runs on the host.  With kDistorted the
 // lane that owns a used layout tag undistorts its chosen record's corners first and leaves the tag out when one fails.
-template <bool kDistorted>
+// With kCov the warp adds the covariance of the result (field_covariance_warp); the variants without it compile to the
+// kernel without the step.
+template <bool kDistorted, bool kCov>
 __global__ void __launch_bounds__(32) k_field_pose(FieldLaunch L) {
   __shared__ int cnt[B200TAG_MAX_FIELD_TAGS], sel[B200TAG_MAX_FIELD_TAGS];
   __shared__ int dup;
@@ -304,6 +368,7 @@ __global__ void __launch_bounds__(32) k_field_pose(FieldLaunch L) {
     };
     field_solve(tags, used, cost, sum, L.rotation, L.offset, &res);
   }
+  if (kCov) field_covariance_warp<kDistorted>(tags, used, res, L, lane, L.cov + frame);
   if (lane == 0) L.out[frame] = res;
 }
 
@@ -312,14 +377,28 @@ __global__ void __launch_bounds__(32) k_field_pose(FieldLaunch L) {
 size_t field_tag_bytes() { return sizeof(FieldTagData); }
 
 void launch_field_pose(const FieldLaunch &L, int frames, Launcher &ln) {
-  const auto kernel = has_distortion(L.dist) ? k_field_pose<true> : k_field_pose<false>;
+  const bool cov = L.sigma > 0;
+  const auto kernel = has_distortion(L.dist) ? (cov ? k_field_pose<true, true> : k_field_pose<true, false>)
+                                             : (cov ? k_field_pose<false, true> : k_field_pose<false, false>);
   ln.timed("field_pose", [&] { kernel<<<static_cast<unsigned>(frames), 32, 0, ln.s>>>(L); });
+}
+
+// One thread per record, all of a frame's records in one pass up to 1024 of them; CTAs past a frame's count exit.
+static unsigned per_record_ctas(const PoseLaunch &L) {
+  return L.counters ? min((L.stride + kIppeThreads - 1) / kIppeThreads, 8u) : (L.count + kIppeThreads - 1) / kIppeThreads;
+}
+
+void launch_pose_cov(const PoseLaunch &L, b200tag_covariance *cov, double sigma, int frames, Launcher &ln) {
+  const unsigned ctas = per_record_ctas(L);
+  const auto kernel = has_distortion(L.dist) ? k_pose_cov<true> : k_pose_cov<false>;
+  ln.timed("pose_cov", [&] {
+    if (ctas > 0) kernel<<<dim3(ctas, static_cast<unsigned>(frames)), kIppeThreads, 0, ln.s>>>(L, cov, sigma);
+  });
 }
 
 void launch_pose(const PoseLaunch &L, int frames, Launcher &ln) {
   if (L.method == B200TAG_POSE_IPPE) {
-    // one thread per record, all of a frame's records in one pass up to 1024 of them; CTAs past a frame's count exit
-    const unsigned ctas = L.counters ? min((L.stride + kIppeThreads - 1) / kIppeThreads, 8u) : (L.count + kIppeThreads - 1) / kIppeThreads;
+    const unsigned ctas = per_record_ctas(L);
     const auto kernel = has_distortion(L.dist) ? k_pose_ippe<true> : k_pose_ippe<false>;
     ln.timed("pose_ippe", [&] {
       if (ctas > 0) kernel<<<dim3(ctas, static_cast<unsigned>(frames)), kIppeThreads, 0, ln.s>>>(L);

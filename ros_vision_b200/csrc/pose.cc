@@ -64,6 +64,8 @@ bool read_distortion(const double *dist, bool *active, pose::Distortion *D) {
   return true;
 }
 
+bool valid_sigma(double sigma) { return std::isfinite(sigma) && sigma > 0; }
+
 }  // namespace b200tag
 
 using namespace b200tag::pose;
@@ -148,10 +150,25 @@ int b200tag_locate_tags(const b200tag_detection *dets, int count, double tagsize
 
 namespace {
 
-// b200tag_estimate_field_pose(_distorted); `lens` null: no undistortion step.
+// The field covariance of result `res` over the corners of the used tags, summed in the solve's slot order.
+void field_covariance_of(const FieldTagData *tags, int ntags, const FieldCamera &cam, const Distortion *lens,
+                         const double *offset, double sigma, const b200tag_field_pose &res, b200tag_field_covariance *cov) {
+  M3 R;
+  V3 t;
+  field_cov_pose(res, &R, &t);
+  double slot[kFieldSlots][kCovSums] = {}, S[kCovSums];
+  for (int k = 0; k < 4 * ntags; k++) {
+    field_cov_corner_terms(tags[k >> 2], k & 3, R, t, cam, lens, slot[k % kFieldSlots]);
+  }
+  field_slot_tree<kCovSums>(slot, S);
+  field_covariance(S, lens != nullptr, res, offset, sigma, cov);
+}
+
+// b200tag_estimate_field_pose(_distorted); `lens` null: no undistortion step.  With `cov`, also the covariance of the
+// result at sigma (b200tag_estimate_field_pose_covariance).
 int field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout, double tagsize,
                double fx, double fy, double cx, double cy, const Distortion *lens, const double *rotation,
-               const double *offset, b200tag_field_pose *out) {
+               const double *offset, b200tag_field_pose *out, double sigma = 0, b200tag_field_covariance *cov = nullptr) {
   if (count < 0 || (count > 0 && !dets) || !out || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
   std::vector<FieldKey> keys(static_cast<size_t>(std::max(nlayout, 0)));
   if (!b200tag::field_layout_keys(layout, nlayout, nullptr, 0, keys.data())) return B200TAG_E_INVALID;
@@ -177,6 +194,7 @@ int field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag
   const int ntags = static_cast<int>(tags.size());
   if (ntags == 0) {
     field_empty(out);
+    if (cov) field_covariance_of(tags.data(), 0, cam, lens, ox, sigma, *out, cov);
     return 0;
   }
   const int ncorr = 4 * ntags;
@@ -201,6 +219,7 @@ int field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag
     field_slot_tree<kFieldSums>(slot, S);
   };
   field_solve(tags.data(), ntags, cost, sum, Rx, ox, out);
+  if (cov) field_covariance_of(tags.data(), ntags, cam, lens, ox, sigma, *out, cov);
   return 0;
 }
 
@@ -264,6 +283,30 @@ int b200tag_estimate_field_pose_distorted(const b200tag_detection *dets, int cou
   Distortion D;
   if (!b200tag::read_distortion(dist, &active, &D)) return B200TAG_E_INVALID;
   return field_pose(dets, count, layout, nlayout, tagsize, fx, fy, cx, cy, active ? &D : nullptr, rotation, offset, out);
+}
+
+int b200tag_estimate_pose_covariances(const b200tag_detection *dets, const b200tag_pose *poses, int count, double tagsize,
+                                      double fx, double fy, double cx, double cy, const double *dist, double sigma,
+                                      b200tag_covariance *out) {
+  bool active;
+  Distortion D;
+  if (!b200tag::valid_sigma(sigma) || !b200tag::read_distortion(dist, &active, &D)) return B200TAG_E_INVALID;
+  if (count < 0 || (count > 0 && (!dets || !poses || !out))) return B200TAG_E_INVALID;
+  if (count > 0 && (!(tagsize > 0) || fx == 0 || fy == 0)) return B200TAG_E_INVALID;
+  const FieldCamera cam{fx, fy, cx, cy};
+  for (int i = 0; i < count; i++) tag_covariance(dets[i].p, poses[i], tagsize, cam, active ? &D : nullptr, sigma, out[i].C);
+  return 0;
+}
+
+int b200tag_estimate_field_pose_covariance(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
+                                           int nlayout, double tagsize, double fx, double fy, double cx, double cy,
+                                           const double *dist, const double *rotation, const double *offset, double sigma,
+                                           b200tag_field_pose *out, b200tag_field_covariance *cov) {
+  bool active;
+  Distortion D;
+  if (!b200tag::valid_sigma(sigma) || !cov || !b200tag::read_distortion(dist, &active, &D)) return B200TAG_E_INVALID;
+  return field_pose(dets, count, layout, nlayout, tagsize, fx, fy, cx, cy, active ? &D : nullptr, rotation, offset, out,
+                    sigma, cov);
 }
 
 }  // extern "C"

@@ -728,15 +728,9 @@ inline void field_slot_tree(double (*slot)[K], double *out) {
   for (int j = 0; j < K; j++) out[j] = slot[0][j];
 }
 
-// Solves (J^T J + lambda diag(J^T J)) d = -J^T r from the sums S by Cholesky; false when the matrix is not positive
-// definite.
-POSE_HD_CALL bool field_step(const double *S, double lambda, double *d) {
-  double A[6][6];
-  int o = 7;
-  POSE_UNROLL for (int i = 0; i < 6; i++)
-    POSE_UNROLL for (int j = i; j < 6; j++) A[i][j] = A[j][i] = S[o++];
-  POSE_UNROLL for (int i = 0; i < 6; i++) A[i][i] = A[i][i] + lambda * A[i][i];
-  double Lm[6][6] = {};
+// The Cholesky factor A = Lm Lm^T of a symmetric 6x6 matrix (only its lower triangle is read); false when A is not
+// positive definite.
+POSE_HD bool cholesky6(const double (*A)[6], double (*Lm)[6]) {
   POSE_UNROLL for (int j = 0; j < 6; j++) {
     double s = A[j][j];
     POSE_UNROLL for (int k = 0; k < j; k++) s -= Lm[j][k] * Lm[j][k];
@@ -748,6 +742,19 @@ POSE_HD_CALL bool field_step(const double *S, double lambda, double *d) {
       Lm[i][j] = r / Lm[j][j];
     }
   }
+  return true;
+}
+
+// Solves (J^T J + lambda diag(J^T J)) d = -J^T r from the sums S by Cholesky; false when the matrix is not positive
+// definite.
+POSE_HD_CALL bool field_step(const double *S, double lambda, double *d) {
+  double A[6][6];
+  int o = 7;
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = i; j < 6; j++) A[i][j] = A[j][i] = S[o++];
+  POSE_UNROLL for (int i = 0; i < 6; i++) A[i][i] = A[i][i] + lambda * A[i][i];
+  double Lm[6][6] = {};
+  if (!cholesky6(A, Lm)) return false;
   double y[6];
   POSE_UNROLL for (int i = 0; i < 6; i++) {
     double r = -S[1 + i];
@@ -884,6 +891,200 @@ POSE_HD void field_solve(const FieldTagData *tags, int ntags, CostFn &cost, SumF
   field_result(R, t, c, HUGE_VAL, ntags, it, rotation, offset, out);
 }
 
+// ---- Covariance (b200tag_estimate_pose_covariances, b200tag_estimate_field_pose_covariance) ----
+// The first-order covariance of the pixel least-squares pose over a set of corners, linearised at a given
+// camera-from-X pose (R, t), for xi = (r, dt): R_true = exp([r]x) R, t_true = t + dt (b200tag.h has the definition):
+//   C = sigma^2 M^-1 B M^-1,   M = sum_i J_i^T J_i,   B = sum_i J_i^T A_i A_i^T J_i,
+// J_i the 2x6 Jacobian of corner i's ideal-image projection, A_i the Jacobian of the undistortion at corner i in pixels.
+// Without distortion A_i = I, B = M and C = sigma^2 M^-1: B is not summed.  The field's sums go through its slot order;
+// only + - * / and sqrt, so host and device agree bit for bit.
+
+constexpr int kCovSums = 43;  // corners behind the camera, the upper triangles of M (21) and of B (21)
+
+// A_i (2x2, row-major) at ideal pixel (u, v): diag(fx, fy) (dx_d/dx_u)^-1 diag(1/fx, 1/fy), with dx_d/dx_u the model's
+// Jacobian at the normalised point; false when its determinant is not positive.
+POSE_HD bool undistortion_jacobian(double u, double v, const FieldCamera &cam, const Distortion &D, double *A) {
+  double xd, yd, j00, j01, j11;
+  distort_normalised(D, (u - cam.cx) / cam.fx, (v - cam.cy) / cam.fy, &xd, &yd, &j00, &j01, &j11);
+  const double det = j00 * j11 - j01 * j01;
+  if (!(det > 0)) return false;
+  A[0] = j11 / det;
+  A[1] = -j01 * cam.fx / (cam.fy * det);
+  A[2] = -j01 * cam.fy / (cam.fx * det);
+  A[3] = j00 / det;
+  return true;
+}
+
+// Adds the terms of the point X seen at pose (R, t) into acc[kCovSums]: 1 into acc[0] when it is not in front of the
+// camera; else J^T J into acc[1..21] and, when A is given, J^T A A^T J into acc[22..42].  d(R X + t) = r x (R X) + dt.
+POSE_HD void cov_corner_terms(const V3 &X, const M3 &R, const V3 &t, const FieldCamera &cam, const double *A, double *acc) {
+  const V3 Y = mul(R, X), P = add(Y, t);
+  if (!(P.v[2] > 0)) {
+    acc[0] += 1;
+    return;
+  }
+  const double iz = 1 / P.v[2];
+  const V3 du{{cam.fx * iz, 0, -cam.fx * (P.v[0] * iz) * iz}}, dv{{0, cam.fy * iz, -cam.fy * (P.v[1] * iz) * iz}};
+  const V3 cu = cross(Y, du), cv = cross(Y, dv);
+  const double Ju[6] = {cu.v[0], cu.v[1], cu.v[2], du.v[0], du.v[1], du.v[2]};
+  const double Jv[6] = {cv.v[0], cv.v[1], cv.v[2], dv.v[0], dv.v[1], dv.v[2]};
+  int o = 1;
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = i; j < 6; j++) acc[o++] += Ju[i] * Ju[j] + Jv[i] * Jv[j];
+  if (!A) return;
+  double K0[6], K1[6];  // the rows of A^T J
+  POSE_UNROLL for (int i = 0; i < 6; i++) {
+    K0[i] = A[0] * Ju[i] + A[2] * Jv[i];
+    K1[i] = A[1] * Ju[i] + A[3] * Jv[i];
+  }
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = i; j < 6; j++) acc[o++] += K0[i] * K0[j] + K1[i] * K1[j];
+}
+
+// cov_corner_terms for corner c of used field tag g (whose px are already undistorted), with A_i through the lens D
+// (null: none); a corner where A_i cannot be formed counts as one behind the camera.
+POSE_HD void field_cov_corner_terms(const FieldTagData &g, int c, const M3 &R, const V3 &t, const FieldCamera &cam,
+                                    const Distortion *D, double *acc) {
+  double A[4] = {1, 0, 0, 1};
+  if (D && !undistortion_jacobian(g.px[c][0], g.px[c][1], cam, *D, A)) {
+    acc[0] += 1;
+    return;
+  }
+  cov_corner_terms(g.X[c], R, t, cam, D ? A : nullptr, acc);
+}
+
+// C = M^-1 B M^-1 (distorted) or M^-1 from the sums S of cov_corner_terms, exactly symmetric; false when a corner is
+// behind the camera or M is not positive definite.
+POSE_HD bool cov_from_sums(const double *S, bool distorted, double *C) {
+  if (!(S[0] == 0)) return false;
+  double M[6][6], Lm[6][6] = {};
+  int o = 1;
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = i; j < 6; j++) M[i][j] = M[j][i] = S[o++];
+  if (!cholesky6(M, Lm)) return false;
+  double Mi[6][6];  // column k solves Lm Lm^T x = e_k
+  POSE_UNROLL for (int k = 0; k < 6; k++) {
+    double y[6];
+    POSE_UNROLL for (int i = 0; i < 6; i++) {
+      double r = i == k ? 1.0 : 0.0;
+      POSE_UNROLL for (int m = 0; m < i; m++) r -= Lm[i][m] * y[m];
+      y[i] = r / Lm[i][i];
+    }
+    POSE_UNROLL for (int i = 5; i >= 0; i--) {
+      double r = y[i];
+      POSE_UNROLL for (int m = i + 1; m < 6; m++) r -= Lm[m][i] * Mi[m][k];
+      Mi[i][k] = r / Lm[i][i];
+    }
+  }
+  if (!distorted) {
+    POSE_UNROLL for (int i = 0; i < 6; i++)
+      POSE_UNROLL for (int j = i; j < 6; j++) C[6 * i + j] = C[6 * j + i] = Mi[i][j];
+    return true;
+  }
+  double B[6][6], T[6][6];
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = i; j < 6; j++) B[i][j] = B[j][i] = S[o++];
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = 0; j < 6; j++) {
+      double s = 0;
+      POSE_UNROLL for (int k = 0; k < 6; k++) s += Mi[i][k] * B[k][j];
+      T[i][j] = s;
+    }
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = i; j < 6; j++) {
+      double s = 0;
+      POSE_UNROLL for (int k = 0; k < 6; k++) s += T[i][k] * Mi[k][j];
+      C[6 * i + j] = C[6 * j + i] = s;
+    }
+  return true;
+}
+
+// out = G C G^T (6x6, row-major), exactly symmetric; out must not alias C.
+POSE_HD void cov_transform(const double *G, const double *C, double *out) {
+  double T[36];
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = 0; j < 6; j++) {
+      double s = 0;
+      POSE_UNROLL for (int k = 0; k < 6; k++) s += G[6 * i + k] * C[6 * k + j];
+      T[6 * i + j] = s;
+    }
+  POSE_UNROLL for (int i = 0; i < 6; i++)
+    POSE_UNROLL for (int j = i; j < 6; j++) {
+      double s = 0;
+      POSE_UNROLL for (int k = 0; k < 6; k++) s += T[6 * i + k] * G[6 * j + k];
+      out[6 * i + j] = out[6 * j + i] = s;
+    }
+}
+
+// The last step: C * sigma^2 when ok, else all HUGE_VAL.  Scaling last makes C(2 sigma) = 4 C(sigma) bit for bit.
+POSE_HD void cov_scale(bool ok, double sigma, double *C) {
+  const double s2 = sigma * sigma;
+  POSE_UNROLL for (int k = 0; k < 36; k++) C[k] = ok ? C[k] * s2 : HUGE_VAL;
+}
+
+// The covariance of tag pose `pose` (camera frame) from the tag's raw image corners `raw`, through the lens D (null:
+// none), into C[36]; all HUGE_VAL for a failed record, a corner that cannot be undistorted or is behind the camera, or
+// an M that is not positive definite.
+POSE_HD void tag_covariance(const double (*raw)[2], const b200tag_pose &pose, double tagsize, const FieldCamera &cam,
+                            const Distortion *D, double sigma, double *C) {
+  bool ok = pose.err < HUGE_VAL;
+  M3 R;
+  POSE_UNROLL for (int k = 0; k < 9; k++) R.a[k] = pose.R[k];
+  const V3 t{{pose.t[0], pose.t[1], pose.t[2]}};
+  const double s = tagsize / 2.0;
+  const V3 X[4] = {V3{{-s, s, 0}}, V3{{s, s, 0}}, V3{{s, -s, 0}}, V3{{-s, -s, 0}}};
+  double S[kCovSums] = {};
+  POSE_UNROLL for (int i = 0; i < 4; i++) {
+    double A[4] = {1, 0, 0, 1}, u[2];
+    if (D) ok = ok && undistort_point(raw[i], cam.fx, cam.fy, cam.cx, cam.cy, *D, u) && undistortion_jacobian(u[0], u[1], cam, *D, A);
+    cov_corner_terms(X[i], R, t, cam, D ? A : nullptr, S);
+  }
+  ok = ok && cov_from_sums(S, D != nullptr, C);
+  cov_scale(ok, sigma, C);
+}
+
+// The camera-from-field pose at which field record `res` is linearised: R = camera_R^T, t = -R camera_t.
+POSE_HD void field_cov_pose(const b200tag_field_pose &res, M3 *R, V3 *t) {
+  M3 Rc;
+  POSE_UNROLL for (int k = 0; k < 9; k++) Rc.a[k] = res.camera_R[k];
+  *R = transpose(Rc);
+  *t = scale(mul(*R, V3{{res.camera_t[0], res.camera_t[1], res.camera_t[2]}}), -1.0);
+}
+
+// The covariances of field record `res` from the reduced sums S (kCovSums; B only when distorted) at field_cov_pose(res).
+// The solve's xi (a, b) perturbs the camera-from-field pose in the camera frame; the camera in the field (Rc, tc) moves
+// by r = -Rc a, dt = -Rc b + [tc]x Rc a, and the robot (Rr, tr = tc - Rr offset) by r, dt + [Rr offset]x r.  All
+// HUGE_VAL when no tag was used or cov_from_sums fails.
+POSE_HD_CALL void field_covariance(const double *S, bool distorted, const b200tag_field_pose &res, const double *offset,
+                                   double sigma, b200tag_field_covariance *out) {
+  double Cs[36] = {};
+  const bool ok = res.num_tags > 0 && cov_from_sums(S, distorted, Cs);
+  const double *Rc = res.camera_R, *tc = res.camera_t;
+  double G[36] = {};
+  POSE_UNROLL for (int i = 0; i < 3; i++)
+    POSE_UNROLL for (int j = 0; j < 3; j++) {
+      G[6 * i + j] = -Rc[3 * i + j];
+      G[6 * (i + 3) + j + 3] = -Rc[3 * i + j];
+      // row i of [tc]x times column j of Rc
+      const int a = (i + 1) % 3, b = (i + 2) % 3;
+      G[6 * (i + 3) + j] = tc[a] * Rc[3 * b + j] - tc[b] * Rc[3 * a + j];
+    }
+  cov_transform(G, Cs, out->camera);
+  double q[3];
+  POSE_UNROLL for (int i = 0; i < 3; i++)
+    q[i] = res.robot_R[3 * i] * offset[0] + res.robot_R[3 * i + 1] * offset[1] + res.robot_R[3 * i + 2] * offset[2];
+  double H[36] = {};
+  POSE_UNROLL for (int i = 0; i < 6; i++) H[7 * i] = 1;
+  POSE_UNROLL for (int i = 0; i < 3; i++) {
+    const int a = (i + 1) % 3, b = (i + 2) % 3;
+    H[6 * (i + 3) + a] = -q[b];  // [q]x: row i has -q[b] at column a and q[a] at column b
+    H[6 * (i + 3) + b] = q[a];
+  }
+  cov_transform(H, out->camera, out->robot);
+  cov_scale(ok, sigma, out->camera);
+  cov_scale(ok, sigma, out->robot);
+}
+
 }  // namespace pose
 
 // Host, pose.cc: the node's records from poses already estimated (robot frame, distance, closest first), the step
@@ -898,6 +1099,9 @@ bool field_layout_keys(const b200tag_field_tag *layout, int nlayout, const uint3
 // Host, pose.cc: the check of a `dist` argument ({k1, k2, p1, p2, k3} or NULL): false when a coefficient is not finite.
 // *active is true when a coefficient is non-zero; only then is there an undistortion step, and *D holds the model.
 bool read_distortion(const double *dist, bool *active, pose::Distortion *D);
+
+// Host, pose.cc: the check of a covariance's sigma: finite and > 0.
+bool valid_sigma(double sigma);
 
 }  // namespace b200tag
 

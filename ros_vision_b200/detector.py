@@ -87,6 +87,8 @@ FIELD_TAG_DT = np.dtype([("family", "<i4"), ("id", "<i4"), ("R", "<f8", (3, 3)),
 FIELD_POSE_DT = np.dtype([("num_tags", "<i4"), ("iterations", "<i4"), ("reserved", "<i4", (2,)), ("camera_R", "<f8", (3, 3)),
                           ("camera_t", "<f8", (3,)), ("robot_R", "<f8", (3, 3)), ("robot_t", "<f8", (3,)), ("rms", "<f8"),
                           ("rms_other", "<f8")])  # b200tag_field_pose
+COVARIANCE_DT = np.dtype([("C", "<f8", (6, 6))])  # b200tag_covariance: xi = (rx, ry, rz, tx, ty, tz), rad and m
+FIELD_COVARIANCE_DT = np.dtype([("camera", "<f8", (6, 6)), ("robot", "<f8", (6, 6))])  # b200tag_field_covariance
 
 _lib = None
 
@@ -170,6 +172,15 @@ def load_library():
     L.b200tag_estimate_field_pose_distorted.argtypes = [vp, i32, vp, i32] + [C.c_double] * 5 + [vp, vp, vp, vp]
     L.b200tag_debug_estimate_field_pose_distorted_device.argtypes = [vp, i32, vp, i32] + [C.c_double] * 5 + [vp, vp, vp, vp]
     L.b200tag_set_pose_distortion.argtypes = [vp, vp]
+    L.b200tag_estimate_pose_covariances.argtypes = [vp, vp, i32] + [C.c_double] * 5 + [vp, C.c_double, vp]
+    L.b200tag_debug_pose_covariances_device.argtypes = [vp, vp, i32] + [C.c_double] * 5 + [vp, C.c_double, vp]
+    L.b200tag_estimate_field_pose_covariance.argtypes = [vp, i32, vp, i32] + [C.c_double] * 5 + [vp, vp, vp, C.c_double, vp, vp]
+    L.b200tag_debug_field_pose_covariance_device.argtypes = [vp, i32, vp, i32] + [C.c_double] * 5 + [vp, vp, vp, C.c_double, vp, vp]
+    L.b200tag_set_pose_covariance.argtypes = [vp, C.c_double]
+    L.b200tag_pose_covariances.argtypes = [vp, i32, C.POINTER(i32)]
+    L.b200tag_pose_covariances.restype = vp
+    L.b200tag_field_covariance_get.argtypes = [vp, i32]
+    L.b200tag_field_covariance_get.restype = vp
     L.b200tag_version.restype = i32
     _lib = L
     return L
@@ -331,6 +342,80 @@ def estimate_field_pose_device(detections: np.ndarray, layout: np.ndarray, tagsi
     """Test hook: estimate_field_pose computed by the device kernel GpuDetector.SetFieldLayout enables."""
     return _field_call("b200tag_debug_estimate_field_pose_device", "b200tag_debug_estimate_field_pose_distorted_device",
                        detections, layout, tagsize, fx, fy, cx, cy, rotation, offset, distortion)
+
+
+def _pose_covariances(fn, detections, poses, tagsize, fx, fy, cx, cy, sigma, distortion) -> np.ndarray:
+    lib = load_library()
+    dist = _distortion(distortion)
+    dets = np.ascontiguousarray(detections, dtype=DETECTION_DT)
+    ps = np.ascontiguousarray(poses, dtype=POSE_DT)
+    if len(ps) != len(dets):
+        raise ValueError(f"{len(dets)} detections but {len(ps)} poses")
+    out = np.zeros(len(dets), dtype=COVARIANCE_DT)
+    n = len(dets)
+    rc = getattr(lib, fn)(_ptr(dets) if n else None, _ptr(ps) if n else None, n, float(tagsize), float(fx), float(fy),
+                          float(cx), float(cy), _ptr(dist), float(sigma), _ptr(out) if n else None)
+    if rc:
+        raise B200TagError(f"{fn}: {lib.b200tag_error_string(rc).decode()}")
+    return out
+
+
+def estimate_pose_covariances(detections: np.ndarray, poses: np.ndarray, tagsize: float, fx: float, fy: float, cx: float,
+                              cy: float, sigma: float, distortion=None) -> np.ndarray:
+    """The covariance of every tag pose (b200tag_estimate_pose_covariances): COVARIANCE_DT records parallel to `poses`
+    (POSE_DT, from estimate_poses with either method and the same `distortion`).  C is the 6x6 covariance of the pose's
+    (rx, ry, rz, tx, ty, tz) in the camera frame for corner noise of `sigma` px per coordinate; all inf on failure."""
+    return _pose_covariances("b200tag_estimate_pose_covariances", detections, poses, tagsize, fx, fy, cx, cy, sigma,
+                             distortion)
+
+
+def estimate_pose_covariances_device(detections, poses, tagsize, fx, fy, cx, cy, sigma, distortion=None) -> np.ndarray:
+    """Test hook: estimate_pose_covariances computed by the device kernel k_pose_cov."""
+    return _pose_covariances("b200tag_debug_pose_covariances_device", detections, poses, tagsize, fx, fy, cx, cy, sigma,
+                             distortion)
+
+
+def _field_covariance_call(fn, detections, layout, tagsize, fx, fy, cx, cy, sigma, rotation, offset, distortion):
+    lib = load_library()
+    dist = _distortion(distortion)
+    dets = np.ascontiguousarray(detections, dtype=DETECTION_DT)
+    lay = np.ascontiguousarray(np.zeros(0, dtype=FIELD_TAG_DT) if layout is None else layout, dtype=FIELD_TAG_DT)
+    rot = None if rotation is None else np.ascontiguousarray(rotation, dtype=np.float64).reshape(9)
+    off = None if offset is None else np.ascontiguousarray(offset, dtype=np.float64).reshape(3)
+    pose = np.zeros(1, dtype=FIELD_POSE_DT)
+    cov = np.zeros(1, dtype=FIELD_COVARIANCE_DT)
+    rc = getattr(lib, fn)(_ptr(dets) if len(dets) else None, len(dets), _ptr(lay) if len(lay) else None, len(lay),
+                          float(tagsize), float(fx), float(fy), float(cx), float(cy), _ptr(dist), _ptr(rot), _ptr(off),
+                          float(sigma), _ptr(pose), _ptr(cov))
+    if rc:
+        raise B200TagError(f"{fn}: {lib.b200tag_error_string(rc).decode()}")
+    return pose[0], cov[0]
+
+
+def estimate_field_pose_covariance(detections: np.ndarray, layout: np.ndarray, tagsize: float, fx: float, fy: float,
+                                   cx: float, cy: float, sigma: float, rotation=None, offset=None, distortion=None):
+    """estimate_field_pose and the covariance of its result (b200tag_estimate_field_pose_covariance): (FIELD_POSE_DT
+    record, FIELD_COVARIANCE_DT record).  The pose is bit-identical to estimate_field_pose's; `camera` and `robot` are
+    the 6x6 covariances of (rx, ry, rz, tx, ty, tz) of camera_R / camera_t and robot_R / robot_t in the field frame, for
+    corner noise of `sigma` px per coordinate.  pose2d_stddevs(cov["robot"]) gives a pose estimator's (x, y, heading)
+    standard deviations."""
+    return _field_covariance_call("b200tag_estimate_field_pose_covariance", detections, layout, tagsize, fx, fy, cx, cy,
+                                  sigma, rotation, offset, distortion)
+
+
+def estimate_field_pose_covariance_device(detections, layout, tagsize, fx, fy, cx, cy, sigma, rotation=None, offset=None,
+                                          distortion=None):
+    """Test hook: estimate_field_pose_covariance computed by k_field_pose's variant with the covariance."""
+    return _field_covariance_call("b200tag_debug_field_pose_covariance_device", detections, layout, tagsize, fx, fy, cx,
+                                  cy, sigma, rotation, offset, distortion)
+
+
+def pose2d_stddevs(cov) -> tuple:
+    """(sigma_x, sigma_y, sigma_yaw) of a robot Pose2d from a 6x6 field-frame pose covariance (e.g. the `robot` field of
+    FIELD_COVARIANCE_DT): sqrt(C[3][3]), sqrt(C[4][4]) and sqrt(C[2][2]), in m, m and rad, as WPILib's
+    addVisionMeasurement takes them."""
+    C6 = np.asarray(cov, dtype=np.float64).reshape(6, 6)
+    return float(np.sqrt(C6[3, 3])), float(np.sqrt(C6[4, 4])), float(np.sqrt(C6[2, 2]))
 
 
 def _records(ptr, n, dtype) -> np.ndarray:
@@ -561,6 +646,22 @@ class GpuDetector:
         """TAG_POSITION_DT records of frame `frame`, closest first, as locate_tags(Detections(frame), ...) returns them."""
         n = C.c_int()
         return _records(self._lib.b200tag_tag_positions(self._h, frame, C.byref(n)), n.value, TAG_POSITION_DT)
+
+    def SetPoseCovariance(self, sigma: float) -> None:
+        """From the next Detect on, the covariance of every pose (PoseCovariances) and of the field pose
+        (FieldCovariance) for corner noise of `sigma` px per coordinate, as estimate_pose_covariances and
+        estimate_field_pose_covariance compute them.  0 turns it off."""
+        self._check(self._lib.b200tag_set_pose_covariance(self._h, float(sigma)), "b200tag_set_pose_covariance")
+
+    def PoseCovariances(self, frame: int = 0) -> np.ndarray:
+        """COVARIANCE_DT records parallel to Poses(frame); empty when the last call ran without the covariance."""
+        n = C.c_int()
+        return _records(self._lib.b200tag_pose_covariances(self._h, frame, C.byref(n)), n.value, COVARIANCE_DT)
+
+    def FieldCovariance(self, frame: int = 0):
+        """The FIELD_COVARIANCE_DT record of FieldPose(frame); None when the last call ran without it."""
+        p = self._lib.b200tag_field_covariance_get(self._h, frame)
+        return None if not p else _records(p, 1, FIELD_COVARIANCE_DT)[0]
 
     def SetFieldLayout(self, layout) -> None:
         """From the next Detect on, while the pose step is on, one field pose per frame from every visible tag of

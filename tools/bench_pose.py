@@ -27,6 +27,13 @@ same run, the pose step on without and with the coefficients, on the same config
   * the arm's kernel (`pose`, `pose_ippe` or `field_pose`) per 128-frame batch, from b200tag_profile_device, alternated
     over rounds; for --field on the synth.field_scene frames of the field arm.
 
+--covariance SIGMA measures the covariance step (GpuDetector.SetPoseCovariance) on top of IPPE: two arms alternating in
+the same run, IPPE without and with the covariance at SIGMA px, on the same config-2 workload:
+  * frames/s of 128-frame batches and kernels per batch;
+  * single-frame p50 and p90;
+  * the `pose_cov` kernel per 128-frame batch, and the `field_pose` kernel per 128-frame batch on the synth.field_scene
+    frames of the --field workload, each arm with that layout, alternated over rounds.
+
 Prints one JSON record, and writes it to --out when given.  Needs a CUDA device."""
 import argparse
 import json
@@ -64,8 +71,13 @@ def main():
     ap.add_argument("--method", choices=("oi", "ippe"), default="oi", help="pose method of the device step")
     ap.add_argument("--field", action="store_true", help="measure the field pose step (IPPE + SetFieldLayout)")
     ap.add_argument("--distortion", help="K1,K2,P1,P2,K3: measure the pose step with these lens coefficients against without")
+    ap.add_argument("--covariance", type=float, help="SIGMA: measure IPPE with the pose covariance at SIGMA px against without")
     ap.add_argument("--out", help="also write the JSON to this file (e.g. profiles/pose_r03.json)")
     args = ap.parse_args()
+    if args.covariance is not None:
+        if not args.covariance > 0:
+            ap.error("--covariance needs SIGMA > 0")
+        return covariance_main(args, args.covariance)
     if args.distortion:
         dist = [float(v) for v in args.distortion.split(",")]
         if len(dist) != 5:
@@ -449,6 +461,101 @@ def distortion_main(args, dist):
             json.dump(res, f, indent=1)
     print(json.dumps(res, indent=1))
     for d in list(big.values()) + list(one.values()):
+        d.close()
+    for pb in pins:
+        pb.close()
+
+
+def covariance_main(args, sigma):
+    import torch
+    from ros_vision_b200 import detector as D, synth
+    arms = ("ippe", "ippe_cov")
+    frames = [np.ascontiguousarray(synth.config_frame(2, i)[0]).reshape(-1) for i in range(UNIQUE)]
+    dev_batch = torch.from_numpy(np.stack([frames[i % UNIQUE] for i in range(BATCH)])).cuda()
+    ptr = dev_batch.data_ptr()
+    fs_lay, fs_frames = field_frames(D, synth, UNIQUE)
+    fs_batch = torch.from_numpy(np.stack([fs_frames[i % UNIQUE] for i in range(BATCH)])).cuda()
+
+    def detector(arm, max_batch, lay=None):
+        d = D.GpuDetector(1280, 800, "yuyv", quad_decimate=2, max_batch=max_batch)
+        d.SetPoseEstimation(TAGSIZE, FX, FY, CX, CY, rotation=ROTATION, offset=OFFSET, method="ippe")
+        if lay is not None:
+            d.SetFieldLayout(lay)
+        d.SetPoseCovariance(sigma if arm == "ippe_cov" else 0.0)
+        return d
+
+    big = {a: detector(a, BATCH) for a in arms}
+    for d in big.values():
+        for _ in range(5):
+            d.DetectDevice(ptr, BATCH)
+    fps = {a: [] for a in arms}
+    for _ in range(args.rounds):
+        for a in arms:
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            for _ in range(args.steps):
+                big[a].DetectDevice(ptr, BATCH)
+            fps[a].append(BATCH * args.steps / (time.perf_counter() - t0))
+    kpb = {a: big[a].kernels_per_batch() for a in arms}
+    raw_per_batch = sum(int(big["ippe_cov"].FrameInfo(f).num_detections) for f in range(BATCH))
+
+    # kernel times: pose_cov on config 2; field_pose on the field_scene frames, off and on alternating
+    fs = {a: detector(a, BATCH, fs_lay) for a in arms}
+    cov_ms, field_ms = [], {a: [] for a in arms}
+    for _ in range(3):
+        cov_ms.append([ms for name, ms in big["ippe_cov"].ProfileDevice(ptr, BATCH, iters=20) if name == "pose_cov"][0])
+        for a in arms:
+            field_ms[a].append([ms for name, ms in fs[a].ProfileDevice(fs_batch.data_ptr(), BATCH, iters=20)
+                                if name == "field_pose"][0])
+    fs_used = [int(fs["ippe_cov"].FieldPose(f)["num_tags"]) for f in range(BATCH)]
+
+    one = {a: detector(a, 1) for a in arms}
+    pins = []
+    for f in frames:
+        pb = D.PinnedBuffer(f.size)
+        pb.array[:] = f
+        pins.append(pb)
+    for d in one.values():
+        for pb in pins:
+            d.DetectPointers([pb.ptr])
+    lat = {a: [] for a in arms}
+    for i in range(args.latency_iters):
+        pb = pins[i % UNIQUE]
+        for a in (arms if i % 2 == 0 else arms[::-1]):
+            t0 = time.perf_counter()
+            one[a].DetectPointers([pb.ptr])
+            lat[a].append((time.perf_counter() - t0) * 1e6)
+
+    med = {a: float(np.median(fps[a])) for a in arms}
+    p50 = {a: float(np.percentile(lat[a], 50)) for a in arms}
+    fmed = {a: float(np.median(field_ms[a])) for a in arms}
+    cmed = float(np.median(cov_ms))
+    res = {
+        "mode": "covariance",
+        "sigma": sigma,
+        "gpu": gpu_identity(),
+        "torch_device": torch.cuda.get_device_name(0),
+        "workload": "config2: 1280x800 YUYV, synth.config_frame(2, 0..15) tiled to 128-frame batches, tag36h11, decimate 2, "
+                    "IPPE; field_pose kernel on synth.field_scene frames of one 6-tag layout (the --field workload)",
+        "batch_frames_per_s": {"rounds": fps, "median": med, "ratio_cov_over_ippe": med["ippe_cov"] / med["ippe"]},
+        "kernels_per_batch": kpb,
+        "raw_detections_per_batch": raw_per_batch,
+        "pose_cov_kernel_ms_per_batch": {"rounds": cov_ms, "median": cmed},
+        "field_pose_kernel_ms_per_batch": {"rounds": field_ms, "median": fmed, "ratio_cov_over_off": fmed["ippe_cov"] / fmed["ippe"],
+                                           "tags_used_per_batch": sum(fs_used)},
+        "single_frame_latency_us": {"p50": p50, "p90": {a: float(np.percentile(lat[a], 90)) for a in arms},
+                                    "iters": args.latency_iters},
+        "targets": {"pose_cov_at_most_0.02ms_per_batch": bool(cmed <= 0.02),
+                    "p50_at_most_p50_without_plus_5us": bool(p50["ippe_cov"] <= p50["ippe"] + 5),
+                    "field_pose_at_most_1.1x_without": bool(fmed["ippe_cov"] <= 1.1 * fmed["ippe"]),
+                    "batch_ratio_at_least_0.98": bool(med["ippe_cov"] >= 0.98 * med["ippe"])},
+    }
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            json.dump(res, f, indent=1)
+    print(json.dumps(res, indent=1))
+    for d in list(big.values()) + list(fs.values()) + list(one.values()):
         d.close()
     for pb in pins:
         pb.close()
