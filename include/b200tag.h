@@ -532,6 +532,83 @@ int b200tag_debug_field_pose_covariance_device(const b200tag_detection *dets, in
                                                const double *dist, const double *rotation, const double *offset,
                                                double sigma, b200tag_field_pose *out, b200tag_field_covariance *cov);
 
+/* Floor pose: the robot's (x, y, heading) on a flat floor from the field pose's correspondences, for a drivetrain pose
+ * estimator's Pose2d, with an optional gyro heading.
+ *
+ * Frames.  Field and layout frames are those of b200tag_set_field_layout (WPILib: z up).  The robot frame is given by
+ * the extrinsics, X_robot = rotation * X_cam + offset; its origin is on the floor and its z axis is the field's.  So
+ * robot_R = Rz(theta), robot_t = (x, y, 0), camera_R = Rz(theta) * rotation and camera_t = (x, y, 0) + Rz(theta) *
+ * offset.  theta is counter-clockwise from field +x in radians, as WPILib's Rotation2d.
+ *
+ * Correspondences: those of the field pose (the same selected detections, undistortion and failure rules), so num_tags
+ * always equals the field pose's.  Cost: E = sum_k |r_k|^2 + rho^2, r_k the ideal-image pixel residual of corner k and
+ * rho the heading prior, rho = w * 2 (s cg - c sg) / (1 + c cg + s sg) = w * 2 tan((theta - theta_g) / 2), (c, s) =
+ * (cos theta, sin theta), (cg, sg) the gyro heading's cos and sin (computed with the host's cos / sin on both paths).
+ * E is HUGE_VAL where 1 + c cg + s sg <= 0.  w is in px per unit of 2 tan(delta / 2): with a gyro of sigma_theta rad
+ * and corner noise of sigma px, w = sigma / sigma_theta.
+ *
+ * Modes, per frame: heading NaN: free (x, y, theta; no rho).  Heading finite and 0 < w < inf: prior (x, y, theta plus
+ * rho).  Heading finite and w = +inf: fixed ((c, s) = (cg, sg); unknowns x, y).
+ *
+ * Seeds, scored by E in this order, the first best winning: for every used tag in layout order and each IPPE candidate
+ * (0 first), the candidate's robot pose projected onto the floor ((x, y) = robot_t's, (c, s) the normalised
+ * (robot_R[0][0], robot_R[1][0]); skipped when both are 0; the gyro's (c, s) in fixed mode); then, with a heading, the
+ * linear least-squares (x, y) at the gyro heading from m_k x (R X_k + t(x, y)) = 0, m_k corner k's ideal normalised
+ * ray, which does not depend on the IPPE branch.  Refinement: Levenberg-Marquardt from the best seed with the field
+ * pose's stop rules and 20-iteration cap; the heading turns by the 2-D Cayley map, cos phi = (1 - d^2/4) / (1 + d^2/4),
+ * sin phi = d / (1 + d^2/4).  In free mode with exactly one tag each candidate's seed is refined, the lower cost returned
+ * (candidate 0 on a tie) and the other reported in rms_other.  Only + - * /, sqrt and fabs, with every pixel sum in the
+ * field pose's order: host and device results are bit-identical.
+ *
+ * Covariance (sigma > 0): the 3x3 covariance of (x, y, theta) in the field frame, row-major,
+ *   C = sigma^2 H^-1 M H^-1,  H = J^T J + g g^T,  M = sum_i J_i^T A_i A_i^T J_i + g g^T,
+ * J the pixel Jacobian with respect to (x, y, theta), A_i the lens term of the pose covariance above, g = d rho /
+ * d(x, y, theta) = (0, 0, 2 w / (1 + cos(theta - theta_g))) in prior mode and 0 in free mode.  Without distortion
+ * C = sigma^2 H^-1.  Fixed mode: the (x, y) block, theta's row and column exactly 0.  Failures as for the field
+ * covariance (no tag, a corner behind the camera or not undistortable, H not positive definite): all nine HUGE_VAL. */
+#define B200TAG_FLOOR_FREE 0
+#define B200TAG_FLOOR_PRIOR 1
+#define B200TAG_FLOOR_FIXED 2
+typedef struct b200tag_floor_pose {
+  int32_t num_tags;     /* layout tags used: always the field pose's num_tags */
+  int32_t iterations;   /* Levenberg-Marquardt iterations run (accepted and rejected steps) */
+  int32_t mode;         /* B200TAG_FLOOR_FREE, _PRIOR or _FIXED */
+  int32_t reserved;
+  double x, y;          /* robot_t's x and y in the field, m */
+  double cos_heading, sin_heading;
+  double heading;       /* atan2(sin_heading, cos_heading), rad */
+  double rms;           /* RMS pixel reprojection error over the corners used (rho not included) */
+  double rms_other;     /* free mode with one tag: the same for the other IPPE candidate after refinement; else HUGE_VAL */
+} b200tag_floor_pose;   /* num_tags == 0: x = y = 0, heading 0, rms = rms_other = HUGE_VAL */
+
+/* One frame on the host.  heading NaN: free mode.  sigma 0: no covariance (cov may be NULL); sigma > 0: cov[9].
+ * B200TAG_E_INVALID as b200tag_estimate_field_pose_distorted, and for an infinite heading, a heading_weight that is not
+ * > 0 (+inf is valid and means fixed), a negative or non-finite sigma, or sigma > 0 with cov NULL. */
+int b200tag_estimate_floor_pose(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout,
+                                double tagsize, double fx, double fy, double cx, double cy, const double *dist,
+                                const double *rotation, const double *offset, double heading, double heading_weight,
+                                double sigma, b200tag_floor_pose *out, double cov[9]);
+/* The floor pose on the device, from the next detect call, whenever the field step runs: heading_weight > 0 (or +inf)
+ * turns it on, 0 off; B200TAG_E_INVALID (state unchanged) for anything else.  Uses the pose step's intrinsics,
+ * extrinsics, distortion and covariance sigma.  One more kernel in b200tag_kernels_per_batch while it runs; off,
+ * nothing changes. */
+int b200tag_set_floor_pose(b200tag_detector *det, double heading_weight);
+/* Per-frame gyro headings (rad) for the next detect or enqueue call only: frame f gets heading[f] for f < count and
+ * none (free mode) otherwise, NaN also meaning none.  A call without a preceding set runs every frame in free mode.
+ * The array is not read after this returns; a batch already enqueued keeps its headings.  B200TAG_E_INVALID (state
+ * unchanged) for count < 0, count > max_batch, NULL with count > 0, or an infinite heading. */
+int b200tag_set_robot_headings(b200tag_detector *det, const double *heading, int count);
+/* The floor pose of frame `frame` of the last call and its 3x3 covariance; NULL when that call ran without the step
+ * (or, for the covariance, without sigma).  Owned by the detector, valid until the next detect call. */
+const b200tag_floor_pose *b200tag_floor_pose_get(const b200tag_detector *det, int frame);
+const double *b200tag_floor_covariance_get(const b200tag_detector *det, int frame);
+/* Test hook: the device kernels on one caller-supplied (raw) list; arguments and results as
+ * b200tag_estimate_floor_pose. */
+int b200tag_debug_floor_pose_device(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
+                                    int nlayout, double tagsize, double fx, double fy, double cx, double cy,
+                                    const double *dist, const double *rotation, const double *offset, double heading,
+                                    double heading_weight, double sigma, b200tag_floor_pose *out, double cov[9]);
+
 /* Pinned host staging memory, so b200tag_detect* can overlap H2D with compute. */
 void *b200tag_alloc_pinned(size_t bytes);
 /* Write-combined pinned memory: for buffers the CPU (or a capture driver) only ever WRITES, such as a camera ring

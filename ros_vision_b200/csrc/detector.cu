@@ -148,6 +148,19 @@ struct b200tag_detector {
   b200tag_field_covariance *d_field_cov_alias = nullptr;
   std::vector<std::vector<b200tag_covariance>> covs;  // parallel to dets
   std::vector<b200tag_field_covariance> field_covs;   // per frame of the last call
+  // the floor pose step (b200tag_set_floor_pose): on while the field step runs and floor_weight > 0
+  double floor_weight = 0;
+  bool last_floor = false;                     // the last enqueue ran the step
+  b200tag_floor_pose *h_floor = nullptr;       // pinned + mapped, max_batch entries; allocated when first turned on
+  b200tag_floor_pose *d_floor_alias = nullptr;
+  double *h_floor_cov = nullptr;               // pinned + mapped, 9 per frame
+  double *d_floor_cov_alias = nullptr;
+  double *h_gyro = nullptr;                    // pinned + mapped, (cos, sin) per frame, NaN: no heading; written by
+  double *d_gyro_alias = nullptr;              // enqueue_impl, when no batch is in flight
+  std::vector<double> next_gyro;               // b200tag_set_robot_headings: (cos, sin) per frame for the next call
+  bool next_gyro_set = false;
+  std::vector<b200tag_floor_pose> floor_poses; // per frame of the last call
+  std::vector<double> floor_covs;              // 9 per frame of the last call
 };
 
 namespace b200tag {
@@ -401,6 +414,12 @@ int finish_impl(b200tag_detector *det) {
     }
     if (det->last_field) det->field_poses[f] = det->h_field[f];
     if (det->last_field && det->last_pose.sigma > 0) det->field_covs[f] = det->h_field_cov[f];
+    if (det->last_floor) {
+      b200tag_floor_pose &fp = det->floor_poses[f];
+      fp = det->h_floor[f];
+      fp.heading = std::atan2(fp.sin_heading, fp.cos_heading);
+      if (det->last_pose.sigma > 0) memcpy(&det->floor_covs[9 * static_cast<size_t>(f)], det->h_floor_cov + 9 * static_cast<size_t>(f), 9 * sizeof(double));
+    }
     det->quads_valid[f] = false;
     if (c.status) rc = B200TAG_E_OVERFLOW;
   }
@@ -444,6 +463,14 @@ int record_sequence(b200tag_detector *det, const void *device_images, size_t str
       fl.cov = det->d_field_cov_alias;
       fl.sigma = ps.sigma;
       launch_field_pose(fl, count, ln);
+      if (det->floor_weight > 0) {
+        FloorLaunch gl{fl.scratch, fl.scratch_stride, det->d_field_alias, det->d_gyro_alias, det->floor_weight,
+                       ps.fx, ps.fy, ps.cx, ps.cy, {}, {}, {}, det->d_floor_alias, det->d_floor_cov_alias, ps.sigma};
+        memcpy(gl.rotation, ps.rotation, sizeof(gl.rotation));
+        memcpy(gl.offset, ps.offset, sizeof(gl.offset));
+        memcpy(gl.dist, ps.dist, sizeof(gl.dist));
+        launch_floor_pose(gl, count, ln);
+      }
     }
   }
   *launches_out = ln.count;
@@ -456,6 +483,16 @@ int record_sequence(b200tag_detector *det, const void *device_images, size_t str
 // single-frame latency path, where the kernels are short).
 int enqueue_impl(b200tag_detector *det, const void *device_images, size_t stride, int count, KernelTimer *kt, bool keep_host_status = false) {
   if (!keep_host_status) det->host_status.assign(static_cast<size_t>(count), 0u);
+  // the headings of b200tag_set_robot_headings belong to this call only; every caller has finished the previous batch,
+  // so no kernel reads h_gyro while it is written
+  const bool floor = det->pose.tagsize > 0 && det->field_n > 0 && det->floor_weight > 0;
+  if (floor)
+    for (int f = 0; f < count; f++) {
+      const bool given = det->next_gyro_set && 2 * static_cast<size_t>(f) < det->next_gyro.size();
+      det->h_gyro[2 * f] = given ? det->next_gyro[2 * f] : NAN;
+      det->h_gyro[2 * f + 1] = given ? det->next_gyro[2 * f + 1] : NAN;
+    }
+  det->next_gyro_set = false;
   det->last_images = static_cast<const uint8_t *>(device_images);
   det->last_stride = stride ? stride : det->in_bytes;
   int launches = 0;
@@ -494,6 +531,7 @@ int enqueue_impl(b200tag_detector *det, const void *device_images, size_t stride
   CK(cudaGetLastError());
   det->last_pose = det->pose;
   det->last_field = det->pose.tagsize > 0 && det->field_n > 0;
+  det->last_floor = floor;
   det->last_count = count;
   det->pending = true;
   return 0;
@@ -824,6 +862,8 @@ int b200tag_create_families(const b200tag_config *cfg, const b200tag_family *fam
   det->field_poses.resize(B);
   det->covs.resize(B);
   det->field_covs.resize(B);
+  det->floor_poses.resize(B);
+  det->floor_covs.resize(9 * B);
   det->quads.resize(B);
   det->quads_valid.assign(B, false);
   memset(det->h_counters, 0, sizeof(Counters) * B);
@@ -866,6 +906,9 @@ void b200tag_destroy(b200tag_detector *det) {
   if (det->h_field) cudaFreeHost(det->h_field);
   if (det->h_cov) cudaFreeHost(det->h_cov);
   if (det->h_field_cov) cudaFreeHost(det->h_field_cov);
+  if (det->h_floor) cudaFreeHost(det->h_floor);
+  if (det->h_floor_cov) cudaFreeHost(det->h_floor_cov);
+  if (det->h_gyro) cudaFreeHost(det->h_gyro);
   delete det;
 }
 
@@ -1298,6 +1341,17 @@ const b200tag_field_pose *b200tag_field_pose_get(const b200tag_detector *det, in
   return &det->field_poses[frame];
 }
 
+const b200tag_floor_pose *b200tag_floor_pose_get(const b200tag_detector *det, int frame) {
+  if (!det || frame < 0 || frame >= det->last_count || det->pending || !det->last_floor) return nullptr;
+  return &det->floor_poses[frame];
+}
+
+const double *b200tag_floor_covariance_get(const b200tag_detector *det, int frame) {
+  if (!det || frame < 0 || frame >= det->last_count || det->pending || !det->last_floor || !(det->last_pose.sigma > 0))
+    return nullptr;
+  return &det->floor_covs[9 * static_cast<size_t>(frame)];
+}
+
 const b200tag_covariance *b200tag_pose_covariances(const b200tag_detector *det, int frame, int *count) {
   if (count) *count = 0;
   if (!det || frame < 0 || frame >= det->last_count || det->pending || !(det->last_pose.tagsize > 0) ||
@@ -1564,6 +1618,49 @@ int b200tag_set_pose_covariance(b200tag_detector *det, double sigma) {
   return 0;
 }
 
+int b200tag_set_floor_pose(b200tag_detector *det, double heading_weight) {
+  if (!det || !(heading_weight == 0 || heading_weight > 0)) return B200TAG_E_INVALID;
+  DeviceGuard on_device(det->device);
+  if (heading_weight > 0 && !det->h_floor) {
+    const size_t B = static_cast<size_t>(det->cfg.max_batch);
+    b200tag_floor_pose *h = nullptr, *d = nullptr;
+    double *hc = nullptr, *dc = nullptr, *hg = nullptr, *dg = nullptr;
+    const bool ok = cudaHostAlloc(reinterpret_cast<void **>(&h), sizeof(b200tag_floor_pose) * B, cudaHostAllocMapped) == cudaSuccess &&
+                    cudaHostGetDevicePointer(reinterpret_cast<void **>(&d), h, 0) == cudaSuccess &&
+                    cudaHostAlloc(reinterpret_cast<void **>(&hc), sizeof(double) * 9 * B, cudaHostAllocMapped) == cudaSuccess &&
+                    cudaHostGetDevicePointer(reinterpret_cast<void **>(&dc), hc, 0) == cudaSuccess &&
+                    cudaHostAlloc(reinterpret_cast<void **>(&hg), sizeof(double) * 2 * B, cudaHostAllocMapped) == cudaSuccess &&
+                    cudaHostGetDevicePointer(reinterpret_cast<void **>(&dg), hg, 0) == cudaSuccess;
+    if (!ok) {
+      cudaGetLastError();
+      if (h) cudaFreeHost(h);
+      if (hc) cudaFreeHost(hc);
+      if (hg) cudaFreeHost(hg);
+      det->err = "allocating the floor pose buffers failed";
+      return B200TAG_E_CUDA;
+    }
+    det->h_floor = h;
+    det->d_floor_alias = d;
+    det->h_floor_cov = hc;
+    det->d_floor_cov_alias = dc;
+    det->h_gyro = hg;
+    det->d_gyro_alias = dg;
+  }
+  drop_graphs(det);  // the kernel and the weight are baked into the captured launches
+  det->floor_weight = heading_weight;
+  return 0;
+}
+
+int b200tag_set_robot_headings(b200tag_detector *det, const double *heading, int count) {
+  if (!det || count < 0 || count > det->cfg.max_batch || (count > 0 && !heading)) return B200TAG_E_INVALID;
+  for (int f = 0; f < count; f++)
+    if (std::isinf(heading[f])) return B200TAG_E_INVALID;
+  det->next_gyro.resize(2 * static_cast<size_t>(count));
+  for (int f = 0; f < count; f++) floor_gyro(heading[f], &det->next_gyro[2 * f], &det->next_gyro[2 * f + 1]);
+  det->next_gyro_set = true;
+  return 0;
+}
+
 int b200tag_set_distortion(b200tag_detector *det, double k1, double k2, double p1, double p2, double k3) {
   if (!det) return B200TAG_E_INVALID;
   DeviceGuard on_device(det->device);
@@ -1718,9 +1815,73 @@ int field_pose_device(const b200tag_detection *dets, int count, const b200tag_fi
   return rc;
 }
 
+// The floor hook: k_field_pose (for its scratch) and k_floor_pose on one caller list.
+int floor_pose_device(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout,
+                      double tagsize, double fx, double fy, double cx, double cy, const double *dist,
+                      const double *rotation, const double *offset, double heading, double heading_weight, double sigma,
+                      b200tag_floor_pose *out, double *cov) {
+  bool active;
+  pose::Distortion D;
+  pose::FloorModel m;
+  if (!read_distortion(dist, &active, &D) || !floor_model(rotation, offset, heading, heading_weight, &m))
+    return B200TAG_E_INVALID;
+  if (!(sigma == 0 || valid_sigma(sigma)) || (sigma > 0 && !cov)) return B200TAG_E_INVALID;
+  if (count < 0 || (count > 0 && !dets) || !out || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
+  std::vector<pose::FieldKey> keys(static_cast<size_t>(std::max(nlayout, 0)));
+  if (!field_layout_keys(layout, nlayout, nullptr, 0, keys.data())) return B200TAG_E_INVALID;
+  const size_t db = sizeof(b200tag_detection) * static_cast<size_t>(count), lb = sizeof(b200tag_field_tag) * nlayout,
+               kb = sizeof(pose::FieldKey) * nlayout, sb = field_tag_bytes() * std::max(count, 1);
+  const size_t o_l = align_up(db, 256), o_k = align_up(o_l + lb, 256), o_s = align_up(o_k + kb, 256), o_o = align_up(o_s + sb, 256);
+  const size_t o_g = align_up(o_o + sizeof(b200tag_field_pose), 256), o_f = align_up(o_g + 2 * sizeof(double), 256);
+  const size_t o_c = align_up(o_f + sizeof(b200tag_floor_pose), 256);
+  uint8_t *d = nullptr;
+  if (cudaMalloc(&d, o_c + 9 * sizeof(double)) != cudaSuccess) {
+    cudaGetLastError();
+    return B200TAG_E_NO_DEVICE;
+  }
+  const double gyro[2] = {m.cg, m.sg};
+  FieldLaunch fl{reinterpret_cast<const b200tag_detection *>(d), nullptr, 0, static_cast<uint32_t>(count),
+                 reinterpret_cast<const b200tag_field_tag *>(d + o_l), reinterpret_cast<const pose::FieldKey *>(d + o_k), nlayout,
+                 reinterpret_cast<pose::FieldTagData *>(d + o_s), 0, tagsize, fx, fy, cx, cy, {}, {},
+                 reinterpret_cast<b200tag_field_pose *>(d + o_o), {D.k1, D.k2, D.p1, D.p2, D.k3}, nullptr, 0};
+  memcpy(fl.rotation, m.rot, sizeof(fl.rotation));
+  memcpy(fl.offset, m.off, sizeof(fl.offset));
+  FloorLaunch gl{fl.scratch, 0, fl.out, reinterpret_cast<const double *>(d + o_g), heading_weight, fx, fy, cx, cy, {}, {},
+                 {D.k1, D.k2, D.p1, D.p2, D.k3}, reinterpret_cast<b200tag_floor_pose *>(d + o_f),
+                 reinterpret_cast<double *>(d + o_c), sigma};
+  memcpy(gl.rotation, m.rot, sizeof(gl.rotation));
+  memcpy(gl.offset, m.off, sizeof(gl.offset));
+  int rc = 0;
+  if ((db && cudaMemcpy(d, dets, db, cudaMemcpyHostToDevice) != cudaSuccess) ||
+      (lb && cudaMemcpy(d + o_l, layout, lb, cudaMemcpyHostToDevice) != cudaSuccess) ||
+      (kb && cudaMemcpy(d + o_k, keys.data(), kb, cudaMemcpyHostToDevice) != cudaSuccess) ||
+      cudaMemcpy(d + o_g, gyro, sizeof(gyro), cudaMemcpyHostToDevice) != cudaSuccess)
+    rc = B200TAG_E_CUDA;
+  if (!rc) {
+    Launcher ln{nullptr, nullptr};
+    launch_field_pose(fl, 1, ln);
+    launch_floor_pose(gl, 1, ln);
+    if (cudaGetLastError() != cudaSuccess || cudaMemcpy(out, d + o_f, sizeof(*out), cudaMemcpyDeviceToHost) != cudaSuccess ||
+        (sigma > 0 && cudaMemcpy(cov, d + o_c, 9 * sizeof(double), cudaMemcpyDeviceToHost) != cudaSuccess))
+      rc = B200TAG_E_CUDA;
+    else
+      out->heading = std::atan2(out->sin_heading, out->cos_heading);
+  }
+  cudaFree(d);
+  return rc;
+}
+
 }  // namespace
 
 extern "C" {
+
+int b200tag_debug_floor_pose_device(const b200tag_detection *dets, int count, const b200tag_field_tag *layout,
+                                    int nlayout, double tagsize, double fx, double fy, double cx, double cy,
+                                    const double *dist, const double *rotation, const double *offset, double heading,
+                                    double heading_weight, double sigma, b200tag_floor_pose *out, double cov[9]) {
+  return floor_pose_device(dets, count, layout, nlayout, tagsize, fx, fy, cx, cy, dist, rotation, offset, heading,
+                           heading_weight, sigma, out, cov);
+}
 
 int b200tag_debug_estimate_poses_device(const b200tag_detection *dets, int count, double tagsize, double fx, double fy,
                                         double cx, double cy, b200tag_pose *out) {

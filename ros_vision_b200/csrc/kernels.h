@@ -123,6 +123,23 @@ inline bool has_distortion(const double *dist) {
 }
 size_t field_tag_bytes();            // sizeof(pose::FieldTagData)
 
+// The floor pose step (kernels_pose.cu, k_floor_pose, b200tag_set_floor_pose): one b200tag_floor_pose per frame from
+// the used tags k_field_pose wrote to its scratch, behind it on the same stream.
+struct FloorLaunch {
+  const pose::FieldTagData *scratch;  // k_field_pose's FieldLaunch::scratch and scratch_stride
+  uint32_t scratch_stride;
+  const b200tag_field_pose *field;    // k_field_pose's records: num_tags is the frame's count of used tags
+  const double *gyro;                 // per frame (cos, sin) of the gyro heading, NaN: none
+  double weight;                      // heading_weight, +inf: fixed
+  double fx, fy, cx, cy;
+  double rotation[9], offset[3];
+  double dist[5];                     // as PoseLaunch::dist
+  b200tag_floor_pose *out;            // one per frame
+  double *cov;                        // 9 per frame; written by the variant with covariance (sigma > 0)
+  double sigma;
+};
+void launch_floor_pose(const FloorLaunch &L, int frames, Launcher &ln);
+
 // JPEG luminance planes of a batch (jpeg.h): the parallel kernels for streams without restart markers, the sequential
 // warp-per-frame kernel for the rest.
 struct JpegBatch;

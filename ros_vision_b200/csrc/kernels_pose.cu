@@ -6,7 +6,8 @@
 // is k_pose_ippe instead: the closed-form IPPE pose, one thread per detection.  With b200tag_set_pose_distortion each
 // kernel's variant with kDistorted = true runs: it undistorts the corners first (pose_core.h's undistort_point); the
 // variant without compiles to the kernel without the step.  With b200tag_set_pose_covariance, k_pose_cov runs behind
-// either pose kernel and writes every pose's covariance.
+// either pose kernel and writes every pose's covariance.  With b200tag_set_floor_pose, k_floor_pose runs behind
+// k_field_pose and fits the robot's (x, y, heading) on the floor to the same corners.
 //
 // A pose depends only on its own record, so computing it before the host's reconcile gives the pose of every
 // detection that survives it.
@@ -372,9 +373,104 @@ __global__ void __launch_bounds__(32) k_field_pose(FieldLaunch L) {
   if (lane == 0) L.out[frame] = res;
 }
 
+// The floor covariance of result `res` over the frame's `ncorr` correspondences (k_floor_pose with kCov): correspondence k
+// on lane k % 32, the sums by warp_sum, then floor_covariance on every lane; lanes 0-8 write an entry each.  Not
+// inlined, so the solve's register allocation is that of the kernel without it.
+template <bool kDistorted>
+__device__ __noinline__ void floor_covariance_warp(const FieldTagData *tags, int ncorr, const b200tag_floor_pose &res,
+                                                   const FloorModel &m, const FloorLaunch &L, int lane, double *dst) {
+  constexpr int kSums = kDistorted ? kFloorCovSums : 7;  // without distortion M is not summed
+  const FieldCamera cam{L.fx, L.fy, L.cx, L.cy};
+  const FloorState st{res.x, res.y, res.cos_heading, res.sin_heading};
+  const Distortion D = lens(L.dist);
+  double acc[kFloorCovSums];
+#pragma unroll
+  for (int j = 0; j < kFloorCovSums; j++) acc[j] = 0;
+  for (int k = lane; k < ncorr; k += 32) floor_cov_corner_terms(tags[k >> 2], k & 3, st, m, cam, kDistorted ? &D : nullptr, acc);
+  double S[kFloorCovSums];
+#pragma unroll
+  for (int j = 0; j < kFloorCovSums; j++) S[j] = j < kSums ? warp_sum(acc[j]) : 0.0;
+  double C[9];
+  floor_covariance(S, kDistorted, res, m, L.sigma, C);
+  if (lane < 9) dst[lane] = C[lane];
+}
+
+// The floor pose (b200tag_set_floor_pose) of every frame, behind k_field_pose: one warp per frame, blockIdx.x = frame,
+// reading the used tags k_field_pose wrote to the frame's scratch (their count is its record's num_tags) and the
+// frame's gyro heading.  Correspondence k on lane k % 32, the sums by warp_sum, floor_solve's 3x3 (or 2x2) step on every
+// lane; the arithmetic is pose_core.h's, the same b200tag_estimate_floor_pose runs on the host.  With kCov the warp
+// adds the 3x3 covariance of the result (kDistorted: through the lens).  heading is filled on the host.
+template <bool kDistorted, bool kCov>
+__global__ void __launch_bounds__(32) k_floor_pose(FloorLaunch L) {
+  const int lane = threadIdx.x;
+  const size_t frame = blockIdx.x;
+  const int used = L.field[frame].num_tags;
+  const FieldTagData *tags = L.scratch + frame * L.scratch_stride;
+  FloorModel m;
+#pragma unroll
+  for (int k = 0; k < 9; k++) m.rot[k] = L.rotation[k];
+#pragma unroll
+  for (int k = 0; k < 3; k++) m.off[k] = L.offset[k];
+  m.cg = L.gyro[2 * frame];
+  m.sg = L.gyro[2 * frame + 1];
+  m.w = L.weight;
+  m.mode = floor_mode(m.cg, m.w);
+  const FieldCamera cam{L.fx, L.fy, L.cx, L.cy};
+  const int ncorr = 4 * used;
+  b200tag_floor_pose res;
+  if (used == 0) {
+    floor_empty(m.mode, &res);
+  } else {
+    auto cost = [&](const FloorState &st) {
+      double acc = 0;
+      for (int k = lane; k < ncorr; k += 32) {
+        const FieldTagData &g = tags[k >> 2];
+        V3 W, P;
+        double ru, rv;
+        acc += floor_corner_cost(g.px[k & 3][0], g.px[k & 3][1], g.X[k & 3], st, m, cam, &W, &P, &ru, &rv);
+      }
+      return warp_sum(acc);
+    };
+    auto sum = [&](const FloorState &st, double *S) {
+      double acc[kFloorSums];
+#pragma unroll
+      for (int j = 0; j < kFloorSums; j++) acc[j] = 0;
+      for (int k = lane; k < ncorr; k += 32) {
+        const FieldTagData &g = tags[k >> 2];
+        floor_corner_terms(g.px[k & 3][0], g.px[k & 3][1], g.X[k & 3], st, m, cam, acc);
+      }
+#pragma unroll
+      for (int j = 0; j < kFloorSums; j++) S[j] = warp_sum(acc[j]);
+    };
+    auto lin = [&](double *S) {
+      double acc[kFloorLinSums];
+#pragma unroll
+      for (int j = 0; j < kFloorLinSums; j++) acc[j] = 0;
+      for (int k = lane; k < ncorr; k += 32) {
+        const FieldTagData &g = tags[k >> 2];
+        floor_lin_terms(g.px[k & 3][0], g.px[k & 3][1], g.X[k & 3], m, cam, acc);
+      }
+#pragma unroll
+      for (int j = 0; j < kFloorLinSums; j++) S[j] = warp_sum(acc[j]);
+    };
+    floor_solve(tags, used, m, cost, sum, lin, &res);
+  }
+  if (kCov) floor_covariance_warp<kDistorted>(tags, ncorr, res, m, L, lane, L.cov + 9 * frame);
+  static_assert(sizeof(b200tag_floor_pose) % 8 == 0 && sizeof(b200tag_floor_pose) / 8 <= 32, "floor copy");
+  if (lane < static_cast<int>(sizeof(b200tag_floor_pose) / 8))
+    reinterpret_cast<double *>(L.out + frame)[lane] = reinterpret_cast<const double *>(&res)[lane];
+}
+
 }  // namespace
 
 size_t field_tag_bytes() { return sizeof(FieldTagData); }
+
+void launch_floor_pose(const FloorLaunch &L, int frames, Launcher &ln) {
+  const bool cov = L.sigma > 0;
+  const auto kernel = has_distortion(L.dist) ? (cov ? k_floor_pose<true, true> : k_floor_pose<true, false>)
+                                             : (cov ? k_floor_pose<false, true> : k_floor_pose<false, false>);
+  ln.timed("floor_pose", [&] { kernel<<<static_cast<unsigned>(frames), 32, 0, ln.s>>>(L); });
+}
 
 void launch_field_pose(const FieldLaunch &L, int frames, Launcher &ln) {
   const bool cov = L.sigma > 0;

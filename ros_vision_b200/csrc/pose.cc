@@ -66,6 +66,22 @@ bool read_distortion(const double *dist, bool *active, pose::Distortion *D) {
 
 bool valid_sigma(double sigma) { return std::isfinite(sigma) && sigma > 0; }
 
+bool floor_model(const double *rotation, const double *offset, double heading, double heading_weight, pose::FloorModel *m) {
+  if (std::isinf(heading) || !(heading_weight > 0)) return false;
+  static const double kEye[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, kZero[3] = {0, 0, 0};
+  memcpy(m->rot, rotation ? rotation : kEye, sizeof(m->rot));
+  memcpy(m->off, offset ? offset : kZero, sizeof(m->off));
+  floor_gyro(heading, &m->cg, &m->sg);
+  m->w = heading_weight;
+  m->mode = pose::floor_mode(m->cg, heading_weight);
+  return true;
+}
+
+void floor_gyro(double heading, double *cg, double *sg) {
+  *cg = std::isnan(heading) ? NAN : std::cos(heading);
+  *sg = std::isnan(heading) ? NAN : std::sin(heading);
+}
+
 }  // namespace b200tag
 
 using namespace b200tag::pose;
@@ -164,6 +180,28 @@ void field_covariance_of(const FieldTagData *tags, int ntags, const FieldCamera 
   field_covariance(S, lens != nullptr, res, offset, sigma, cov);
 }
 
+// The used tags of b200tag_estimate_field_pose(_distorted), in layout order: per layout tag the detection reconcile
+// prefers, its corners undistorted through `lens` (null: none); a tag whose corners fail or whose IPPE candidates cannot
+// be formed is left out.
+void field_tags(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout,
+                const FieldKey *keys, double tagsize, const FieldCamera &cam, const Distortion *lens,
+                std::vector<FieldTagData> *tags) {
+  std::vector<int> sel(static_cast<size_t>(nlayout), -1);
+  for (int i = 0; i < count; i++) {
+    const int L = field_lookup(keys, nlayout, dets[i].family, dets[i].id);
+    if (L >= 0 && (sel[L] < 0 || field_prefers(dets[i], dets[sel[L]]))) sel[L] = i;
+  }
+  for (int L = 0; L < nlayout; L++) {
+    if (sel[L] < 0) continue;
+    // only the chosen record's corners are undistorted; one that fails leaves the tag out
+    double px[4][2];
+    if (!lens) memcpy(px, dets[sel[L]].p, sizeof(px));
+    else if (!undistort_corners(dets[sel[L]].p, cam.fx, cam.fy, cam.cx, cam.cy, *lens, px)) continue;
+    FieldTagData d;
+    if (field_tag_data(layout[L], px, tagsize, cam, &d)) tags->push_back(d);
+  }
+}
+
 // b200tag_estimate_field_pose(_distorted); `lens` null: no undistortion step.  With `cov`, also the covariance of the
 // result at sigma (b200tag_estimate_field_pose_covariance).
 int field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout, double tagsize,
@@ -174,23 +212,9 @@ int field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag
   if (!b200tag::field_layout_keys(layout, nlayout, nullptr, 0, keys.data())) return B200TAG_E_INVALID;
   static const double kEye[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, kZero[3] = {0, 0, 0};
   const double *Rx = rotation ? rotation : kEye, *ox = offset ? offset : kZero;
-  // the detection reconcile prefers, per layout tag
-  std::vector<int> sel(static_cast<size_t>(nlayout), -1);
-  for (int i = 0; i < count; i++) {
-    const int L = field_lookup(keys.data(), nlayout, dets[i].family, dets[i].id);
-    if (L >= 0 && (sel[L] < 0 || field_prefers(dets[i], dets[sel[L]]))) sel[L] = i;
-  }
   const FieldCamera cam{fx, fy, cx, cy};
   std::vector<FieldTagData> tags;
-  for (int L = 0; L < nlayout; L++) {
-    if (sel[L] < 0) continue;
-    // only the chosen record's corners are undistorted; one that fails leaves the tag out
-    double px[4][2];
-    if (!lens) memcpy(px, dets[sel[L]].p, sizeof(px));
-    else if (!undistort_corners(dets[sel[L]].p, fx, fy, cx, cy, *lens, px)) continue;
-    FieldTagData d;
-    if (field_tag_data(layout[L], px, tagsize, cam, &d)) tags.push_back(d);
-  }
+  field_tags(dets, count, layout, nlayout, keys.data(), tagsize, cam, lens, &tags);
   const int ntags = static_cast<int>(tags.size());
   if (ntags == 0) {
     field_empty(out);
@@ -221,6 +245,52 @@ int field_pose(const b200tag_detection *dets, int count, const b200tag_field_tag
   field_solve(tags.data(), ntags, cost, sum, Rx, ox, out);
   if (cov) field_covariance_of(tags.data(), ntags, cam, lens, ox, sigma, *out, cov);
   return 0;
+}
+
+// b200tag_estimate_floor_pose after its checks; `lens` null: no undistortion step; cov (9) only when sigma > 0.
+void floor_pose(const std::vector<FieldTagData> &tags, const FieldCamera &cam, const Distortion *lens, const FloorModel &m,
+                double sigma, b200tag_floor_pose *out, double *cov) {
+  const int ntags = static_cast<int>(tags.size()), ncorr = 4 * ntags;
+  if (ntags == 0) {
+    floor_empty(m.mode, out);
+  } else {
+    auto cost = [&](const FloorState &st) {
+      double slot[kFieldSlots][1] = {};
+      for (int k = 0; k < ncorr; k++) {
+        const FieldTagData &g = tags[k >> 2];
+        V3 W, P;
+        double ru, rv;
+        slot[k % kFieldSlots][0] += floor_corner_cost(g.px[k & 3][0], g.px[k & 3][1], g.X[k & 3], st, m, cam, &W, &P, &ru, &rv);
+      }
+      double total;
+      field_slot_tree<1>(slot, &total);
+      return total;
+    };
+    auto sum = [&](const FloorState &st, double *S) {
+      double slot[kFieldSlots][kFloorSums] = {};
+      for (int k = 0; k < ncorr; k++) {
+        const FieldTagData &g = tags[k >> 2];
+        floor_corner_terms(g.px[k & 3][0], g.px[k & 3][1], g.X[k & 3], st, m, cam, slot[k % kFieldSlots]);
+      }
+      field_slot_tree<kFloorSums>(slot, S);
+    };
+    auto lin = [&](double *S) {
+      double slot[kFieldSlots][kFloorLinSums] = {};
+      for (int k = 0; k < ncorr; k++) {
+        const FieldTagData &g = tags[k >> 2];
+        floor_lin_terms(g.px[k & 3][0], g.px[k & 3][1], g.X[k & 3], m, cam, slot[k % kFieldSlots]);
+      }
+      field_slot_tree<kFloorLinSums>(slot, S);
+    };
+    floor_solve(tags.data(), ntags, m, cost, sum, lin, out);
+  }
+  out->heading = std::atan2(out->sin_heading, out->cos_heading);
+  if (!(sigma > 0)) return;
+  const FloorState st{out->x, out->y, out->cos_heading, out->sin_heading};
+  double slot[kFieldSlots][kFloorCovSums] = {}, S[kFloorCovSums];
+  for (int k = 0; k < ncorr; k++) floor_cov_corner_terms(tags[k >> 2], k & 3, st, m, cam, lens, slot[k % kFieldSlots]);
+  field_slot_tree<kFloorCovSums>(slot, S);
+  floor_covariance(S, lens != nullptr, *out, m, sigma, cov);
 }
 
 }  // namespace
@@ -307,6 +377,26 @@ int b200tag_estimate_field_pose_covariance(const b200tag_detection *dets, int co
   if (!b200tag::valid_sigma(sigma) || !cov || !b200tag::read_distortion(dist, &active, &D)) return B200TAG_E_INVALID;
   return field_pose(dets, count, layout, nlayout, tagsize, fx, fy, cx, cy, active ? &D : nullptr, rotation, offset, out,
                     sigma, cov);
+}
+
+int b200tag_estimate_floor_pose(const b200tag_detection *dets, int count, const b200tag_field_tag *layout, int nlayout,
+                                double tagsize, double fx, double fy, double cx, double cy, const double *dist,
+                                const double *rotation, const double *offset, double heading, double heading_weight,
+                                double sigma, b200tag_floor_pose *out, double cov[9]) {
+  bool active;
+  Distortion D;
+  FloorModel m;
+  if (!b200tag::read_distortion(dist, &active, &D) || !b200tag::floor_model(rotation, offset, heading, heading_weight, &m))
+    return B200TAG_E_INVALID;
+  if (!(sigma == 0 || b200tag::valid_sigma(sigma)) || (sigma > 0 && !cov)) return B200TAG_E_INVALID;
+  if (count < 0 || (count > 0 && !dets) || !out || !(tagsize > 0) || fx == 0 || fy == 0) return B200TAG_E_INVALID;
+  std::vector<FieldKey> keys(static_cast<size_t>(std::max(nlayout, 0)));
+  if (!b200tag::field_layout_keys(layout, nlayout, nullptr, 0, keys.data())) return B200TAG_E_INVALID;
+  const FieldCamera cam{fx, fy, cx, cy};
+  std::vector<FieldTagData> tags;
+  field_tags(dets, count, layout, nlayout, keys.data(), tagsize, cam, active ? &D : nullptr, &tags);
+  floor_pose(tags, cam, active ? &D : nullptr, m, sigma, out, cov);
+  return 0;
 }
 
 }  // extern "C"

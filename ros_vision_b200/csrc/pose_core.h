@@ -1085,6 +1085,450 @@ POSE_HD_CALL void field_covariance(const double *S, bool distorted, const b200ta
   cov_scale(ok, sigma, out->robot);
 }
 
+// ---- Floor pose (b200tag_estimate_floor_pose, b200tag_set_floor_pose) ----
+// The robot on a flat floor: robot_R = Rz(theta), robot_t = (x, y, 0), so the camera-from-field pose maps a field point
+// X to P = rotation^T (Rz^T (X - (x, y, 0)) - offset).  The heading is held as (c, s) = (cos theta, sin theta) and
+// turned by the 2-D Cayley map.  The correspondences are the field pose's (FieldTagData, its slot order); the optional
+// heading prior rho = w 2 (s cg - c sg) / (1 + c cg + s sg) is added once, after the reduction.  Unknowns (x, y, theta),
+// or (x, y) in fixed mode, where (c, s) = (cg, sg).  Only + - * /, sqrt and fabs: host and device agree bit for bit.
+
+constexpr int kFloorSums = 10;     // cost, J^T r (3), the upper triangle of J^T J (6): xx xy xt yy yt tt
+constexpr int kFloorLinSums = 5;   // the heading seed's normal matrix (xx, xy, yy) and right-hand side (2)
+constexpr int kFloorCovSums = 13;  // corners behind the camera, the upper triangles of H (6) and of M (6)
+
+// The setting of one solve: extrinsics, mode (B200TAG_FLOOR_*), gyro heading (cg, sg; unused in free mode), weight w.
+struct FloorModel {
+  double rot[9], off[3];
+  int mode;
+  double cg, sg, w;
+};
+
+struct FloorState {
+  double x, y, c, s;
+};
+
+// The mode of heading (cg, sg) (NaN: none) at weight w (+inf: fixed).
+POSE_HD int floor_mode(double cg, double w) {
+  return cg != cg ? B200TAG_FLOOR_FREE : (w < HUGE_VAL ? B200TAG_FLOOR_PRIOR : B200TAG_FLOOR_FIXED);
+}
+
+// Pixel residual of one correspondence (image point u, v; field point X) at state st, HUGE_VAL when the point is not
+// in front of the camera.  *W = Rz^T (X - p), *P the camera-frame point.
+POSE_HD double floor_corner_cost(double u, double v, const V3 &X, const FloorState &st, const FloorModel &m,
+                                 const FieldCamera &cam, V3 *W, V3 *P, double *ru, double *rv) {
+  const double dx = X.v[0] - st.x, dy = X.v[1] - st.y;
+  *W = V3{{st.c * dx + st.s * dy, st.c * dy - st.s * dx, X.v[2]}};
+  const V3 Q{{W->v[0] - m.off[0], W->v[1] - m.off[1], W->v[2] - m.off[2]}};
+  POSE_UNROLL for (int i = 0; i < 3; i++) P->v[i] = m.rot[i] * Q.v[0] + m.rot[3 + i] * Q.v[1] + m.rot[6 + i] * Q.v[2];
+  if (!(P->v[2] > 0)) return HUGE_VAL;
+  const double iz = 1 / P->v[2];
+  *ru = cam.fx * (P->v[0] * iz) + cam.cx - u;
+  *rv = cam.fy * (P->v[1] * iz) + cam.cy - v;
+  return *ru * *ru + *rv * *rv;
+}
+
+// The 1x3 rows Ju, Jv of d(ru, rv)/d(x, y, theta) at (W, P): dW/dx = (-c, s, 0), dW/dy = (-s, -c, 0),
+// dW/dtheta = (W1, -W0, 0), dP = rotation^T dW.
+POSE_HD void floor_jacobian(const V3 &W, const V3 &P, const FloorState &st, const FloorModel &m, const FieldCamera &cam,
+                            double *Ju, double *Jv) {
+  const double iz = 1 / P.v[2];
+  const V3 du{{cam.fx * iz, 0, -cam.fx * (P.v[0] * iz) * iz}}, dv{{0, cam.fy * iz, -cam.fy * (P.v[1] * iz) * iz}};
+  double a[2], b[2];  // the first two entries of rotation du, rotation dv
+  POSE_UNROLL for (int j = 0; j < 2; j++) {
+    a[j] = m.rot[3 * j] * du.v[0] + m.rot[3 * j + 1] * du.v[1] + m.rot[3 * j + 2] * du.v[2];
+    b[j] = m.rot[3 * j] * dv.v[0] + m.rot[3 * j + 1] * dv.v[1] + m.rot[3 * j + 2] * dv.v[2];
+  }
+  Ju[0] = st.s * a[1] - st.c * a[0];
+  Ju[1] = -(st.s * a[0] + st.c * a[1]);
+  Ju[2] = a[0] * W.v[1] - a[1] * W.v[0];
+  Jv[0] = st.s * b[1] - st.c * b[0];
+  Jv[1] = -(st.s * b[0] + st.c * b[1]);
+  Jv[2] = b[0] * W.v[1] - b[1] * W.v[0];
+}
+
+// Adds one correspondence's cost, J^T r and J^T J into acc[kFloorSums].
+POSE_HD void floor_corner_terms(double u, double v, const V3 &X, const FloorState &st, const FloorModel &m,
+                                const FieldCamera &cam, double *acc) {
+  V3 W, P;
+  double ru = 0, rv = 0;
+  const double e = floor_corner_cost(u, v, X, st, m, cam, &W, &P, &ru, &rv);
+  acc[0] += e;
+  if (!(e < HUGE_VAL)) return;
+  double Ju[3], Jv[3];
+  floor_jacobian(W, P, st, m, cam, Ju, Jv);
+  POSE_UNROLL for (int i = 0; i < 3; i++) acc[1 + i] += Ju[i] * ru + Jv[i] * rv;
+  int o = 4;
+  POSE_UNROLL for (int i = 0; i < 3; i++)
+    POSE_UNROLL for (int j = i; j < 3; j++) acc[o++] += Ju[i] * Ju[j] + Jv[i] * Jv[j];
+}
+
+// The heading prior at st: false when 1 + cos(theta - theta_g) <= 0; else rho and g = d rho / d theta.
+POSE_HD bool floor_prior(const FloorState &st, const FloorModel &m, double *rho, double *g) {
+  const double D = 1 + st.c * m.cg + st.s * m.sg;
+  if (!(D > 0)) return false;
+  *rho = m.w * (2 * (st.s * m.cg - st.c * m.sg)) / D;
+  *g = 2 * m.w / D;
+  return true;
+}
+
+// The prior's terms added to reduced sums S (kFloorSums) in prior mode; S[0] = HUGE_VAL where it is not defined.
+POSE_HD void floor_add_prior(const FloorState &st, const FloorModel &m, double *S) {
+  if (m.mode != B200TAG_FLOOR_PRIOR) return;
+  double rho, g;
+  if (!floor_prior(st, m, &rho, &g)) {
+    S[0] = HUGE_VAL;
+    return;
+  }
+  S[0] = S[0] + rho * rho;
+  S[3] = S[3] + g * rho;
+  S[9] = S[9] + g * g;
+}
+
+// The seed score E from the reduced pixel cost e at st.
+POSE_HD double floor_score(double e, const FloorState &st, const FloorModel &m) {
+  if (m.mode != B200TAG_FLOOR_PRIOR) return e;
+  double rho, g;
+  return floor_prior(st, m, &rho, &g) ? e + rho * rho : HUGE_VAL;
+}
+
+// The Cholesky factor of a symmetric N x N matrix (lower triangle read), N = 2 or 3; false when not positive definite.
+template <int N>
+POSE_HD bool cholesky_small(const double (*A)[N], double (*Lm)[N]) {
+  POSE_UNROLL for (int j = 0; j < N; j++) {
+    double s = A[j][j];
+    POSE_UNROLL for (int k = 0; k < j; k++) s -= Lm[j][k] * Lm[j][k];
+    if (!(s > 0)) return false;
+    Lm[j][j] = sqrt(s);
+    POSE_UNROLL for (int i = j + 1; i < N; i++) {
+      double r = A[i][j];
+      POSE_UNROLL for (int k = 0; k < j; k++) r -= Lm[i][k] * Lm[j][k];
+      Lm[i][j] = r / Lm[j][j];
+    }
+  }
+  return true;
+}
+
+// Solves Lm Lm^T x = b.
+template <int N>
+POSE_HD void cholesky_solve(const double (*Lm)[N], const double *b, double *x) {
+  double y[N];
+  POSE_UNROLL for (int i = 0; i < N; i++) {
+    double r = b[i];
+    POSE_UNROLL for (int k = 0; k < i; k++) r -= Lm[i][k] * y[k];
+    y[i] = r / Lm[i][i];
+  }
+  POSE_UNROLL for (int i = N - 1; i >= 0; i--) {
+    double r = y[i];
+    POSE_UNROLL for (int k = i + 1; k < N; k++) r -= Lm[k][i] * x[k];
+    x[i] = r / Lm[i][i];
+  }
+}
+
+// The full 3x3 matrix of an upper triangle (xx xy xt yy yt tt).
+POSE_HD void floor_sym3(const double *u, double (*A)[3]) {
+  A[0][0] = u[0]; A[0][1] = A[1][0] = u[1]; A[0][2] = A[2][0] = u[2];
+  A[1][1] = u[3]; A[1][2] = A[2][1] = u[4]; A[2][2] = u[5];
+}
+
+// Solves (J^T J + lambda diag(J^T J)) d = -J^T r over the first N unknowns; false when not positive definite.
+template <int N>
+POSE_HD bool floor_step(const double *S, double lambda, double *d) {
+  double F[3][3], A[N][N], Lm[N][N] = {}, b[N];
+  floor_sym3(S + 4, F);
+  POSE_UNROLL for (int i = 0; i < N; i++) {
+    POSE_UNROLL for (int j = 0; j < N; j++) A[i][j] = F[i][j];
+    A[i][i] = A[i][i] + lambda * A[i][i];
+    b[i] = -S[1 + i];
+  }
+  if (!cholesky_small<N>(A, Lm)) return false;
+  cholesky_solve<N>(Lm, b, d);
+  return true;
+}
+
+// x, y += d[0], d[1]; with N = 3 the heading turns by phi, cos phi = (1 - d^2/4) / (1 + d^2/4),
+// sin phi = d / (1 + d^2/4) for d = d[2].
+template <int N>
+POSE_HD FloorState floor_update(const FloorState &st, const double *d) {
+  FloorState n{st.x + d[0], st.y + d[1], st.c, st.s};
+  if (N == 3) {
+    const double q = d[N - 1] * d[N - 1] / 4, den = 1 + q, cp = (1 - q) / den, sp = d[N - 1] / den;
+    n.c = st.c * cp - st.s * sp;
+    n.s = st.s * cp + st.c * sp;
+  }
+  return n;
+}
+
+// Levenberg-Marquardt from *st over the first N unknowns, with field_refine's stop rules.  sum(st, S) fills
+// S[kFloorSums] with the reduced pixel sums at st; the prior is added here.  Returns the final E; *pixel is its pixel
+// part and *iterations counts accepted and rejected steps.
+template <int N, class SumFn>
+POSE_HD double floor_refine(SumFn &sum, const FloorModel &m, FloorState *st, double *pixel, int *iterations) {
+  double S[kFloorSums];
+  sum(*st, S);
+  *pixel = S[0];
+  floor_add_prior(*st, m, S);
+  double cost = S[0];
+  int it = 0;
+  if (cost < HUGE_VAL) {
+    double lambda = 1e-3;
+    while (it < kFieldMaxIterations) {
+      it++;
+      double d[N];
+      if (floor_step<N>(S, lambda, d)) {
+        const FloorState sn = floor_update<N>(*st, d);
+        double Sn[kFloorSums];
+        sum(sn, Sn);
+        const double pn = Sn[0];
+        floor_add_prior(sn, m, Sn);
+        bool small = true;
+        POSE_UNROLL for (int j = 0; j < N; j++) small = small && fabs(d[j]) <= 1e-10;
+        if (Sn[0] < cost) {
+          small = small || cost - Sn[0] <= 1e-12 * cost;
+          *st = sn;
+          cost = Sn[0];
+          *pixel = pn;
+          POSE_UNROLL for (int j = 0; j < kFloorSums; j++) S[j] = Sn[j];
+          lambda = lambda * 0.1;
+          if (small) break;
+          continue;
+        }
+        if (small) break;
+      }
+      lambda = lambda * 10;
+      if (lambda > 1e8) break;
+    }
+  }
+  *iterations = it;
+  return cost;
+}
+
+// The floor seed of camera-from-field pose (R, t): the robot pose projected onto the floor, (c, s) the normalised
+// horizontal part of robot_R's first column (the gyro's in fixed mode); false when that part is zero.
+POSE_HD bool floor_seed(const M3 &R, const V3 &t, const FloorModel &m, FloorState *st) {
+  const M3 Rc = transpose(R);
+  const V3 tc = scale(mul(Rc, t), -1.0);
+  M3 Rx;
+  POSE_UNROLL for (int k = 0; k < 9; k++) Rx.a[k] = m.rot[k];
+  const M3 Rr = mul(Rc, transpose(Rx));
+  const V3 tr = sub(tc, mul(Rr, V3{{m.off[0], m.off[1], m.off[2]}}));
+  const double h = sqrt(Rr(0, 0) * Rr(0, 0) + Rr(1, 0) * Rr(1, 0));
+  if (!(h > 0)) return false;
+  *st = FloorState{tr.v[0], tr.v[1], Rr(0, 0) / h, Rr(1, 0) / h};
+  if (m.mode == B200TAG_FLOOR_FIXED) {
+    st->c = m.cg;
+    st->s = m.sg;
+  }
+  return true;
+}
+
+// Adds one correspondence's terms of the heading seed into acc[kFloorLinSums]: m_k x (P0 + x bx + y by) = 0 with m_k
+// the ideal normalised ray, P0 = rotation^T (Rz^T X - offset), bx = -rotation^T Rz^T e_x, by = -rotation^T Rz^T e_y
+// at the gyro heading.
+POSE_HD void floor_lin_terms(double u, double v, const V3 &X, const FloorModel &m, const FieldCamera &cam, double *acc) {
+  const V3 ray{{(u - cam.cx) / cam.fx, (v - cam.cy) / cam.fy, 1}};
+  const FloorState g{0, 0, m.cg, m.sg};
+  V3 W, P0;
+  double ru, rv;
+  floor_corner_cost(u, v, X, g, m, cam, &W, &P0, &ru, &rv);
+  const double qx[3] = {-m.cg, m.sg, 0}, qy[3] = {-m.sg, -m.cg, 0};
+  V3 bx, by;
+  POSE_UNROLL for (int i = 0; i < 3; i++) {
+    bx.v[i] = m.rot[i] * qx[0] + m.rot[3 + i] * qx[1];
+    by.v[i] = m.rot[i] * qy[0] + m.rot[3 + i] * qy[1];
+  }
+  const V3 ex = cross(ray, bx), ey = cross(ray, by), e0 = cross(ray, P0);
+  acc[0] += dot(ex, ex);
+  acc[1] += dot(ex, ey);
+  acc[2] += dot(ey, ey);
+  acc[3] += dot(ex, e0);
+  acc[4] += dot(ey, e0);
+}
+
+// The heading seed from the reduced sums S (kFloorLinSums); false when the normal matrix is not positive definite.
+POSE_HD bool floor_lin_seed(const double *S, const FloorModel &m, FloorState *st) {
+  const double A[2][2] = {{S[0], S[1]}, {S[1], S[2]}};
+  double Lm[2][2] = {}, q[2];
+  if (!cholesky_small<2>(A, Lm)) return false;
+  const double b[2] = {-S[3], -S[4]};
+  cholesky_solve<2>(Lm, b, q);
+  *st = FloorState{q[0], q[1], m.cg, m.sg};
+  return true;
+}
+
+POSE_HD void floor_empty(int mode, b200tag_floor_pose *out) {
+  out->num_tags = 0;
+  out->iterations = 0;
+  out->mode = mode;
+  out->reserved = 0;
+  out->x = out->y = 0;
+  out->cos_heading = 1;
+  out->sin_heading = 0;
+  out->heading = 0;
+  out->rms = out->rms_other = HUGE_VAL;
+}
+
+POSE_HD void floor_result(const FloorState &st, double pixel, double pixel_other, int ntags, int iterations, int mode,
+                          b200tag_floor_pose *out) {
+  out->num_tags = ntags;
+  out->iterations = iterations;
+  out->mode = mode;
+  out->reserved = 0;
+  out->x = st.x;
+  out->y = st.y;
+  out->cos_heading = st.c;
+  out->sin_heading = st.s;
+  out->heading = 0;  // atan2(sin, cos), filled on the host
+  const double n = 4.0 * ntags;
+  out->rms = pixel < HUGE_VAL ? sqrt(pixel / n) : HUGE_VAL;
+  out->rms_other = pixel_other < HUGE_VAL ? sqrt(pixel_other / n) : HUGE_VAL;
+}
+
+// The solve over `ntags` used tags (ntags >= 1).  cost(st) returns the reduced pixel cost, sum(st, S) the reduced pixel
+// sums of floor_refine, lin(S) the reduced sums of floor_lin_terms.  Seeds, scored by E in order with the first best
+// winning: every used tag's IPPE candidates (0 first), then, with a heading, the linear (x, y) at the gyro heading.  In
+// free mode with one tag each candidate's seed is refined and the lower cost returned (candidate 0 on a tie), the other
+// in rms_other.  Without any seed the start is x = y = 0 at heading 0.
+template <class CostFn, class SumFn, class LinFn>
+POSE_HD void floor_solve(const FieldTagData *tags, int ntags, const FloorModel &m, CostFn &cost, SumFn &sum, LinFn &lin,
+                         b200tag_floor_pose *out) {
+  if (m.mode == B200TAG_FLOOR_FREE && ntags == 1) {
+    FloorState st[2];
+    double c[2], p[2];
+    int it[2];
+    POSE_UNROLL for (int k = 0; k < 2; k++) {
+      st[k] = FloorState{0, 0, 1, 0};
+      c[k] = p[k] = HUGE_VAL;
+      it[k] = 0;
+      if (floor_seed(tags[0].R[k], tags[0].t[k], m, &st[k])) c[k] = floor_refine<3>(sum, m, &st[k], &p[k], &it[k]);
+    }
+    const int b = c[1] < c[0] ? 1 : 0;
+    floor_result(st[b], p[b], p[1 - b], 1, it[b], m.mode, out);
+    return;
+  }
+  FloorState best{0, 0, 1, 0};
+  if (m.mode == B200TAG_FLOOR_FIXED) {
+    best.c = m.cg;
+    best.s = m.sg;
+  }
+  double best_cost = HUGE_VAL;
+  bool any = false;
+  for (int s = 0; s < 2 * ntags; s++) {
+    FloorState st;
+    if (!floor_seed(tags[s >> 1].R[s & 1], tags[s >> 1].t[s & 1], m, &st)) continue;
+    const double e = floor_score(cost(st), st, m);
+    if (!any || e < best_cost) {
+      best = st;
+      best_cost = e;
+      any = true;
+    }
+  }
+  if (m.mode != B200TAG_FLOOR_FREE) {
+    double S[kFloorLinSums];
+    lin(S);
+    FloorState st;
+    if (floor_lin_seed(S, m, &st)) {
+      const double e = floor_score(cost(st), st, m);
+      if (!any || e < best_cost) best = st;
+    }
+  }
+  double pixel;
+  int it = 0;
+  if (m.mode == B200TAG_FLOOR_FIXED) floor_refine<2>(sum, m, &best, &pixel, &it);
+  else floor_refine<3>(sum, m, &best, &pixel, &it);
+  floor_result(best, pixel, HUGE_VAL, ntags, it, m.mode, out);
+}
+
+// Adds the covariance terms of corner c of used tag g at state st into acc[kFloorCovSums]: 1 into acc[0] when it is
+// behind the camera or A_i cannot be formed; else J^T J into acc[1..6] and, with the lens D, J^T A A^T J into
+// acc[7..12].
+POSE_HD void floor_cov_corner_terms(const FieldTagData &g, int c, const FloorState &st, const FloorModel &m,
+                                    const FieldCamera &cam, const Distortion *D, double *acc) {
+  double A[4] = {1, 0, 0, 1};
+  if (D && !undistortion_jacobian(g.px[c][0], g.px[c][1], cam, *D, A)) {
+    acc[0] += 1;
+    return;
+  }
+  V3 W, P;
+  double ru, rv;
+  if (!(floor_corner_cost(g.px[c][0], g.px[c][1], g.X[c], st, m, cam, &W, &P, &ru, &rv) < HUGE_VAL)) {
+    acc[0] += 1;
+    return;
+  }
+  double Ju[3], Jv[3];
+  floor_jacobian(W, P, st, m, cam, Ju, Jv);
+  int o = 1;
+  POSE_UNROLL for (int i = 0; i < 3; i++)
+    POSE_UNROLL for (int j = i; j < 3; j++) acc[o++] += Ju[i] * Ju[j] + Jv[i] * Jv[j];
+  if (!D) return;
+  double K0[3], K1[3];  // the rows of A^T J
+  POSE_UNROLL for (int i = 0; i < 3; i++) {
+    K0[i] = A[0] * Ju[i] + A[2] * Jv[i];
+    K1[i] = A[1] * Ju[i] + A[3] * Jv[i];
+  }
+  POSE_UNROLL for (int i = 0; i < 3; i++)
+    POSE_UNROLL for (int j = i; j < 3; j++) acc[o++] += K0[i] * K0[j] + K1[i] * K1[j];
+}
+
+// C = Hi M Hi (distorted) or Hi over the first N unknowns, Hi = H^-1; the rest of the 3x3 C is 0.
+template <int N>
+POSE_HD bool floor_cov_solve(const double (*H)[3], const double (*M)[3], bool distorted, double *C) {
+  double A[N][N], Lm[N][N] = {}, Hi[N][N];
+  POSE_UNROLL for (int i = 0; i < N; i++)
+    POSE_UNROLL for (int j = 0; j < N; j++) A[i][j] = H[i][j];
+  if (!cholesky_small<N>(A, Lm)) return false;
+  POSE_UNROLL for (int k = 0; k < N; k++) {
+    double e[N], x[N];
+    POSE_UNROLL for (int i = 0; i < N; i++) e[i] = i == k ? 1.0 : 0.0;
+    cholesky_solve<N>(Lm, e, x);
+    POSE_UNROLL for (int i = 0; i < N; i++) Hi[i][k] = x[i];
+  }
+  POSE_UNROLL for (int k = 0; k < 9; k++) C[k] = 0;
+  if (!distorted) {
+    POSE_UNROLL for (int i = 0; i < N; i++)
+      POSE_UNROLL for (int j = i; j < N; j++) C[3 * i + j] = C[3 * j + i] = Hi[i][j];
+    return true;
+  }
+  double T[N][N];
+  POSE_UNROLL for (int i = 0; i < N; i++)
+    POSE_UNROLL for (int j = 0; j < N; j++) {
+      double s = 0;
+      POSE_UNROLL for (int k = 0; k < N; k++) s += Hi[i][k] * M[k][j];
+      T[i][j] = s;
+    }
+  POSE_UNROLL for (int i = 0; i < N; i++)
+    POSE_UNROLL for (int j = i; j < N; j++) {
+      double s = 0;
+      POSE_UNROLL for (int k = 0; k < N; k++) s += T[i][k] * Hi[k][j];
+      C[3 * i + j] = C[3 * j + i] = s;
+    }
+  return true;
+}
+
+// The 3x3 covariance of (x, y, theta) of floor record `res` from the reduced sums S (kFloorCovSums; M only when
+// distorted): sigma^2 H^-1 M H^-1, H = J^T J + g g^T, M = sum J_i^T A_i A_i^T J_i + g g^T, g the prior's gradient
+// (prior mode only).  Fixed mode: the (x, y) block, theta's row and column 0.  All HUGE_VAL when no tag was used, a
+// corner failed, the prior is undefined or H is not positive definite.
+POSE_HD_CALL void floor_covariance(const double *S, bool distorted, const b200tag_floor_pose &res, const FloorModel &m,
+                                   double sigma, double *C) {
+  bool ok = res.num_tags > 0 && S[0] == 0;
+  double H[3][3], M[3][3];
+  floor_sym3(S + 1, H);
+  floor_sym3(distorted ? S + 7 : S + 1, M);
+  if (m.mode == B200TAG_FLOOR_PRIOR) {
+    double rho, g;
+    const FloorState st{res.x, res.y, res.cos_heading, res.sin_heading};
+    if (floor_prior(st, m, &rho, &g)) {
+      H[2][2] = H[2][2] + g * g;
+      M[2][2] = M[2][2] + g * g;
+    } else {
+      ok = false;
+    }
+  }
+  if (ok) ok = m.mode == B200TAG_FLOOR_FIXED ? floor_cov_solve<2>(H, M, distorted, C) : floor_cov_solve<3>(H, M, distorted, C);
+  const double s2 = sigma * sigma;
+  POSE_UNROLL for (int k = 0; k < 9; k++) C[k] = ok ? C[k] * s2 : HUGE_VAL;
+}
+
 }  // namespace pose
 
 // Host, pose.cc: the node's records from poses already estimated (robot frame, distance, closest first), the step
@@ -1102,6 +1546,13 @@ bool read_distortion(const double *dist, bool *active, pose::Distortion *D);
 
 // Host, pose.cc: the check of a covariance's sigma: finite and > 0.
 bool valid_sigma(double sigma);
+
+// Host, pose.cc: the gyro heading's (cos, sin) with the host's libm, both NaN for a NaN heading.
+void floor_gyro(double heading, double *cg, double *sg);
+
+// Host, pose.cc: the checks of b200tag_estimate_floor_pose on heading (not infinite) and heading_weight (> 0, +inf
+// allowed); on success fills *m (rotation / offset NULL: identity / zero).
+bool floor_model(const double *rotation, const double *offset, double heading, double heading_weight, pose::FloorModel *m);
 
 }  // namespace b200tag
 

@@ -89,6 +89,10 @@ FIELD_POSE_DT = np.dtype([("num_tags", "<i4"), ("iterations", "<i4"), ("reserved
                           ("rms_other", "<f8")])  # b200tag_field_pose
 COVARIANCE_DT = np.dtype([("C", "<f8", (6, 6))])  # b200tag_covariance: xi = (rx, ry, rz, tx, ty, tz), rad and m
 FIELD_COVARIANCE_DT = np.dtype([("camera", "<f8", (6, 6)), ("robot", "<f8", (6, 6))])  # b200tag_field_covariance
+FLOOR_POSE_DT = np.dtype([("num_tags", "<i4"), ("iterations", "<i4"), ("mode", "<i4"), ("reserved", "<i4"), ("x", "<f8"),
+                          ("y", "<f8"), ("cos_heading", "<f8"), ("sin_heading", "<f8"), ("heading", "<f8"), ("rms", "<f8"),
+                          ("rms_other", "<f8")])  # b200tag_floor_pose; mode 0 free, 1 prior, 2 fixed
+FLOOR_MODES = {0: "free", 1: "prior", 2: "fixed"}
 
 _lib = None
 
@@ -181,6 +185,14 @@ def load_library():
     L.b200tag_pose_covariances.restype = vp
     L.b200tag_field_covariance_get.argtypes = [vp, i32]
     L.b200tag_field_covariance_get.restype = vp
+    L.b200tag_estimate_floor_pose.argtypes = [vp, i32, vp, i32] + [C.c_double] * 5 + [vp, vp, vp] + [C.c_double] * 3 + [vp, vp]
+    L.b200tag_debug_floor_pose_device.argtypes = L.b200tag_estimate_floor_pose.argtypes
+    L.b200tag_set_floor_pose.argtypes = [vp, C.c_double]
+    L.b200tag_set_robot_headings.argtypes = [vp, vp, i32]
+    L.b200tag_floor_pose_get.argtypes = [vp, i32]
+    L.b200tag_floor_pose_get.restype = vp
+    L.b200tag_floor_covariance_get.argtypes = [vp, i32]
+    L.b200tag_floor_covariance_get.restype = vp
     L.b200tag_version.restype = i32
     _lib = L
     return L
@@ -410,11 +422,55 @@ def estimate_field_pose_covariance_device(detections, layout, tagsize, fx, fy, c
                                   cy, sigma, rotation, offset, distortion)
 
 
+def _floor_call(fn, detections, layout, tagsize, fx, fy, cx, cy, rotation, offset, heading, heading_weight, distortion,
+                sigma):
+    lib = load_library()
+    dist = _distortion(distortion)
+    dets = np.ascontiguousarray(detections, dtype=DETECTION_DT)
+    lay = np.ascontiguousarray(np.zeros(0, dtype=FIELD_TAG_DT) if layout is None else layout, dtype=FIELD_TAG_DT)
+    rot = None if rotation is None else np.ascontiguousarray(rotation, dtype=np.float64).reshape(9)
+    off = None if offset is None else np.ascontiguousarray(offset, dtype=np.float64).reshape(3)
+    out = np.zeros(1, dtype=FLOOR_POSE_DT)
+    cov = np.zeros((3, 3), dtype=np.float64)
+    rc = getattr(lib, fn)(_ptr(dets) if len(dets) else None, len(dets), _ptr(lay) if len(lay) else None, len(lay),
+                          float(tagsize), float(fx), float(fy), float(cx), float(cy), _ptr(dist), _ptr(rot), _ptr(off),
+                          float(heading), float(heading_weight), float(sigma), _ptr(out), _ptr(cov) if sigma > 0 else None)
+    if rc:
+        raise B200TagError(f"{fn}: {lib.b200tag_error_string(rc).decode()}")
+    return out[0], (cov if sigma > 0 else None)
+
+
+def estimate_floor_pose(detections: np.ndarray, layout: np.ndarray, tagsize: float, fx: float, fy: float, cx: float,
+                        cy: float, rotation=None, offset=None, heading=float("nan"), heading_weight=float("inf"),
+                        distortion=None, sigma=0.0):
+    """The robot's (x, y, heading) on a flat floor (b200tag_estimate_floor_pose): (FLOOR_POSE_DT record, 3x3 covariance
+    of (x, y, heading) in the field frame or None when sigma is 0).  Correspondences as estimate_field_pose; rotation /
+    offset are the camera's extrinsics with the robot frame's origin on the floor.  `heading` (rad, counter-clockwise
+    from field +x) is the gyro's: NaN solves for it (free), a finite heading with heading_weight = inf fixes it, and
+    with 0 < heading_weight < inf adds it as a prior of heading_weight px per unit of 2 tan(delta / 2) (corner noise
+    over gyro noise in rad).  Pure host math in libb200tag.so."""
+    return _floor_call("b200tag_estimate_floor_pose", detections, layout, tagsize, fx, fy, cx, cy, rotation, offset,
+                       heading, heading_weight, distortion, sigma)
+
+
+def estimate_floor_pose_device(detections: np.ndarray, layout: np.ndarray, tagsize: float, fx: float, fy: float,
+                               cx: float, cy: float, rotation=None, offset=None, heading=float("nan"),
+                               heading_weight=float("inf"), distortion=None, sigma=0.0):
+    """Test hook: estimate_floor_pose computed by the device kernels GpuDetector.SetFloorPose enables."""
+    return _floor_call("b200tag_debug_floor_pose_device", detections, layout, tagsize, fx, fy, cx, cy, rotation, offset,
+                       heading, heading_weight, distortion, sigma)
+
+
 def pose2d_stddevs(cov) -> tuple:
-    """(sigma_x, sigma_y, sigma_yaw) of a robot Pose2d from a 6x6 field-frame pose covariance (e.g. the `robot` field of
-    FIELD_COVARIANCE_DT): sqrt(C[3][3]), sqrt(C[4][4]) and sqrt(C[2][2]), in m, m and rad, as WPILib's
-    addVisionMeasurement takes them."""
-    C6 = np.asarray(cov, dtype=np.float64).reshape(6, 6)
+    """(sigma_x, sigma_y, sigma_yaw) of a robot Pose2d, in m, m and rad, as WPILib's addVisionMeasurement takes them:
+    from a 6x6 field-frame pose covariance (e.g. the `robot` field of FIELD_COVARIANCE_DT) sqrt(C[3][3]),
+    sqrt(C[4][4]) and sqrt(C[2][2]); from the 3x3 (x, y, heading) covariance of a floor pose the square roots of its
+    diagonal."""
+    C = np.asarray(cov, dtype=np.float64)
+    if C.size == 9:
+        C3 = C.reshape(3, 3)
+        return float(np.sqrt(C3[0, 0])), float(np.sqrt(C3[1, 1])), float(np.sqrt(C3[2, 2]))
+    C6 = C.reshape(6, 6)
     return float(np.sqrt(C6[3, 3])), float(np.sqrt(C6[4, 4])), float(np.sqrt(C6[2, 2]))
 
 
@@ -676,6 +732,30 @@ class GpuDetector:
         the last call ran without the field step."""
         p = self._lib.b200tag_field_pose_get(self._h, frame)
         return None if not p else _records(p, 1, FIELD_POSE_DT)[0]
+
+    def SetFloorPose(self, heading_weight) -> None:
+        """From the next Detect on, whenever the field step runs, the robot's floor pose per frame (FloorPose) with
+        estimate_floor_pose's model, from the field step's corners.  heading_weight > 0 (inf: the gyro heading is
+        fixed) turns it on, 0 off; SetPoseCovariance's sigma adds FloorCovariance."""
+        self._check(self._lib.b200tag_set_floor_pose(self._h, float(heading_weight)), "b200tag_set_floor_pose")
+
+    def SetRobotHeadings(self, headings) -> None:
+        """Gyro headings (rad) for the next Detect / Enqueue call only, one per frame; frames past the list or NaN run
+        in free mode, and so does every frame of a call without a preceding SetRobotHeadings."""
+        h = np.ascontiguousarray(np.zeros(0) if headings is None else headings, dtype=np.float64).reshape(-1)
+        self._check(self._lib.b200tag_set_robot_headings(self._h, _ptr(h) if len(h) else None, len(h)),
+                    "b200tag_set_robot_headings")
+
+    def FloorPose(self, frame: int = 0):
+        """The FLOOR_POSE_DT record of frame `frame`, as estimate_floor_pose(Detections(frame), ...) returns it; None
+        when the last call ran without the floor step."""
+        p = self._lib.b200tag_floor_pose_get(self._h, frame)
+        return None if not p else _records(p, 1, FLOOR_POSE_DT)[0]
+
+    def FloorCovariance(self, frame: int = 0):
+        """The 3x3 covariance of FloorPose(frame)'s (x, y, heading); None when the last call ran without it."""
+        p = self._lib.b200tag_floor_covariance_get(self._h, frame)
+        return None if not p else np.frombuffer((C.c_char * 72).from_address(p), dtype=np.float64).reshape(3, 3).copy()
 
     def ReinitializeDetections(self) -> None:
         """apriltag_gpu.cu:202-220 frees and re-creates the zarray; results here are plain arrays."""

@@ -34,6 +34,15 @@ the same run, IPPE without and with the covariance at SIGMA px, on the same conf
   * the `pose_cov` kernel per 128-frame batch, and the `field_pose` kernel per 128-frame batch on the synth.field_scene
     frames of the --field workload, each arm with that layout, alternated over rounds.
 
+--floor measures the floor pose step (GpuDetector.SetFloorPose, the `floor_pose` kernel) on top of IPPE + field, on the
+synth.field_scene frames of the --field workload in 128-frame batches, with each frame's true heading passed by
+SetRobotHeadings before every call: three arms alternating in the same run, IPPE + field, IPPE + field + floor with the
+heading fixed, and IPPE + field + floor with the heading as a prior of weight 0.3 / 0.02:
+  * frames/s of 128-frame batches and kernels per batch;
+  * single-frame p50 and p90;
+  * the `floor_pose` kernel per 128-frame batch (b200tag_profile_device), the median of three rounds of 20 calls;
+  * the host estimate_floor_pose per field_scene frame on one CPU core.
+
 Prints one JSON record, and writes it to --out when given.  Needs a CUDA device."""
 import argparse
 import json
@@ -72,8 +81,11 @@ def main():
     ap.add_argument("--field", action="store_true", help="measure the field pose step (IPPE + SetFieldLayout)")
     ap.add_argument("--distortion", help="K1,K2,P1,P2,K3: measure the pose step with these lens coefficients against without")
     ap.add_argument("--covariance", type=float, help="SIGMA: measure IPPE with the pose covariance at SIGMA px against without")
+    ap.add_argument("--floor", action="store_true", help="measure the floor pose step (IPPE + field + SetFloorPose)")
     ap.add_argument("--out", help="also write the JSON to this file (e.g. profiles/pose_r03.json)")
     args = ap.parse_args()
+    if args.floor:
+        return floor_main(args)
     if args.covariance is not None:
         if not args.covariance > 0:
             ap.error("--covariance needs SIGMA > 0")
@@ -221,9 +233,9 @@ def all_ids_layout(D, seed=1):
     return lay
 
 
-def field_frames(D, synth, n):
+def field_frames(D, synth, n, yaws=None):
     """One layout of 6 tags 1.5-4 m in front of a nominal robot pose, and `n` field_scene frames (YUYV) from robot poses
-    within 0.3 m / 5 deg of it."""
+    within 0.3 m / 5 deg of it.  The robot headings (rad) are appended to `yaws` when given."""
     rng = np.random.default_rng(6)
     R0 = np.array(ROTATION, dtype=np.float64)
     lay = np.zeros(6, dtype=D.FIELD_TAG_DT)
@@ -238,6 +250,8 @@ def field_frames(D, synth, n):
     frames = []
     for i in range(n):
         yaw = np.radians(rng.uniform(-5, 5))
+        if yaws is not None:
+            yaws.append(float(yaw))
         Rz = np.array([[np.cos(yaw), -np.sin(yaw), 0], [np.sin(yaw), np.cos(yaw), 0], [0, 0, 1]])
         t = np.array([rng.uniform(-0.3, 0.3), rng.uniform(-0.3, 0.3), 0.6])
         sc = synth.field_scene(1280, 800, lay, TAGSIZE, Rz @ R0, t, FX, FY, CX, CY, seed=i, noise_sigma=4.0)
@@ -556,6 +570,137 @@ def covariance_main(args, sigma):
             json.dump(res, f, indent=1)
     print(json.dumps(res, indent=1))
     for d in list(big.values()) + list(fs.values()) + list(one.values()):
+        d.close()
+    for pb in pins:
+        pb.close()
+
+
+
+def floor_main(args):
+    import torch
+    from ros_vision_b200 import detector as D, synth
+    arms = ("ippe_field", "floor_fixed", "floor_prior")
+    weight = {"floor_fixed": float("inf"), "floor_prior": 0.3 / 0.02}
+    yaws = []
+    lay, frames = field_frames(D, synth, UNIQUE, yaws)
+    heads = [yaws[i % UNIQUE] for i in range(BATCH)]
+    offset = [OFFSET[0], OFFSET[1], 0.6]  # field_frames' cameras are 0.6 m up: the robot frame's origin on the floor
+    dev_batch = torch.from_numpy(np.stack([frames[i % UNIQUE] for i in range(BATCH)])).cuda()
+    ptr = dev_batch.data_ptr()
+
+    def detector(arm, max_batch):
+        d = D.GpuDetector(1280, 800, "yuyv", quad_decimate=2, max_batch=max_batch)
+        d.SetPoseEstimation(TAGSIZE, FX, FY, CX, CY, rotation=ROTATION, offset=offset, method="ippe")
+        d.SetFieldLayout(lay)
+        if arm in weight:
+            d.SetFloorPose(weight[arm])
+        return d
+
+    def run(d, arm, p, n, hs):
+        if arm in weight:
+            d.SetRobotHeadings(hs)
+        d.DetectDevice(p, n) if n > 1 else d.DetectPointers([p])
+
+    big = {a: detector(a, BATCH) for a in arms}
+    for a, d in big.items():
+        for _ in range(5):
+            run(d, a, ptr, BATCH, heads)
+    fps = {a: [] for a in arms}
+    for _ in range(args.rounds):
+        for a in arms:
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            for _ in range(args.steps):
+                run(big[a], a, ptr, BATCH, heads)
+            fps[a].append(BATCH * args.steps / (time.perf_counter() - t0))
+    kpb = {a: big[a].kernels_per_batch() for a in arms}
+    floor_stats = {a: {"tags_used_per_batch": sum(int(big[a].FloorPose(f)["num_tags"]) for f in range(BATCH)),
+                       "iterations_median": float(np.median([int(big[a].FloorPose(f)["iterations"]) for f in range(BATCH)])),
+                       "modes": sorted({int(big[a].FloorPose(f)["mode"]) for f in range(BATCH)})} for a in weight}
+
+    # floor_pose per batch: headings hold for one call, so each profile call runs one iteration after its own set
+    def kernel_ms(a):
+        vals = []
+        for _ in range(20):
+            big[a].SetRobotHeadings(heads)
+            prof = big[a].ProfileDevice(ptr, BATCH, iters=1)
+            vals.append([ms for name, ms in prof if name == "floor_pose"][0])
+        return float(np.mean(vals))
+    rounds_ms = {a: [kernel_ms(a) for _ in range(3)] for a in weight}
+    floor_ms = {a: float(np.median(v)) for a, v in rounds_ms.items()}
+    field_ms = float(np.median([[ms for name, ms in big["ippe_field"].ProfileDevice(ptr, BATCH, iters=20)
+                                 if name == "field_pose"][0] for _ in range(3)]))
+
+    # single-frame latency from a pinned host frame, the three arms in rotating order
+    one = {a: detector(a, 1) for a in arms}
+    pins = []
+    for f in frames:
+        pb = D.PinnedBuffer(f.size)
+        pb.array[:] = f
+        pins.append(pb)
+    for a, d in one.items():
+        for i, pb in enumerate(pins):
+            run(d, a, pb.ptr, 1, [yaws[i]])
+    lat = {a: [] for a in arms}
+    for i in range(args.latency_iters):
+        pb = pins[i % UNIQUE]
+        for k in range(3):
+            a = arms[(i + k) % 3]
+            t0 = time.perf_counter()
+            run(one[a], a, pb.ptr, 1, [yaws[i % UNIQUE]])
+            lat[a].append((time.perf_counter() - t0) * 1e6)
+
+    # the host solve on the same frames' detections, one core: the median of 20 calls per frame
+    per_frame = []
+    for i in range(UNIQUE):
+        run(one["ippe_field"], "ippe_field", pins[i].ptr, 1, None)
+        per_frame.append(one["ippe_field"].Detections(0))
+    cpu = sorted(os.sched_getaffinity(0))[0]
+    saved = os.sched_getaffinity(0)
+    host_us = {a: [] for a in weight}
+    os.sched_setaffinity(0, {cpu})
+    try:
+        for a in weight:
+            for i, dets in enumerate(per_frame):
+                reps = []
+                for _ in range(21):
+                    t0 = time.perf_counter()
+                    D.estimate_floor_pose(dets, lay, TAGSIZE, FX, FY, CX, CY, ROTATION, offset, heading=yaws[i],
+                                          heading_weight=weight[a])
+                    reps.append((time.perf_counter() - t0) * 1e6)
+                host_us[a].append(float(np.median(reps[1:])))
+    finally:
+        os.sched_setaffinity(0, saved)
+
+    med = {a: float(np.median(fps[a])) for a in arms}
+    p50 = {a: float(np.percentile(lat[a], 50)) for a in arms}
+    res = {
+        "mode": "floor",
+        "gpu": gpu_identity(),
+        "torch_device": torch.cuda.get_device_name(0),
+        "workload": "synth.field_scene frames of one 6-tag layout seen from 16 robot poses (the --field workload), YUYV "
+                    "1280x800, tiled to 128-frame batches, IPPE; each frame's true heading set before every call; "
+                    "prior weight 0.3 / 0.02 px per unit of 2 tan(delta / 2)",
+        "batch_frames_per_s": {"rounds": fps, "median": med,
+                               "ratio_over_ippe_field": {a: med[a] / med["ippe_field"] for a in weight}},
+        "kernels_per_batch": kpb,
+        "single_frame_latency_us": {"p50": p50, "p90": {a: float(np.percentile(lat[a], 90)) for a in arms},
+                                    "iters": args.latency_iters},
+        "floor_pose_kernel_ms_per_batch": {"median_of_3_rounds": floor_ms, "rounds": rounds_ms},
+        "field_pose_kernel_ms_per_batch": field_ms,
+        "floor": floor_stats,
+        "host_estimate_floor_pose_us_per_frame": {a: {"per_frame": v, "median": float(np.median(v))} for a, v in host_us.items()}
+                                                 | {"tags": [int(len(d)) for d in per_frame], "cpu": cpu},
+        "targets": {f"{a}_kernel_at_most_0.03ms_per_batch": bool(floor_ms[a] <= 0.03) for a in weight}
+                   | {f"{a}_batch_ratio_at_least_0.98": bool(med[a] >= 0.98 * med["ippe_field"]) for a in weight}
+                   | {f"{a}_p50_at_most_ippe_field_plus_10us": bool(p50[a] <= p50["ippe_field"] + 10) for a in weight},
+    }
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            json.dump(res, f, indent=1)
+    print(json.dumps(res, indent=1))
+    for d in list(big.values()) + list(one.values()):
         d.close()
     for pb in pins:
         pb.close()
